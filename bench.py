@@ -26,6 +26,9 @@ library's stream).
               same run is the `cpu_baseline` -- and the discrete-log property; N > 1: the discrete-log property per slice).
 `cpu_baseline` / `--impl reference`: the reference's arkworks algorithm restated in C (oracle/), timed on the host cores at
               the SAME size (one 2^24-point MSM per step).  The reference itself is Rust and cannot run here.
+
+`--dump-outputs DIR` writes the result of the last timed step (rank 0; either arm) to DIR/msm_result.npy, so that two builds
+run with the same arguments (same derived generators, same seeded scalars) can be compared output for output.
 """
 import argparse
 import json
@@ -70,6 +73,18 @@ def bench_scalars(n, seed_offset):
     a = rng.integers(0, 1 << 64, size=(n, 4), dtype=np.uint64)
     a[:, 3] &= np.uint64((1 << 62) - 1)
     return a
+
+
+def dump_outputs(out_dir, point_jac):
+    """Writes an MSM result as DIR/msm_result.npy: float64 [2, 8], the affine x and y as canonical integers in eight
+    little-endian 32-bit words each (exact in float64).  Affine, because two builds may return different Jacobian
+    representatives of the same point; (0, 0) is not on y^2 = x^3 + 5 and stands for the point at infinity."""
+    from oracle import oracle as O
+
+    xy = O.pt_to_affine_ints(point_jac) or (0, 0)
+    words = np.array([[(v >> (32 * i)) & 0xFFFFFFFF for i in range(8)] for v in xy], dtype=np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "msm_result.npy"), words)
 
 
 class ClockSampler(threading.Thread):
@@ -177,6 +192,8 @@ def run_reference(args):
     for _ in range(args.steps):
         res = O.msm_affine(bases, scalars, threads=threads)
     dt = (time.perf_counter() - t) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res)
     ok = bool(O.pt_eq(res, O.msm_derived_by_dlog(0, scalars, threads=threads)))
     val = n / dt
     sample = (f"one MSM of 2^{args.log_n} points per step = the full per-GPU workload, {args.steps} timed steps after "
@@ -293,6 +310,8 @@ def run_ours(args):
     launches = ctx.kernel_launches() - l0
     clocks = sampler.summary()
     ms_step = max(ev_ms, 0.0) / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res)  # `res` is the collected (and, with N > 1, all-gathered) result of the last step
 
     # ---- e2e (host buffers through the C ABI) ----
     def timed_host(f, steps, warm):
@@ -588,7 +607,12 @@ def main():
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling sweep (one MSM of 2^16 .. 2^log_n points over the GPUs)")
     ap.add_argument("--no-precompute", action="store_true", help="variable-base path only (no tables of precomputed multiples)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the result of the last timed step to DIR/msm_result.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    # the tree may be read-only and is never written: no bytecode caches next to the modules imported below
+    sys.dont_write_bytecode = True
     if args.impl == "reference":
         run_reference(args)
     else:
