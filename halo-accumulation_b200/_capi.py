@@ -12,6 +12,7 @@ u64p = C.POINTER(C.c_uint64)
 u8p = C.POINTER(C.c_uint8)
 
 HALO_OK, HALO_EINVAL, HALO_ELEN, HALO_ECUDA, HALO_ENCCL, HALO_ENOMEM, HALO_ESTATE, HALO_EIO = 0, -1, -2, -3, -4, -5, -6, -7
+HALO_EINTERNAL = -8
 
 
 class HaloError(RuntimeError):
@@ -61,6 +62,7 @@ def load():
     lib.halo_mgpu_msm_gens.argtypes = [C.c_void_p, u64p, C.c_uint64, u64p]
     lib.halo_mgpu_last_error.argtypes = [C.c_void_p]
     lib.halo_mgpu_last_error.restype = C.c_char_p
+    lib.halo_h_msm_batch.argtypes = [C.c_void_p, u64p, C.POINTER(C.c_uint32), u64p, C.c_uint64, u64p, u8p, u64p, C.c_uint64, u64p]
     if lib.halo_curve_name().decode() != _build.CURVE:
         raise RuntimeError(f"{path} was built for {lib.halo_curve_name().decode()}, HALO_B200_CURVE asks for {_build.CURVE}")
     _lib = lib

@@ -6,7 +6,7 @@ import os
 import numpy as np
 
 from . import _build
-from ._capi import HaloError, arr, load, p64
+from ._capi import HaloError, arr, load, p64, u64p
 
 MAX_LG = 32
 REJECT_SUCCINCT, REJECT_U, REJECT_U0, REJECT_D, REJECT_CBAR, REJECT_Z, REJECT_V = -10, -11, -12, -13, -14, -15, -17
@@ -23,11 +23,13 @@ _REJECT_TEXT = {
 
 
 class Rejected(Exception):
-    """The analogue of the reference's `ensure!` Err (anyhow::Error) from a verifier-style function."""
+    """The analogue of the reference's `ensure!` Err (anyhow::Error) from a verifier-style function.  `index`: the
+    rejected claim of a batch decision (check_batch / decider_batch), None for the single calls."""
 
-    def __init__(self, code):
+    def __init__(self, code, index=None):
         super().__init__(_REJECT_TEXT.get(code, f"rejected ({code})"))
         self.code = code
+        self.index = index
 
 
 class EvalProof(C.Structure):  # pcdl.rs:22-30
@@ -72,15 +74,17 @@ def lib():
             raise RuntimeError(f"{path} is missing: build it with __graft_entry__.build()")
         _lib = C.CDLL(path)
         _lib.halo_host_last_error.restype = C.c_char_p
+        _lib.halo_pcdl_check_batch.argtypes = [C.c_void_p, C.POINTER(Instance), C.c_uint64, u64p, u64p]
+        _lib.halo_acc_decider_batch.argtypes = [C.c_void_p, C.POINTER(Accumulator), C.c_uint64, u64p, u64p]
     return _lib
 
 
-def chk(rc):
+def chk(rc, index=None):
     """0 -> ok; HALO_REJECT_* -> Rejected (Err in the reference); HALO_E* -> HaloError (panic in the reference)."""
     if rc == 0:
         return
     if rc <= -10:
-        raise Rejected(rc)
+        raise Rejected(rc, index)
     raise HaloError(rc, lib().halo_host_last_error().decode())
 
 

@@ -45,3 +45,13 @@ def verifier(ctx, d, qs, acc):
 def decider(ctx, acc):
     """acc.rs:245-255; raises Rejected"""
     _host.chk(_host.lib().halo_acc_decider(ctx._h, C.byref(acc)))
+
+
+def decider_batch(ctx, accs, rho):
+    """check_batch over (C_bar, d, z, v, pi) of every accumulator (include/halo_pcdl.h halo_acc_decider_batch); raises
+    Rejected with .code and .index exactly as a loop of `decider` calls would."""
+    a = (Accumulator * max(1, len(accs)))(*accs)
+    rho = arr(rho, (4,))
+    idx = C.c_uint64()
+    rc = _host.lib().halo_acc_decider_batch(ctx._h, a, C.c_uint64(len(accs)), p64(rho), C.byref(idx))
+    _host.chk(rc, idx.value)

@@ -198,6 +198,7 @@ void halo_ctx_destroy(halo_ctx* ctx) {
     ctx->stage_bases.release();
     ctx->stage_misc.release();
     ctx->poly_dev.release();
+    ctx->lincomb_claims.release();
     for (halo::DevBuf* b : {&ctx->ipa_G, &ctx->ipa_cs, &ctx->ipa_zs, &ctx->ipa_pbar, &ctx->ipa_tail, &ctx->ipa_frozen,
                            &ctx->ipa_sums, &ctx->ipa_den, &ctx->ipa_inv_scratch, &ctx->ipa_bx, &ctx->ipa_diff, &ctx->ipa_den2, &ctx->ipa_ops}) b->release();
     for (MsmWorkspace* wsp : {&ctx->ws, &ctx->ws2}) {
@@ -795,15 +796,20 @@ static int check_lg(halo_ctx* ctx, uint32_t lg_n, bool need_gens) {
     return HALO_OK;
 }
 
+// d = coeffs(h), the n = 2^lg_n coefficients of one claim
+static void h_expand_one(halo_ctx* ctx, const uint64_t* xis, uint32_t lg_n, fr_t* d) {
+    fr_t one;
+    fp_one(one);
+    vec_h_lincomb(ctx, reinterpret_cast<const fr_t*>(xis), &lg_n, &one, 1, (uint64_t)1 << lg_n, false, d);
+}
+
 int halo_h_expand(halo_ctx* ctx, const uint64_t* xis, uint32_t lg_n, uint64_t* out) {
     if (!ctx || !xis || !out) return HALO_EINVAL;
     if (int rc = check_lg(ctx, lg_n, false)) return rc;
     HALO_TRY(ctx)
     uint64_t n = (uint64_t)1 << lg_n;
     ctx->stage_scalars.reserve(n * sizeof(fr_t));
-    fr_t one;
-    fp_one(one);
-    vec_h_expand(ctx, reinterpret_cast<const fr_t*>(xis), (int)lg_n, one, false, ctx->stage_scalars.as<fr_t>());
+    h_expand_one(ctx, xis, lg_n, ctx->stage_scalars.as<fr_t>());
     HALO_CUDA(cudaMemcpyAsync(out, ctx->stage_scalars.p, n * sizeof(fr_t), cudaMemcpyDeviceToHost, ctx->stream));
     HALO_CUDA(cudaStreamSynchronize(ctx->stream));
     HALO_CATCH(ctx)
@@ -815,26 +821,17 @@ int halo_h_msm(halo_ctx* ctx, const uint64_t* xis, uint32_t lg_n, uint64_t out_j
     HALO_TRY(ctx)
     uint64_t n = (uint64_t)1 << lg_n;
     ctx->stage_scalars.reserve(n * sizeof(fr_t));
-    fr_t one;
-    fp_one(one);
-    vec_h_expand(ctx, reinterpret_cast<const fr_t*>(xis), (int)lg_n, one, false, ctx->stage_scalars.as<fr_t>());
+    h_expand_one(ctx, xis, lg_n, ctx->stage_scalars.as<fr_t>());
     xyzz_t r;
     msm_gens_device(ctx, ctx->stage_scalars.as<fr_t>(), 0, n, r);
     out_jac_from_xyzz(r, out_jac);
     HALO_CATCH(ctx)
 }
 
-int halo_h_msm_with(halo_ctx* ctx, const uint64_t* xis, uint32_t lg_n, const uint64_t* bases_affine, const uint8_t* inf_flags,
-                    const uint64_t* scalars, uint64_t k, uint64_t out_h_jac[12], uint64_t out_small_jac[12]) {
-    if (!ctx || !xis || !out_h_jac || !out_small_jac || ((!bases_affine || !scalars) && k)) return HALO_EINVAL;
-    if (int rc = check_lg(ctx, lg_n, true)) return rc;
-    if (k > 4096) return fail(ctx, HALO_EINVAL, "halo_h_msm_with: the companion MSM is meant to be small (k <= 4096)");
-    HALO_TRY(ctx)
-    uint64_t n = (uint64_t)1 << lg_n;
-    ctx->stage_scalars.reserve(n * sizeof(fr_t));
-    fr_t one;
-    fp_one(one);
-    vec_h_expand(ctx, reinterpret_cast<const fr_t*>(xis), (int)lg_n, one, false, ctx->stage_scalars.as<fr_t>());
+// <GS[0..n), stage_scalars> and the companion MSM sum_i scalars[i] * bases[i] (i < m, staged in stage_misc) on the two lanes
+// of msm_batch; the generator MSM takes the FIXED-base tables under the same condition as msm_gens_device.
+static void h_msm_pair(halo_ctx* ctx, uint64_t n, const uint64_t* bases_affine, const uint8_t* inf_flags, const uint64_t* scalars,
+                       uint64_t m, xyzz_t out[2]) {
     MsmInput in[2];
     in[0].scalars = ctx->stage_scalars.as<fr_t>();
     in[0].n = (uint32_t)n;
@@ -846,25 +843,24 @@ int halo_h_msm_with(halo_ctx* ctx, const uint64_t* xis, uint32_t lg_n, const uin
         in[0].bases = ctx->gens.as<affine_t>();
     }
     // companion: bases | scalars | infinity flags staged in stage_misc
-    const size_t kk = k ? k : 1;
-    ctx->stage_misc.reserve(kk * (sizeof(affine_t) + sizeof(fr_t) + 1));
+    const size_t mm = m ? m : 1;
+    ctx->stage_misc.reserve(mm * (sizeof(affine_t) + sizeof(fr_t) + 1));
     affine_t* d_b = ctx->stage_misc.as<affine_t>();
-    fr_t* d_s = reinterpret_cast<fr_t*>(d_b + kk);
-    uint8_t* d_i = reinterpret_cast<uint8_t*>(d_s + kk);
-    if (k) {
-        HALO_CUDA(cudaMemcpyAsync(d_b, bases_affine, k * sizeof(affine_t), cudaMemcpyHostToDevice, ctx->stream));
-        HALO_CUDA(cudaMemcpyAsync(d_s, scalars, k * sizeof(fr_t), cudaMemcpyHostToDevice, ctx->stream));
+    fr_t* d_s = reinterpret_cast<fr_t*>(d_b + mm);
+    uint8_t* d_i = reinterpret_cast<uint8_t*>(d_s + mm);
+    if (m) {
+        HALO_CUDA(cudaMemcpyAsync(d_b, bases_affine, m * sizeof(affine_t), cudaMemcpyHostToDevice, ctx->stream));
+        HALO_CUDA(cudaMemcpyAsync(d_s, scalars, m * sizeof(fr_t), cudaMemcpyHostToDevice, ctx->stream));
         if (inf_flags) {
-            HALO_CUDA(cudaMemcpyAsync(d_i, inf_flags, k, cudaMemcpyHostToDevice, ctx->stream));
-            k_mark_infinity<<<(unsigned)((k + 255) / 256), 256, 0, ctx->stream>>>(d_b, d_i, k);
+            HALO_CUDA(cudaMemcpyAsync(d_i, inf_flags, m, cudaMemcpyHostToDevice, ctx->stream));
+            k_mark_infinity<<<(unsigned)((m + 255) / 256), 256, 0, ctx->stream>>>(d_b, d_i, m);
             ctx->kernel_launches++;
         }
     }
     in[1].bases = d_b;
     in[1].scalars = d_s;
-    in[1].n = (uint32_t)k;
-    xyzz_t out[2];
-    ctx->force_two_lanes = k > 0;
+    in[1].n = (uint32_t)m;
+    ctx->force_two_lanes = m > 0;
     try {
         msm_batch(ctx, in, 2, out);
     } catch (...) {
@@ -872,8 +868,42 @@ int halo_h_msm_with(halo_ctx* ctx, const uint64_t* xis, uint32_t lg_n, const uin
         throw;
     }
     ctx->force_two_lanes = false;
+}
+
+int halo_h_msm_with(halo_ctx* ctx, const uint64_t* xis, uint32_t lg_n, const uint64_t* bases_affine, const uint8_t* inf_flags,
+                    const uint64_t* scalars, uint64_t k, uint64_t out_h_jac[12], uint64_t out_small_jac[12]) {
+    if (!ctx || !xis || !out_h_jac || !out_small_jac || ((!bases_affine || !scalars) && k)) return HALO_EINVAL;
+    if (int rc = check_lg(ctx, lg_n, true)) return rc;
+    if (k > 4096) return fail(ctx, HALO_EINVAL, "halo_h_msm_with: the companion MSM is meant to be small (k <= 4096)");
+    HALO_TRY(ctx)
+    uint64_t n = (uint64_t)1 << lg_n;
+    ctx->stage_scalars.reserve(n * sizeof(fr_t));
+    h_expand_one(ctx, xis, lg_n, ctx->stage_scalars.as<fr_t>());
+    xyzz_t out[2];
+    h_msm_pair(ctx, n, bases_affine, inf_flags, scalars, k, out);
     out_jac_from_xyzz(out[0], out_h_jac);
     out_jac_from_xyzz(out[1], out_small_jac);
+    HALO_CATCH(ctx)
+}
+
+int halo_h_msm_batch(halo_ctx* ctx, const uint64_t* xis, const uint32_t* lg_ns, const uint64_t* weights, uint64_t k,
+                     const uint64_t* bases_affine, const uint8_t* inf_flags, const uint64_t* scalars, uint64_t m,
+                     uint64_t out_jac[12]) {
+    if (!ctx || !out_jac || ((!xis || !lg_ns || !weights) && k) || ((!bases_affine || !scalars) && m)) return HALO_EINVAL;
+    if ((k | m) >> 32) return fail(ctx, HALO_EINVAL, "halo_h_msm_batch: k or m is 2^32 or more");
+    uint64_t n = 0;
+    for (uint64_t j = 0; j < k; j++) {
+        if (int rc = check_lg(ctx, lg_ns[j], true)) return rc;
+        if (((uint64_t)1 << lg_ns[j]) > n) n = (uint64_t)1 << lg_ns[j];
+    }
+    HALO_TRY(ctx)
+    ctx->stage_scalars.reserve((n ? n : 1) * sizeof(fr_t));
+    vec_h_lincomb(ctx, reinterpret_cast<const fr_t*>(xis), lg_ns, reinterpret_cast<const fr_t*>(weights), k, n, false,
+                  ctx->stage_scalars.as<fr_t>());
+    xyzz_t out[2];
+    h_msm_pair(ctx, n, bases_affine, inf_flags, scalars, m, out);
+    xyzz_add(out[0], out[1]);
+    out_jac_from_xyzz(out[0], out_jac);
     HALO_CATCH(ctx)
 }
 
@@ -942,9 +972,9 @@ static int h_lincomb_impl(halo_ctx* ctx, const uint64_t* h0, uint64_t n_h0, cons
     fr_t* d = buf.as<fr_t>();
     HALO_CUDA(cudaMemsetAsync(d, 0, n * sizeof(fr_t), ctx->stream));
     if (n_h0) HALO_CUDA(cudaMemcpyAsync(d, h0, n_h0 * sizeof(fr_t), cudaMemcpyHostToDevice, ctx->stream));
-    const fr_t* al = reinterpret_cast<const fr_t*>(alphas);
-    const fr_t* xs = reinterpret_cast<const fr_t*>(xis);
-    for (uint64_t i = 0; i < m; i++) vec_h_expand(ctx, xs + i * (lg_n + 1), (int)lg_n, al[i + 1], true, d);  // acc.rs:90-92
+    std::vector<uint32_t> lgs(m, lg_n);
+    if (m)  // acc.rs:90-92: h_0 + sum_i alphas[i + 1] coeffs(h_i)
+        vec_h_lincomb(ctx, reinterpret_cast<const fr_t*>(xis), lgs.data(), reinterpret_cast<const fr_t*>(alphas) + 1, m, n, true, d);
     if (out) {
         HALO_CUDA(cudaMemcpyAsync(out, d, n * sizeof(fr_t), cudaMemcpyDeviceToHost, ctx->stream));
         HALO_CUDA(cudaStreamSynchronize(ctx->stream));

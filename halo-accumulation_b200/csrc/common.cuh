@@ -163,6 +163,7 @@ struct halo_ctx {
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     halo::DevBuf stage_scalars, stage_bases, stage_misc;
     halo::DevBuf poly_dev;  // polynomial left on the device by halo_h_lincomb_resident for halo_ipa_begin_resident
+    halo::DevBuf lincomb_claims;  // claim descriptors of vec_h_lincomb
     uint64_t poly_n = 0;
     // buffers of the (single) in-flight PCDL opening, kept across openings: cudaMalloc / cudaFree of 100+ MB per open
     // costs tens of milliseconds

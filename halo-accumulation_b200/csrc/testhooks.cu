@@ -429,7 +429,10 @@ int halo_test_vec_bench(halo_ctx* ctx, int kind, uint64_t n, float* ms) {
     for (int rep = 0; rep < 6; rep++) {
         HALO_CUDA(cudaEventRecord(e0, ctx->stream));
         if (kind == 0) vec_fold_scalars(ctx, a.as<fr_t>(), b.as<fr_t>(), n / 2, z, xis[3]);
-        else if (kind == 1) vec_h_expand(ctx, xis, lg, z, false, a.as<fr_t>());
+        else if (kind == 1) {
+            const uint32_t ulg = (uint32_t)lg;
+            vec_h_lincomb(ctx, xis, &ulg, &z, 1, (uint64_t)1 << lg, false, a.as<fr_t>());
+        }
         else if (kind == 2) vec_dot(ctx, a.as<fr_t>(), b.as<fr_t>(), n, scratch.as<fr_t>() + 2, scratch.as<fr_t>());
         else vec_powers(ctx, z, n, a.as<fr_t>());
         HALO_CUDA(cudaEventRecord(e1, ctx->stream));
@@ -444,6 +447,42 @@ int halo_test_vec_bench(halo_ctx* ctx, int kind, uint64_t n, float* ms) {
     a.release();
     b.release();
     scratch.release();
+    T_CATCH(ctx)
+}
+
+// k_h_lincomb over k claims of 2^lg_n coefficients, writing (CUDA events on the context stream, best of 5 after a warm-up;
+// the H2D copy of the claim descriptors included).
+int halo_test_h_lincomb_bench(halo_ctx* ctx, uint32_t lg_n, uint64_t k, float* ms) {
+    if (!ctx || !ms || lg_n > LINCOMB_MAX_LG || k == 0) return HALO_EINVAL;
+    T_TRY(ctx)
+    const uint64_t n = (uint64_t)1 << lg_n;
+    DevBuf a;
+    a.reserve(n * sizeof(fr_t));
+    std::vector<fr_t> xis(k * (lg_n + 1)), w(k);
+    std::vector<uint32_t> lgs(k, lg_n);
+    for (size_t i = 0; i < xis.size(); i++) {
+        fp_one(xis[i]);
+        xis[i].v[1] ^= (uint32_t)i * 2654435761u;
+        xis[i].v[7] &= 0x0fffffffu;
+    }
+    for (uint64_t j = 0; j < k; j++) w[j] = xis[j * (lg_n + 1)];
+    cudaEvent_t e0, e1;
+    HALO_CUDA(cudaEventCreate(&e0));
+    HALO_CUDA(cudaEventCreate(&e1));
+    float best = 1e30f;
+    for (int rep = 0; rep < 6; rep++) {
+        HALO_CUDA(cudaEventRecord(e0, ctx->stream));
+        vec_h_lincomb(ctx, xis.data(), lgs.data(), w.data(), k, n, false, a.as<fr_t>());
+        HALO_CUDA(cudaEventRecord(e1, ctx->stream));
+        HALO_CUDA(cudaStreamSynchronize(ctx->stream));
+        float t;
+        HALO_CUDA(cudaEventElapsedTime(&t, e0, e1));
+        if (rep > 0 && t < best) best = t;
+    }
+    *ms = best;
+    cudaEventDestroy(e0);
+    cudaEventDestroy(e1);
+    a.release();
     T_CATCH(ctx)
 }
 }

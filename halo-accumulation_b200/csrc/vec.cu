@@ -1,12 +1,13 @@
-// vec.cu -- Fr vector kernels: dot products, powers, folds, and the h(X) expansion (K5).
+// vec.cu -- Fr vector kernels: dot products, powers, folds, and the expansion of h(X) and of sums of them (K5, K5b).
 //
 // Replaces the serial scalar loops of the reference:
 //   group.rs:13-15  scalar_dot            -> k_dot_partial + k_dot_final
 //   group.rs:29-37  construct_powers      -> k_powers
 //   pcdl.rs:221-223 c / z folds           -> k_fold_scalars   (HBM bound: 2 x (64 B read + 32 B write) per j)
-//   pcdl.rs:56-77   HPoly::get_poly       -> k_h_expand       (closed form pinned by pcdl.rs:496-508:
+//   pcdl.rs:56-77   HPoly::get_poly       -> k_h_lincomb, one claim of weight 1 (closed form pinned by pcdl.rs:496-508:
 //                                             coeff[j] = prod_{b: bit b of j set} xi_{lg n - b})
-//   acc.rs:85-94    AccumulatedHPolys::get_poly -> k_h_expand with scale = alpha^{i+1}, accumulating
+//   acc.rs:85-94    AccumulatedHPolys::get_poly -> k_h_lincomb with weights alpha^{i+1}, accumulating onto h_0
+//   (batch decider)  sum_j w_j coeffs(h_j) over claims of mixed size -> k_h_lincomb (DESIGN.md K5b)
 //   pcdl.rs:140-142,156  p_bar = q (X - z), p' = p + alpha p_bar -> k_pbar, k_axpy
 #include "common.cuh"
 #include "vec.cuh"
@@ -118,57 +119,124 @@ void vec_fold_scalars(halo_ctx* ctx, fr_t* d_c, fr_t* d_z, uint64_t m, const fr_
     HALO_CUDA(cudaGetLastError());
 }
 
-// ---- h(X) expansion (K5) -------------------------------------------------------------------------------
-struct XiTable {
-    fr_t x[32];  // x[b] = xi_{lg_n - b}: the factor contributed by bit b of the coefficient index
-};
+// ---- sum of weighted h(X) of several claims (K5b) ------------------------------------------------------------
+// out[i] (+)= sum_j w_j prod_{b: bit b of i} x_j[b] for i < 2^lg_j.  A block owns 2^11 consecutive coefficients, a thread 8
+// of them: bits 0-2 of the index are the thread's own, bits 3-10 its thread index, the bits above the block's.  Per chunk of
+// claims the block first builds, in shared memory, the block-uniform product of the high bits with w_j folded in, two
+// 16-entry tables over the thread-index bits (the high one with that product folded in) and an 8-entry table over the low
+// bits; a thread then pays 1 multiplication for its base and 7 for its 8 coefficients, about 1 per coefficient and claim.
+constexpr int LC_THREADS = 256;
+constexpr int LC_SPAN_LG = 11;  // lg of the coefficients of one block: 8 per thread
+constexpr int LC_CHUNK = 32;    // claims whose tables are in shared memory at a time (41 KiB)
+constexpr uint32_t LC_DEAD = 0xFFFFFFFFu;
 
-// Each thread produces 8 consecutive coefficients: one product for the high index bits, then the 8 subset
-// products of the three low-bit factors (7 multiplications).
-__global__ void __launch_bounds__(VEC_THREADS) k_h_expand(XiTable tab, int lg_n, uint64_t n, fr_t scale, int accumulate,
-                                                          fr_t* __restrict__ out) {
-    uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    uint64_t j0 = t * 8;
-    if (j0 >= n) return;
-    fr_t v[8];
-    v[0] = scale;
+__global__ void __launch_bounds__(LC_THREADS) k_h_lincomb(const LincombClaim* __restrict__ claims, uint32_t k, uint64_t n_out,
+                                                          int accumulate, fr_t* __restrict__ out) {
+    __shared__ fr_t t_hi[LC_CHUNK][16];   // w_j * (high bits) * subset products of x[7..10]
+    __shared__ fr_t t_mid[LC_CHUNK][16];  // subset products of x[3..6]
+    __shared__ fr_t t_lo[LC_CHUNK][8];    // subset products of x[0..2]
+    __shared__ fr_t high[LC_CHUNK];
+    __shared__ uint32_t lgs[LC_CHUNK];    // lg n_j, or LC_DEAD when the claim ends below this block
+    const uint32_t tid = threadIdx.x;
+    const uint64_t base = (uint64_t)blockIdx.x << LC_SPAN_LG;
+    const uint64_t i0 = base + 8 * (uint64_t)tid;
+    fr_t acc[8];
+#pragma unroll
+    for (int s = 0; s < 8; s++) fp_zero(acc[s]);
 #pragma unroll 1
-    for (int b = 3; b < lg_n; b++)
-        if ((j0 >> b) & 1) fp_mul(v[0], v[0], tab.x[b]);
-    fp_mul(v[1], v[0], tab.x[0]);
-    fp_mul(v[2], v[0], tab.x[1]);
-    fp_mul(v[3], v[2], tab.x[0]);
-    fp_mul(v[4], v[0], tab.x[2]);
-    fp_mul(v[5], v[4], tab.x[0]);
-    fp_mul(v[6], v[4], tab.x[1]);
-    fp_mul(v[7], v[6], tab.x[0]);
+    for (uint32_t c0 = 0; c0 < k; c0 += LC_CHUNK) {
+        const uint32_t cn = k - c0 < (uint32_t)LC_CHUNK ? k - c0 : (uint32_t)LC_CHUNK;
+        __syncthreads();  // the previous chunk's tables are consumed
+        if (tid < cn) {
+            const LincombClaim& cl = claims[c0 + tid];
+            const uint32_t lg = cl.lg_n;
+            const bool live = (base >> lg) == 0;
+            fr_t h = cl.w;
+#pragma unroll 1
+            for (uint32_t b = LC_SPAN_LG; live && b < lg; b++)
+                if ((base >> b) & 1) fp_mul(h, h, cl.x[b]);
+            high[tid] = h;
+            lgs[tid] = live ? lg : LC_DEAD;
+        }
+        __syncthreads();
+#pragma unroll 1
+        for (uint32_t e = tid; e < cn * 40; e += LC_THREADS) {
+            const uint32_t c = e / 40, r = e % 40;
+            if (lgs[c] == LC_DEAD) continue;
+            const fr_t* x = claims[c0 + c].x;
+            fr_t v;
+            uint32_t sub, first;
+            if (r < 16) {
+                v = high[c];
+                sub = r, first = 7;
+            } else if (r < 32) {
+                fp_one(v);
+                sub = r - 16, first = 3;
+            } else {
+                fp_one(v);
+                sub = r - 32, first = 0;
+            }
+#pragma unroll 1
+            for (uint32_t b = 0; b < 4; b++)
+                if ((sub >> b) & 1) fp_mul(v, v, x[first + b]);
+            if (r < 16)
+                t_hi[c][sub] = v;
+            else if (r < 32)
+                t_mid[c][sub] = v;
+            else
+                t_lo[c][sub] = v;
+        }
+        __syncthreads();
+#pragma unroll 1
+        for (uint32_t c = 0; c < cn; c++) {
+            const uint32_t lg = lgs[c];
+            if (lg == LC_DEAD || (i0 >> lg) != 0) continue;
+            const uint32_t cnt = lg < 3 ? 1u << lg : 8u;  // claims shorter than 8 coefficients
+            fr_t b, v;
+            fp_mul(b, t_hi[c][tid >> 4], t_mid[c][tid & 15]);
+            fp_add(acc[0], acc[0], b);
+#pragma unroll
+            for (uint32_t s = 1; s < 8; s++) {
+                if (s < cnt) {
+                    fp_mul(v, b, t_lo[c][s]);
+                    fp_add(acc[s], acc[s], v);
+                }
+            }
+        }
+    }
 #pragma unroll
     for (int s = 0; s < 8; s++) {
-        if (j0 + s < n) {
+        if (i0 + s < n_out) {
             if (accumulate) {
-                fr_t o = out[j0 + s];
-                fp_add(o, o, v[s]);
-                out[j0 + s] = o;
+                fr_t o = out[i0 + s];
+                fp_add(o, o, acc[s]);
+                out[i0 + s] = o;
             } else {
-                out[j0 + s] = v[s];
+                out[i0 + s] = acc[s];
             }
         }
     }
 }
 
-void vec_h_expand(halo_ctx* ctx, const fr_t* xis /*host, lg_n + 1*/, int lg_n, const fr_t& scale, bool accumulate,
-                  fr_t* d_out) {
-    XiTable tab;
-    for (int b = 0; b < 32; b++) {
-        if (b < lg_n)
-            tab.x[b] = xis[lg_n - b];
-        else
-            fp_one(tab.x[b]);
+void vec_h_lincomb(halo_ctx* ctx, const fr_t* xis, const uint32_t* lg_ns, const fr_t* weights, uint64_t k, uint64_t n_out,
+                   bool accumulate, fr_t* d_out) {
+    if (n_out == 0) return;
+    std::vector<LincombClaim> h(k ? k : 1);
+    fr_t one;
+    fp_one(one);
+    const fr_t* x = xis;
+    for (uint64_t j = 0; j < k; j++) {
+        const uint32_t lg = lg_ns[j];
+        h[j].w = weights[j];
+        for (uint32_t b = 0; b < LINCOMB_MAX_LG; b++) h[j].x[b] = b < lg ? x[lg - b] : one;
+        h[j].lg_n = lg;
+        x += lg + 1;
     }
-    uint64_t n = (uint64_t)1 << lg_n;
-    uint64_t threads = (n + 7) / 8;
-    k_h_expand<<<(unsigned)((threads + VEC_THREADS - 1) / VEC_THREADS), VEC_THREADS, 0, ctx->stream>>>(tab, lg_n, n, scale,
-                                                                                                     accumulate ? 1 : 0, d_out);
+    ctx->lincomb_claims.reserve(h.size() * sizeof(LincombClaim));
+    HALO_CUDA(cudaMemcpyAsync(ctx->lincomb_claims.p, h.data(), k * sizeof(LincombClaim), cudaMemcpyHostToDevice, ctx->stream));
+    const unsigned blocks = (unsigned)((n_out + (1u << LC_SPAN_LG) - 1) >> LC_SPAN_LG);
+    k_h_lincomb<<<blocks, LC_THREADS, 0, ctx->stream>>>(ctx->lincomb_claims.as<LincombClaim>(), (uint32_t)k, n_out,
+                                                        accumulate ? 1 : 0, d_out);
     ctx->kernel_launches++;
     HALO_CUDA(cudaGetLastError());
 }

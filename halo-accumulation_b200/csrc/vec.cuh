@@ -1,4 +1,4 @@
-// vec.cuh -- internal interface of vec.cu (Fr vector kernels and the h(X) expansion).
+// vec.cuh -- internal interface of vec.cu (Fr vector kernels and the expansion of sums of h(X)).
 #pragma once
 #include "common.cuh"
 namespace halo {
@@ -9,8 +9,18 @@ void vec_powers(halo_ctx* ctx, const fr_t& z, uint64_t n, fr_t* d_out);
 void vec_dot(halo_ctx* ctx, const fr_t* d_a, const fr_t* d_b, uint64_t n, fr_t* d_partials, fr_t* d_out);
 // c[j] += xi_inv c[j+m]; z[j] += xi z[j+m], j < m
 void vec_fold_scalars(halo_ctx* ctx, fr_t* d_c, fr_t* d_z, uint64_t m, const fr_t& xi, const fr_t& xi_inv);
-// d_out[j] (+)= scale * prod_{b: bit b of j} xis[lg_n - b], j < 2^lg_n   (xis on the host)
-void vec_h_expand(halo_ctx* ctx, const fr_t* xis, int lg_n, const fr_t& scale, bool accumulate, fr_t* d_out);
+// One claim of vec_h_lincomb on the device: weight, x[b] = xi_{lg_n - b} for b < lg_n (one above), lg_n.
+constexpr uint32_t LINCOMB_MAX_LG = 30;
+struct LincombClaim {
+    fr_t w;
+    fr_t x[LINCOMB_MAX_LG];
+    uint32_t lg_n;
+    uint32_t pad[7];
+};
+// d_out[i] (+)= sum_j weights[j] * coeffs(h_j)[i], i < n_out (coefficients of h_j zero from 2^lg_ns[j] on); claim j's
+// challenges xi_0 .. xi_{lg_ns[j]} are the next lg_ns[j] + 1 rows of xis; xis, lg_ns, weights on the host, lg_ns[j] <= 30
+void vec_h_lincomb(halo_ctx* ctx, const fr_t* xis, const uint32_t* lg_ns, const fr_t* weights, uint64_t k, uint64_t n_out,
+                   bool accumulate, fr_t* d_out);
 void vec_pbar(halo_ctx* ctx, const fr_t* d_q, uint64_t n_q, const fr_t& z, uint64_t n, fr_t* d_out);
 void vec_axpy(halo_ctx* ctx, fr_t* d_y, const fr_t* d_x, const fr_t& alpha, uint64_t n);
 }  // namespace halo

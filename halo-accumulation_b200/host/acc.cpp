@@ -172,6 +172,13 @@ void decider(halo_ctx* ctx, const Accumulator& acc) {
     pcdl::check(ctx, acc.C_bar, acc.d, acc.z, acc.v, acc.pi);  // :254
 }
 
+void decider_batch(halo_ctx* ctx, const std::vector<Accumulator>& accs, const PallasScalar& rho, uint64_t* rejected_index) {
+    std::vector<pcdl::Query> qs;
+    qs.reserve(accs.size());
+    for (const Accumulator& a : accs) qs.push_back(pcdl::Query{&a.C_bar, a.d, &a.z, &a.v, &a.pi});
+    pcdl::check_batch(ctx, qs, rho, rejected_index);
+}
+
 Instance instance_from_c(const halo_instance& q) {
     return Instance{point_load(q.C), q.d, scalar_load(q.z), scalar_load(q.v), pcdl::proof_from_c(q.pi)};
 }

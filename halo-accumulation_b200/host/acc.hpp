@@ -57,6 +57,8 @@ Accumulator prover(halo_ctx* ctx, uint64_t d, const std::vector<Instance>& qs, c
 void verifier(halo_ctx* ctx, uint64_t D, const std::vector<Instance>& qs, const Accumulator& acc);
 // acc.rs:245-255
 void decider(halo_ctx* ctx, const Accumulator& acc);
+// pcdl::check_batch over (C_bar, d, z, v, pi) of every accumulator (acc.rs:254); the reference has no batch decider
+void decider_batch(halo_ctx* ctx, const std::vector<Accumulator>& accs, const PallasScalar& rho, uint64_t* rejected_index);
 
 Instance instance_from_c(const halo_instance& q);
 Accumulator accumulator_from_c(const halo_accumulator& a);

@@ -119,6 +119,24 @@ int halo_pcdl_check(halo_ctx* ctx, const uint64_t C_jac[12], uint64_t d, const u
     });
 }
 
+int halo_pcdl_check_batch(halo_ctx* ctx, const halo_instance* claims, uint64_t k, const uint64_t rho[4], uint64_t* rejected_index) {
+    return guarded([&] {
+        if (k == 0) return;
+        ensure(claims && rho && rejected_index, HALO_EINVAL, "null claims / rho / rejected_index");
+        const PallasScalar r = scalar_load_checked(rho, "rho is not a canonical scalar");
+        std::vector<acc::Instance> v;
+        v.reserve(k);
+        for (uint64_t j = 0; j < k; j++) {
+            validate(claims[j]);
+            v.push_back(acc::instance_from_c(claims[j]));
+        }
+        std::vector<pcdl::Query> qs;
+        qs.reserve(k);
+        for (const acc::Instance& q : v) qs.push_back(pcdl::Query{&q.C, q.d, &q.z, &q.v, &q.pi});
+        pcdl::check_batch(ctx, qs, r, rejected_index);
+    });
+}
+
 int halo_h_eval(const uint64_t* xis, uint32_t lg_n, const uint64_t z[4], uint64_t out[4]) {
     return guarded([&] {
         std::vector<PallasScalar> x(lg_n + 1);
@@ -160,6 +178,21 @@ int halo_acc_decider(halo_ctx* ctx, const halo_accumulator* acc) {
         ensure(acc != nullptr, HALO_EINVAL, "null accumulator");
         validate(*acc);
         acc::decider(ctx, acc::accumulator_from_c(*acc));
+    });
+}
+
+int halo_acc_decider_batch(halo_ctx* ctx, const halo_accumulator* accs, uint64_t k, const uint64_t rho[4], uint64_t* rejected_index) {
+    return guarded([&] {
+        if (k == 0) return;
+        ensure(accs && rho && rejected_index, HALO_EINVAL, "null accumulators / rho / rejected_index");
+        const PallasScalar r = scalar_load_checked(rho, "rho is not a canonical scalar");
+        std::vector<acc::Accumulator> v;
+        v.reserve(k);
+        for (uint64_t j = 0; j < k; j++) {
+            validate(accs[j]);
+            v.push_back(acc::accumulator_from_c(accs[j]));
+        }
+        acc::decider_batch(ctx, v, r, rejected_index);
     });
 }
 

@@ -2,6 +2,12 @@
 // call into libhalo_b200.so.
 #include "pcdl.hpp"
 
+#include <algorithm>
+#include <exception>
+#include <optional>
+#include <system_error>
+#include <thread>
+
 #include "pedersen.hpp"
 
 namespace halo {
@@ -252,6 +258,95 @@ void check(halo_ctx* ctx, const PallasPoint& C, uint64_t d, const PallasScalar& 
     PallasPoint lhs = sp.C_prime + point_load(out_s);
     ensure(xyzz_is_inf(lhs.p), HALO_REJECT_SUCCINCT, "C_(log_n) != CM.Commit_Sigma(c || v')");  // :307-310
     ensure(sp.U == point_load(out_h), HALO_REJECT_U, "U != CM.Commit(ck, h_vec)");                // :339
+}
+
+void check_batch(halo_ctx* ctx, const std::vector<Query>& qs, const PallasScalar& rho, uint64_t* rejected_index) {
+    ensure(!fp_is_zero(rho), HALO_EINVAL, "rho is zero");
+    const size_t k = qs.size();
+    if (k == 0) return;
+    PallasPoint S, H;
+    params_SH(ctx, S, H);  // missing parameters fail here, before any worker thread reads the context
+    // succinct_prepare of every claim: the transcript of check, unchanged.  A hiding claim pays two scalar multiplications
+    // for C', so the claims are spread over host threads; the first malformed claim in claim order is the error raised.
+    std::vector<std::optional<SuccinctPrep>> preps(k);
+    std::vector<std::exception_ptr> errs(k);
+    auto work = [&](size_t t, size_t T) {
+        for (size_t j = t; j < k; j += T) {
+            try {
+                preps[j].emplace(succinct_prepare(ctx, *qs[j].C, qs[j].d, *qs[j].z, *qs[j].v, *qs[j].pi));
+            } catch (...) {
+                errs[j] = std::current_exception();
+            }
+        }
+    };
+    const size_t hw = std::thread::hardware_concurrency();
+    const size_t T = std::min(k, std::max<size_t>(1, std::min<size_t>(hw, 16)));
+    std::vector<std::thread> th;
+    std::vector<size_t> unspawned;
+    for (size_t t = 1; t < T; t++) {
+        try {
+            th.emplace_back(work, t, T);
+        } catch (const std::system_error&) {
+            unspawned.push_back(t);  // no thread available: this thread takes that share as well
+        }
+    }
+    work(0, T);
+    for (size_t t : unspawned) work(t, T);
+    for (auto& x : th) x.join();
+    for (size_t j = 0; j < k; j++)
+        if (errs[j]) std::rethrow_exception(errs[j]);
+
+    // sum_j rho^2j E_j + rho^(2j+1) F_j with E_j = C'_j + sum_i s_{j,i} P_{j,i} (L, R, H, U) and F_j = U_j - <G, h_j>
+    std::vector<PallasScalar> rp(2 * k);
+    rp[0] = scalar_one();
+    for (size_t i = 1; i < 2 * k; i++) rp[i] = rp[i - 1] * rho;
+    std::vector<PallasPoint> c_primes(k);
+    for (size_t j = 0; j < k; j++) c_primes[j] = preps[j]->C_prime;
+    std::vector<affine_t> c_aff = batch_to_affine(c_primes);
+    std::vector<affine_t> aff;
+    std::vector<uint8_t> inf;
+    std::vector<PallasScalar> sc, xis, weights;
+    std::vector<uint32_t> lgs(k);
+    PallasScalar s_H = scalar_zero();
+    for (size_t j = 0; j < k; j++) {
+        const SuccinctPrep& sp = *preps[j];
+        const size_t lr = sp.aff.size() - 2;  // L_0, R_0, .., then H, U
+        for (size_t i = 0; i < lr; i++) {
+            aff.push_back(sp.aff[i]);
+            inf.push_back(sp.inf[i]);
+            sc.push_back(rp[2 * j] * sp.scalars[i]);
+        }
+        s_H = s_H + rp[2 * j] * sp.scalars[lr];
+        aff.push_back(sp.aff[lr + 1]);  // U_j: - rho^2j c_j from E_j, + rho^(2j+1) from F_j
+        inf.push_back(sp.inf[lr + 1]);
+        sc.push_back(rp[2 * j] * sp.scalars[lr + 1] + rp[2 * j + 1]);
+        aff.push_back(c_aff[j]);  // C'_j
+        inf.push_back(affine_is_inf(c_aff[j]) ? 1 : 0);
+        sc.push_back(rp[2 * j]);
+        lgs[j] = (uint32_t)sp.h.xis.size() - 1;
+        xis.insert(xis.end(), sp.h.xis.begin(), sp.h.xis.end());
+        weights.push_back(-rp[2 * j + 1]);
+    }
+    const size_t h_at = preps[0]->aff.size() - 2;  // H, the same point in every claim
+    aff.push_back(preps[0]->aff[h_at]);
+    inf.push_back(preps[0]->inf[h_at]);
+    sc.push_back(s_H);
+    uint64_t out[12];
+    check_rc(ctx, halo_h_msm_batch(ctx, reinterpret_cast<const uint64_t*>(xis.data()), lgs.data(),
+                                   reinterpret_cast<const uint64_t*>(weights.data()), k, reinterpret_cast<const uint64_t*>(aff.data()),
+                                   inf.data(), reinterpret_cast<const uint64_t*>(sc.data()), aff.size(), out));
+    if (xyzz_is_inf(point_load(out).p)) return;
+
+    // rejected: the claims one by one, in order, so that (index, code) is what a loop of single deciders returns
+    for (size_t j = 0; j < k; j++) {
+        try {
+            check(ctx, *qs[j].C, qs[j].d, *qs[j].z, *qs[j].v, *qs[j].pi);
+        } catch (const HaloFailure& e) {
+            if (e.code <= HALO_REJECT_SUCCINCT && rejected_index) *rejected_index = j;
+            throw;
+        }
+    }
+    throw HaloFailure(HALO_EINTERNAL, "check_batch: the combined equation fails but every claim accepts on its own");
 }
 
 EvalProof proof_from_c(const halo_eval_proof& p) {

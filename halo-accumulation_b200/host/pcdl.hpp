@@ -58,6 +58,13 @@ SuccinctMany succinct_check_many(halo_ctx* ctx, const std::vector<Query>& qs, co
 void check(halo_ctx* ctx, const PallasPoint& C, uint64_t d, const PallasScalar& z, const PallasScalar& v,
            const EvalProof& pi);
 
+// Batch decider (DESIGN.md K5b; the reference has none): the claims' succinct equations E_j and U checks F_j are combined
+// with powers of the caller's rho != 0 into sum_j (rho^2j E_j + rho^(2j+1) F_j) = O, ONE halo_h_msm_batch.  Accepts iff that
+// point is O.  Otherwise runs `check` on the claims in order and throws the first reject with *rejected_index = its claim;
+// if every claim then accepts, the batch contradicted them: HALO_EINTERNAL.  Malformed input in any claim throws
+// HALO_EINVAL before any decision.
+void check_batch(halo_ctx* ctx, const std::vector<Query>& claims, const PallasScalar& rho, uint64_t* rejected_index);
+
 // wire conversion
 EvalProof proof_from_c(const halo_eval_proof& p);
 void proof_to_c(const EvalProof& p, halo_eval_proof& out);

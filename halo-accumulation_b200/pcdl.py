@@ -5,7 +5,7 @@ import numpy as np
 
 from . import _host
 from ._capi import arr, p64
-from ._host import EvalProof, Rejected  # noqa: F401
+from ._host import EvalProof, Instance, Rejected  # noqa: F401
 
 
 class HPoly:
@@ -63,3 +63,14 @@ def check(ctx, Cm, d, z, v, pi):
     """pcdl.rs:323-342; raises Rejected"""
     Cm, z, v = arr(Cm, (12,)), arr(z, (4,)), arr(v, (4,))
     _host.chk(_host.lib().halo_pcdl_check(ctx._h, p64(Cm), C.c_uint64(d), p64(z), p64(v), C.byref(pi)))
+
+
+def check_batch(ctx, claims, rho):
+    """Batch decider over claims built by acc.new_instance (include/halo_pcdl.h halo_pcdl_check_batch; the reference has
+    none): one MSM over the generators for all claims, combined with the caller's random rho != 0.  Raises Rejected with
+    .code and .index of the first claim that `check` rejects, exactly as a loop of `check` calls would."""
+    a = (Instance * max(1, len(claims)))(*claims)
+    rho = arr(rho, (4,))
+    idx = C.c_uint64()
+    rc = _host.lib().halo_pcdl_check_batch(ctx._h, a, C.c_uint64(len(claims)), p64(rho), C.byref(idx))
+    _host.chk(rc, idx.value)

@@ -43,6 +43,7 @@ extern "C" {
 #define HALO_ENOMEM (-5)
 #define HALO_ESTATE (-6) /* call out of order (e.g. generators not loaded) */
 #define HALO_EIO (-7)    /* generator store: file cannot be opened / read / written */
+#define HALO_EINTERNAL (-8) /* the library contradicts itself (a batch decision that its one-by-one checks do not confirm) */
 
 typedef struct halo_ctx halo_ctx;
 
@@ -208,6 +209,17 @@ int halo_h_msm(halo_ctx *ctx, const uint64_t *xis /*[lg_n+1][4]*/, uint32_t lg_n
 int halo_h_msm_with(halo_ctx *ctx, const uint64_t *xis /*[lg_n+1][4]*/, uint32_t lg_n, const uint64_t *bases_affine /*[k][8]*/,
                     const uint8_t *inf_flags /*[k] or NULL*/, const uint64_t *scalars /*[k][4]*/, uint64_t k,
                     uint64_t out_h_jac[12], uint64_t out_small_jac[12]);
+/* Batch decider core (K5b): ONE point
+ *   <GS[0..n), sum_j weights[j] coeffs(h_j)> + sum_{i<m} scalars[i] * bases[i],   n = max_j 2^lg_ns[j],
+ * where h_j is the h(X) of claim j with challenges xi_0 .. xi_{lg_ns[j]} (the next lg_ns[j] + 1 rows of xis, concatenated
+ * in claim order; xi_0 unused as in halo_h_expand) and its coefficients are zero from 2^lg_ns[j] on.  The coefficient sum
+ * is built on the device in one kernel, then the generator MSM (FIXED-base tables under the same condition as halo_h_msm)
+ * and the companion MSM over caller-supplied affine points run on two streams.  m is not limited to 4096 (k claims at
+ * lg n = 20 bring 42 k + 1 points, DESIGN.md K5b).  Each lg_ns[j] is checked like halo_h_msm's lg_n; k, m < 2^32.
+ * k = m = 0 gives infinity. */
+int halo_h_msm_batch(halo_ctx *ctx, const uint64_t *xis /*sum_j (lg_ns[j]+1) rows of [4]*/, const uint32_t *lg_ns /*[k]*/,
+                     const uint64_t *weights /*[k][4]*/, uint64_t k, const uint64_t *bases_affine /*[m][8]*/,
+                     const uint8_t *inf_flags /*[m] or NULL*/, const uint64_t *scalars /*[m][4]*/, uint64_t m, uint64_t out_jac[12]);
 /* A batch of small, independent MSMs with ONE host round trip (SURVEY 8(f).2): the accumulation verifier's
  * common_subroutine (acc.rs:135-188) needs commit(h_0) (acc.rs:153) and, per instance q_i, the 2 lg n + 2 point MSM that
  * succinct_check's group equation reduces to (pcdl.rs:285-310); none depends on another's result, so they are enqueued

@@ -37,6 +37,9 @@ int halo_test_gather_throughput(halo_ctx *ctx, uint64_t table_bytes, int blocks,
  * one IPA round over 2 x n/2 outputs (pcdl.rs:221-223), 1 = h-expansion to 2^floor(lg n) coefficients (pcdl.rs:56-77),
  * 2 = dot product of two n-vectors (group.rs:13-15), 3 = powers of z (group.rs:29-37). */
 int halo_test_vec_bench(halo_ctx *ctx, int kind, uint64_t n, float *ms);
+/* Times k_h_lincomb (DESIGN.md K5b) over k claims of 2^lg_n coefficients each, lg_n <= 30 (ms, best of 5, CUDA events; the
+ * copy of the claim descriptors included). */
+int halo_test_h_lincomb_bench(halo_ctx *ctx, uint32_t lg_n, uint64_t k, float *ms);
 /* Host-side GLV decomposition of a challenge used by the generator fold (K4): xi = k1 + k2 * lambda (mod r), written in
  * joint sparse form (digits in {0, +-1}, LSB first; at most half of the positions non-zero on average).  Runs without a GPU. */
 int halo_test_glv_decompose_jsf(const uint64_t xi[4], int8_t d1[136], int8_t d2[136], int *top);

@@ -82,6 +82,24 @@ int halo_pcdl_succinct_check(halo_ctx *ctx, const uint64_t C_jac[12], uint64_t d
 /* pcdl.rs:323-342 */
 int halo_pcdl_check(halo_ctx *ctx, const uint64_t C_jac[12], uint64_t d, const uint64_t z[4], const uint64_t v[4],
                     const halo_eval_proof *pi);
+/* Batch decider (an extension: the reference decides one claim at a time, DESIGN.md K5b).  Decides the k claims
+ * (C, d, z, v, pi) -- each what halo_pcdl_check takes -- with ONE MSM over the generators: with the caller's rho != 0 the
+ * succinct equations E_j (pcdl.rs:307-310) and the U checks F_j (pcdl.rs:339) of all claims are combined into
+ *   sum_j (rho^2j E_j + rho^(2j+1) F_j) = O.
+ * Honest claims satisfy it for every rho; if some E_j or F_j != O it holds for at most 2k - 1 values of rho, so a false
+ * accept has probability <= (2k - 1) / r when rho is drawn after the claims are fixed (from a CSPRNG, or by hashing all k
+ * claims).  rho is an explicit argument like every other random draw here.
+ * Returns
+ *   HALO_OK         accept, iff the combined point is O;
+ *   HALO_REJECT_*   otherwise halo_pcdl_check runs on claims 0, 1, .. in order and the first reject is returned, with
+ *                   *rejected_index = its claim: the (index, code) pair a loop of single checks returns;
+ *   HALO_EINTERNAL  the combined equation failed but every claim accepts on its own (a bug, not a decision);
+ *   HALO_EINVAL     before any decision, wherever the claim sits: a point or scalar of a claim that is not canonical / not
+ *                   on the curve, d + 1 not a power of two, d >= the resident generators, a proof with the wrong number
+ *                   of rounds, a zero challenge; rho = 0 or not canonical; claims / rho / rejected_index NULL with k > 0.
+ * k = 0 accepts and reads no other argument.  *rejected_index is written on a reject only. */
+int halo_pcdl_check_batch(halo_ctx *ctx, const halo_instance *claims, uint64_t k, const uint64_t rho[4],
+                          uint64_t *rejected_index);
 /* HPoly::eval pcdl.rs:79-91 */
 int halo_h_eval(const uint64_t *xis, uint32_t lg_n, const uint64_t z[4], uint64_t out[4]);
 
@@ -92,6 +110,10 @@ int halo_acc_prover(halo_ctx *ctx, uint64_t d, const halo_instance *qs, uint64_t
 int halo_acc_verifier(halo_ctx *ctx, uint64_t d, const halo_instance *qs, uint64_t m, const halo_accumulator *acc);
 /* acc.rs:245-255 */
 int halo_acc_decider(halo_ctx *ctx, const halo_accumulator *acc);
+/* halo_pcdl_check_batch over (C_bar, d, z, v, pi) of each accumulator (the claim of acc.rs:254), same results and errors;
+ * every accumulator is validated like halo_acc_decider's. */
+int halo_acc_decider_batch(halo_ctx *ctx, const halo_accumulator *accs, uint64_t k, const uint64_t rho[4],
+                           uint64_t *rejected_index);
 /* impl From<Accumulator> for Instance, acc.rs:121-131 */
 void halo_acc_to_instance(const halo_accumulator *acc, halo_instance *q);
 
