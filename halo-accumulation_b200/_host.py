@@ -24,7 +24,7 @@ _REJECT_TEXT = {
 
 class Rejected(Exception):
     """The analogue of the reference's `ensure!` Err (anyhow::Error) from a verifier-style function.  `index`: the
-    rejected claim of a batch decision (check_batch / decider_batch), None for the single calls."""
+    rejected claim of a batch decision (check_batch / decider_batch) or step (verifier_batch), None for the single calls."""
 
     def __init__(self, code, index=None):
         super().__init__(_REJECT_TEXT.get(code, f"rejected ({code})"))
@@ -76,6 +76,8 @@ def lib():
         _lib.halo_host_last_error.restype = C.c_char_p
         _lib.halo_pcdl_check_batch.argtypes = [C.c_void_p, C.POINTER(Instance), C.c_uint64, u64p, u64p]
         _lib.halo_acc_decider_batch.argtypes = [C.c_void_p, C.POINTER(Accumulator), C.c_uint64, u64p, u64p]
+        _lib.halo_acc_verifier_batch.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(Instance), u64p, C.POINTER(Accumulator),
+                                                 C.c_uint64, u64p, u64p]
     return _lib
 
 

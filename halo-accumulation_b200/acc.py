@@ -55,3 +55,18 @@ def decider_batch(ctx, accs, rho):
     idx = C.c_uint64()
     rc = _host.lib().halo_acc_decider_batch(ctx._h, a, C.c_uint64(len(accs)), p64(rho), C.byref(idx))
     _host.chk(rc, idx.value)
+
+
+def verifier_batch(ctx, d, steps, rho):
+    """k `verifier` calls at once (include/halo_pcdl.h halo_acc_verifier_batch): steps = [(qs, acc), ..], each checked against
+    d; one MSM for all steps, combined with the caller's random rho != 0.  Raises Rejected with .code and .index (the step)
+    exactly as a loop of `verifier` calls would."""
+    qs = [q for s in steps for q in s[0]]
+    a = (Instance * max(1, len(qs)))(*qs)
+    accs = (Accumulator * max(1, len(steps)))(*[s[1] for s in steps])
+    ms = np.array([len(s[0]) for s in steps] or [0], dtype=np.uint64)
+    rho = arr(rho, (4,))
+    idx = C.c_uint64()
+    rc = _host.lib().halo_acc_verifier_batch(ctx._h, C.c_uint64(d), a, p64(ms), accs, C.c_uint64(len(steps)), p64(rho),
+                                             C.byref(idx))
+    _host.chk(rc, idx.value)

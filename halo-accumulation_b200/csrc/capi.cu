@@ -199,6 +199,7 @@ void halo_ctx_destroy(halo_ctx* ctx) {
     ctx->stage_misc.release();
     ctx->poly_dev.release();
     ctx->lincomb_claims.release();
+    for (halo::DevBuf* b : {&ctx->combine_in, &ctx->combine_work, &ctx->combine_inv_scratch}) b->release();
     for (halo::DevBuf* b : {&ctx->ipa_G, &ctx->ipa_cs, &ctx->ipa_zs, &ctx->ipa_pbar, &ctx->ipa_tail, &ctx->ipa_frozen,
                            &ctx->ipa_sums, &ctx->ipa_den, &ctx->ipa_inv_scratch, &ctx->ipa_bx, &ctx->ipa_diff, &ctx->ipa_den2, &ctx->ipa_ops}) b->release();
     for (MsmWorkspace* wsp : {&ctx->ws, &ctx->ws2}) {
@@ -266,6 +267,7 @@ int halo_set_tuning(halo_ctx* ctx, const char* key, int value) {
     else if (!strcmp(key, "ipa_two_lanes")) ctx->tune_ipa_two_lanes = value;
     else if (!strcmp(key, "ipa_freeze_len")) ctx->tune_ipa_freeze_len = value;
     else if (!strcmp(key, "ipa_frozen_c")) ctx->tune_ipa_frozen_c = value;
+    else if (!strcmp(key, "combine_min_outputs")) ctx->tune_combine_min_outputs = value;
     else return fail(ctx, HALO_EINVAL, "halo_set_tuning: unknown key");
     return HALO_OK;
 }

@@ -164,6 +164,7 @@ struct halo_ctx {
     halo::DevBuf stage_scalars, stage_bases, stage_misc;
     halo::DevBuf poly_dev;  // polynomial left on the device by halo_h_lincomb_resident for halo_ipa_begin_resident
     halo::DevBuf lincomb_claims;  // claim descriptors of vec_h_lincomb
+    halo::DevBuf combine_in, combine_work, combine_inv_scratch;  // k_point_combine (combine.cu): inputs, work and outputs, inversions
     uint64_t poly_n = 0;
     // buffers of the (single) in-flight PCDL opening, kept across openings: cudaMalloc / cudaFree of 100+ MB per open
     // costs tens of milliseconds
@@ -205,6 +206,7 @@ struct halo_ctx {
                                  // with the two-level quad reduction 11 was (8192-point MSM 0.46 / 0.38 / 0.41 ms at c = 10 / 11 / 12), with
                                  // four lanes per bucket 10 again (0.32 / 0.35 ms at c = 10 / 11), and once the host's Horner finish halved
                                  // (assembly field core) 9: open at 2^20 46.0 -> 45.6 ms in three alternating runs
+    int tune_combine_min_outputs = 1024;  // halo_test_point_combine: the device from this many outputs on, host GLV below (-1: never); measured crossover, DESIGN.md K5c
     int tune_fold_call_min_lg = 17;  // generator folds of >= 2^this outputs use the copy of k_fold_multi with the multiplication out of line (-1: never)
     int tune_ipa_defer = -1;    // -1: automatic (3 rounds when the FIXED-base tables cover the opening); 0: off; D: force
     int tune_ipa_defer2 = 0;    // later deferred stages over the materialised vector, at most this many rounds each; 0 = off: measured slower at 2^20

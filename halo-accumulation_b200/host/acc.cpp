@@ -1,6 +1,10 @@
 // host/acc.cpp -- see acc.hpp.  Control flow follows code/src/acc.rs step by step.
 #include "acc.hpp"
 
+#include <algorithm>
+#include <cstdint>
+#include <optional>
+
 namespace halo {
 namespace acc {
 
@@ -177,6 +181,202 @@ void decider_batch(halo_ctx* ctx, const std::vector<Accumulator>& accs, const Pa
     qs.reserve(accs.size());
     for (const Accumulator& a : accs) qs.push_back(pcdl::Query{&a.C_bar, a.d, &a.z, &a.v, &a.pi});
     pcdl::check_batch(ctx, qs, rho, rejected_index);
+}
+
+// DESIGN.md K5c.  Step i (instances q_{i,j}, accumulator acc_i) holds iff the group equations
+//   A_i = U0_i - h0_i[0] G_0 - h0_i[1] G_1                       (acc.rs:152-155)
+//   E_ij = the succinct equation of q_{i,j}                       (pcdl.rs:307-310)
+//   B_i = sum_{j=0..m_i} alpha_i^j U_{i,j} + omega_i S - C_bar_i  (acc.rs:178, :184, :237; U_{i,0} = U0_i)
+// are O and the host checks d_{i,j} = D, d_i = D, rho_1(C*_i, alpha_i) = z_i with C*_i = C_bar_i - omega_i S, h_i(z_i) = v_i
+// hold.  z' = rho_1(C_i, alpha_i) hashes C_i = sum_j alpha_i^j U_{i,j} itself, which a random combination cannot stand for;
+// C*_i is the only C_i that passes (B_i = O <=> C_i = C*_i), so it is hashed instead.  The T = sum_i (m_i + 2) equations are
+// combined in the order A_0, E_0*, B_0, A_1, .. with the powers of rho into ONE halo_msm.
+void verifier_batch(halo_ctx* ctx, uint64_t D, const std::vector<Step>& steps, const PallasScalar& rho, uint64_t* rejected_index) {
+    ensure(!fp_is_zero(rho), HALO_EINVAL, "rho is zero");
+    const size_t k = steps.size();
+    if (k == 0) return;
+    PallasPoint S, H;
+    params_SH(ctx, S, H);  // missing parameters fail here, before any worker thread reads the context
+    // what the single verifier refuses as malformed, wherever it sits (pcdl::commit of h_0: pcdl.rs:102-104)
+    const uint64_t n = D + 1;
+    ensure(n != 0 && !(n & (n - 1)), HALO_EINVAL, "d+1 is not a power of 2");
+    ensure(n <= halo_num_generators(ctx), HALO_EINVAL, "d > D");
+    std::vector<const Instance*> inst;
+    std::vector<size_t> first(k + 1, 0);
+    for (size_t i = 0; i < k; i++) {
+        const Accumulator& a = *steps[i].acc;
+        ensure(a.pi_V.h.size() == 2, HALO_EINVAL, "h_0 must have two coefficients");
+        ensure(D >= 1 || fp_is_zero(a.pi_V.h[1]), HALO_EINVAL, "p.degree() > d");
+        first[i] = inst.size();
+        for (const Instance& q : *steps[i].qs) inst.push_back(&q);
+    }
+    first[k] = inst.size();
+    const size_t M = inst.size();
+
+    // validation + alpha of every instance; then C' of the hiding instances and C*_i of every step in ONE combine call
+    // (the second pass runs on the instances ahead of the first one this pass refused, so the error raised is that of the first
+    // malformed instance in order)
+    std::vector<PallasScalar> alphas(M);
+    const auto errs1 = pcdl::parallel_each(M, [&](size_t j) {
+        const Instance& q = *inst[j];
+        alphas[j] = pcdl::succinct_alpha(ctx, q.C, q.d, q.z, q.v, q.pi);
+    });
+    const size_t f1 = pcdl::first_error(errs1);
+    std::vector<PallasPoint> cP, cQ;
+    std::vector<PallasScalar> ca, cb;
+    std::vector<size_t> slot(M, SIZE_MAX);
+    for (size_t j = 0; j < f1; j++) {
+        if (!inst[j]->pi.hiding) continue;
+        slot[j] = cP.size();
+        cP.push_back(inst[j]->C);
+        cQ.push_back(inst[j]->pi.C_bar);
+        ca.push_back(alphas[j]);
+        cb.push_back(-inst[j]->pi.w_prime);
+    }
+    const size_t star = cP.size();
+    for (size_t i = 0; i < k; i++) {  // C*_i = C_bar_i - omega_i S
+        cP.push_back(steps[i].acc->C_bar);
+        cQ.push_back(point_zero());
+        ca.push_back(scalar_zero());
+        cb.push_back(-steps[i].acc->pi_V.w);
+    }
+    const std::vector<affine_t> c_out = pcdl::combine(ctx, cP, cQ, ca, cb);
+
+    // per step: the rest of every transcript, alpha_i = rho_1(hs_i) (acc.rs:173) and the host checks
+    std::vector<std::optional<pcdl::SuccinctPrep>> preps(M);
+    std::vector<std::vector<PallasScalar>> step_alphas(k);
+    std::vector<uint8_t> host_ok(k, 0);
+    std::vector<std::exception_ptr> errs2(M);
+    const auto step_errs = pcdl::parallel_each(k, [&](size_t i) {
+        const Accumulator& a = *steps[i].acc;
+        const size_t m = first[i + 1] - first[i];
+        AccumulatedHPolys hs(m);
+        hs.h_0 = a.pi_V.h;
+        hs.have_h0 = true;
+        bool ok = a.d == D;  // acc.rs:239
+        for (size_t j = first[i]; j < first[i + 1]; j++) {
+            if (j >= f1) return;
+            const Instance& q = *inst[j];
+            PallasPoint C_prime = q.C;
+            if (slot[j] != SIZE_MAX) xyzz_from_affine(C_prime.p, c_out[slot[j]]);
+            try {
+                preps[j].emplace(pcdl::succinct_finish(ctx, C_prime, q.d, q.z, q.v, q.pi));
+            } catch (...) {
+                errs2[j] = std::current_exception();
+                return;
+            }
+            hs.hs.push_back(preps[j]->h);
+            ok = ok && q.d == D;  // acc.rs:169
+        }
+        Transcript t;
+        hs.serialize(t);
+        hs.set_alpha(t.finish(1));
+        ok = ok && Transcript().point_affine(c_out[star + i]).scalar(hs.alpha).finish(1) == a.z;  // acc.rs:181, :238
+        ok = ok && hs.eval(a.z) == a.v;                                                            // acc.rs:240
+        host_ok[i] = ok;
+        step_alphas[i] = std::move(hs.alphas);
+    });
+
+    const size_t f2 = pcdl::first_error(errs2);
+    if (f2 < f1) std::rethrow_exception(errs2[f2]);
+    if (f1 < M) std::rethrow_exception(errs1[f1]);
+    if (pcdl::first_error(step_errs) < k) std::rethrow_exception(step_errs[pcdl::first_error(step_errs)]);
+
+    // sum_t rho^t X_t over A_i, E_i1 .. E_im_i, B_i
+    std::vector<PallasPoint> acc_pts;  // U0_i, C_bar_i of every step, normalised together
+    for (size_t i = 0; i < k; i++) {
+        acc_pts.push_back(steps[i].acc->pi_V.U);
+        acc_pts.push_back(steps[i].acc->C_bar);
+    }
+    const std::vector<affine_t> acc_aff = batch_to_affine(acc_pts);
+    std::vector<affine_t> cp_aff(M);  // C'_ij affine: the combined ones as they come, the others (= C) normalised together
+    std::vector<PallasPoint> plain;
+    std::vector<size_t> plain_at;
+    for (size_t j = 0; j < M; j++) {
+        if (slot[j] != SIZE_MAX)
+            cp_aff[j] = c_out[slot[j]];
+        else
+            plain.push_back(preps[j]->C_prime), plain_at.push_back(j);
+    }
+    const std::vector<affine_t> plain_aff = batch_to_affine(plain);
+    for (size_t i = 0; i < plain_at.size(); i++) cp_aff[plain_at[i]] = plain_aff[i];
+    std::vector<affine_t> aff;
+    std::vector<PallasScalar> sc;
+    PallasScalar s_G0 = scalar_zero(), s_G1 = scalar_zero(), s_H = scalar_zero(), s_S = scalar_zero();
+    PallasScalar r_t = scalar_one();  // rho^t of the current equation
+    for (size_t i = 0; i < k; i++) {
+        const Accumulator& a = *steps[i].acc;
+        const PallasScalar rA = r_t;
+        r_t = r_t * rho;
+        std::vector<PallasScalar> rE;
+        for (size_t j = first[i]; j < first[i + 1]; j++) {
+            rE.push_back(r_t);
+            r_t = r_t * rho;
+        }
+        const PallasScalar rB = r_t;
+        r_t = r_t * rho;
+        const std::vector<PallasScalar>& al = step_alphas[i];
+        // A_i and B_i's alpha^0 U0_i
+        s_G0 = s_G0 - rA * a.pi_V.h[0];
+        s_G1 = s_G1 - rA * a.pi_V.h[1];
+        aff.push_back(acc_aff[2 * i]);
+        sc.push_back(rA + rB * al[0]);
+        for (size_t j = first[i]; j < first[i + 1]; j++) {
+            const pcdl::SuccinctPrep& sp = *preps[j];
+            const PallasScalar& re = rE[j - first[i]];
+            const size_t lr = sp.aff.size() - 2;  // L_0, R_0, .., then H, U
+            for (size_t l = 0; l < lr; l++) {
+                aff.push_back(sp.aff[l]);
+                sc.push_back(re * sp.scalars[l]);
+            }
+            s_H = s_H + re * sp.scalars[lr];
+            aff.push_back(sp.aff[lr + 1]);  // U_ij: - rho^tE c from E_ij, + rho^tB alpha_i^j from B_i
+            sc.push_back(re * sp.scalars[lr + 1] + rB * al[j - first[i] + 1]);
+            aff.push_back(cp_aff[j]);  // C'_ij
+            sc.push_back(re);
+        }
+        s_S = s_S + rB * a.pi_V.w;
+        aff.push_back(acc_aff[2 * i + 1]);  // - C_bar_i
+        sc.push_back(-rB);
+    }
+    affine_t g[2];
+    check_rc(ctx, halo_get_generators(ctx, 0, n >= 2 ? 2 : 1, reinterpret_cast<uint64_t*>(g)));
+    aff.push_back(g[0]);
+    sc.push_back(s_G0);
+    if (n >= 2) {
+        aff.push_back(g[1]);
+        sc.push_back(s_G1);
+    }
+    const std::vector<affine_t> sh = batch_to_affine({S, H});
+    aff.push_back(sh[0]);
+    sc.push_back(s_S);
+    aff.push_back(sh[1]);
+    sc.push_back(s_H);
+    std::vector<uint8_t> inf(aff.size());
+    for (size_t i = 0; i < aff.size(); i++) inf[i] = affine_is_inf(aff[i]) ? 1 : 0;
+    PallasPoint sum = point_zero();
+    const uint64_t chunk = halo_num_generators(ctx);  // halo_msm takes at most the context's max_n >= generators points per call
+    for (uint64_t off = 0; off < aff.size(); off += chunk) {
+        const uint64_t len = std::min<uint64_t>(chunk, aff.size() - off);
+        uint64_t out[12];
+        check_rc(ctx, halo_msm(ctx, reinterpret_cast<const uint64_t*>(aff.data() + off), inf.data() + off,
+                               reinterpret_cast<const uint64_t*>(sc.data() + off), len, out));
+        sum = sum + point_load(out);
+    }
+    bool all_ok = true;
+    for (size_t i = 0; i < k; i++) all_ok = all_ok && host_ok[i];
+    if (all_ok && xyzz_is_inf(sum.p)) return;
+
+    // rejected: the steps one by one, in order, so that (index, code) is what a loop of single verifiers returns
+    for (size_t i = 0; i < k; i++) {
+        try {
+            verifier(ctx, D, *steps[i].qs, *steps[i].acc);
+        } catch (const HaloFailure& e) {
+            if (e.code <= HALO_REJECT_SUCCINCT && rejected_index) *rejected_index = i;
+            throw;
+        }
+    }
+    throw HaloFailure(HALO_EINTERNAL, "verifier_batch: the combined equation fails but every step accepts on its own");
 }
 
 Instance instance_from_c(const halo_instance& q) {

@@ -60,6 +60,17 @@ void decider(halo_ctx* ctx, const Accumulator& acc);
 // pcdl::check_batch over (C_bar, d, z, v, pi) of every accumulator (acc.rs:254); the reference has no batch decider
 void decider_batch(halo_ctx* ctx, const std::vector<Accumulator>& accs, const PallasScalar& rho, uint64_t* rejected_index);
 
+// Batch verifier (DESIGN.md K5c; the reference has none): k accumulation steps (qs_i, acc_i), each against D as `verifier`,
+// with ONE halo_msm over all their group equations combined with the powers of the caller's rho != 0.  Accepts iff that point is
+// O and every step's host checks hold.  Otherwise runs `verifier` on the steps in order and throws the first reject with
+// *rejected_index = its step; if every step then accepts: HALO_EINTERNAL.  Malformed input anywhere throws HALO_EINVAL before
+// any decision.
+struct Step {
+    const std::vector<Instance>* qs;
+    const Accumulator* acc;
+};
+void verifier_batch(halo_ctx* ctx, uint64_t D, const std::vector<Step>& steps, const PallasScalar& rho, uint64_t* rejected_index);
+
 Instance instance_from_c(const halo_instance& q);
 Accumulator accumulator_from_c(const halo_accumulator& a);
 void accumulator_to_c(const Accumulator& a, halo_accumulator& out);

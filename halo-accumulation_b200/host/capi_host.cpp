@@ -196,6 +196,36 @@ int halo_acc_decider_batch(halo_ctx* ctx, const halo_accumulator* accs, uint64_t
     });
 }
 
+int halo_acc_verifier_batch(halo_ctx* ctx, uint64_t d, const halo_instance* qs, const uint64_t* ms, const halo_accumulator* accs,
+                            uint64_t k, const uint64_t rho[4], uint64_t* rejected_index) {
+    return guarded([&] {
+        if (k == 0) return;
+        ensure(ms && accs && rho && rejected_index, HALO_EINVAL, "null ms / accumulators / rho / rejected_index");
+        const PallasScalar r = scalar_load_checked(rho, "rho is not a canonical scalar");
+        uint64_t total = 0;
+        for (uint64_t i = 0; i < k; i++) {
+            ensure(ms[i] <= UINT64_MAX - total, HALO_EINVAL, "instance count overflows");
+            total += ms[i];
+        }
+        ensure(qs != nullptr || total == 0, HALO_EINVAL, "null instance list");
+        std::vector<std::vector<acc::Instance>> qv(k);
+        std::vector<acc::Accumulator> av;
+        av.reserve(k);
+        uint64_t at = 0;
+        for (uint64_t i = 0; i < k; i++) {
+            validate(accs[i]);
+            av.push_back(acc::accumulator_from_c(accs[i]));
+            for (uint64_t j = 0; j < ms[i]; j++, at++) {
+                validate(qs[at]);
+                qv[i].push_back(acc::instance_from_c(qs[at]));
+            }
+        }
+        std::vector<acc::Step> steps(k);
+        for (uint64_t i = 0; i < k; i++) steps[i] = acc::Step{&qv[i], &av[i]};
+        acc::verifier_batch(ctx, d, steps, r, rejected_index);
+    });
+}
+
 void halo_acc_to_instance(const halo_accumulator* acc, halo_instance* q) {
     std::memcpy(q->C, acc->C_bar, 96);
     q->d = acc->d;

@@ -3,11 +3,14 @@
 #include "pcdl.hpp"
 
 #include <algorithm>
+#include <cstdint>
 #include <exception>
+#include <functional>
 #include <optional>
 #include <system_error>
 #include <thread>
 
+#include "../../include/halo_b200_test.h"
 #include "pedersen.hpp"
 
 namespace halo {
@@ -142,31 +145,24 @@ static EvalProof open_impl(halo_ctx* ctx, const PolyView* p, uint64_t deg, const
     return pi;
 }
 
-// Everything of succinct_check (pcdl.rs:252-314) up to its group equation, which is left as one small MSM:
+// succinct_check (pcdl.rs:252-314) up to its group equation is succinct_alpha, C' (:272-279) and succinct_finish; the group
+// equation is left as one small MSM:
 //   C_lg == c U + v' H'   <=>   C' + sum_k scalars[k] * aff[k] == 0
-struct SuccinctPrep {
-    HPoly h;
-    PallasPoint U, C_prime;
-    std::vector<affine_t> aff;
-    std::vector<uint8_t> inf;
-    std::vector<PallasScalar> scalars;
-};
-static SuccinctPrep succinct_prepare(halo_ctx* ctx, const PallasPoint& C, uint64_t d, const PallasScalar& z, const PallasScalar& v,
-                                     const EvalProof& pi) {
+PallasScalar succinct_alpha(halo_ctx* ctx, const PallasPoint& C, uint64_t d, const PallasScalar& z, const PallasScalar& v,
+                            const EvalProof& pi) {
     uint64_t n = d + 1;
     ensure(is_pow2(n), HALO_EINVAL, "d+1 is not a power of 2!");           // :261
     ensure(n <= halo_num_generators(ctx), HALO_EINVAL, "d was larger than D!");  // :262
     uint32_t lg_n = ilog2(n);
     ensure(pi.Ls.size() == lg_n && pi.Rs.size() == lg_n, HALO_EINVAL, "proof has the wrong number of rounds");
+    return pi.hiding ? Transcript().point(C).scalar(z).scalar(v).point(pi.C_bar).finish(0) : scalar_zero();  // :272-276
+}
+
+SuccinctPrep succinct_finish(halo_ctx* ctx, const PallasPoint& C_prime, uint64_t d, const PallasScalar& z, const PallasScalar& v,
+                             const EvalProof& pi) {
+    uint32_t lg_n = ilog2(d + 1);
     PallasPoint S, H;
     params_SH(ctx, S, H);
-
-    // C' = C + alpha C_bar - w' S  (:272-279)
-    PallasPoint C_prime = C;
-    if (pi.hiding) {
-        PallasScalar a = Transcript().point(C).scalar(z).scalar(v).point(pi.C_bar).finish(0);
-        C_prime = C + pi.C_bar * a - S * pi.w_prime;
-    }
     // xi_0, challenges (:282-293); the group arithmetic of :285-298 and :307-310 is one small MSM:
     //   C_lg == c U + v' H'   <=>   C' + (xi_0 v - xi_0 v') H + sum_i (xi_{i+1}^-1 L_i + xi_{i+1} R_i) - c U == 0
     // all points that enter the transcript or the MSM are normalised with ONE field inversion (the reference normalises
@@ -203,6 +199,67 @@ static SuccinctPrep succinct_prepare(halo_ctx* ctx, const PallasPoint& C, uint64
     scalars.push_back(xis[0] * v - xis[0] * v_prime);  // v H' - v' H' with H' = xi_0 H  (:285, :288, :308)
     scalars.push_back(-pi.c);                          // - c U
     return SuccinctPrep{std::move(h), pi.U, C_prime, std::move(aff), std::move(inf), std::move(scalars)};
+}
+
+static SuccinctPrep succinct_prepare(halo_ctx* ctx, const PallasPoint& C, uint64_t d, const PallasScalar& z, const PallasScalar& v,
+                                     const EvalProof& pi) {
+    PallasScalar a = succinct_alpha(ctx, C, d, z, v, pi);
+    // C' = C + alpha C_bar - w' S  (:272-279)
+    PallasPoint C_prime = C;
+    if (pi.hiding) {
+        PallasPoint S, H;
+        params_SH(ctx, S, H);
+        C_prime = C + pi.C_bar * a - S * pi.w_prime;
+    }
+    return succinct_finish(ctx, C_prime, d, z, v, pi);
+}
+
+std::vector<affine_t> combine(halo_ctx* ctx, const std::vector<PallasPoint>& P, const std::vector<PallasPoint>& Q,
+                              const std::vector<PallasScalar>& a, const std::vector<PallasScalar>& b) {
+    const size_t n = P.size();
+    std::vector<uint64_t> pj(12 * n), qj(12 * n);
+    for (size_t o = 0; o < n; o++) {
+        point_store(&pj[12 * o], P[o]);
+        point_store(&qj[12 * o], Q[o]);
+    }
+    std::vector<affine_t> out(n);
+    check_rc(ctx, halo_test_point_combine(ctx, -1, pj.data(), qj.data(), reinterpret_cast<const uint64_t*>(a.data()),
+                                          reinterpret_cast<const uint64_t*>(b.data()), n, reinterpret_cast<uint64_t*>(out.data())));
+    return out;
+}
+
+std::vector<std::exception_ptr> parallel_each(size_t k, const std::function<void(size_t)>& f) {
+    std::vector<std::exception_ptr> errs(k);
+    auto work = [&](size_t t, size_t T) {
+        for (size_t j = t; j < k; j += T) {
+            try {
+                f(j);
+            } catch (...) {
+                errs[j] = std::current_exception();
+            }
+        }
+    };
+    const size_t hw = std::thread::hardware_concurrency();
+    const size_t T = std::min(k, std::max<size_t>(1, std::min<size_t>(hw, 16)));
+    std::vector<std::thread> th;
+    std::vector<size_t> unspawned;
+    for (size_t t = 1; t < T; t++) {
+        try {
+            th.emplace_back(work, t, T);
+        } catch (const std::system_error&) {
+            unspawned.push_back(t);  // no thread available: this thread takes that share as well
+        }
+    }
+    work(0, T);
+    for (size_t t : unspawned) work(t, T);
+    for (auto& x : th) x.join();
+    return errs;
+}
+
+size_t first_error(const std::vector<std::exception_ptr>& errs) {
+    for (size_t j = 0; j < errs.size(); j++)
+        if (errs[j]) return j;
+    return errs.size();
 }
 
 std::pair<HPoly, PallasPoint> succinct_check(halo_ctx* ctx, const PallasPoint& C, uint64_t d, const PallasScalar& z,
@@ -266,43 +323,57 @@ void check_batch(halo_ctx* ctx, const std::vector<Query>& qs, const PallasScalar
     if (k == 0) return;
     PallasPoint S, H;
     params_SH(ctx, S, H);  // missing parameters fail here, before any worker thread reads the context
-    // succinct_prepare of every claim: the transcript of check, unchanged.  A hiding claim pays two scalar multiplications
-    // for C', so the claims are spread over host threads; the first malformed claim in claim order is the error raised.
+    // succinct_prepare of every claim: the transcript of check, unchanged, spread over host threads.  Without hiding claims
+    // that is one pass.  Otherwise validation + alpha of every claim come first, then C' = C + alpha C_bar - w' S of the hiding
+    // claims in ONE combine call (on the device from "combine_min_outputs"), then the rest of the transcripts.  The second pass
+    // runs on the claims ahead of the first one the first pass refused, so the error raised is always that of the first
+    // malformed claim in claim order.
     std::vector<std::optional<SuccinctPrep>> preps(k);
-    std::vector<std::exception_ptr> errs(k);
-    auto work = [&](size_t t, size_t T) {
-        for (size_t j = t; j < k; j += T) {
-            try {
-                preps[j].emplace(succinct_prepare(ctx, *qs[j].C, qs[j].d, *qs[j].z, *qs[j].v, *qs[j].pi));
-            } catch (...) {
-                errs[j] = std::current_exception();
-            }
+    std::vector<affine_t> c_aff(k);     // C'_j affine: the combined ones as they come, the others normalised below
+    std::vector<uint8_t> have_aff(k, 0);
+    bool any_hiding = false;
+    for (const Query& q : qs) any_hiding = any_hiding || q.pi->hiding;
+    if (!any_hiding) {
+        const auto errs = parallel_each(k, [&](size_t j) { preps[j].emplace(succinct_prepare(ctx, *qs[j].C, qs[j].d, *qs[j].z, *qs[j].v, *qs[j].pi)); });
+        if (first_error(errs) < k) std::rethrow_exception(errs[first_error(errs)]);
+    } else {
+        std::vector<PallasScalar> alphas(k);
+        const auto errs1 = parallel_each(k, [&](size_t j) { alphas[j] = succinct_alpha(ctx, *qs[j].C, qs[j].d, *qs[j].z, *qs[j].v, *qs[j].pi); });
+        const size_t f1 = first_error(errs1);
+        std::vector<PallasPoint> cP, cQ;
+        std::vector<PallasScalar> ca, cb;
+        std::vector<size_t> slot(k, SIZE_MAX);
+        for (size_t j = 0; j < f1; j++) {
+            if (!qs[j].pi->hiding) continue;
+            slot[j] = cP.size();
+            cP.push_back(*qs[j].C);
+            cQ.push_back(qs[j].pi->C_bar);
+            ca.push_back(alphas[j]);
+            cb.push_back(-qs[j].pi->w_prime);
         }
-    };
-    const size_t hw = std::thread::hardware_concurrency();
-    const size_t T = std::min(k, std::max<size_t>(1, std::min<size_t>(hw, 16)));
-    std::vector<std::thread> th;
-    std::vector<size_t> unspawned;
-    for (size_t t = 1; t < T; t++) {
-        try {
-            th.emplace_back(work, t, T);
-        } catch (const std::system_error&) {
-            unspawned.push_back(t);  // no thread available: this thread takes that share as well
-        }
+        const std::vector<affine_t> c_out = combine(ctx, cP, cQ, ca, cb);
+        const auto errs2 = parallel_each(f1, [&](size_t j) {
+            PallasPoint C_prime = *qs[j].C;
+            if (slot[j] != SIZE_MAX) xyzz_from_affine(C_prime.p, c_out[slot[j]]);
+            preps[j].emplace(succinct_finish(ctx, C_prime, qs[j].d, *qs[j].z, *qs[j].v, *qs[j].pi));
+        });
+        const size_t f2 = first_error(errs2);
+        if (f2 < f1) std::rethrow_exception(errs2[f2]);
+        if (f1 < k) std::rethrow_exception(errs1[f1]);
+        for (size_t j = 0; j < k; j++)
+            if (slot[j] != SIZE_MAX) c_aff[j] = c_out[slot[j]], have_aff[j] = 1;
     }
-    work(0, T);
-    for (size_t t : unspawned) work(t, T);
-    for (auto& x : th) x.join();
-    for (size_t j = 0; j < k; j++)
-        if (errs[j]) std::rethrow_exception(errs[j]);
 
     // sum_j rho^2j E_j + rho^(2j+1) F_j with E_j = C'_j + sum_i s_{j,i} P_{j,i} (L, R, H, U) and F_j = U_j - <G, h_j>
     std::vector<PallasScalar> rp(2 * k);
     rp[0] = scalar_one();
     for (size_t i = 1; i < 2 * k; i++) rp[i] = rp[i - 1] * rho;
-    std::vector<PallasPoint> c_primes(k);
-    for (size_t j = 0; j < k; j++) c_primes[j] = preps[j]->C_prime;
-    std::vector<affine_t> c_aff = batch_to_affine(c_primes);
+    std::vector<PallasPoint> plain;
+    std::vector<size_t> plain_at;
+    for (size_t j = 0; j < k; j++)
+        if (!have_aff[j]) plain.push_back(preps[j]->C_prime), plain_at.push_back(j);
+    const std::vector<affine_t> plain_aff = batch_to_affine(plain);
+    for (size_t i = 0; i < plain_at.size(); i++) c_aff[plain_at[i]] = plain_aff[i];
     std::vector<affine_t> aff;
     std::vector<uint8_t> inf;
     std::vector<PallasScalar> sc, xis, weights;

@@ -1,5 +1,8 @@
 // host/pcdl.hpp -- host mirror of code/src/pcdl.rs (Bulletproofs-style polynomial commitment, DL based).
 #pragma once
+#include <exception>
+#include <functional>
+
 #include "../../include/halo_pcdl.h"
 #include "group.hpp"
 
@@ -34,6 +37,30 @@ EvalProof open(halo_ctx* ctx, PolyView p, const PallasPoint& C, uint64_t d, cons
 // Same for a polynomial of degree `deg` that already sits on the device (halo_h_lincomb_resident): acc.rs:209.
 EvalProof open_resident(halo_ctx* ctx, uint64_t deg, const PallasPoint& C, uint64_t d, const PallasScalar& z,
                         const PallasScalar* w, const PolyView* q, const PallasScalar* w_bar);
+// succinct_check (pcdl.rs:252-314) without its group equation, in two halves around C' = C + alpha C_bar - w' S (:272-279) so
+// that a batch can compute every C' with one `combine` call.  succinct_alpha validates (d + 1 a power of two, d <= D, the
+// number of rounds) and returns alpha = rho_0(C, z, v, C_bar) of a hiding proof (zero otherwise); succinct_finish runs the rest
+// of the transcript from C' and leaves the group equation as C' + sum_k scalars[k] aff[k] == O (aff: L_0, R_0, .., H, U).
+struct SuccinctPrep {
+    HPoly h;
+    PallasPoint U, C_prime;
+    std::vector<affine_t> aff;
+    std::vector<uint8_t> inf;
+    std::vector<PallasScalar> scalars;
+};
+PallasScalar succinct_alpha(halo_ctx* ctx, const PallasPoint& C, uint64_t d, const PallasScalar& z, const PallasScalar& v,
+                            const EvalProof& pi);
+SuccinctPrep succinct_finish(halo_ctx* ctx, const PallasPoint& C_prime, uint64_t d, const PallasScalar& z, const PallasScalar& v,
+                             const EvalProof& pi);
+// R_o = P_o + a_o Q_o + b_o S for every o, exact and affine: halo_test_point_combine, on the device from "combine_min_outputs"
+// outputs on (one launch), on host threads below
+std::vector<affine_t> combine(halo_ctx* ctx, const std::vector<PallasPoint>& P, const std::vector<PallasPoint>& Q,
+                              const std::vector<PallasScalar>& a, const std::vector<PallasScalar>& b);
+// f(0) .. f(k - 1) spread over up to 16 host threads; returns what each call threw (null: nothing)
+std::vector<std::exception_ptr> parallel_each(size_t k, const std::function<void(size_t)>& f);
+// index of the first non-null entry (errs.size() if none)
+size_t first_error(const std::vector<std::exception_ptr>& errs);
+
 // pcdl.rs:252-314; throws HaloFailure(HALO_REJECT_SUCCINCT) on reject
 std::pair<HPoly, PallasPoint> succinct_check(halo_ctx* ctx, const PallasPoint& C, uint64_t d, const PallasScalar& z,
                                              const PallasScalar& v, const EvalProof& pi);

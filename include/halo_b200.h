@@ -69,6 +69,8 @@ int halo_set_msm_window(halo_ctx *ctx, int c);
  *                  "split_second_16ths" (0 = two slices), "stage_pageable", "stage_threads" (1 .. 8)
  *   opening        "ipa_defer_rounds" (-1 = automatic), "ipa_defer2_rounds", "ipa_two_lanes", "ipa_freeze_len", "ipa_frozen_c",
  *                  "ipa_fold_call_min_lg" (folds of >= 2^v outputs use the kernel copy with the multiplication out of line)
+ *   batch checks   "combine_min_outputs" (the exact C' = C + alpha C_bar - w' S of hiding claims and C* = C_bar - omega S of
+ *                  accumulation steps run as one device launch from this many points on, on host threads below; -1 = never)
  * Unknown keys return HALO_EINVAL. */
 int halo_set_tuning(halo_ctx *ctx, const char *key, int value);
 /* Enable per-phase CUDA-event timing of the MSM; read back with halo_last_msm_timings (ms):

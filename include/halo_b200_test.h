@@ -43,6 +43,15 @@ int halo_test_h_lincomb_bench(halo_ctx *ctx, uint32_t lg_n, uint64_t k, float *m
 /* Host-side GLV decomposition of a challenge used by the generator fold (K4): xi = k1 + k2 * lambda (mod r), written in
  * joint sparse form (digits in {0, +-1}, LSB first; at most half of the positions non-zero on average).  Runs without a GPU. */
 int halo_test_glv_decompose_jsf(const uint64_t xi[4], int8_t d1[136], int8_t d2[136], int *top);
+/* K5c (DESIGN.md): R_o = P_o + a_o Q_o + b_o S for o < n, S of the context's parameters, each exact, returned affine
+ * (out_affine[n][8], infinity = (0, 0)).  P, Q: Jacobian [n][12]; a, b: [n][4].  path 1: k_point_combine, one launch for all
+ * outputs (GLV + joint sparse form digits written on the host); 0: host GLV on up to 16 threads; -1: the device from
+ * "combine_min_outputs" outputs on (halo_set_tuning), the host below.
+ * Unlike the other hooks this one is load-bearing: the batch checks of libhalo_host.so (halo_pcdl_check_batch,
+ * halo_acc_decider_batch, halo_acc_verifier_batch) take every C' and C* through it with path -1.  It stays out of
+ * halo_b200.h because only that library calls it; removing or changing it breaks those entry points. */
+int halo_test_point_combine(halo_ctx *ctx, int path, const uint64_t *P_jac, const uint64_t *Q_jac, const uint64_t *a,
+                            const uint64_t *b, uint64_t n, uint64_t *out_affine);
 #ifdef __cplusplus
 }
 #endif

@@ -114,6 +114,28 @@ int halo_acc_decider(halo_ctx *ctx, const halo_accumulator *acc);
  * every accumulator is validated like halo_acc_decider's. */
 int halo_acc_decider_batch(halo_ctx *ctx, const halo_accumulator *accs, uint64_t k, const uint64_t rho[4],
                            uint64_t *rejected_index);
+/* Batch verifier (an extension: the reference verifies one accumulation step at a time, DESIGN.md K5c).  Verifies the k
+ * steps (qs_i, accs[i]) against D -- each what halo_acc_verifier takes, step i owning the next ms[i] instances of qs -- with
+ * ONE variable-base MSM: with the caller's rho != 0 the group equations of all steps, in the order
+ *   A_i = U0_i - h0_i[0] G_0 - h0_i[1] G_1                        (acc.rs:152-155)
+ *   E_ij = the succinct equation of instance j                    (pcdl.rs:307-310), j = 1 .. ms[i]
+ *   B_i = sum_{j=0..m_i} alpha_i^j U_ij + omega_i S - C_bar_i     (acc.rs:178, :184, :237; U_i0 = U0_i, omega_i = accs[i].w)
+ * for i = 0, 1, .., are combined into sum_t rho^t X_t = O over T = sum_i (ms[i] + 2) equations; the host checks d_ij = D,
+ * d_i = D, z_i = rho_1(C_bar_i - omega_i S, alpha_i) and h_i(z_i) = v_i.  Honest steps pass for every rho; if some equation
+ * != O the sum is O for at most T - 1 values of rho, so a false accept has probability <= (T - 1) / r when rho is drawn after
+ * the steps are fixed (from a CSPRNG, or by hashing all steps).
+ * Returns
+ *   HALO_OK         accept, iff the combined point is O and every host check holds;
+ *   HALO_REJECT_*   otherwise halo_acc_verifier runs on steps 0, 1, .. in order and the first reject is returned, with
+ *                   *rejected_index = its step: the (index, code) pair a loop of single verifiers returns;
+ *   HALO_EINTERNAL  the combined check failed but every step accepts on its own (a bug, not a decision);
+ *   HALO_EINVAL     before any decision, wherever the step sits: a point or scalar that is not canonical / not on the
+ *                   curve, d + 1 or D + 1 not a power of two, d or D >= the resident generators, a proof with the wrong
+ *                   number of rounds, a zero challenge, h_0 of degree > D; rho = 0 or not canonical; qs / ms / accs / rho /
+ *                   rejected_index NULL with k > 0 (qs may be NULL when every ms[i] is 0).
+ * k = 0 accepts and reads no other argument.  *rejected_index is written on a reject only. */
+int halo_acc_verifier_batch(halo_ctx *ctx, uint64_t d, const halo_instance *qs /*[sum ms]*/, const uint64_t *ms /*[k]*/,
+                            const halo_accumulator *accs /*[k]*/, uint64_t k, const uint64_t rho[4], uint64_t *rejected_index);
 /* impl From<Accumulator> for Instance, acc.rs:121-131 */
 void halo_acc_to_instance(const halo_accumulator *acc, halo_instance *q);
 
