@@ -63,6 +63,8 @@ def load():
     lib.halo_mgpu_last_error.argtypes = [C.c_void_p]
     lib.halo_mgpu_last_error.restype = C.c_char_p
     lib.halo_h_msm_batch.argtypes = [C.c_void_p, u64p, C.POINTER(C.c_uint32), u64p, C.c_uint64, u64p, u8p, u64p, C.c_uint64, u64p]
+    lib.halo_h_msm_batch_submit.argtypes = [C.c_void_p, u64p, C.POINTER(C.c_uint32), u64p, C.c_uint64, C.POINTER(C.c_int)]
+    lib.halo_h_msm_batch_collect.argtypes = [C.c_void_p, C.c_int, u64p, u8p, u64p, C.c_uint64, u64p]
     lib.halo_test_point_combine.argtypes = [C.c_void_p, C.c_int, u64p, u64p, u64p, u64p, C.c_uint64, u64p]
     if lib.halo_curve_name().decode() != _build.CURVE:
         raise RuntimeError(f"{path} was built for {lib.halo_curve_name().decode()}, HALO_B200_CURVE asks for {_build.CURVE}")

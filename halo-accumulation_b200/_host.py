@@ -78,6 +78,8 @@ def lib():
         _lib.halo_acc_decider_batch.argtypes = [C.c_void_p, C.POINTER(Accumulator), C.c_uint64, u64p, u64p]
         _lib.halo_acc_verifier_batch.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(Instance), u64p, C.POINTER(Accumulator),
                                                  C.c_uint64, u64p, u64p]
+        _lib.halo_acc_verify_decide_batch.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(Instance), u64p, C.POINTER(Accumulator),
+                                                      C.c_uint64, C.POINTER(Accumulator), C.c_uint64, u64p, u64p]
     return _lib
 
 

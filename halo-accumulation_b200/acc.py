@@ -70,3 +70,19 @@ def verifier_batch(ctx, d, steps, rho):
     rc = _host.lib().halo_acc_verifier_batch(ctx._h, C.c_uint64(d), a, p64(ms), accs, C.c_uint64(len(steps)), p64(rho),
                                              C.byref(idx))
     _host.chk(rc, idx.value)
+
+
+def verify_decide_batch(ctx, d, steps, decide_accs, rho):
+    """verifier_batch(ctx, d, steps, rho) followed by decider_batch(ctx, decide_accs, rho) in one call
+    (include/halo_pcdl.h halo_acc_verify_decide_batch).  Raises Rejected with .code and .index exactly as a loop of `verifier`
+    calls followed by a loop of `decider` calls would: step i is index i, decided accumulator j is index len(steps) + j."""
+    qs = [q for s in steps for q in s[0]]
+    a = (Instance * max(1, len(qs)))(*qs)
+    accs = (Accumulator * max(1, len(steps)))(*[s[1] for s in steps])
+    dec = (Accumulator * max(1, len(decide_accs)))(*decide_accs)
+    ms = np.array([len(s[0]) for s in steps] or [0], dtype=np.uint64)
+    rho = arr(rho, (4,))
+    idx = C.c_uint64()
+    rc = _host.lib().halo_acc_verify_decide_batch(ctx._h, C.c_uint64(d), a, p64(ms), accs, C.c_uint64(len(steps)), dec,
+                                                  C.c_uint64(len(decide_accs)), p64(rho), C.byref(idx))
+    _host.chk(rc, idx.value)

@@ -227,6 +227,9 @@ void halo_ctx_destroy(halo_ctx* ctx) {
         if (s.done) cudaEventDestroy(s.done);
         if (s.h_parts) cudaFreeHost(s.h_parts);
     }
+    for (DevBuf* b : {&ctx->hb.scalars, &ctx->hb.companion, &ctx->hb.parts}) b->release();
+    if (ctx->hb.done) cudaEventDestroy(ctx->hb.done);
+    if (ctx->hb.h_parts) cudaFreeHost(ctx->hb.h_parts);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
     if (ctx->sort_stream) cudaStreamDestroy(ctx->sort_stream);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -830,20 +833,27 @@ int halo_h_msm(halo_ctx* ctx, const uint64_t* xis, uint32_t lg_n, uint64_t out_j
     HALO_CATCH(ctx)
 }
 
+// <GS[0..n), d_scalars>: the FIXED-base tables under the same condition as msm_gens_device
+static MsmInput gens_input(halo_ctx* ctx, const fr_t* d_scalars, uint64_t n) {
+    MsmInput in;
+    in.scalars = d_scalars;
+    in.n = (uint32_t)n;
+    if (ctx->use_fixed && ctx->pre_n == ctx->n_gens && ctx->gens_pre.p && n >= (1u << 17) && n * 8 >= ctx->pre_n) {
+        in.bases = ctx->gens_pre.as<affine_t>();
+        in.fixed_stride = (uint32_t)ctx->pre_n;
+        in.fixed_first = 0;
+    } else {
+        in.bases = ctx->gens.as<affine_t>();
+    }
+    return in;
+}
+
 // <GS[0..n), stage_scalars> and the companion MSM sum_i scalars[i] * bases[i] (i < m, staged in stage_misc) on the two lanes
-// of msm_batch; the generator MSM takes the FIXED-base tables under the same condition as msm_gens_device.
+// of msm_batch.
 static void h_msm_pair(halo_ctx* ctx, uint64_t n, const uint64_t* bases_affine, const uint8_t* inf_flags, const uint64_t* scalars,
                        uint64_t m, xyzz_t out[2]) {
     MsmInput in[2];
-    in[0].scalars = ctx->stage_scalars.as<fr_t>();
-    in[0].n = (uint32_t)n;
-    if (ctx->use_fixed && ctx->pre_n == ctx->n_gens && ctx->gens_pre.p && n >= (1u << 17) && n * 8 >= ctx->pre_n) {
-        in[0].bases = ctx->gens_pre.as<affine_t>();
-        in[0].fixed_stride = (uint32_t)ctx->pre_n;
-        in[0].fixed_first = 0;
-    } else {
-        in[0].bases = ctx->gens.as<affine_t>();
-    }
+    in[0] = gens_input(ctx, ctx->stage_scalars.as<fr_t>(), n);
     // companion: bases | scalars | infinity flags staged in stage_misc
     const size_t mm = m ? m : 1;
     ctx->stage_misc.reserve(mm * (sizeof(affine_t) + sizeof(fr_t) + 1));
@@ -888,25 +898,107 @@ int halo_h_msm_with(halo_ctx* ctx, const uint64_t* xis, uint32_t lg_n, const uin
     HALO_CATCH(ctx)
 }
 
-int halo_h_msm_batch(halo_ctx* ctx, const uint64_t* xis, const uint32_t* lg_ns, const uint64_t* weights, uint64_t k,
-                     const uint64_t* bases_affine, const uint8_t* inf_flags, const uint64_t* scalars, uint64_t m,
-                     uint64_t out_jac[12]) {
-    if (!ctx || !out_jac || ((!xis || !lg_ns || !weights) && k) || ((!bases_affine || !scalars) && m)) return HALO_EINVAL;
-    if ((k | m) >> 32) return fail(ctx, HALO_EINVAL, "halo_h_msm_batch: k or m is 2^32 or more");
+// The generator half (k_h_lincomb, then the generator MSM on lane 0) is enqueued by submit; collect runs the companion on
+// lane 1, so it starts at once even while the generator MSM still runs, and finishes both.
+static constexpr size_t HB_SLOT = 3 * MSM_MAX_WINDOWS;
+
+int halo_h_msm_batch_submit(halo_ctx* ctx, const uint64_t* xis, const uint32_t* lg_ns, const uint64_t* weights, uint64_t k,
+                            int* ticket) {
+    if (!ctx || !ticket || ((!xis || !lg_ns || !weights) && k)) return HALO_EINVAL;
+    if (k >> 32) return fail(ctx, HALO_EINVAL, "halo_h_msm_batch_submit: k is 2^32 or more");
+    if (ctx->hb.active) return fail(ctx, HALO_ESTATE, "halo_h_msm_batch_submit: a batch is outstanding; collect it first");
     uint64_t n = 0;
     for (uint64_t j = 0; j < k; j++) {
         if (int rc = check_lg(ctx, lg_ns[j], true)) return rc;
         if (((uint64_t)1 << lg_ns[j]) > n) n = (uint64_t)1 << lg_ns[j];
     }
     HALO_TRY(ctx)
-    ctx->stage_scalars.reserve((n ? n : 1) * sizeof(fr_t));
-    vec_h_lincomb(ctx, reinterpret_cast<const fr_t*>(xis), lg_ns, reinterpret_cast<const fr_t*>(weights), k, n, false,
-                  ctx->stage_scalars.as<fr_t>());
-    xyzz_t out[2];
-    h_msm_pair(ctx, n, bases_affine, inf_flags, scalars, m, out);
-    xyzz_add(out[0], out[1]);
-    out_jac_from_xyzz(out[0], out_jac);
+    halo_ctx::HBatch& b = ctx->hb;
+    if (!b.h_parts) {
+        HALO_CUDA(cudaEventCreateWithFlags(&b.done, cudaEventDisableTiming));
+        HALO_CUDA(cudaMallocHost(reinterpret_cast<void**>(&b.h_parts), 2 * HB_SLOT * sizeof(xyzz_t)));
+    }
+    b.parts.reserve(2 * HB_SLOT * sizeof(xyzz_t));
+    b.empty = n == 0;
+    if (!b.empty) {
+        b.scalars.reserve(n * sizeof(fr_t));
+        vec_h_lincomb(ctx, reinterpret_cast<const fr_t*>(xis), lg_ns, reinterpret_cast<const fr_t*>(weights), k, n, false,
+                      b.scalars.as<fr_t>());
+        const MsmInput in = gens_input(ctx, b.scalars.as<fr_t>(), n);
+        b.plan = in.fixed_stride ? ctx->pre_plan : msm_make_plan(n, ctx->force_c);
+        msm_enqueue(ctx, in, b.plan, b.parts.as<xyzz_t>(), 0);
+        const int nwin = b.plan.fixed ? 1 : b.plan.W;
+        HALO_CUDA(cudaMemcpyAsync(b.h_parts, b.parts.p, (size_t)3 * nwin * sizeof(xyzz_t), cudaMemcpyDeviceToHost, ctx->stream));
+        HALO_CUDA(cudaEventRecord(b.done, ctx->stream));
+    }
+    b.active = true;
+    *ticket = 0;
     HALO_CATCH(ctx)
+}
+
+int halo_h_msm_batch_collect(halo_ctx* ctx, int ticket, const uint64_t* bases_affine, const uint8_t* inf_flags,
+                             const uint64_t* scalars, uint64_t m, uint64_t out_jac[12]) {
+    if (!ctx || !out_jac || ticket != 0 || ((!bases_affine || !scalars) && m)) return HALO_EINVAL;
+    if (m >> 32) return fail(ctx, HALO_EINVAL, "halo_h_msm_batch_collect: m is 2^32 or more");
+    halo_ctx::HBatch& b = ctx->hb;
+    if (!b.active) return fail(ctx, HALO_ESTATE, "halo_h_msm_batch_collect: no batch submitted");
+    b.active = false;  // from here on the batch is collected, whatever the outcome
+    HALO_TRY(ctx)
+    xyzz_t gen, comp;
+    xyzz_set_inf(gen);
+    xyzz_set_inf(comp);
+    if (m) {
+        b.companion.reserve(m * (sizeof(affine_t) + sizeof(fr_t) + 1));
+        affine_t* d_b = b.companion.as<affine_t>();
+        fr_t* d_s = reinterpret_cast<fr_t*>(d_b + m);
+        uint8_t* d_i = reinterpret_cast<uint8_t*>(d_s + m);
+        HALO_CUDA(cudaMemcpyAsync(d_b, bases_affine, m * sizeof(affine_t), cudaMemcpyHostToDevice, ctx->stream2));
+        HALO_CUDA(cudaMemcpyAsync(d_s, scalars, m * sizeof(fr_t), cudaMemcpyHostToDevice, ctx->stream2));
+        if (inf_flags) {
+            HALO_CUDA(cudaMemcpyAsync(d_i, inf_flags, m, cudaMemcpyHostToDevice, ctx->stream2));
+            k_mark_infinity<<<(unsigned)((m + 255) / 256), 256, 0, ctx->stream2>>>(d_b, d_i, m);
+            ctx->kernel_launches++;
+        }
+        MsmInput in;
+        in.bases = d_b;
+        in.scalars = d_s;
+        in.n = (uint32_t)m;
+        MsmPlan plan = msm_make_plan(m, ctx->force_c);
+        msm_enqueue(ctx, in, plan, b.parts.as<xyzz_t>() + HB_SLOT, 1);
+        HALO_CUDA(cudaMemcpyAsync(b.h_parts + HB_SLOT, b.parts.as<xyzz_t>() + HB_SLOT, (size_t)3 * plan.W * sizeof(xyzz_t),
+                                  cudaMemcpyDeviceToHost, ctx->stream2));
+        // the companion is the smaller MSM as a rule: its host finish overlaps the generator MSM
+        HALO_CUDA(cudaStreamSynchronize(ctx->stream2));
+        msm_finish_host(b.h_parts + HB_SLOT, plan, comp);
+    }
+    if (!b.empty) {
+        HALO_CUDA(cudaEventSynchronize(b.done));
+        msm_finish_host(b.h_parts, b.plan, gen);
+        if (ctx->profile) {  // phase timings of the generator MSM (lane 0)
+            float t[5];
+            for (int i = 0; i < 5; i++) HALO_CUDA(cudaEventElapsedTime(&t[i], ctx->ev[i], ctx->ev[i + 1]));
+            ctx->last.digits_ms = t[0];
+            ctx->last.scan_ms = t[1];
+            ctx->last.scatter_ms = t[2];
+            ctx->last.accumulate_ms = t[3];
+            ctx->last.reduce_ms = t[4];
+            HALO_CUDA(cudaEventElapsedTime(&ctx->last.total_ms, ctx->ev[0], ctx->ev[5]));
+        }
+    }
+    xyzz_add(gen, comp);
+    out_jac_from_xyzz(gen, out_jac);
+    HALO_CATCH(ctx)
+}
+
+int halo_h_msm_batch(halo_ctx* ctx, const uint64_t* xis, const uint32_t* lg_ns, const uint64_t* weights, uint64_t k,
+                     const uint64_t* bases_affine, const uint8_t* inf_flags, const uint64_t* scalars, uint64_t m,
+                     uint64_t out_jac[12]) {
+    // the companion's arguments are checked ahead of the submit: a refused collect would leave the batch outstanding
+    if (!ctx || !out_jac || ((!bases_affine || !scalars) && m)) return HALO_EINVAL;
+    if (m >> 32) return fail(ctx, HALO_EINVAL, "halo_h_msm_batch: m is 2^32 or more");
+    int ticket = 0;
+    if (int rc = halo_h_msm_batch_submit(ctx, xis, lg_ns, weights, k, &ticket)) return rc;
+    return halo_h_msm_batch_collect(ctx, ticket, bases_affine, inf_flags, scalars, m, out_jac);
 }
 
 int halo_msm_multi(halo_ctx* ctx, const halo_msm_desc* descs, uint32_t count, uint64_t* out_jac) {

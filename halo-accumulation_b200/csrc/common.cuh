@@ -186,6 +186,18 @@ struct halo_ctx {
     } slots[2];
     cudaStream_t copy_stream = nullptr, sort_stream = nullptr;  // sort_stream: highest priority
     int next_slot = 0;
+    // the outstanding batch of halo_h_msm_batch_submit / _collect: its own buffers, so that calls made between the two
+    // (the verifier's C' on the device, other MSMs) neither wait for nor overwrite it
+    struct HBatch {
+        halo::DevBuf scalars;    // sum_j w_j coeffs(h_j)
+        halo::DevBuf companion;  // bases | scalars | infinity flags of the companion MSM
+        halo::DevBuf parts;      // window partials: generator MSM | companion MSM
+        halo::xyzz_t* h_parts = nullptr;  // pinned, same layout
+        cudaEvent_t done = nullptr;
+        halo::MsmPlan plan;
+        bool active = false;
+        bool empty = false;  // no claims: the generator part is infinity
+    } hb;
     // staging ring for host-to-device copies out of PAGEABLE caller memory (h2d_copy, capi.cu)
     static constexpr int STAGE_THREADS = 8, STAGE_SLOTS = 2;  // upper bound of threads; tune_stage_threads of them work
     static constexpr size_t STAGE_CHUNK = 8u << 20;

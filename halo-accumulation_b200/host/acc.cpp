@@ -189,64 +189,61 @@ void decider_batch(halo_ctx* ctx, const std::vector<Accumulator>& accs, const Pa
 //   B_i = sum_{j=0..m_i} alpha_i^j U_{i,j} + omega_i S - C_bar_i  (acc.rs:178, :184, :237; U_{i,0} = U0_i)
 // are O and the host checks d_{i,j} = D, d_i = D, rho_1(C*_i, alpha_i) = z_i with C*_i = C_bar_i - omega_i S, h_i(z_i) = v_i
 // hold.  z' = rho_1(C_i, alpha_i) hashes C_i = sum_j alpha_i^j U_{i,j} itself, which a random combination cannot stand for;
-// C*_i is the only C_i that passes (B_i = O <=> C_i = C*_i), so it is hashed instead.  The T = sum_i (m_i + 2) equations are
-// combined in the order A_0, E_0*, B_0, A_1, .. with the powers of rho into ONE halo_msm.
-void verifier_batch(halo_ctx* ctx, uint64_t D, const std::vector<Step>& steps, const PallasScalar& rho, uint64_t* rejected_index) {
+// C*_i is the only C_i that passes (B_i = O <=> C_i = C*_i), so it is hashed instead.  The T_v = sum_i (m_i + 2) equations
+// are combined in the order A_0, E_0*, B_0, A_1, .. with the powers of rho.  DESIGN.md K5d: the decided claims' E_j, F_j
+// (pcdl::check_batch) follow with rho^(T_v + 2j), rho^(T_v + 2j + 1), and everything is ONE halo_h_msm_batch.
+void verify_decide_batch(halo_ctx* ctx, uint64_t D, const std::vector<Step>& steps, const std::vector<pcdl::Query>& claims,
+                         const PallasScalar& rho, uint64_t* rejected_index) {
     ensure(!fp_is_zero(rho), HALO_EINVAL, "rho is zero");
     const size_t k = steps.size();
-    if (k == 0) return;
+    if (k == 0 && claims.empty()) return;
     PallasPoint S, H;
     params_SH(ctx, S, H);  // missing parameters fail here, before any worker thread reads the context
-    // what the single verifier refuses as malformed, wherever it sits (pcdl::commit of h_0: pcdl.rs:102-104)
     const uint64_t n = D + 1;
-    ensure(n != 0 && !(n & (n - 1)), HALO_EINVAL, "d+1 is not a power of 2");
-    ensure(n <= halo_num_generators(ctx), HALO_EINVAL, "d > D");
-    std::vector<const Instance*> inst;
+    affine_t g[2];
+    pcdl::QueryBatch inst, dec;  // the steps' instances, the decided claims
     std::vector<size_t> first(k + 1, 0);
-    for (size_t i = 0; i < k; i++) {
-        const Accumulator& a = *steps[i].acc;
-        ensure(a.pi_V.h.size() == 2, HALO_EINVAL, "h_0 must have two coefficients");
-        ensure(D >= 1 || fp_is_zero(a.pi_V.h[1]), HALO_EINVAL, "p.degree() > d");
-        first[i] = inst.size();
-        for (const Instance& q : *steps[i].qs) inst.push_back(&q);
+    if (k > 0) {
+        // what the single verifier refuses as malformed, wherever it sits (pcdl::commit of h_0: pcdl.rs:102-104)
+        ensure(n != 0 && !(n & (n - 1)), HALO_EINVAL, "d+1 is not a power of 2");
+        ensure(n <= halo_num_generators(ctx), HALO_EINVAL, "d > D");
+        for (size_t i = 0; i < k; i++) {
+            const Accumulator& a = *steps[i].acc;
+            ensure(a.pi_V.h.size() == 2, HALO_EINVAL, "h_0 must have two coefficients");
+            ensure(D >= 1 || fp_is_zero(a.pi_V.h[1]), HALO_EINVAL, "p.degree() > d");
+            first[i] = inst.qs.size();
+            for (const Instance& q : *steps[i].qs) inst.qs.push_back(pcdl::Query{&q.C, q.d, &q.z, &q.v, &q.pi});
+        }
+        // G_0, G_1 of the A_i: read now, as the read waits for the context's stream, which the generator part will occupy
+        check_rc(ctx, halo_get_generators(ctx, 0, n >= 2 ? 2 : 1, reinterpret_cast<uint64_t*>(g)));
     }
-    first[k] = inst.size();
-    const size_t M = inst.size();
+    first[k] = inst.qs.size();
+    dec.qs = claims;
 
-    // validation + alpha of every instance; then C' of the hiding instances and C*_i of every step in ONE combine call
-    // (the second pass runs on the instances ahead of the first one this pass refused, so the error raised is that of the first
-    // malformed instance in order)
-    std::vector<PallasScalar> alphas(M);
-    const auto errs1 = pcdl::parallel_each(M, [&](size_t j) {
-        const Instance& q = *inst[j];
-        alphas[j] = pcdl::succinct_alpha(ctx, q.C, q.d, q.z, q.v, q.pi);
-    });
-    const size_t f1 = pcdl::first_error(errs1);
-    std::vector<PallasPoint> cP, cQ;
-    std::vector<PallasScalar> ca, cb;
-    std::vector<size_t> slot(M, SIZE_MAX);
-    for (size_t j = 0; j < f1; j++) {
-        if (!inst[j]->pi.hiding) continue;
-        slot[j] = cP.size();
-        cP.push_back(inst[j]->C);
-        cQ.push_back(inst[j]->pi.C_bar);
-        ca.push_back(alphas[j]);
-        cb.push_back(-inst[j]->pi.w_prime);
+    // validation + alpha of every query; then C' of the hiding ones and C*_i of every step in ONE combine call
+    inst.validate(ctx, false);
+    dec.validate(ctx, true);
+    pcdl::CombineList cl;
+    inst.request(cl);
+    dec.request(cl);
+    const size_t star = cl.P.size();
+    for (size_t i = 0; i < k; i++) cl.push(steps[i].acc->C_bar, point_zero(), scalar_zero(), -steps[i].acc->pi_V.w);
+    const std::vector<affine_t> c_out = cl.run(ctx);
+
+    // the decided claims' transcripts; their generator part then runs on the device while the steps' transcripts run here
+    pcdl::parallel_each(dec.valid, [&](size_t j) { dec.finish(ctx, j, c_out); });
+    PallasScalar r_dec = scalar_one();  // rho^T_v
+    for (size_t t = 0; t < inst.qs.size() + 2 * k; t++) r_dec = r_dec * rho;
+    pcdl::BatchTerms terms;
+    pcdl::GeneratorPart gen(ctx);
+    if (!inst.failed() && !dec.failed()) {
+        terms.add_claims(dec, dec.c_prime_affine(c_out), r_dec, rho);
+        gen.submit(terms);
     }
-    const size_t star = cP.size();
-    for (size_t i = 0; i < k; i++) {  // C*_i = C_bar_i - omega_i S
-        cP.push_back(steps[i].acc->C_bar);
-        cQ.push_back(point_zero());
-        ca.push_back(scalar_zero());
-        cb.push_back(-steps[i].acc->pi_V.w);
-    }
-    const std::vector<affine_t> c_out = pcdl::combine(ctx, cP, cQ, ca, cb);
 
     // per step: the rest of every transcript, alpha_i = rho_1(hs_i) (acc.rs:173) and the host checks
-    std::vector<std::optional<pcdl::SuccinctPrep>> preps(M);
     std::vector<std::vector<PallasScalar>> step_alphas(k);
     std::vector<uint8_t> host_ok(k, 0);
-    std::vector<std::exception_ptr> errs2(M);
     const auto step_errs = pcdl::parallel_each(k, [&](size_t i) {
         const Accumulator& a = *steps[i].acc;
         const size_t m = first[i + 1] - first[i];
@@ -255,18 +252,11 @@ void verifier_batch(halo_ctx* ctx, uint64_t D, const std::vector<Step>& steps, c
         hs.have_h0 = true;
         bool ok = a.d == D;  // acc.rs:239
         for (size_t j = first[i]; j < first[i + 1]; j++) {
-            if (j >= f1) return;
-            const Instance& q = *inst[j];
-            PallasPoint C_prime = q.C;
-            if (slot[j] != SIZE_MAX) xyzz_from_affine(C_prime.p, c_out[slot[j]]);
-            try {
-                preps[j].emplace(pcdl::succinct_finish(ctx, C_prime, q.d, q.z, q.v, q.pi));
-            } catch (...) {
-                errs2[j] = std::current_exception();
-                return;
-            }
-            hs.hs.push_back(preps[j]->h);
-            ok = ok && q.d == D;  // acc.rs:169
+            if (j >= inst.valid) return;
+            inst.finish(ctx, j, c_out);
+            if (!inst.preps[j]) return;
+            hs.hs.push_back(inst.preps[j]->h);
+            ok = ok && inst.qs[j].d == D;  // acc.rs:169
         }
         Transcript t;
         hs.serialize(t);
@@ -276,11 +266,9 @@ void verifier_batch(halo_ctx* ctx, uint64_t D, const std::vector<Step>& steps, c
         host_ok[i] = ok;
         step_alphas[i] = std::move(hs.alphas);
     });
-
-    const size_t f2 = pcdl::first_error(errs2);
-    if (f2 < f1) std::rethrow_exception(errs2[f2]);
-    if (f1 < M) std::rethrow_exception(errs1[f1]);
+    inst.rethrow_first();
     if (pcdl::first_error(step_errs) < k) std::rethrow_exception(step_errs[pcdl::first_error(step_errs)]);
+    dec.rethrow_first();
 
     // sum_t rho^t X_t over A_i, E_i1 .. E_im_i, B_i
     std::vector<PallasPoint> acc_pts;  // U0_i, C_bar_i of every step, normalised together
@@ -289,20 +277,8 @@ void verifier_batch(halo_ctx* ctx, uint64_t D, const std::vector<Step>& steps, c
         acc_pts.push_back(steps[i].acc->C_bar);
     }
     const std::vector<affine_t> acc_aff = batch_to_affine(acc_pts);
-    std::vector<affine_t> cp_aff(M);  // C'_ij affine: the combined ones as they come, the others (= C) normalised together
-    std::vector<PallasPoint> plain;
-    std::vector<size_t> plain_at;
-    for (size_t j = 0; j < M; j++) {
-        if (slot[j] != SIZE_MAX)
-            cp_aff[j] = c_out[slot[j]];
-        else
-            plain.push_back(preps[j]->C_prime), plain_at.push_back(j);
-    }
-    const std::vector<affine_t> plain_aff = batch_to_affine(plain);
-    for (size_t i = 0; i < plain_at.size(); i++) cp_aff[plain_at[i]] = plain_aff[i];
-    std::vector<affine_t> aff;
-    std::vector<PallasScalar> sc;
-    PallasScalar s_G0 = scalar_zero(), s_G1 = scalar_zero(), s_H = scalar_zero(), s_S = scalar_zero();
+    const std::vector<affine_t> cp_aff = inst.c_prime_affine(c_out);
+    PallasScalar s_G0 = scalar_zero(), s_G1 = scalar_zero(), s_S = scalar_zero();
     PallasScalar r_t = scalar_one();  // rho^t of the current equation
     for (size_t i = 0; i < k; i++) {
         const Accumulator& a = *steps[i].acc;
@@ -319,55 +295,32 @@ void verifier_batch(halo_ctx* ctx, uint64_t D, const std::vector<Step>& steps, c
         // A_i and B_i's alpha^0 U0_i
         s_G0 = s_G0 - rA * a.pi_V.h[0];
         s_G1 = s_G1 - rA * a.pi_V.h[1];
-        aff.push_back(acc_aff[2 * i]);
-        sc.push_back(rA + rB * al[0]);
-        for (size_t j = first[i]; j < first[i + 1]; j++) {
-            const pcdl::SuccinctPrep& sp = *preps[j];
-            const PallasScalar& re = rE[j - first[i]];
-            const size_t lr = sp.aff.size() - 2;  // L_0, R_0, .., then H, U
-            for (size_t l = 0; l < lr; l++) {
-                aff.push_back(sp.aff[l]);
-                sc.push_back(re * sp.scalars[l]);
-            }
-            s_H = s_H + re * sp.scalars[lr];
-            aff.push_back(sp.aff[lr + 1]);  // U_ij: - rho^tE c from E_ij, + rho^tB alpha_i^j from B_i
-            sc.push_back(re * sp.scalars[lr + 1] + rB * al[j - first[i] + 1]);
-            aff.push_back(cp_aff[j]);  // C'_ij
-            sc.push_back(re);
-        }
+        terms.aff.push_back(acc_aff[2 * i]);
+        terms.sc.push_back(rA + rB * al[0]);
+        // E_ij, and U_ij's + rho^tB alpha_i^j from B_i
+        for (size_t j = first[i]; j < first[i + 1]; j++) terms.add_succinct(*inst.preps[j], cp_aff[j], rE[j - first[i]], rB * al[j - first[i] + 1]);
         s_S = s_S + rB * a.pi_V.w;
-        aff.push_back(acc_aff[2 * i + 1]);  // - C_bar_i
-        sc.push_back(-rB);
-    }
-    affine_t g[2];
-    check_rc(ctx, halo_get_generators(ctx, 0, n >= 2 ? 2 : 1, reinterpret_cast<uint64_t*>(g)));
-    aff.push_back(g[0]);
-    sc.push_back(s_G0);
-    if (n >= 2) {
-        aff.push_back(g[1]);
-        sc.push_back(s_G1);
+        terms.aff.push_back(acc_aff[2 * i + 1]);  // - C_bar_i
+        terms.sc.push_back(-rB);
     }
     const std::vector<affine_t> sh = batch_to_affine({S, H});
-    aff.push_back(sh[0]);
-    sc.push_back(s_S);
-    aff.push_back(sh[1]);
-    sc.push_back(s_H);
-    std::vector<uint8_t> inf(aff.size());
-    for (size_t i = 0; i < aff.size(); i++) inf[i] = affine_is_inf(aff[i]) ? 1 : 0;
-    PallasPoint sum = point_zero();
-    const uint64_t chunk = halo_num_generators(ctx);  // halo_msm takes at most the context's max_n >= generators points per call
-    for (uint64_t off = 0; off < aff.size(); off += chunk) {
-        const uint64_t len = std::min<uint64_t>(chunk, aff.size() - off);
-        uint64_t out[12];
-        check_rc(ctx, halo_msm(ctx, reinterpret_cast<const uint64_t*>(aff.data() + off), inf.data() + off,
-                               reinterpret_cast<const uint64_t*>(sc.data() + off), len, out));
-        sum = sum + point_load(out);
+    if (k > 0) {
+        terms.aff.push_back(g[0]);
+        terms.sc.push_back(s_G0);
+        if (n >= 2) {
+            terms.aff.push_back(g[1]);
+            terms.sc.push_back(s_G1);
+        }
+        terms.aff.push_back(sh[0]);
+        terms.sc.push_back(s_S);
     }
+    const bool zero = gen.is_zero(terms, sh[1]);
     bool all_ok = true;
     for (size_t i = 0; i < k; i++) all_ok = all_ok && host_ok[i];
-    if (all_ok && xyzz_is_inf(sum.p)) return;
+    if (all_ok && zero) return;
 
-    // rejected: the steps one by one, in order, so that (index, code) is what a loop of single verifiers returns
+    // rejected: the steps one by one, in order, then the claims, so that (index, code) is what a loop of single verifiers
+    // followed by a loop of single deciders returns
     for (size_t i = 0; i < k; i++) {
         try {
             verifier(ctx, D, *steps[i].qs, *steps[i].acc);
@@ -376,7 +329,12 @@ void verifier_batch(halo_ctx* ctx, uint64_t D, const std::vector<Step>& steps, c
             throw;
         }
     }
-    throw HaloFailure(HALO_EINTERNAL, "verifier_batch: the combined equation fails but every step accepts on its own");
+    pcdl::check_in_order(ctx, claims, k, rejected_index);
+    throw HaloFailure(HALO_EINTERNAL, "verify_decide_batch: the combined equation fails but every item accepts on its own");
+}
+
+void verifier_batch(halo_ctx* ctx, uint64_t D, const std::vector<Step>& steps, const PallasScalar& rho, uint64_t* rejected_index) {
+    verify_decide_batch(ctx, D, steps, {}, rho, rejected_index);
 }
 
 Instance instance_from_c(const halo_instance& q) {

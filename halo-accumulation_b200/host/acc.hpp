@@ -70,6 +70,12 @@ struct Step {
     const Accumulator* acc;
 };
 void verifier_batch(halo_ctx* ctx, uint64_t D, const std::vector<Step>& steps, const PallasScalar& rho, uint64_t* rejected_index);
+// verifier_batch(steps) followed by pcdl::check_batch(claims) in one call (DESIGN.md K5d): the claims' equations follow the
+// steps' with the next powers of rho, and the generator MSM of the claims runs on the device while the steps' transcripts run
+// on the host.  Decisions and errors are those of the pair, a claim j counting as item k + j of the concatenated sequence
+// "steps, then claims": on a reject *rejected_index = that position.
+void verify_decide_batch(halo_ctx* ctx, uint64_t D, const std::vector<Step>& steps, const std::vector<pcdl::Query>& claims,
+                         const PallasScalar& rho, uint64_t* rejected_index);
 
 Instance instance_from_c(const halo_instance& q);
 Accumulator accumulator_from_c(const halo_accumulator& a);

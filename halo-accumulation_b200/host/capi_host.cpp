@@ -198,9 +198,17 @@ int halo_acc_decider_batch(halo_ctx* ctx, const halo_accumulator* accs, uint64_t
 
 int halo_acc_verifier_batch(halo_ctx* ctx, uint64_t d, const halo_instance* qs, const uint64_t* ms, const halo_accumulator* accs,
                             uint64_t k, const uint64_t rho[4], uint64_t* rejected_index) {
+    return halo_acc_verify_decide_batch(ctx, d, qs, ms, accs, k, nullptr, 0, rho, rejected_index);
+}
+
+int halo_acc_verify_decide_batch(halo_ctx* ctx, uint64_t d, const halo_instance* qs, const uint64_t* ms,
+                                 const halo_accumulator* steps_accs, uint64_t k, const halo_accumulator* decide_accs, uint64_t k_dec,
+                                 const uint64_t rho[4], uint64_t* rejected_index) {
     return guarded([&] {
-        if (k == 0) return;
-        ensure(ms && accs && rho && rejected_index, HALO_EINVAL, "null ms / accumulators / rho / rejected_index");
+        if (k == 0 && k_dec == 0) return;
+        ensure((ms && steps_accs) || k == 0, HALO_EINVAL, "null ms / step accumulators");
+        ensure(decide_accs || k_dec == 0, HALO_EINVAL, "null decided accumulators");
+        ensure(rho && rejected_index, HALO_EINVAL, "null rho / rejected_index");
         const PallasScalar r = scalar_load_checked(rho, "rho is not a canonical scalar");
         uint64_t total = 0;
         for (uint64_t i = 0; i < k; i++) {
@@ -213,16 +221,25 @@ int halo_acc_verifier_batch(halo_ctx* ctx, uint64_t d, const halo_instance* qs, 
         av.reserve(k);
         uint64_t at = 0;
         for (uint64_t i = 0; i < k; i++) {
-            validate(accs[i]);
-            av.push_back(acc::accumulator_from_c(accs[i]));
+            validate(steps_accs[i]);
+            av.push_back(acc::accumulator_from_c(steps_accs[i]));
             for (uint64_t j = 0; j < ms[i]; j++, at++) {
                 validate(qs[at]);
                 qv[i].push_back(acc::instance_from_c(qs[at]));
             }
         }
+        std::vector<acc::Accumulator> dv;
+        dv.reserve(k_dec);
+        for (uint64_t j = 0; j < k_dec; j++) {
+            validate(decide_accs[j]);
+            dv.push_back(acc::accumulator_from_c(decide_accs[j]));
+        }
         std::vector<acc::Step> steps(k);
         for (uint64_t i = 0; i < k; i++) steps[i] = acc::Step{&qv[i], &av[i]};
-        acc::verifier_batch(ctx, d, steps, r, rejected_index);
+        std::vector<pcdl::Query> claims;
+        claims.reserve(k_dec);
+        for (const acc::Accumulator& a : dv) claims.push_back(pcdl::Query{&a.C_bar, a.d, &a.z, &a.v, &a.pi});
+        acc::verify_decide_batch(ctx, d, steps, claims, r, rejected_index);
     });
 }
 

@@ -317,106 +317,146 @@ void check(halo_ctx* ctx, const PallasPoint& C, uint64_t d, const PallasScalar& 
     ensure(sp.U == point_load(out_h), HALO_REJECT_U, "U != CM.Commit(ck, h_vec)");                // :339
 }
 
-void check_batch(halo_ctx* ctx, const std::vector<Query>& qs, const PallasScalar& rho, uint64_t* rejected_index) {
-    ensure(!fp_is_zero(rho), HALO_EINVAL, "rho is zero");
+void QueryBatch::validate(halo_ctx* ctx, bool finish_plain) {
     const size_t k = qs.size();
-    if (k == 0) return;
-    PallasPoint S, H;
-    params_SH(ctx, S, H);  // missing parameters fail here, before any worker thread reads the context
-    // succinct_prepare of every claim: the transcript of check, unchanged, spread over host threads.  Without hiding claims
-    // that is one pass.  Otherwise validation + alpha of every claim come first, then C' = C + alpha C_bar - w' S of the hiding
-    // claims in ONE combine call (on the device from "combine_min_outputs"), then the rest of the transcripts.  The second pass
-    // runs on the claims ahead of the first one the first pass refused, so the error raised is always that of the first
-    // malformed claim in claim order.
-    std::vector<std::optional<SuccinctPrep>> preps(k);
-    std::vector<affine_t> c_aff(k);     // C'_j affine: the combined ones as they come, the others normalised below
-    std::vector<uint8_t> have_aff(k, 0);
-    bool any_hiding = false;
-    for (const Query& q : qs) any_hiding = any_hiding || q.pi->hiding;
-    if (!any_hiding) {
-        const auto errs = parallel_each(k, [&](size_t j) { preps[j].emplace(succinct_prepare(ctx, *qs[j].C, qs[j].d, *qs[j].z, *qs[j].v, *qs[j].pi)); });
-        if (first_error(errs) < k) std::rethrow_exception(errs[first_error(errs)]);
-    } else {
-        std::vector<PallasScalar> alphas(k);
-        const auto errs1 = parallel_each(k, [&](size_t j) { alphas[j] = succinct_alpha(ctx, *qs[j].C, qs[j].d, *qs[j].z, *qs[j].v, *qs[j].pi); });
-        const size_t f1 = first_error(errs1);
-        std::vector<PallasPoint> cP, cQ;
-        std::vector<PallasScalar> ca, cb;
-        std::vector<size_t> slot(k, SIZE_MAX);
-        for (size_t j = 0; j < f1; j++) {
-            if (!qs[j].pi->hiding) continue;
-            slot[j] = cP.size();
-            cP.push_back(*qs[j].C);
-            cQ.push_back(qs[j].pi->C_bar);
-            ca.push_back(alphas[j]);
-            cb.push_back(-qs[j].pi->w_prime);
-        }
-        const std::vector<affine_t> c_out = combine(ctx, cP, cQ, ca, cb);
-        const auto errs2 = parallel_each(f1, [&](size_t j) {
-            PallasPoint C_prime = *qs[j].C;
-            if (slot[j] != SIZE_MAX) xyzz_from_affine(C_prime.p, c_out[slot[j]]);
-            preps[j].emplace(succinct_finish(ctx, C_prime, qs[j].d, *qs[j].z, *qs[j].v, *qs[j].pi));
-        });
-        const size_t f2 = first_error(errs2);
-        if (f2 < f1) std::rethrow_exception(errs2[f2]);
-        if (f1 < k) std::rethrow_exception(errs1[f1]);
-        for (size_t j = 0; j < k; j++)
-            if (slot[j] != SIZE_MAX) c_aff[j] = c_out[slot[j]], have_aff[j] = 1;
-    }
+    alphas.assign(k, scalar_zero());
+    errs2.assign(k, nullptr);
+    slot.assign(k, SIZE_MAX);
+    preps.clear();
+    preps.resize(k);
+    errs1 = parallel_each(k, [&](size_t j) {
+        const Query& q = qs[j];
+        alphas[j] = succinct_alpha(ctx, *q.C, q.d, *q.z, *q.v, *q.pi);
+        if (finish_plain && !q.pi->hiding) finish(ctx, j, {});
+    });
+    valid = first_error(errs1);
+}
 
-    // sum_j rho^2j E_j + rho^(2j+1) F_j with E_j = C'_j + sum_i s_{j,i} P_{j,i} (L, R, H, U) and F_j = U_j - <G, h_j>
-    std::vector<PallasScalar> rp(2 * k);
-    rp[0] = scalar_one();
-    for (size_t i = 1; i < 2 * k; i++) rp[i] = rp[i - 1] * rho;
+void QueryBatch::request(CombineList& cl) {
+    for (size_t j = 0; j < valid; j++)
+        if (qs[j].pi->hiding && !errs2[j]) slot[j] = cl.push(*qs[j].C, qs[j].pi->C_bar, alphas[j], -qs[j].pi->w_prime);
+}
+
+void QueryBatch::finish(halo_ctx* ctx, size_t j, const std::vector<affine_t>& c_out) {
+    if (preps[j] || errs2[j]) return;
+    const Query& q = qs[j];
+    PallasPoint C_prime = *q.C;
+    if (slot[j] != SIZE_MAX) xyzz_from_affine(C_prime.p, c_out[slot[j]]);
+    try {
+        preps[j].emplace(succinct_finish(ctx, C_prime, q.d, *q.z, *q.v, *q.pi));
+    } catch (...) {
+        errs2[j] = std::current_exception();
+    }
+}
+
+bool QueryBatch::failed() const { return valid < qs.size() || first_error(errs2) < qs.size(); }
+
+void QueryBatch::rethrow_first() const {
+    for (size_t j = 0; j < valid; j++)
+        if (errs2[j]) std::rethrow_exception(errs2[j]);
+    if (valid < qs.size()) std::rethrow_exception(errs1[valid]);
+}
+
+std::vector<affine_t> QueryBatch::c_prime_affine(const std::vector<affine_t>& c_out) const {
+    std::vector<affine_t> out(qs.size());  // the combined ones as they come, the others (C' = C) normalised together
     std::vector<PallasPoint> plain;
     std::vector<size_t> plain_at;
-    for (size_t j = 0; j < k; j++)
-        if (!have_aff[j]) plain.push_back(preps[j]->C_prime), plain_at.push_back(j);
-    const std::vector<affine_t> plain_aff = batch_to_affine(plain);
-    for (size_t i = 0; i < plain_at.size(); i++) c_aff[plain_at[i]] = plain_aff[i];
-    std::vector<affine_t> aff;
-    std::vector<uint8_t> inf;
-    std::vector<PallasScalar> sc, xis, weights;
-    std::vector<uint32_t> lgs(k);
-    PallasScalar s_H = scalar_zero();
-    for (size_t j = 0; j < k; j++) {
-        const SuccinctPrep& sp = *preps[j];
-        const size_t lr = sp.aff.size() - 2;  // L_0, R_0, .., then H, U
-        for (size_t i = 0; i < lr; i++) {
-            aff.push_back(sp.aff[i]);
-            inf.push_back(sp.inf[i]);
-            sc.push_back(rp[2 * j] * sp.scalars[i]);
-        }
-        s_H = s_H + rp[2 * j] * sp.scalars[lr];
-        aff.push_back(sp.aff[lr + 1]);  // U_j: - rho^2j c_j from E_j, + rho^(2j+1) from F_j
-        inf.push_back(sp.inf[lr + 1]);
-        sc.push_back(rp[2 * j] * sp.scalars[lr + 1] + rp[2 * j + 1]);
-        aff.push_back(c_aff[j]);  // C'_j
-        inf.push_back(affine_is_inf(c_aff[j]) ? 1 : 0);
-        sc.push_back(rp[2 * j]);
-        lgs[j] = (uint32_t)sp.h.xis.size() - 1;
-        xis.insert(xis.end(), sp.h.xis.begin(), sp.h.xis.end());
-        weights.push_back(-rp[2 * j + 1]);
+    for (size_t j = 0; j < qs.size(); j++) {
+        if (slot[j] != SIZE_MAX)
+            out[j] = c_out[slot[j]];
+        else
+            plain.push_back(preps[j]->C_prime), plain_at.push_back(j);
     }
-    const size_t h_at = preps[0]->aff.size() - 2;  // H, the same point in every claim
-    aff.push_back(preps[0]->aff[h_at]);
-    inf.push_back(preps[0]->inf[h_at]);
-    sc.push_back(s_H);
-    uint64_t out[12];
-    check_rc(ctx, halo_h_msm_batch(ctx, reinterpret_cast<const uint64_t*>(xis.data()), lgs.data(),
-                                   reinterpret_cast<const uint64_t*>(weights.data()), k, reinterpret_cast<const uint64_t*>(aff.data()),
-                                   inf.data(), reinterpret_cast<const uint64_t*>(sc.data()), aff.size(), out));
-    if (xyzz_is_inf(point_load(out).p)) return;
+    const std::vector<affine_t> plain_aff = batch_to_affine(plain);
+    for (size_t i = 0; i < plain_at.size(); i++) out[plain_at[i]] = plain_aff[i];
+    return out;
+}
 
-    // rejected: the claims one by one, in order, so that (index, code) is what a loop of single deciders returns
-    for (size_t j = 0; j < k; j++) {
+void BatchTerms::add_succinct(const SuccinctPrep& sp, const affine_t& c_prime, const PallasScalar& re, const PallasScalar& u_extra) {
+    const size_t lr = sp.aff.size() - 2;  // L_0, R_0, .., then H, U
+    for (size_t l = 0; l < lr; l++) {
+        aff.push_back(sp.aff[l]);
+        sc.push_back(re * sp.scalars[l]);
+    }
+    s_H = s_H + re * sp.scalars[lr];
+    aff.push_back(sp.aff[lr + 1]);
+    sc.push_back(re * sp.scalars[lr + 1] + u_extra);
+    aff.push_back(c_prime);
+    sc.push_back(re);
+}
+
+void BatchTerms::add_claims(const QueryBatch& qb, const std::vector<affine_t>& c_aff, PallasScalar r, const PallasScalar& rho) {
+    for (size_t j = 0; j < qb.qs.size(); j++) {
+        const SuccinctPrep& sp = *qb.preps[j];
+        const PallasScalar rf = r * rho;
+        add_succinct(sp, c_aff[j], r, rf);  // U_j: - rho^t c_j from E_j, + rho^(t+1) from F_j
+        lgs.push_back((uint32_t)sp.h.xis.size() - 1);
+        xis.insert(xis.end(), sp.h.xis.begin(), sp.h.xis.end());
+        weights.push_back(-rf);
+        r = rf * rho;
+    }
+}
+
+GeneratorPart::~GeneratorPart() {
+    if (ticket_ < 0) return;
+    uint64_t out[12];
+    halo_h_msm_batch_collect(ctx_, ticket_, nullptr, nullptr, nullptr, 0, out);
+}
+
+void GeneratorPart::submit(const BatchTerms& t) {
+    check_rc(ctx_, halo_h_msm_batch_submit(ctx_, reinterpret_cast<const uint64_t*>(t.xis.data()), t.lgs.data(),
+                                           reinterpret_cast<const uint64_t*>(t.weights.data()), t.lgs.size(), &ticket_));
+}
+
+bool GeneratorPart::is_zero(BatchTerms& t, const affine_t& H) {
+    t.aff.push_back(H);  // H, the same point in every succinct equation
+    t.sc.push_back(t.s_H);
+    std::vector<uint8_t> inf(t.aff.size());
+    for (size_t i = 0; i < t.aff.size(); i++) inf[i] = affine_is_inf(t.aff[i]) ? 1 : 0;
+    const int ticket = ticket_;
+    ticket_ = -1;
+    uint64_t out[12];
+    check_rc(ctx_, halo_h_msm_batch_collect(ctx_, ticket, reinterpret_cast<const uint64_t*>(t.aff.data()), inf.data(),
+                                            reinterpret_cast<const uint64_t*>(t.sc.data()), t.aff.size(), out));
+    return xyzz_is_inf(point_load(out).p);
+}
+
+void check_in_order(halo_ctx* ctx, const std::vector<Query>& qs, uint64_t index_base, uint64_t* rejected_index) {
+    for (size_t j = 0; j < qs.size(); j++) {
         try {
             check(ctx, *qs[j].C, qs[j].d, *qs[j].z, *qs[j].v, *qs[j].pi);
         } catch (const HaloFailure& e) {
-            if (e.code <= HALO_REJECT_SUCCINCT && rejected_index) *rejected_index = j;
+            if (e.code <= HALO_REJECT_SUCCINCT && rejected_index) *rejected_index = index_base + j;
             throw;
         }
     }
+}
+
+void check_batch(halo_ctx* ctx, const std::vector<Query>& qs, const PallasScalar& rho, uint64_t* rejected_index) {
+    ensure(!fp_is_zero(rho), HALO_EINVAL, "rho is zero");
+    if (qs.empty()) return;
+    PallasPoint S, H;
+    params_SH(ctx, S, H);  // missing parameters fail here, before any worker thread reads the context
+    // the transcript of check, unchanged, spread over host threads: the claims without hiding in one pass; C' = C + alpha C_bar
+    // - w' S of the hiding ones in ONE combine call (on the device from "combine_min_outputs"), then their transcripts
+    QueryBatch qb;
+    qb.qs = qs;
+    qb.validate(ctx, true);
+    CombineList cl;
+    qb.request(cl);
+    const std::vector<affine_t> c_out = cl.run(ctx);
+    parallel_each(qb.valid, [&](size_t j) { qb.finish(ctx, j, c_out); });
+    qb.rethrow_first();
+
+    // sum_j rho^2j E_j + rho^(2j+1) F_j with E_j = C'_j + sum_i s_{j,i} P_{j,i} (L, R, H, U) and F_j = U_j - <G, h_j>
+    BatchTerms t;
+    t.add_claims(qb, qb.c_prime_affine(c_out), scalar_one(), rho);
+    GeneratorPart gen(ctx);
+    gen.submit(t);
+    if (gen.is_zero(t, batch_to_affine({S, H})[1])) return;
+
+    // rejected: the claims one by one, in order, so that (index, code) is what a loop of single deciders returns
+    check_in_order(ctx, qs, 0, rejected_index);
     throw HaloFailure(HALO_EINTERNAL, "check_batch: the combined equation fails but every claim accepts on its own");
 }
 

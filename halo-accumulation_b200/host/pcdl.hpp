@@ -2,6 +2,7 @@
 #pragma once
 #include <exception>
 #include <functional>
+#include <optional>
 
 #include "../../include/halo_pcdl.h"
 #include "group.hpp"
@@ -91,6 +92,66 @@ void check(halo_ctx* ctx, const PallasPoint& C, uint64_t d, const PallasScalar& 
 // if every claim then accepts, the batch contradicted them: HALO_EINTERNAL.  Malformed input in any claim throws
 // HALO_EINVAL before any decision.
 void check_batch(halo_ctx* ctx, const std::vector<Query>& claims, const PallasScalar& rho, uint64_t* rejected_index);
+
+// ---- the stages shared by the batch checks (check_batch, acc::verifier_batch, acc::verify_decide_batch; DESIGN.md K5d) ----
+// Inputs of ONE `combine` call, gathered from every part of a batch.
+struct CombineList {
+    std::vector<PallasPoint> P, Q;
+    std::vector<PallasScalar> a, b;
+    size_t push(const PallasPoint& p, const PallasPoint& q, const PallasScalar& x, const PallasScalar& y) {
+        P.push_back(p), Q.push_back(q), a.push_back(x), b.push_back(y);
+        return P.size() - 1;
+    }
+    std::vector<affine_t> run(halo_ctx* ctx) const { return combine(ctx, P, Q, a, b); }
+};
+// The succinct equations of a list of queries, prepared in three steps around the one `combine` call of the batch:
+// validate() (every query's validation and alpha, on host threads), request() (C' of the hiding queries that passed) and
+// finish(j) (query j's transcript from its C').  The error of a batch is that of its first malformed query in order:
+// rethrow_first() raises it, whichever step found it.
+struct QueryBatch {
+    std::vector<Query> qs;
+    std::vector<PallasScalar> alphas;
+    std::vector<std::exception_ptr> errs1, errs2;  // validate() / finish() failures
+    size_t valid = 0;                              // queries ahead of the first one validate() refused
+    std::vector<size_t> slot;                      // C' in the combine output (SIZE_MAX: C' = C)
+    std::vector<std::optional<SuccinctPrep>> preps;
+    void validate(halo_ctx* ctx, bool finish_plain);  // finish_plain: finish the queries without hiding in the same pass
+    void request(CombineList& cl);
+    void finish(halo_ctx* ctx, size_t j, const std::vector<affine_t>& c_out);  // j < valid
+    bool failed() const;                           // some query is malformed
+    void rethrow_first() const;                    // no-op if none is
+    std::vector<affine_t> c_prime_affine(const std::vector<affine_t>& c_out) const;  // C'_j of every query, affine
+};
+// Terms of one combined equation sum_t rho^t X_t = O: the companion MSM (points and scalars; H once, with its scalars summed)
+// and the generator part <GS, sum_j w_j coeffs(h_j)> (the claims' xi rows, lg n and weights).
+struct BatchTerms {
+    std::vector<affine_t> aff;
+    std::vector<PallasScalar> sc;
+    PallasScalar s_H = scalar_zero();
+    std::vector<PallasScalar> xis, weights;
+    std::vector<uint32_t> lgs;
+    // re E + u_extra U for the succinct equation E = C' + sum_i s_i P_i (L, R, H, U) of one query
+    void add_succinct(const SuccinctPrep& sp, const affine_t& c_prime, const PallasScalar& re, const PallasScalar& u_extra);
+    // the claims' E_j and F_j = U_j - <G, h_j> with rho^t, rho^(t+1) for claim j, t = 2 j from rho_first on
+    void add_claims(const QueryBatch& qb, const std::vector<affine_t>& c_aff, PallasScalar rho_first, const PallasScalar& rho);
+};
+// The decide stage: the generator part is submitted ahead of the host work that builds the companion terms; is_zero()
+// collects with them and tells whether the combined point is O.  A batch left outstanding (the caller threw) is drained on
+// destruction.
+class GeneratorPart {
+  public:
+    explicit GeneratorPart(halo_ctx* ctx) : ctx_(ctx) {}
+    GeneratorPart(const GeneratorPart&) = delete;
+    GeneratorPart& operator=(const GeneratorPart&) = delete;
+    ~GeneratorPart();
+    void submit(const BatchTerms& t);
+    bool is_zero(BatchTerms& t, const affine_t& H);
+  private:
+    halo_ctx* ctx_;
+    int ticket_ = -1;
+};
+// `check` on claims in order; a reject is thrown with *rejected_index = index_base + its claim
+void check_in_order(halo_ctx* ctx, const std::vector<Query>& claims, uint64_t index_base, uint64_t* rejected_index);
 
 // wire conversion
 EvalProof proof_from_c(const halo_eval_proof& p);

@@ -218,10 +218,20 @@ int halo_h_msm_with(halo_ctx *ctx, const uint64_t *xis /*[lg_n+1][4]*/, uint32_t
  * is built on the device in one kernel, then the generator MSM (FIXED-base tables under the same condition as halo_h_msm)
  * and the companion MSM over caller-supplied affine points run on two streams.  m is not limited to 4096 (k claims at
  * lg n = 20 bring 42 k + 1 points, DESIGN.md K5b).  Each lg_ns[j] is checked like halo_h_msm's lg_n; k, m < 2^32.
- * k = m = 0 gives infinity. */
+ * k = m = 0 gives infinity.  Same as halo_h_msm_batch_submit followed by halo_h_msm_batch_collect. */
 int halo_h_msm_batch(halo_ctx *ctx, const uint64_t *xis /*sum_j (lg_ns[j]+1) rows of [4]*/, const uint32_t *lg_ns /*[k]*/,
                      const uint64_t *weights /*[k][4]*/, uint64_t k, const uint64_t *bases_affine /*[m][8]*/,
                      const uint8_t *inf_flags /*[m] or NULL*/, const uint64_t *scalars /*[m][4]*/, uint64_t m, uint64_t out_jac[12]);
+/* halo_h_msm_batch in two calls (K5d), so that the caller's host work runs while the device computes the generator part.
+ * submit enqueues the coefficient sum and the generator MSM and returns without waiting for the device; the caller's
+ * buffers are read before it returns.  collect runs the companion MSM on the second stream, waits for both and returns
+ * their sum, which is what halo_h_msm_batch returns for the same arguments.  One batch may be outstanding per context:
+ * a second submit, or a collect without a submit, is HALO_ESTATE.  A caller that gives up after a submit collects with
+ * m = 0 to leave the context idle.  Other calls of the library may be made between the two. */
+int halo_h_msm_batch_submit(halo_ctx *ctx, const uint64_t *xis /*sum_j (lg_ns[j]+1) rows of [4]*/, const uint32_t *lg_ns /*[k]*/,
+                            const uint64_t *weights /*[k][4]*/, uint64_t k, int *ticket);
+int halo_h_msm_batch_collect(halo_ctx *ctx, int ticket, const uint64_t *bases_affine /*[m][8]*/, const uint8_t *inf_flags /*[m] or NULL*/,
+                             const uint64_t *scalars /*[m][4]*/, uint64_t m, uint64_t out_jac[12]);
 /* A batch of small, independent MSMs with ONE host round trip (SURVEY 8(f).2): the accumulation verifier's
  * common_subroutine (acc.rs:135-188) needs commit(h_0) (acc.rs:153) and, per instance q_i, the 2 lg n + 2 point MSM that
  * succinct_check's group equation reduces to (pcdl.rs:285-310); none depends on another's result, so they are enqueued

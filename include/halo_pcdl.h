@@ -136,6 +136,25 @@ int halo_acc_decider_batch(halo_ctx *ctx, const halo_accumulator *accs, uint64_t
  * k = 0 accepts and reads no other argument.  *rejected_index is written on a reject only. */
 int halo_acc_verifier_batch(halo_ctx *ctx, uint64_t d, const halo_instance *qs /*[sum ms]*/, const uint64_t *ms /*[k]*/,
                             const halo_accumulator *accs /*[k]*/, uint64_t k, const uint64_t rho[4], uint64_t *rejected_index);
+/* Batch verify-and-decide (DESIGN.md K5d): halo_acc_verifier_batch(d, qs, ms, steps_accs, k) followed by
+ * halo_acc_decider_batch(decide_accs, k_dec) in ONE call, with the same decisions and errors as that pair.  The combined
+ * equation is the T_v = sum_i (ms[i] + 2) equations of the steps, in the order of halo_acc_verifier_batch, followed by the
+ * pair E_j, F_j of halo_acc_decider_batch for each decided accumulator, the powers of rho running on across the boundary;
+ * a false accept has probability <= (T - 1) / r, T = T_v + 2 k_dec, when rho is drawn after both lists are fixed.  The
+ * generator MSM of the decided accumulators runs on the device while the steps' transcripts run on the host.
+ * Returns
+ *   HALO_OK         accept, iff the combined point is O and every host check of every step holds;
+ *   HALO_REJECT_*   otherwise halo_acc_verifier runs on steps 0, 1, .., then halo_acc_decider on the decided accumulators
+ *                   0, 1, .., and the first reject is returned with *rejected_index = its position in the sequence "steps,
+ *                   then decided accumulators": step i is i, decided accumulator j is k + j;
+ *   HALO_EINTERNAL  the combined check failed but every item accepts on its own (a bug, not a decision);
+ *   HALO_EINVAL     before any decision, for malformed input anywhere in either list (what either batch call refuses), the
+ *                   error of the first malformed item in the same order; rho = 0 or not canonical; ms / steps_accs NULL with
+ *                   k > 0, decide_accs NULL with k_dec > 0, rho / rejected_index NULL.
+ * k = k_dec = 0 accepts and reads no other argument.  A decided accumulator may also be one of the steps' accumulators. */
+int halo_acc_verify_decide_batch(halo_ctx *ctx, uint64_t d, const halo_instance *qs /*[sum ms]*/, const uint64_t *ms /*[k]*/,
+                                 const halo_accumulator *steps_accs /*[k]*/, uint64_t k, const halo_accumulator *decide_accs /*[k_dec]*/,
+                                 uint64_t k_dec, const uint64_t rho[4], uint64_t *rejected_index);
 /* impl From<Accumulator> for Instance, acc.rs:121-131 */
 void halo_acc_to_instance(const halo_accumulator *acc, halo_instance *q);
 

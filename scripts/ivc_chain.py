@@ -49,6 +49,8 @@ t = time.perf_counter(); acc.decider(ctx, accs[-1]); t_dec = time.perf_counter()
 # the same fast path with ONE batch verifier over the k steps (rho drawn after the steps are fixed)
 rho = rs(1)[0]
 t = time.perf_counter(); acc.verifier_batch(ctx, d, list(zip(qss, accs)), rho); acc.decider(ctx, accs[-1]); t_fast_batch = time.perf_counter() - t
+# and with ONE fused call: the steps verified and the last accumulator decided together (DESIGN.md K5d)
+t = time.perf_counter(); acc.verify_decide_batch(ctx, d, list(zip(qss, accs)), [accs[-1]], rho); t_fast_fused = time.perf_counter() - t
 # ---- the oracle's view of the same chain (checker only, untimed) ----
 from oracle import oracle as O
 S, Hh = ctx.get_SH()
@@ -62,7 +64,7 @@ all_accept = all(rc == 0 for rc in oracle_verifier.values()) and oracle_decider 
 print(json.dumps({"config": f"ivc_chain_2^{lg}_k{k}", "setup_s": setup_s, "random_instance_ms": t_inst / k * 1e3, "prover_ms": t_prov / k * 1e3,
                   "random_instance_ms_median": float(np.median(inst_ms)), "prover_ms_median": float(np.median(prov_ms)),
                   "random_instance_ms_first3": inst_ms[:3], "verifier_ms": t_ver / k * 1e3, "decider_ms": t_dec * 1e3, "fast_path_total_s": t_ver + t_dec,
-                  "fast_path_batch_s": t_fast_batch,
+                  "fast_path_batch_s": t_fast_batch, "fast_path_fused_s": t_fast_fused,
                   "chain_total_s": t_inst + t_prov, "kernel_launches": ctx.kernel_launches(), "all_accept": all_accept,
                   "oracle": {"acc_verifier_rc_at_steps": {str(s): rc for s, rc in oracle_verifier.items()}, "acc_decider_rc": oracle_decider,
                              "acc_decider_cpu_ms": t_odec * 1e3, "threads": T}}))
