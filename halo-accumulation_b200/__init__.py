@@ -328,6 +328,14 @@ class Context:
         self._chk(self._lib.halo_test_add_chain(self._h, p64(a), C.c_uint64(a.shape[0]), int(dbls), p64(out)))
         return out
 
+    MSM_ROUTE_KEYS = ("c", "fixed", "P", "pass0_async", "acc", "quad_lanes", "quad_blocks", "acc_grid", "reduce_quad", "two_lanes")
+
+    def test_msm_route(self, lane=0):
+        """What the last MSM on `lane` ran (halo_test_msm_route); acc: 2 quad, 1 static, 0 lane claiming.  Reading clears it."""
+        out = (C.c_int * 10)()
+        self._chk(self._lib.halo_test_msm_route(self._h, int(lane), out))
+        return dict(zip(self.MSM_ROUTE_KEYS, list(out)))
+
     def test_fp_mul_throughput(self, blocks, threads, iters, ilp=1):
         ms, ck = C.c_float(), C.c_uint64()
         self._chk(self._lib.halo_test_fp_mul_throughput(self._h, blocks, threads, iters, ilp, C.byref(ms), C.byref(ck)))

@@ -247,6 +247,16 @@ int halo_set_msm_window(halo_ctx* ctx, int c) {
 }
 int halo_set_tuning(halo_ctx* ctx, const char* key, int value) {
     if (!ctx || !key) return HALO_EINVAL;
+    // values that become a plan or a launch geometry are checked, not cast or silently replaced
+    bool ok = true;
+    if (!strcmp(key, "acc_static")) ok = value >= 0 && value <= 2;
+    else if (!strcmp(key, "acc_blocks_per_sm")) ok = value >= 0 && value <= 32;
+    else if (!strcmp(key, "acc_quad_max_buckets")) ok = value >= 0;
+    else if (!strcmp(key, "acc_quad_lanes")) ok = value == 0 || value == 2 || value == 4;
+    else if (!strcmp(key, "acc_quad_blocks")) ok = value == 0 || value == 4 || value == 6;
+    else if (!strcmp(key, "pair_passes")) ok = value >= -1;
+    else if (!strcmp(key, "ipa_frozen_c")) ok = value == 0 || (value >= 4 && value <= 20);  // the range of halo_set_msm_window
+    if (!ok) return fail(ctx, HALO_EINVAL, "halo_set_tuning: value out of range for this key (include/halo_b200.h)");
     if (!strcmp(key, "acc_static")) ctx->tune_acc_static = value;
     else if (!strcmp(key, "acc_blocks_per_sm")) ctx->tune_acc_blocks_per_sm = value;
     else if (!strcmp(key, "acc_quad")) ctx->tune_acc_quad = value;

@@ -235,6 +235,9 @@ struct halo_ctx {
                                   // accumulation phase at 2^24 27.39 -> 26.75 ms; profiles/r02_pair_bwd_async_ab.jsonl), 0 = per-lane gathers
     int tune_reduce_quad = 1;   // 0: one-lane bucket reduction (k_reduce_slabs), for A/B measurements
     int tune_pair_passes = -1;  // -1: automatic; 0: XYZZ accumulation only; P > 0: force P pair-tree passes
+    // what msm_enqueue chose for the last MSM on each lane (halo_test_msm_route, layout in include/halo_b200_test.h); host
+    // bookkeeping only, written next to the decisions themselves
+    int msm_route[2][10] = {};
     uint64_t kernel_launches = 0;
     halo::Timings last;
     bool profile = false;

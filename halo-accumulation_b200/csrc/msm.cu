@@ -1402,6 +1402,8 @@ void msm_enqueue(halo_ctx* ctx, const MsmInput& in, MsmPlan& plan, xyzz_t* d_out
     // measured (profiles/r02_acc_quad_ab.jsonl): 2^8 .. 2^14 points (<= 24 576 buckets) 0.080 -> 0.041, 0.108 -> 0.055, 0.197 -> 0.165,
     // 0.324 -> 0.229 ms; at 2^15 / 2^16 (82 k buckets: 4.3 waves of quads, two extra full additions per bucket) it loses
     const bool quad_lanes = !P && ctx->tune_acc_quad != 0 && NB <= (uint32_t)ctx->tune_acc_quad_max_buckets && ctx->tune_acc_static == 0 && !deep;
+    int acc_kind = 0, acc_lanes = 0, acc_minb = 0;  // 2 = k_accumulate_quad, 1 = k_accumulate_static, 0 = k_accumulate
+    uint32_t acc_grid = 0;
     if (quad_lanes) {
         // lanes per bucket and CTAs per SM (tunables acc_quad_lanes / acc_quad_blocks; 0 = the policy below)
         int lanes = ctx->tune_acc_quad_lanes, minb = ctx->tune_acc_quad_blocks;
@@ -1411,7 +1413,9 @@ void msm_enqueue(halo_ctx* ctx, const MsmInput& in, MsmPlan& plan, xyzz_t* d_out
         if (lanes != 2 && lanes != 4) lanes = 4;
         if (minb != 4 && minb != 6) minb = 4;
         launch_accumulate_quad(st, lanes, minb, acc_bases, acc_n, in.tail_bases, acc_offsets, entries, NB, buckets, split_len);
+        acc_kind = 2, acc_lanes = lanes, acc_minb = minb;
     } else if (ctx->tune_acc_static == 1 || (ctx->tune_acc_static == 0 && deep)) {
+        acc_kind = 1;
         if (P)
             k_accumulate_static<true><<<(NB + 127) / 128, 128, 0, st>>>(acc_bases, acc_n, in.tail_bases, acc_offsets, entries, NB,
                                                                        buckets, split_len);
@@ -1423,6 +1427,7 @@ void msm_enqueue(halo_ctx* ctx, const MsmInput& in, MsmPlan& plan, xyzz_t* d_out
         uint32_t want_blocks = (NB + 127) / 128;
         uint32_t max_blocks = (uint32_t)ctx->sm_count * (ctx->tune_acc_blocks_per_sm ? ctx->tune_acc_blocks_per_sm : HALO_ACC_MIN_BLOCKS);
         uint32_t blocks = want_blocks < max_blocks ? want_blocks : max_blocks;
+        acc_grid = blocks;
         uint32_t* next_bucket = counts + NB;  // spare slot at the end of the counter array (zeroed above)
         if (P)
             k_accumulate<true><<<blocks, 128, 0, st>>>(acc_bases, acc_n, in.tail_bases, acc_offsets, entries, NB, buckets, next_bucket,
@@ -1480,6 +1485,17 @@ void msm_enqueue(halo_ctx* ctx, const MsmInput& in, MsmPlan& plan, xyzz_t* d_out
     mark(5);
     ctx->kernel_launches += 1;  // the accumulation kernel (the sort counted its own above)
     HALO_CUDA(cudaGetLastError());
+    int* route = ctx->msm_route[lane ? 1 : 0];
+    route[0] = plan.c;
+    route[1] = plan.fixed ? 1 : 0;
+    route[2] = P;
+    route[3] = P ? (ctx->tune_pair_bwd_async ? 1 : 0) : -1;
+    route[4] = acc_kind;
+    route[5] = acc_kind == 2 ? acc_lanes : 0;
+    route[6] = acc_kind == 2 ? acc_minb : 0;
+    route[7] = acc_kind == 0 ? (int)acc_grid : 0;
+    route[8] = plan.red_quad ? 1 : 0;
+    route[9] = -1;  // msm_batch overwrites it with its lane decision
 }
 
 // Host finish: per window S = E + slab * (A2 - R2), then Horner over the windows (a single term in FIXED mode).
@@ -1538,6 +1554,7 @@ void msm_batch(halo_ctx* ctx, const MsmInput* ins, int count, xyzz_t* outs, cons
         const int lane = two_lanes ? (k & 1) : 0;
         cudaStream_t st = lane ? ctx->stream2 : ctx->stream;
         msm_enqueue(ctx, ins[k], plans[k], d_parts + k * SLOT, lane);
+        ctx->msm_route[lane][9] = two_lanes ? 1 : 0;
         const int nwin = plans[k].fixed ? 1 : plans[k].W;
         HALO_CUDA(cudaMemcpyAsync(h_parts + k * SLOT, d_parts + k * SLOT, (size_t)3 * nwin * sizeof(xyzz_t), cudaMemcpyDeviceToHost, st));
         any = true;

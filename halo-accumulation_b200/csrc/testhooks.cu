@@ -331,6 +331,13 @@ int halo_test_check_canaries(int* live_buffers) {
     return bad;
 }
 
+int halo_test_msm_route(halo_ctx* ctx, int lane, int out[10]) {
+    if (!ctx || !out || lane < 0 || lane > 1) return HALO_EINVAL;
+    memcpy(out, ctx->msm_route[lane], sizeof ctx->msm_route[lane]);
+    memset(ctx->msm_route[lane], 0, sizeof ctx->msm_route[lane]);  // c = 0 until the next MSM on this lane
+    return HALO_OK;
+}
+
 int halo_test_gather_throughput(halo_ctx* ctx, uint64_t table_bytes, int blocks, int threads, int iters, int bytes, float* ms) {
     if (!ctx || !ms || table_bytes < 4096 || threads > 256) return HALO_EINVAL;
     T_TRY(ctx)

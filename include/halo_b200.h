@@ -60,18 +60,25 @@ const char *halo_curve_name(void);
 uint64_t halo_kernel_launches(halo_ctx *ctx);
 /* Tuning / diagnostics: force the Pippenger window width (0 = automatic). */
 int halo_set_msm_window(halo_ctx *ctx, int c);
-/* Measurement knobs (no effect on results; every value is exercised against the oracle in tests/).  Keys:
- *   accumulation   "acc_static" 1 / 2 = force thread-per-bucket / lane-level bucket claiming (0 = automatic), "acc_blocks_per_sm",
- *                  "acc_quad" (four lanes per bucket for small MSMs), "acc_quad_max_buckets", "acc_quad_lanes" (2 / 4), "acc_quad_blocks"
- *                  (4 / 6 CTAs per SM), "pair_passes" (-1 = policy by bucket fill), "pair_bwd_async", "reduce_quad"
- *   counting sort  "sort_ahead" (CTAs per SM of the sort of the next pipelined call), "sort2", "sort2_min_lg" (two-level staged sort)
- *   host buffers   "split_blocking" (lg of the size from which the blocking call runs as point slices), "split_first_16ths",
- *                  "split_second_16ths" (0 = two slices), "stage_pageable", "stage_threads" (1 .. 8)
- *   opening        "ipa_defer_rounds" (-1 = automatic), "ipa_defer2_rounds", "ipa_two_lanes", "ipa_freeze_len", "ipa_frozen_c",
- *                  "ipa_fold_call_min_lg" (folds of >= 2^v outputs use the kernel copy with the multiplication out of line)
+/* Measurement knobs: they select alternative kernels, launch geometries and schedules, not results.  The MSM and opening
+ * variants are compared with the oracle, and with each other, in tests/test_gpu_tuning.py (which also checks that this list
+ * matches the keys the library accepts); the host-buffer, sort and batch-check knobs in the tests named there.  Keys and values:
+ *   accumulation   "acc_static" 0 .. 2: 1 / 2 = force thread-per-bucket / lane-level bucket claiming (0 = automatic);
+ *                  "acc_blocks_per_sm" 0 .. 32 (CTAs per SM of the lane-claiming kernel, 0 = 4); "acc_quad" 0 / other (four
+ *                  lanes per bucket for small MSMs); "acc_quad_max_buckets" >= 0; "acc_quad_lanes" 0 / 2 / 4 and "acc_quad_blocks"
+ *                  0 / 4 / 6 (CTAs per SM; 0 = policy); "pair_passes" >= -1 (-1 = policy by bucket fill, above 8 means 8);
+ *                  "pair_bwd_async" 0 / other; "reduce_quad" 0 / other (refused above the size limit of the quad reduction)
+ *   counting sort  "sort_ahead" (CTAs per SM of the sort of the next pipelined call, 0 = off), "sort2" 0 / other, "sort2_min_lg"
+ *                  (two-level staged sort)
+ *   host buffers   "split_blocking" (lg of the size from which the blocking call runs as point slices, 0 = never),
+ *                  "split_first_16ths" (clamped to 1 .. 15), "split_second_16ths" (clamped to 0 .. 14; 0 = two slices),
+ *                  "stage_pageable" 0 / other, "stage_threads" (clamped to 1 .. 8)
+ *   opening        "ipa_defer_rounds" (-1 = automatic), "ipa_defer2_rounds", "ipa_two_lanes" 0 / other, "ipa_freeze_len" (0 = 8192),
+ *                  "ipa_frozen_c" 0 or 4 .. 20 (0 = automatic window), "ipa_fold_call_min_lg" (folds of >= 2^v outputs use the
+ *                  kernel copy with the multiplication out of line; -1 = never)
  *   batch checks   "combine_min_outputs" (the exact C' = C + alpha C_bar - w' S of hiding claims and C* = C_bar - omega S of
  *                  accumulation steps run as one device launch from this many points on, on host threads below; -1 = never)
- * Unknown keys return HALO_EINVAL. */
+ * Unknown keys and values outside the ranges given return HALO_EINVAL. */
 int halo_set_tuning(halo_ctx *ctx, const char *key, int value);
 /* Enable per-phase CUDA-event timing of the MSM; read back with halo_last_msm_timings (ms):
  * [digits, scan, scatter, accumulate, bucket_reduce, total]. */

@@ -27,6 +27,18 @@ int halo_test_imad_throughput(halo_ctx *ctx, int kind, int blocks, int threads, 
 /* Every device buffer of the library is allocated with a 256-byte canary behind its end.  Returns the number of live
  * buffers whose canary was overwritten (0 = no kernel wrote past a buffer); *live_buffers = how many were checked. */
 int halo_test_check_canaries(int *live_buffers);
+/* Route of the last MSM enqueued on `lane` (0: the context's stream; 1: the second stream of two-lane batches and of the
+ * companion MSM of halo_h_msm_batch), as the host code chose it from the plan, the size and halo_set_tuning:
+ *   out[0] window c            out[1] 1 = FIXED base, 0 = variable base     out[2] P, pair-tree passes (after the clamp to 8)
+ *   out[3] pass-0 kernel of the pair tree: 1 = k_pair_bwd0 (cp.async), 0 = k_pair_bwd<true> (per-lane gathers), -1 = P == 0
+ *   out[4] accumulation kernel: 2 = k_accumulate_quad, 1 = k_accumulate_static, 0 = k_accumulate (lane claiming)
+ *   out[5] lanes per bucket and out[6] CTAs per SM of k_accumulate_quad (0 for the other kernels)
+ *   out[7] grid of k_accumulate (0 for the other kernels)
+ *   out[8] bucket reduction: 1 = k_reduce_slabs_quad, 0 = k_reduce_slabs (one lane per addition)
+ *   out[9] 1 / 0: the msm_batch that enqueued it ran on two lanes / one; -1: enqueued outside msm_batch
+ * Reading clears the record (out[0] = 0 until the next MSM on that lane).  Host bookkeeping only: no kernel, launch or device
+ * memory. */
+int halo_test_msm_route(halo_ctx *ctx, int lane, int out[10]);
 /* Random-gather ceiling of HBM: blocks * threads threads each read `iters` pseudo-random 64-byte-aligned slots (16, 32 or
  * 64 bytes of each; bytes = -64: four adjacent lanes fetch one 64-byte slot with one instruction, blocks * threads / 4 *
  * iters gathers; bytes = -32: two adjacent lanes fetch one 32-byte slot, blocks * threads / 2 * iters gathers) of a table of
