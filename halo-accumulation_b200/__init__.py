@@ -10,7 +10,7 @@ import os
 import numpy as np
 
 from . import _build
-from ._capi import HaloError, arr, load, p64, u8p
+from ._capi import HaloError, arr, load, p64, pack, u8p
 
 __all__ = ["Context", "Comm", "MultiGpu", "HaloError", "build", "points_sum", "points_equal", "comm_slice"]
 
@@ -219,6 +219,13 @@ class Context:
         out = np.zeros(12, dtype=np.uint64)
         self._chk(self._lib.halo_msm_gens(self._h, p64(s), C.c_uint64(off), C.c_uint64(s.shape[0]), p64(out)))
         return out
+
+    def msm_gens_many(self, scalar_vectors):
+        """halo_msm_gens_many: row j of the (k, 12) result is sum_i scalar_vectors[j][i] * G_i (one segmented MSM per group)."""
+        packed, lens = pack(scalar_vectors)
+        out = np.zeros((max(1, len(lens)), 12), dtype=np.uint64)
+        self._chk(self._lib.halo_msm_gens_many(self._h, p64(packed), p64(lens), C.c_uint64(len(lens)), p64(out)))
+        return out[:len(lens)]
 
     def msm_gens_submit(self, scalars, off=0):
         """Pipelined halo_msm_gens: returns a ticket; `scalars` must stay alive (ideally pinned) until collect."""

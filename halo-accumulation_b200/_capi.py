@@ -65,6 +65,7 @@ def load():
     lib.halo_h_msm_batch.argtypes = [C.c_void_p, u64p, C.POINTER(C.c_uint32), u64p, C.c_uint64, u64p, u8p, u64p, C.c_uint64, u64p]
     lib.halo_h_msm_batch_submit.argtypes = [C.c_void_p, u64p, C.POINTER(C.c_uint32), u64p, C.c_uint64, C.POINTER(C.c_int)]
     lib.halo_h_msm_batch_collect.argtypes = [C.c_void_p, C.c_int, u64p, u8p, u64p, C.c_uint64, u64p]
+    lib.halo_msm_gens_many.argtypes = [C.c_void_p, u64p, u64p, C.c_uint64, u64p]
     lib.halo_test_point_combine.argtypes = [C.c_void_p, C.c_int, u64p, u64p, u64p, u64p, C.c_uint64, u64p]
     if lib.halo_curve_name().decode() != _build.CURVE:
         raise RuntimeError(f"{path} was built for {lib.halo_curve_name().decode()}, HALO_B200_CURVE asks for {_build.CURVE}")
@@ -75,6 +76,19 @@ def load():
 def p64(a):
     assert a.dtype == np.uint64 and a.flags["C_CONTIGUOUS"], (a.dtype, a.flags)
     return a.ctypes.data_as(u64p)
+
+
+def pack(vectors):
+    """Scalar vectors -> (packed [sum len][4] array, lengths [k]) for the batch entry points.  A (k, n, 4) array is used in
+    place; a list is copied into one buffer."""
+    if isinstance(vectors, np.ndarray) and vectors.ndim == 3:
+        k, n = vectors.shape[:2]
+        packed = arr(vectors).reshape(-1, 4) if k * n else np.zeros((1, 4), dtype=np.uint64)
+        return packed, np.full(k, n, dtype=np.uint64)
+    vs = [arr(v).reshape(-1, 4) for v in vectors]
+    lens = np.array([v.shape[0] for v in vs], dtype=np.uint64)
+    packed = np.concatenate(vs) if vs and int(lens.sum()) else np.zeros((1, 4), dtype=np.uint64)
+    return np.ascontiguousarray(packed), lens
 
 
 def arr(x, shape=None):

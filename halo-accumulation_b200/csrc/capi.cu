@@ -1,4 +1,5 @@
 // capi.cu -- extern "C" entry points of libhalo_b200.so (include/halo_b200.h).
+#include <algorithm>
 #include <cstdio>
 #include <cstring>
 #include <system_error>
@@ -230,6 +231,13 @@ void halo_ctx_destroy(halo_ctx* ctx) {
     for (DevBuf* b : {&ctx->hb.scalars, &ctx->hb.companion, &ctx->hb.parts}) b->release();
     if (ctx->hb.done) cudaEventDestroy(ctx->hb.done);
     if (ctx->hb.h_parts) cudaFreeHost(ctx->hb.h_parts);
+    for (auto& b : ctx->many) {
+        for (DevBuf* d : {&b.scalars, &b.seg_off, &b.parts}) d->release();
+        if (b.h_seg_off) cudaFreeHost(b.h_seg_off);
+        if (b.h_parts) cudaFreeHost(b.h_parts);
+        if (b.copied) cudaEventDestroy(b.copied);
+        if (b.done) cudaEventDestroy(b.done);
+    }
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
     if (ctx->sort_stream) cudaStreamDestroy(ctx->sort_stream);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -648,6 +656,221 @@ int halo_msm_gens(halo_ctx* ctx, const uint64_t* scalars, uint64_t off, uint64_t
     HALO_CATCH(ctx)
 }
 
+// ---- halo_msm_gens_many (DESIGN.md K2c): k MSMs over the resident generators as segmented MSMs ----
+namespace {
+constexpr uint64_t MANY_MAX_SCALARS = (uint64_t)1 << 24;  // per group: the scalars, entries and buckets of the library's 2^24-point MSM
+constexpr uint64_t MANY_MAX_ENTRIES = (uint64_t)1 << 28;
+constexpr uint64_t MANY_MAX_BUCKETS = (uint64_t)1 << 23;  // the scan's limit, (NB + 4095) / 4096 <= 2048
+constexpr uint64_t MANY_SORT2_BUCKETS = (uint64_t)1 << 21;  // the two-level sort's 2048 coarse bins of 1024 buckets
+constexpr uint32_t MANY_MAX_SEGS = 256;  // bounds the window partials of a group (3 W segs points, pinned on the host)
+
+// One segmented MSM: the non-empty outputs jobs[j0 .. j1) (their scalars are adjacent in the packed buffer, from s0 on).
+struct ManyGroup {
+    size_t j0, j1;
+    uint64_t s0, ns, max_len;
+    MsmPlan plan;
+};
+
+// Plan of one output of the batch by its length: FIXED base under the conditions of a single MSM, else the variable-base
+// window of a single MSM of that length; groups of short segments then narrow it (many_groups).
+MsmPlan many_seg_plan(halo_ctx* ctx, uint64_t len) { return gens_use_fixed(ctx, len) ? ctx->pre_plan : msm_make_plan(len, ctx->force_c); }
+
+// Outputs in caller order, cut into groups of one plan within the limits above; a group of one output is an ordinary MSM.
+std::vector<ManyGroup> many_groups(halo_ctx* ctx, const std::vector<uint64_t>& jobs, const uint64_t* lens, const uint64_t* starts) {
+    std::vector<ManyGroup> gs;
+    for (size_t j = 0; j < jobs.size(); j++) {
+        const uint64_t len = lens[jobs[j]];
+        const MsmPlan p = many_seg_plan(ctx, len);
+        if (!gs.empty()) {
+            ManyGroup& g = gs.back();
+            const uint64_t segs = g.j1 - g.j0 + 1, ns = g.ns + len, nb = segs * g.plan.NB, entries = ns * (uint64_t)p.W;
+            const bool fits = p.c == g.plan.c && p.fixed == g.plan.fixed && segs <= MANY_MAX_SEGS && ns <= MANY_MAX_SCALARS &&
+                              entries <= MANY_MAX_ENTRIES && nb <= MANY_MAX_BUCKETS &&
+                              (entries < ((uint64_t)1 << ctx->tune_sort2_min_lg) || nb <= MANY_SORT2_BUCKETS);
+            if (fits) {
+                g.j1++;
+                g.ns = ns;
+                g.max_len = std::max(g.max_len, len);
+                continue;
+            }
+        }
+        gs.push_back(ManyGroup{j, j + 1, starts[jobs[j]], len, len, p});
+    }
+    for (ManyGroup& g : gs) {
+        const uint32_t segs = (uint32_t)(g.j1 - g.j0);
+        if (segs == 1) continue;
+        // Window sweep of the segmented MSM (profiles/r06_commit_batch.jsonl, B200): 2^12-point segments, window 7 .. 13, best
+        // at 8 -- 8 segments 0.77 ms (c = 11, the single-MSM window: 1.07), 64 segments 2.98 ms (4.56).  A batch fills the
+        // machine, so the narrow window's smaller bucket reduction wins over the latency-bound single MSM's choice.  At 2^16 (8 /
+        // 64 segments) the single-MSM window is within 3 % of the best: kept.  (2^13 .. 2^15: not measured.)
+        if (!g.plan.fixed && !ctx->force_c && segs >= 8 && g.max_len <= 4096 && g.plan.c > 8) g.plan = msm_make_plan(g.max_len, 8);
+        plan_set_segments(g.plan, segs);
+    }
+    return gs;
+}
+
+// f(0) .. f(k - 1) on up to 16 host threads (the host finish of a group's segments)
+void many_parallel(size_t k, const std::function<void(size_t)>& f) {
+    const size_t hw = std::thread::hardware_concurrency();
+    const size_t T = std::min(k, std::max<size_t>(1, std::min<size_t>(hw, 16)));
+    std::vector<std::thread> th;
+    std::vector<size_t> unspawned;
+    auto work = [&](size_t t) {
+        for (size_t j = t; j < k; j += T) f(j);
+    };
+    for (size_t t = 1; t < T; t++) {
+        try {
+            th.emplace_back(work, t);
+        } catch (const std::system_error&) {
+            unspawned.push_back(t);  // no thread available: this thread takes that share as well
+        }
+    }
+    work(0);
+    for (size_t t : unspawned) work(t);
+    for (auto& x : th) x.join();
+}
+}  // namespace
+
+int halo_msm_gens_many(halo_ctx* ctx, const uint64_t* scalars, const uint64_t* lens, uint64_t k, uint64_t* out_jac) {
+    if (!ctx) return HALO_EINVAL;
+    if (k == 0) return HALO_OK;
+    if (!scalars || !lens || !out_jac) return HALO_EINVAL;
+    std::vector<uint64_t> starts, jobs;  // packed position of every output; the outputs with scalars
+    try {
+        starts.resize(k);
+        uint64_t total = 0;
+        for (uint64_t j = 0; j < k; j++) {
+            if (lens[j] > ctx->n_gens) return fail(ctx, HALO_ESTATE, "halo_msm_gens_many: length exceeds resident generators");
+            starts[j] = total;
+            total += lens[j];
+            if (total < lens[j] || total > UINT64_MAX / sizeof(fr_t)) return fail(ctx, HALO_EINVAL, "halo_msm_gens_many: packed size overflows");
+            if (lens[j]) jobs.push_back(j);
+        }
+    } catch (const std::bad_alloc&) {
+        return fail(ctx, HALO_ENOMEM, "out of host memory");
+    }
+    HALO_TRY(ctx)
+    for (uint64_t j = 0; j < k; j++)
+        if (!lens[j]) {
+            xyzz_t inf;
+            xyzz_set_inf(inf);
+            out_jac_from_xyzz(inf, out_jac + 12 * j);
+        }
+    std::vector<ManyGroup> groups = many_groups(ctx, jobs, lens, starts.data());
+    const size_t G = groups.size();
+    auto multi = [&](size_t g) { return groups[g].j1 - groups[g].j0 > 1; };
+    auto n_parts = [](const MsmPlan& p) { return (size_t)3 * (p.fixed ? 1 : p.W) * p.segs; };
+    // both buffers at the size of the largest group, before anything is in flight
+    uint64_t max_ns = 0;
+    size_t max_parts = 0;
+    for (size_t g = 0; g < G; g++)
+        if (multi(g)) {
+            max_ns = std::max(max_ns, groups[g].ns);
+            max_parts = std::max(max_parts, n_parts(groups[g].plan));
+        }
+    if (max_ns) {
+        async_init(ctx);
+        for (auto& b : ctx->many) {
+            if (!b.copied) {
+                HALO_CUDA(cudaEventCreateWithFlags(&b.copied, cudaEventDisableTiming));
+                HALO_CUDA(cudaEventCreateWithFlags(&b.done, cudaEventDisableTiming));
+                HALO_CUDA(cudaMallocHost(reinterpret_cast<void**>(&b.h_seg_off), (size_t)(MANY_MAX_SEGS + 1) * 4));
+            }
+            b.scalars.reserve(max_ns * sizeof(fr_t));
+            b.seg_off.reserve((size_t)(MANY_MAX_SEGS + 1) * 4);
+            b.parts.reserve(max_parts * sizeof(xyzz_t));
+            if (b.h_parts_cap < max_parts) {
+                if (b.h_parts) HALO_CUDA(cudaFreeHost(b.h_parts));
+                b.h_parts = nullptr;
+                b.h_parts_cap = 0;
+                HALO_CUDA(cudaMallocHost(reinterpret_cast<void**>(&b.h_parts), max_parts * sizeof(xyzz_t)));
+                b.h_parts_cap = max_parts;
+            }
+        }
+    }
+    // Whatever happens below, nothing may still read the caller's scalars or write its outputs once this call returns.
+    struct Drain {
+        halo_ctx* c;
+        ~Drain() {
+            if (!c) return;
+            cudaStreamSynchronize(c->copy_stream);
+            cudaStreamSynchronize(c->stream);
+        }
+    } drain{max_ns ? ctx : nullptr};
+    // group g's scalars and segment starts into buffer g & 1 on the copy stream, once the group two back has released it
+    auto issue_copy = [&](size_t g) {
+        const ManyGroup& gr = groups[g];
+        halo_ctx::ManyBuf& b = ctx->many[g & 1];
+        const uint32_t segs = (uint32_t)(gr.j1 - gr.j0);
+        HALO_CUDA(cudaEventSynchronize(b.copied));  // the pinned segment starts of that group have left
+        HALO_CUDA(cudaStreamWaitEvent(ctx->copy_stream, b.done, 0));
+        for (uint32_t s = 0; s <= segs; s++) b.h_seg_off[s] = (uint32_t)((s < segs ? starts[jobs[gr.j0 + s]] : gr.s0 + gr.ns) - gr.s0);
+        HALO_CUDA(cudaMemcpyAsync(b.seg_off.p, b.h_seg_off, (size_t)(segs + 1) * 4, cudaMemcpyHostToDevice, ctx->copy_stream));
+        h2d_copy(ctx, b.scalars.p, scalars + 4 * gr.s0, gr.ns * sizeof(fr_t), ctx->copy_stream);
+        HALO_CUDA(cudaEventRecord(b.copied, ctx->copy_stream));
+    };
+    // group g's segmented MSM on the context stream, its window partials to the pinned host buffer
+    auto launch = [&](size_t g) {
+        ManyGroup& gr = groups[g];
+        halo_ctx::ManyBuf& b = ctx->many[g & 1];
+        MsmPlan& plan = gr.plan;  // msm_enqueue settles the reduction geometry in it
+        const size_t nparts = n_parts(plan);
+        MsmInput in;
+        in.scalars = b.scalars.as<fr_t>();
+        in.n = (uint32_t)gr.ns;
+        in.segs = plan.segs;
+        in.seg_off = b.seg_off.as<uint32_t>();
+        if (plan.fixed) {
+            in.bases = ctx->gens_pre.as<affine_t>();
+            in.fixed_stride = (uint32_t)ctx->pre_n;
+        } else {
+            in.bases = ctx->gens.as<affine_t>();
+        }
+        HALO_CUDA(cudaStreamWaitEvent(ctx->stream, b.copied, 0));
+        msm_enqueue(ctx, in, plan, b.parts.as<xyzz_t>(), 0);
+        HALO_CUDA(cudaMemcpyAsync(b.h_parts, b.parts.p, nparts * sizeof(xyzz_t), cudaMemcpyDeviceToHost, ctx->stream));
+        HALO_CUDA(cudaEventRecord(b.done, ctx->stream));
+    };
+    // host finish of group g, one segment per task (a variable-base finish is ~255 doublings)
+    auto finish = [&](size_t g) {
+        const ManyGroup& gr = groups[g];
+        halo_ctx::ManyBuf& b = ctx->many[g & 1];
+        HALO_CUDA(cudaEventSynchronize(b.done));
+        const size_t per = (size_t)3 * (gr.plan.fixed ? 1 : gr.plan.W);
+        auto one = [&](size_t s) {
+            xyzz_t r;
+            msm_finish_host(b.h_parts + per * s, gr.plan, r);
+            out_jac_from_xyzz(r, out_jac + 12 * jobs[gr.j0 + s]);
+        };
+        if (gr.plan.fixed)
+            for (size_t s = 0; s < gr.plan.segs; s++) one(s);
+        else
+            many_parallel(gr.plan.segs, one);
+    };
+    // Pipeline: the copy of group g+1 and the host finish of group g-1 run while group g is on the device.  A group of one
+    // output drains the pipeline and takes the halo_msm_gens route.
+    if (G && multi(0)) issue_copy(0);
+    size_t pend = SIZE_MAX;  // group whose partials are outstanding
+    for (size_t g = 0; g < G; g++) {
+        if (!multi(g)) {
+            if (pend != SIZE_MAX) finish(pend);
+            pend = SIZE_MAX;
+            const uint64_t j = jobs[groups[g].j0];
+            const int rc = halo_msm_gens(ctx, scalars + 4 * starts[j], 0, lens[j], out_jac + 12 * j);
+            if (rc) return rc;
+        } else {
+            launch(g);
+        }
+        if (g + 1 < G && multi(g + 1)) issue_copy(g + 1);
+        if (multi(g)) {
+            if (pend != SIZE_MAX) finish(pend);
+            pend = g;
+        }
+    }
+    if (pend != SIZE_MAX) finish(pend);
+    HALO_CATCH(ctx)
+}
+
 // Shared body of the two submit entry points: host scalars are copied on the copy stream first; device-resident
 // scalars (resident = true) are used in place and must stay untouched until the ticket is collected.
 static int submit_impl(halo_ctx* ctx, const uint64_t* scalars, bool resident, uint64_t off, uint64_t n, int* ticket) {
@@ -676,8 +899,7 @@ static int submit_impl(halo_ctx* ctx, const uint64_t* scalars, bool resident, ui
             in.scalars = s.scalars.as<fr_t>();
         }
         in.n = (uint32_t)n;
-        const bool fixed = ctx->use_fixed && ctx->pre_n == ctx->n_gens && ctx->gens_pre.p && n >= (1u << 17) && n * 8 >= ctx->pre_n;
-        if (fixed) {
+        if (gens_use_fixed(ctx, n)) {
             in.bases = ctx->gens_pre.as<affine_t>();
             in.fixed_stride = (uint32_t)ctx->pre_n;
             in.fixed_first = (uint32_t)off;

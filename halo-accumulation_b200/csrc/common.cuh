@@ -100,7 +100,8 @@ struct MsmPlan {
     int c = 0;
     int W = 0;
     uint32_t M = 0;
-    uint32_t NB = 0;  // W * M (variable base) or M (fixed base: one shared bucket set)
+    uint32_t NB = 0;  // segs * (W * M (variable base) or M (fixed base: one shared bucket set))
+    uint32_t segs = 1;  // segmented MSM (halo_msm_gens_many): one bucket set per segment, segment s owns buckets [s NB / segs, ..)
     bool fixed = false;
     MsmWidths widths;
     // bucket reduction geometry: slabs of red_T << red_log_s buckets
@@ -110,6 +111,8 @@ struct MsmPlan {
 };
 void plan_set_reduce(MsmPlan& p, bool quad);
 MsmPlan msm_make_plan(uint64_t n, int force_c);
+// p (a one-segment plan) turned into the plan of `segs` segments of the same window
+void plan_set_segments(MsmPlan& p, uint32_t segs);
 
 struct MsmWorkspace {
     DevBuf counts, offsets, cursor, entries, buckets, wsums, scan_tmp;
@@ -198,6 +201,15 @@ struct halo_ctx {
         bool active = false;
         bool empty = false;  // no claims: the generator part is infinity
     } hb;
+    // halo_msm_gens_many: two group buffers, so that the copy of group g+1 and the host finish of group g-1 overlap the
+    // kernels of group g
+    struct ManyBuf {
+        halo::DevBuf scalars, seg_off, parts;
+        uint32_t* h_seg_off = nullptr;  // pinned
+        halo::xyzz_t* h_parts = nullptr;  // pinned
+        size_t h_parts_cap = 0;  // points; h_seg_off holds MANY_MAX_SEGS + 1 starts
+        cudaEvent_t copied = nullptr, done = nullptr;
+    } many[2];
     // staging ring for host-to-device copies out of PAGEABLE caller memory (h2d_copy, capi.cu)
     static constexpr int STAGE_THREADS = 8, STAGE_SLOTS = 2;  // upper bound of threads; tune_stage_threads of them work
     static constexpr size_t STAGE_CHUNK = 8u << 20;

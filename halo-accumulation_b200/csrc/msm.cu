@@ -54,7 +54,7 @@ void plan_set_reduce(MsmPlan& p, bool quad) {
     // partials, hence at most 128 slabs per window and none for small windows.  The quad-cooperative kernel has the
     // shorter dependent chain but issues ~40 % more instructions per addition: it wins while the reduction is latency
     // bound (<= 3 * 2^17 buckets in all), the one-lane kernel wins beyond (2^22 variable base: 0.69 against 0.83 ms).
-    const uint32_t nwin = p.fixed ? 1u : (uint32_t)p.W;
+    const uint32_t nwin = (p.fixed ? 1u : (uint32_t)p.W) * p.segs;  // every window of every segment
     quad = quad && (uint64_t)nwin * p.M <= (p.fixed ? 524288u : 393216u);  // (one bucket set of 2^19: 0.80 -> 0.67 ms)
     p.red_quad = quad;
     if (!quad) {
@@ -77,6 +77,12 @@ void plan_set_reduce(MsmPlan& p, bool quad) {
     p.red_log_s = 0;
     while ((T << p.red_log_s) < B) p.red_log_s++;
     p.red_slabs = p.M / (T << p.red_log_s);
+}
+
+void plan_set_segments(MsmPlan& p, uint32_t segs) {
+    p.NB = p.NB / p.segs * segs;
+    p.segs = segs;
+    plan_set_reduce(p, true);
 }
 
 static int ceil_lg(uint64_t n) {
@@ -119,15 +125,33 @@ MsmPlan msm_make_fixed_plan(uint64_t n, int force_c) {
 // ------------------------------------------------------------------------------------------------
 // VARIABLE: bucket = w * M + |d| - 1, entry = i.   FIXED: bucket = |d| - 1, entry = w * stride + first + i (the index of
 // the precomputed multiple 2^(off_w) G_{first+i}).
-template <bool SCATTER>
-__global__ void __launch_bounds__(256) k_digits(const fr_t* __restrict__ scalars, uint32_t n,
+// SEG (segmented MSM): scalar i of segment s (seg_off[s] <= i < seg_off[s + 1]) goes to bucket s * NB1 + (the bucket above)
+// with i - seg_off[s] in place of i; the entry does not record the segment, so every later stage reads bases unchanged.
+__device__ __forceinline__ uint32_t seg_of(const uint32_t* __restrict__ seg_off, uint32_t segs, uint32_t i) {
+    uint32_t a = 0, b = segs;  // the last segment starting at or before i
+    while (b - a > 1) {
+        const uint32_t m = (a + b) >> 1;
+        if (seg_off[m] <= i) a = m; else b = m;
+    }
+    return a;
+}
+// (the segmented scatter needs ~47 registers: at the 32 that full occupancy leaves it spilled; minBlocks 0 = no bound)
+template <bool SCATTER, bool SEG>
+__global__ void __launch_bounds__(256, SEG ? 4 : 0) k_digits(const fr_t* __restrict__ scalars, uint32_t n,
                                                 const fr_t* __restrict__ tail_scalars, uint32_t n_tail, const MsmWidths widths,
                                                 int W, uint32_t M, uint32_t fixed_stride, uint32_t fixed_first,
-                                                uint32_t* __restrict__ counts, uint32_t* __restrict__ entries) {
+                                                uint32_t* __restrict__ counts, uint32_t* __restrict__ entries,
+                                                const uint32_t* __restrict__ seg_off, uint32_t segs, uint32_t NB1) {
     // grid-stride: the launch normally covers every scalar with one thread; the pipelined path (SortAhead) runs the sort
     // of the NEXT MSM with a few CTAs per SM beside the accumulation kernels of the current one
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n + n_tail; i += gridDim.x * blockDim.x) {
     fr_t s = i < n ? scalars[i] : tail_scalars[i - n];
+    uint32_t li = i, bofs = 0;  // index of the base, first bucket of the segment
+    if (SEG) {
+        const uint32_t sg = seg_of(seg_off, segs, i);
+        li = i - seg_off[sg];
+        bofs = sg * NB1;
+    }
     uint32_t k[8];
     fp_to_canon(k, s);  // arkworks `into_bigint`
     uint32_t carry = 0;
@@ -145,13 +169,13 @@ __global__ void __launch_bounds__(256) k_digits(const fr_t* __restrict__ scalars
             carry = 1;
         }
         if (d != 0) {
-            uint32_t b = fixed_stride ? (d - 1) : (uint32_t)w * M + (d - 1);
+            uint32_t b = bofs + (fixed_stride ? (d - 1) : (uint32_t)w * M + (d - 1));
             // COUNT: histogram (a fire-and-forget RED).  SCATTER: `counts` holds the running write cursor of every bucket,
             // initialised to the bucket offsets, so the returned value is the absolute slot (one random L2 access less per
             // entry than offsets[b] + slot).
             uint32_t pos = atomicAdd(&counts[b], 1u);
             if (SCATTER) {
-                uint32_t idx = fixed_stride ? (uint32_t)w * fixed_stride + fixed_first + i : i;
+                uint32_t idx = fixed_stride ? (uint32_t)w * fixed_stride + fixed_first + li : li;
                 entries[pos] = idx | (neg << 31);
             }
         }
@@ -301,11 +325,11 @@ constexpr uint32_t S2_TILE = S2_THREADS * S2_SPT;        // scalars per tile: CT
 constexpr int S2_BIN_SHIFT = 42;                         // staged record: entry (32) | fine bucket (10) | coarse bin (12)
 constexpr uint64_t S2_REC_MASK = ((uint64_t)1 << S2_BIN_SHIFT) - 1;
 
-// Calls f(bucket, entry) for every non-zero digit of scalar i (the digit rule of k_digits).  Bits are picked straight out of
-// the canonical limbs (no 256-bit shift per window).
+// Calls f(bucket, entry) for every non-zero digit of scalar i (the digit rule of k_digits; bofs: first bucket of the scalar's
+// segment, i: its index in the segment).  Bits are picked straight out of the canonical limbs (no 256-bit shift per window).
 template <class F>
-__device__ __forceinline__ void s2_for_digits(const fr_t& s, uint32_t i, const MsmWidths& widths, int W, uint32_t M, uint32_t fixed_stride,
-                                              uint32_t fixed_first, F&& f) {
+__device__ __forceinline__ void s2_for_digits(const fr_t& s, uint32_t i, uint32_t bofs, const MsmWidths& widths, int W, uint32_t M,
+                                              uint32_t fixed_stride, uint32_t fixed_first, F&& f) {
     uint32_t k[9];
     fp_to_canon(k, s);
     k[8] = 0;
@@ -324,17 +348,32 @@ __device__ __forceinline__ void s2_for_digits(const fr_t& s, uint32_t i, const M
             carry = 1;
         }
         if (d != 0) {
-            const uint32_t b = fixed_stride ? (d - 1) : (uint32_t)w * M + (d - 1);
+            const uint32_t b = bofs + (fixed_stride ? (d - 1) : (uint32_t)w * M + (d - 1));
             const uint32_t idx = fixed_stride ? (uint32_t)w * fixed_stride + fixed_first + i : i;
             f(b, idx | (neg << 31));
         }
     }
 }
 
+// s2_for_digits on packed scalar i of a (SEG: segmented) MSM
+template <bool SEG, class F>
+__device__ __forceinline__ void s2_for_digits_at(const fr_t& s, uint32_t i, const uint32_t* __restrict__ seg_off, uint32_t segs, uint32_t NB1,
+                                                 const MsmWidths& widths, int W, uint32_t M, uint32_t fixed_stride, uint32_t fixed_first, F&& f) {
+    uint32_t li = i, bofs = 0;
+    if (SEG) {
+        const uint32_t sg = seg_of(seg_off, segs, i);
+        li = i - seg_off[sg];
+        bofs = sg * NB1;
+    }
+    s2_for_digits(s, li, bofs, widths, W, M, fixed_stride, fixed_first, f);
+}
+
+template <bool SEG>
 __global__ void __launch_bounds__(S2_THREADS) k_sort_coarse_count(const fr_t* __restrict__ scalars, uint32_t n,
                                                                   const fr_t* __restrict__ tail_scalars, uint32_t n_tail,
                                                                   const MsmWidths widths, int W, uint32_t M, uint32_t fixed_stride,
-                                                                  uint32_t fixed_first, uint32_t NC, uint32_t* __restrict__ cta_hist) {
+                                                                  uint32_t fixed_first, uint32_t NC, uint32_t* __restrict__ cta_hist,
+                                                                  const uint32_t* __restrict__ seg_off, uint32_t segs, uint32_t NB1) {
     __shared__ uint32_t hist[S2_MAX_NC];
     for (uint32_t t = threadIdx.x; t < NC; t += blockDim.x) hist[t] = 0;
     __syncthreads();
@@ -345,7 +384,8 @@ __global__ void __launch_bounds__(S2_THREADS) k_sort_coarse_count(const fr_t* __
             const uint32_t i = tile * S2_TILE + (uint32_t)r * S2_THREADS + threadIdx.x;
             if (i < ntot) {
                 const fr_t s = i < n ? scalars[i] : tail_scalars[i - n];
-                s2_for_digits(s, i, widths, W, M, fixed_stride, fixed_first, [&](uint32_t b, uint32_t) { atomicAdd(&hist[b >> S2_NF_LOG], 1u); });
+                s2_for_digits_at<SEG>(s, i, seg_off, segs, NB1, widths, W, M, fixed_stride, fixed_first,
+                                      [&](uint32_t b, uint32_t) { atomicAdd(&hist[b >> S2_NF_LOG], 1u); });
             }
         }
     __syncthreads();
@@ -424,11 +464,13 @@ __device__ __forceinline__ void s2_block_scan(const uint32_t* __restrict__ v, ui
 // 208 bytes per bin and tile at 2^24): what limits a scatter on this part is the number of store transactions, ~45 G/s,
 // whatever their size, so a record must not be its own transaction.  Dynamic shared memory: gcur[NC] | hist[NC] | toff[NC + 1]
 // | stage[S2_TILE * W] (8 bytes each).
+template <bool SEG>
 __global__ void __launch_bounds__(S2_THREADS) k_sort_coarse_scatter(const fr_t* __restrict__ scalars, uint32_t n,
                                                                     const fr_t* __restrict__ tail_scalars, uint32_t n_tail,
                                                                     const MsmWidths widths, int W, uint32_t M, uint32_t fixed_stride,
                                                                     uint32_t fixed_first, uint32_t NC, const uint32_t* __restrict__ cta_base,
-                                                                    uint64_t* __restrict__ tmp) {
+                                                                    uint64_t* __restrict__ tmp, const uint32_t* __restrict__ seg_off,
+                                                                    uint32_t segs, uint32_t NB1) {
     extern __shared__ __align__(16) unsigned char s2_smem[];
     uint32_t* gcur = reinterpret_cast<uint32_t*>(s2_smem);
     uint32_t* hist = gcur + NC;
@@ -444,7 +486,8 @@ __global__ void __launch_bounds__(S2_THREADS) k_sort_coarse_scatter(const fr_t* 
             const uint32_t i = tile * S2_TILE + (uint32_t)r * S2_THREADS + threadIdx.x;
             if (i < ntot) {
                 const fr_t s = i < n ? scalars[i] : tail_scalars[i - n];
-                s2_for_digits(s, i, widths, W, M, fixed_stride, fixed_first, [&](uint32_t b, uint32_t) { atomicAdd(&hist[b >> S2_NF_LOG], 1u); });
+                s2_for_digits_at<SEG>(s, i, seg_off, segs, NB1, widths, W, M, fixed_stride, fixed_first,
+                                      [&](uint32_t b, uint32_t) { atomicAdd(&hist[b >> S2_NF_LOG], 1u); });
             }
         }
         __syncthreads();
@@ -457,7 +500,7 @@ __global__ void __launch_bounds__(S2_THREADS) k_sort_coarse_scatter(const fr_t* 
             const uint32_t i = tile * S2_TILE + (uint32_t)r * S2_THREADS + threadIdx.x;
             if (i < ntot) {
                 const fr_t s = i < n ? scalars[i] : tail_scalars[i - n];
-                s2_for_digits(s, i, widths, W, M, fixed_stride, fixed_first, [&](uint32_t b, uint32_t ent) {
+                s2_for_digits_at<SEG>(s, i, seg_off, segs, NB1, widths, W, M, fixed_stride, fixed_first, [&](uint32_t b, uint32_t ent) {
                     const uint32_t bin = b >> S2_NF_LOG;
                     const uint32_t pos = toff[bin] + atomicAdd(&hist[bin], 1u);
                     stage[pos] = ((uint64_t)bin << S2_BIN_SHIFT) | ((uint64_t)(b & (S2_NF - 1u)) << 32) | ent;
@@ -1252,7 +1295,12 @@ void msm_enqueue(halo_ctx* ctx, const MsmInput& in, MsmPlan& plan, xyzz_t* d_out
     MsmWorkspace& sws = ahead ? *ahead->ws : ws;
     cudaStream_t sst = ahead ? ahead->stream : st;
     const uint32_t NB = plan.NB;
-    const int nwin = plan.fixed ? 1 : plan.W;
+    // a segmented MSM is one MSM over segs bucket sets: from the sort on, windows of all segments are handled alike
+    const bool seg = in.segs > 1;
+    if (in.segs != plan.segs || (seg && (in.n_tail || !in.seg_off)))
+        throw CudaError{cudaErrorInvalidValue, "segmented MSM: plan / input mismatch", __FILE__, __LINE__};
+    const uint32_t NB1 = NB / plan.segs;
+    const int nwin = (plan.fixed ? 1 : plan.W) * (int)plan.segs;
     const uint64_t total_entries_max = (uint64_t)ntot * plan.W;
     // pair-tree passes (msm_pairs.cu): worthwhile once the per-pass fixed costs (7 launches and one ~0.1 ms inversion
     // latency) are small against the additions saved; bucket segments are then padded to multiples of 2^P slots
@@ -1323,18 +1371,27 @@ void msm_enqueue(halo_ctx* ctx, const MsmInput& in, MsmPlan& plan, xyzz_t* d_out
         uint32_t* chunk_pre = coarse_off + (S2_MAX_NC + 1);
         uint64_t* tmp = sws.sort_tmp.as<uint64_t>();
         uint32_t* fine = sws.sort_fine.as<uint32_t>();
-        k_sort_coarse_count<<<g1, S2_THREADS, 0, sst>>>(in.scalars, n, in.tail_scalars, in.n_tail, plan.widths, plan.W, plan.M, fstride,
-                                                         in.fixed_first, NC, cta_hist);
+        if (seg)
+            k_sort_coarse_count<true><<<g1, S2_THREADS, 0, sst>>>(in.scalars, n, in.tail_scalars, in.n_tail, plan.widths, plan.W, plan.M, fstride,
+                                                                   in.fixed_first, NC, cta_hist, in.seg_off, in.segs, NB1);
+        else
+            k_sort_coarse_count<false><<<g1, S2_THREADS, 0, sst>>>(in.scalars, n, in.tail_scalars, in.n_tail, plan.widths, plan.W, plan.M, fstride,
+                                                                    in.fixed_first, NC, cta_hist, nullptr, 1, NB1);
         k_sort_coarse_scan<<<1, 1024, 0, sst>>>(cta_hist, g1, NC, coarse_off, chunk_pre);
         const size_t smem_b = (((size_t)(3 * NC + 1) * 4 + 15) & ~(size_t)15) + (size_t)S2_TILE * plan.W * 8;
         const size_t smem_d = (size_t)S2_CHUNK * 8 + (size_t)(3 * S2_NF + 1) * 4;
         if (!ctx->sort2_attr) {  // per device: opt in to more than 48 KiB of dynamic shared memory
-            HALO_CUDA(cudaFuncSetAttribute(k_sort_coarse_scatter, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+            HALO_CUDA(cudaFuncSetAttribute(k_sort_coarse_scatter<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+            HALO_CUDA(cudaFuncSetAttribute(k_sort_coarse_scatter<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
             HALO_CUDA(cudaFuncSetAttribute(k_sort_fine_scatter, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
             ctx->sort2_attr = true;
         }
-        k_sort_coarse_scatter<<<g1, S2_THREADS, smem_b, sst>>>(in.scalars, n, in.tail_scalars, in.n_tail, plan.widths, plan.W, plan.M, fstride,
-                                                                in.fixed_first, NC, cta_hist, tmp);
+        if (seg)
+            k_sort_coarse_scatter<true><<<g1, S2_THREADS, smem_b, sst>>>(in.scalars, n, in.tail_scalars, in.n_tail, plan.widths, plan.W, plan.M,
+                                                                          fstride, in.fixed_first, NC, cta_hist, tmp, in.seg_off, in.segs, NB1);
+        else
+            k_sort_coarse_scatter<false><<<g1, S2_THREADS, smem_b, sst>>>(in.scalars, n, in.tail_scalars, in.n_tail, plan.widths, plan.W, plan.M,
+                                                                           fstride, in.fixed_first, NC, cta_hist, tmp, nullptr, 1, NB1);
         mark(1);
         k_sort_fine_count<<<g2, S2_THREADS, 0, sst>>>(tmp, chunk_pre, coarse_off, NC, fine);
         k_sort_fine_total<<<(NB + 255) / 256, 256, 0, sst>>>(fine, chunk_pre, NB, counts);
@@ -1349,8 +1406,12 @@ void msm_enqueue(halo_ctx* ctx, const MsmInput& in, MsmPlan& plan, xyzz_t* d_out
         k_sort_fine_scatter<<<g2, S2_THREADS, smem_d, sst>>>(tmp, chunk_pre, coarse_off, NC, fine, entries);
         ctx->kernel_launches += 7;
     } else {
-    k_digits<false><<<grid, TPB, 0, sst>>>(in.scalars, n, in.tail_scalars, in.n_tail, plan.widths, plan.W, plan.M, fstride,
-                                           in.fixed_first, counts, nullptr);
+    if (seg)
+        k_digits<false, true><<<grid, TPB, 0, sst>>>(in.scalars, n, in.tail_scalars, in.n_tail, plan.widths, plan.W, plan.M, fstride,
+                                                     in.fixed_first, counts, nullptr, in.seg_off, in.segs, NB1);
+    else
+        k_digits<false, false><<<grid, TPB, 0, sst>>>(in.scalars, n, in.tail_scalars, in.n_tail, plan.widths, plan.W, plan.M, fstride,
+                                                      in.fixed_first, counts, nullptr, nullptr, 1, NB1);
     mark(1);
     exclusive_scan(counts, offsets, NB, rmask, sws.scan_tmp.as<uint32_t>(), sst, &ctx->kernel_launches);
     if (P) {  // pad slots of every bucket segment stand for the point at infinity
@@ -1361,8 +1422,12 @@ void msm_enqueue(halo_ctx* ctx, const MsmInput& in, MsmPlan& plan, xyzz_t* d_out
     HALO_CUDA(cudaMemcpyAsync(counts, offsets, (size_t)NB * 4, cudaMemcpyDeviceToDevice, sst));
     HALO_CUDA(cudaMemsetAsync(counts + NB, 0, 4, sst));
     mark(2);
-    k_digits<true><<<grid, TPB, 0, sst>>>(in.scalars, n, in.tail_scalars, in.n_tail, plan.widths, plan.W, plan.M, fstride,
-                                          in.fixed_first, counts, entries);
+    if (seg)
+        k_digits<true, true><<<grid, TPB, 0, sst>>>(in.scalars, n, in.tail_scalars, in.n_tail, plan.widths, plan.W, plan.M, fstride,
+                                                    in.fixed_first, counts, entries, in.seg_off, in.segs, NB1);
+    else
+        k_digits<true, false><<<grid, TPB, 0, sst>>>(in.scalars, n, in.tail_scalars, in.n_tail, plan.widths, plan.W, plan.M, fstride,
+                                                     in.fixed_first, counts, entries, nullptr, 1, NB1);
     ctx->kernel_launches += 2;
     }
     if (ahead) {
@@ -1628,11 +1693,15 @@ void msm_device(halo_ctx* ctx, const affine_t* d_bases, const fr_t* d_scalars, u
 
 // sum_i scalars[i] * G_{first+i} over the resident generators; takes the FIXED-base path when tables exist and the
 // problem is large enough to amortise the (n-independent) bucket reduction of the wide window.
+bool gens_use_fixed(const halo_ctx* ctx, uint64_t n) {
+    return ctx->use_fixed && ctx->pre_n == ctx->n_gens && ctx->gens_pre.p && n >= (1u << 17) && n * 8 >= ctx->pre_n;
+}
+
 void msm_gens_device(halo_ctx* ctx, const fr_t* d_scalars, uint64_t first, uint64_t n, xyzz_t& out) {
     MsmInput in;
     in.scalars = d_scalars;
     in.n = (uint32_t)n;
-    if (ctx->use_fixed && ctx->pre_n == ctx->n_gens && ctx->gens_pre.p && n >= (1u << 17) && n * 8 >= ctx->pre_n) {
+    if (gens_use_fixed(ctx, n)) {
         in.bases = ctx->gens_pre.as<affine_t>();
         in.fixed_stride = ctx->pre_n;
         in.fixed_first = (uint32_t)first;

@@ -17,8 +17,15 @@ struct MsmInput {
     // FIXED-base mode: bases = table of precomputed multiples, table[w * fixed_stride + fixed_first + i]
     uint32_t fixed_stride = 0;
     uint32_t fixed_first = 0;
+    // Segmented MSM (segs > 1, no tail): segs independent MSMs over the same bases in one pass.  The scalar at packed position
+    // seg_off[s] <= i < seg_off[s + 1] (device array of segs + 1 entries) multiplies base i - seg_off[s]; segment s has its own
+    // bucket set and its own window partials (msm_enqueue: 3 W partials per segment, segment-major).
+    uint32_t segs = 1;
+    const uint32_t* seg_off = nullptr;
 };
 MsmPlan msm_make_fixed_plan(uint64_t n, int force_c);
+// FIXED base for an MSM of n points over the resident generators (tables present, enough points to amortise the wide window)
+bool gens_use_fixed(const halo_ctx* ctx, uint64_t n);
 // Counting sort of an MSM ahead of its accumulation: own stream (high priority), own sort buffers, throttled grid.
 struct SortAhead {
     MsmWorkspace* ws;
@@ -26,7 +33,7 @@ struct SortAhead {
     cudaEvent_t sorted;
     int ctas_per_sm;  // 0: full grid
 };
-// Device part of one MSM: 3 partial points per window into d_out (see msm.cu).
+// Device part of one MSM: 3 partial points per window (and segment) into d_out (see msm.cu).
 // (`plan` is the caller's copy: the reduction geometry in it is settled here and read back by msm_finish_host)
 void msm_enqueue(halo_ctx* ctx, const MsmInput& in, MsmPlan& plan, xyzz_t* d_out, int lane = 0, const SortAhead* ahead = nullptr);
 // First `passes` levels of the bucket sums as flat pairwise affine additions with batched inversion (msm_pairs.cu).

@@ -77,6 +77,24 @@ int halo_pcdl_commit(halo_ctx* ctx, const uint64_t* coeffs, uint64_t n_coeffs, u
     });
 }
 
+int halo_pcdl_commit_batch(halo_ctx* ctx, const uint64_t* coeffs, const uint64_t* n_coeffs, uint64_t k, uint64_t d, const uint64_t* ws,
+                           uint64_t* out_jac) {
+    return guarded([&] {
+        if (k == 0) return;
+        ensure(coeffs && n_coeffs && out_jac, HALO_EINVAL, "halo_pcdl_commit_batch: NULL pointer");
+        std::vector<PolyView> ps;
+        ps.reserve(k);
+        uint64_t off = 0;
+        for (uint64_t j = 0; j < k; j++) {
+            ensure(n_coeffs[j] <= UINT64_MAX / 32 - off, HALO_EINVAL, "halo_pcdl_commit_batch: packed size overflows");
+            ps.push_back(poly_from(coeffs + 4 * off, n_coeffs[j]));
+            off += n_coeffs[j];
+        }
+        const std::vector<PallasPoint> C = pcdl::commit_batch(ctx, ps, d, reinterpret_cast<const PallasScalar*>(ws));
+        for (uint64_t j = 0; j < k; j++) point_store(out_jac + 12 * j, C[j]);
+    });
+}
+
 int halo_pcdl_open(halo_ctx* ctx, const uint64_t* coeffs, uint64_t n_coeffs, const uint64_t C_jac[12], uint64_t d,
                    const uint64_t z[4], const uint64_t* w, const uint64_t* q, uint64_t n_q, const uint64_t* w_bar,
                    halo_eval_proof* pi) {

@@ -57,6 +57,52 @@ PallasPoint commit(halo_ctx* ctx, PolyView p, uint64_t d, const PallasScalar* w)
     return pedersen::commit(ctx, w, nullptr, n, p.data(), n_coeffs, true);
 }
 
+std::vector<PallasPoint> commit_batch(halo_ctx* ctx, const std::vector<PolyView>& ps, uint64_t d, const PallasScalar* ws) {
+    const size_t k = ps.size();
+    const uint64_t n = d + 1;
+    std::vector<uint64_t> lens(k);
+    bool packed = true;  // the uploaded prefixes already lie back to back in memory (no host copy)
+    const PallasScalar* end = nullptr;  // one past the uploaded prefix of the last non-empty polynomial
+    for (size_t j = 0; j < k; j++) {
+        ensure(is_pow2(n), HALO_EINVAL, "d+1 is not a power of 2");  // pcdl.rs:102
+        ensure(degree(ps[j]) <= d, HALO_EINVAL, "p.degree() > d");   // pcdl.rs:103
+        ensure(n <= halo_num_generators(ctx), HALO_EINVAL, "d > D");  // pcdl.rs:104
+        lens[j] = ps[j].size() < n ? ps[j].size() : n;  // coeffs.resize(n, ZERO) (pcdl.rs:106-107): the zero tail is implied
+        if (!lens[j]) continue;  // an empty polynomial uploads nothing, wherever its view points
+        if (end && ps[j].data() != end) packed = false;
+        end = ps[j].data() + lens[j];
+    }
+    if (k == 0) return {};
+    if (k == 1) return {commit(ctx, ps[0], d, ws)};  // the single call, exactly
+    size_t first = 0;  // the first polynomial with coefficients to upload anchors the packed buffer
+    while (first < k && !lens[first]) first++;
+    std::vector<PallasScalar> copy;
+    const PallasScalar* base = first < k ? ps[first].data() : nullptr;
+    if (!packed) {
+        uint64_t total = 0;
+        for (uint64_t l : lens) total += l;
+        copy.resize(total);
+        uint64_t o = 0;
+        for (size_t j = 0; j < k; j++) {
+            std::copy(ps[j].data(), ps[j].data() + lens[j], copy.begin() + o);
+            o += lens[j];
+        }
+        base = copy.data();
+    }
+    std::vector<uint64_t> out(12 * k);
+    static const PallasScalar none = scalar_zero();
+    check_rc(ctx, halo_msm_gens_many(ctx, reinterpret_cast<const uint64_t*>(base ? base : &none), lens.data(), k, out.data()));
+    std::vector<PallasPoint> C(k);
+    for (size_t j = 0; j < k; j++) C[j] = point_load(&out[12 * j]);
+    if (ws) {  // pedersen.rs:15-16: C_j + w_j S for every j in ONE combine (host threads or k_point_combine by the output count)
+        CombineList cl;
+        for (size_t j = 0; j < k; j++) cl.push(C[j], point_zero(), scalar_zero(), ws[j]);
+        const std::vector<affine_t> r = cl.run(ctx);
+        for (size_t j = 0; j < k; j++) xyzz_from_affine(C[j].p, r[j]);
+    }
+    return C;
+}
+
 static EvalProof open_impl(halo_ctx* ctx, const PolyView* p, uint64_t deg, const PallasPoint& C, uint64_t d, const PallasScalar& z,
                            const PallasScalar* w, const PolyView* q, const PallasScalar* w_bar);
 

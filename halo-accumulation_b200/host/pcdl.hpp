@@ -32,6 +32,9 @@ struct HPoly {
 
 // pcdl.rs:99-110
 PallasPoint commit(halo_ctx* ctx, PolyView p, uint64_t d, const PallasScalar* w);
+// `commit` of every polynomial (w: one blinding scalar per polynomial, or null): validated in order as commit does, then one
+// halo_msm_gens_many over all of them and w_j S added by one `combine` call (DESIGN.md K2c)
+std::vector<PallasPoint> commit_batch(halo_ctx* ctx, const std::vector<PolyView>& ps, uint64_t d, const PallasScalar* ws);
 // pcdl.rs:120-242; rng draws made explicit: q (deg p coefficients), w_bar
 EvalProof open(halo_ctx* ctx, PolyView p, const PallasPoint& C, uint64_t d, const PallasScalar& z, const PallasScalar* w,
                const PolyView* q, const PallasScalar* w_bar);

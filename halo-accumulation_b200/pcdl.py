@@ -4,7 +4,7 @@ import ctypes as C
 import numpy as np
 
 from . import _host
-from ._capi import arr, p64
+from ._capi import arr, p64, pack
 from ._host import EvalProof, Instance, Rejected  # noqa: F401
 
 
@@ -34,6 +34,20 @@ def commit(ctx, p, d, w=None):
     wk, wp = _host.opt(w)
     _host.chk(_host.lib().halo_pcdl_commit(ctx._h, p64(p), C.c_uint64(p.shape[0]), C.c_uint64(d), wp, p64(out)))
     return out
+
+
+def commit_batch(ctx, ps, d, ws=None):
+    """`commit` of every polynomial in `ps` (ws: one blinding scalar per polynomial, or None) -> (k, 12) array.  Raises on the
+    first malformed polynomial, before any device work, as a loop of `commit` calls would."""
+    if len(ps) == 1:  # the single call, exactly (as pcdl::commit_batch does for k = 1)
+        return commit(ctx, ps[0], d, None if ws is None else arr(ws).reshape(1, 4)[0])[None]
+    packed, lens = pack(ps)
+    k = len(lens)
+    wa = arr(ws).reshape(k, 4) if ws is not None else None
+    out = np.zeros((max(1, k), 12), dtype=np.uint64)
+    _host.chk(_host.lib().halo_pcdl_commit_batch(ctx._h, p64(packed), p64(lens), C.c_uint64(k), C.c_uint64(d),
+                                                 p64(wa) if wa is not None else None, p64(out)))
+    return out[:k]
 
 
 def open(ctx, p, Cm, d, z, w=None, q=None, w_bar=None):

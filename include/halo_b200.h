@@ -121,6 +121,14 @@ int halo_derive_points(halo_ctx *ctx, uint64_t start, uint64_t count, uint64_t *
 /* sum_i scalars[i] * G_{off+i}, i < n.   Replaces group.rs:24-26 `point_dot_affine` as called by
  * pedersen.rs:14 over GS[0..n] (pcdl.rs:109, :338; acc.rs:153, :195). */
 int halo_msm_gens(halo_ctx *ctx, const uint64_t *scalars /*[n][4]*/, uint64_t off, uint64_t n, uint64_t out_jac[12]);
+/* k MSMs over the resident generators: out_jac[j] = sum_{i < lens[j]} scalars_j[i] * G_i, the scalar vectors packed back to
+ * back in output order (a batch of commitments: ark-poly-commit's `commit` over a list, the columns of a circuit).  Runs as
+ * segmented MSMs -- one sort, accumulation and bucket reduction for a group of outputs -- with the copy of the next group and
+ * the host finish of the previous one beside each group's kernels (DESIGN.md K2c); a group of one output is a halo_msm_gens
+ * call.  lens[j] = 0 gives infinity; k = 0 does nothing.  HALO_EINVAL: NULL pointers with k > 0, a packed size that
+ * overflows; HALO_ESTATE: a length beyond the resident generators (nothing runs in either case). */
+int halo_msm_gens_many(halo_ctx *ctx, const uint64_t *scalars /*packed, [sum lens][4]*/, const uint64_t *lens /*[k]*/, uint64_t k,
+                       uint64_t *out_jac /*[k][12]*/);
 /* sum_i scalars[i] * bases[i] for caller-supplied affine bases; inf_flags may be NULL.
  * Replaces group.rs:24-26 for arbitrary bases and, after the caller's normalisation, group.rs:18-21. */
 int halo_msm(halo_ctx *ctx, const uint64_t *bases_affine /*[n][8]*/, const uint8_t *inf_flags /*[n] or NULL*/,

@@ -72,6 +72,12 @@ int halo_pedersen_commit(halo_ctx *ctx, const uint64_t *w /*nullable*/, const ui
 /* pcdl.rs:99-110 */
 int halo_pcdl_commit(halo_ctx *ctx, const uint64_t *coeffs, uint64_t n_coeffs, uint64_t d, const uint64_t *w /*nullable*/,
                      uint64_t out_jac[12]);
+/* halo_pcdl_commit of k polynomials of one degree bound d (the reference has no batch form): polynomial j has n_coeffs[j]
+ * coefficients, packed back to back in `coeffs`; ws holds w_j for every output (hiding) or is NULL.  The polynomials are
+ * validated in order as commit does, and the first malformed one fails the call with HALO_EINVAL before any device work and
+ * before any output is written.  One halo_msm_gens_many for all of them; the hiding terms w_j S in one combined step. */
+int halo_pcdl_commit_batch(halo_ctx *ctx, const uint64_t *coeffs /*packed*/, const uint64_t *n_coeffs /*[k]*/, uint64_t k, uint64_t d,
+                           const uint64_t *ws /*[k][4] or NULL*/, uint64_t *out_jac /*[k][12]*/);
 /* pcdl.rs:120-242; hiding iff w != NULL, then q (n_q = deg p coefficients) and w_bar are the rng draws. */
 int halo_pcdl_open(halo_ctx *ctx, const uint64_t *coeffs, uint64_t n_coeffs, const uint64_t C_jac[12], uint64_t d,
                    const uint64_t z[4], const uint64_t *w /*nullable*/, const uint64_t *q, uint64_t n_q,
