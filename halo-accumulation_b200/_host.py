@@ -75,6 +75,9 @@ def lib():
         _lib = C.CDLL(path)
         _lib.halo_host_last_error.restype = C.c_char_p
         _lib.halo_pcdl_commit_batch.argtypes = [C.c_void_p, u64p, u64p, C.c_uint64, C.c_uint64, u64p, u64p]
+        _lib.halo_pcdl_open_batch.argtypes = [C.c_void_p, u64p, u64p, C.c_uint64, u64p, C.c_uint64, u64p, u64p, u64p, C.c_uint64,
+                                              u64p, u64p, u64p, u64p, C.POINTER(EvalProof)]
+        _lib.halo_pcdl_batch_claim.argtypes = [C.c_void_p, u64p, u64p, C.c_uint64, u64p, u64p, u64p]
         _lib.halo_pcdl_check_batch.argtypes = [C.c_void_p, C.POINTER(Instance), C.c_uint64, u64p, u64p]
         _lib.halo_acc_decider_batch.argtypes = [C.c_void_p, C.POINTER(Accumulator), C.c_uint64, u64p, u64p]
         _lib.halo_acc_verifier_batch.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(Instance), u64p, C.POINTER(Accumulator),

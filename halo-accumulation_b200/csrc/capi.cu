@@ -199,6 +199,8 @@ void halo_ctx_destroy(halo_ctx* ctx) {
     ctx->stage_bases.release();
     ctx->stage_misc.release();
     ctx->poly_dev.release();
+    ctx->polys_dev.release();
+    ctx->polys_off.release();
     ctx->lincomb_claims.release();
     for (halo::DevBuf* b : {&ctx->combine_in, &ctx->combine_work, &ctx->combine_inv_scratch}) b->release();
     for (halo::DevBuf* b : {&ctx->ipa_G, &ctx->ipa_cs, &ctx->ipa_zs, &ctx->ipa_pbar, &ctx->ipa_tail, &ctx->ipa_frozen,
@@ -1284,6 +1286,22 @@ int halo_msm_multi(halo_ctx* ctx, const halo_msm_desc* descs, uint32_t count, ui
     HALO_CATCH(ctx)
 }
 
+// DensePolynomial::degree of the n device coefficients d (index of the highest non-zero one, 0 for the zero polynomial):
+// scanned down from the top in chunks (the leading coefficient is non-zero except with negligible probability)
+static uint64_t device_degree(halo_ctx* ctx, const fr_t* d, uint64_t n) {
+    uint64_t hi = n;
+    std::vector<fr_t> chunk(64);
+    while (hi > 0) {
+        uint64_t lo = hi > 64 ? hi - 64 : 0;
+        HALO_CUDA(cudaMemcpyAsync(chunk.data(), d + lo, (hi - lo) * sizeof(fr_t), cudaMemcpyDeviceToHost, ctx->stream));
+        HALO_CUDA(cudaStreamSynchronize(ctx->stream));
+        for (uint64_t i = hi; i-- > lo;)
+            if (!fp_is_zero(chunk[i - lo])) return i;
+        hi = lo;
+    }
+    return 0;
+}
+
 // out != NULL: coefficients to the host.  out == NULL: the polynomial stays on the device (ctx->poly_dev) and
 // *degree_out receives its degree (DensePolynomial::degree: index of the highest non-zero coefficient).
 static int h_lincomb_impl(halo_ctx* ctx, const uint64_t* h0, uint64_t n_h0, const uint64_t* alphas, const uint64_t* xis,
@@ -1305,24 +1323,8 @@ static int h_lincomb_impl(halo_ctx* ctx, const uint64_t* h0, uint64_t n_h0, cons
         HALO_CUDA(cudaMemcpyAsync(out, d, n * sizeof(fr_t), cudaMemcpyDeviceToHost, ctx->stream));
         HALO_CUDA(cudaStreamSynchronize(ctx->stream));
     } else {
-        // degree: scan down from the top in chunks (the leading coefficient is non-zero except with negligible probability)
         ctx->poly_n = n;
-        uint64_t hi = n, deg = 0;
-        bool found = false;
-        std::vector<fr_t> chunk(64);
-        while (hi > 0 && !found) {
-            uint64_t lo = hi > 64 ? hi - 64 : 0;
-            HALO_CUDA(cudaMemcpyAsync(chunk.data(), d + lo, (hi - lo) * sizeof(fr_t), cudaMemcpyDeviceToHost, ctx->stream));
-            HALO_CUDA(cudaStreamSynchronize(ctx->stream));
-            for (uint64_t i = hi; i-- > lo;)
-                if (!fp_is_zero(chunk[i - lo])) {
-                    deg = i;
-                    found = true;
-                    break;
-                }
-            hi = lo;
-        }
-        *degree_out = deg;
+        *degree_out = device_degree(ctx, d, n);
     }
     HALO_CATCH(ctx)
 }
@@ -1337,6 +1339,72 @@ int halo_h_lincomb_resident(halo_ctx* ctx, const uint64_t* h0, uint64_t n_h0, co
                             uint64_t m, uint32_t lg_n, uint64_t* degree_out) {
     if (!degree_out) return HALO_EINVAL;
     return h_lincomb_impl(ctx, h0, n_h0, alphas, xis, m, lg_n, nullptr, degree_out);
+}
+
+// ---- K3b: k polynomials opened at one point ------------------------------------------------------------------
+// Grows a buffer; false when the device has no memory for it (the error is cleared: the context stays usable)
+static bool reserve_or_nomem(DevBuf& b, size_t bytes) {
+    try {
+        b.reserve(bytes);
+        return true;
+    } catch (const CudaError& e) {
+        if (e.err != cudaErrorMemoryAllocation) throw;
+        cudaGetLastError();
+        return false;
+    }
+}
+
+int halo_poly_eval_many(halo_ctx* ctx, const uint64_t* coeffs, const uint64_t* n_coeffs, uint64_t k, uint64_t n, const uint64_t z[4],
+                        uint64_t* vs_out) {
+    if (!ctx || !n_coeffs || !z || !vs_out) return HALO_EINVAL;
+    if (k == 0 || (k >> 31)) return fail(ctx, HALO_EINVAL, "halo_poly_eval_many: k must be 1 .. 2^31 - 1");
+    if (n > ctx->n_gens) return fail(ctx, HALO_EINVAL, "halo_poly_eval_many: n exceeds the resident generators");
+    std::vector<uint64_t> off(k + 1, 0);
+    uint64_t n_max = 0;
+    for (uint64_t j = 0; j < k; j++) {
+        if (n_coeffs[j] > n) return fail(ctx, HALO_EINVAL, "halo_poly_eval_many: a polynomial has more than n coefficients");
+        off[j + 1] = off[j] + n_coeffs[j];  // k < 2^31 polynomials of at most n < 2^32 coefficients: no wrap
+        n_max = std::max(n_max, n_coeffs[j]);
+    }
+    const uint64_t total = off[k];
+    if (!coeffs && total) return HALO_EINVAL;
+    if (total > (UINT64_MAX >> 6)) return fail(ctx, HALO_ENOMEM, "halo_poly_eval_many: out of device memory");
+    ctx->polys_k = 0;  // the previous evaluation is gone from here on, whatever the outcome
+    HALO_TRY(ctx)
+    const uint32_t bps = vec_eval_many_blocks(k, n_max);
+    if (!reserve_or_nomem(ctx->polys_dev, (total ? total : 1) * sizeof(fr_t)) ||
+        !reserve_or_nomem(ctx->polys_off, (k + 1) * sizeof(uint64_t)) ||
+        !reserve_or_nomem(ctx->stage_scalars, (n_max + (uint64_t)bps * k + k) * sizeof(fr_t)))
+        return fail(ctx, HALO_ENOMEM, "halo_poly_eval_many: out of device memory");
+    HALO_CUDA(cudaMemcpyAsync(ctx->polys_off.p, off.data(), (k + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
+    h2d_copy(ctx, ctx->polys_dev.p, coeffs, total * sizeof(fr_t), ctx->stream);
+    fr_t zz;
+    memcpy(&zz, z, 32);
+    fr_t* pows = ctx->stage_scalars.as<fr_t>();
+    fr_t* partials = pows + n_max;
+    fr_t* vs = partials + (uint64_t)bps * k;
+    vec_powers(ctx, zz, n_max, pows);
+    vec_eval_many(ctx, ctx->polys_dev.as<fr_t>(), ctx->polys_off.as<uint64_t>(), k, n_max, pows, partials, vs);
+    HALO_CUDA(cudaMemcpyAsync(vs_out, vs, k * sizeof(fr_t), cudaMemcpyDeviceToHost, ctx->stream));
+    HALO_CUDA(cudaStreamSynchronize(ctx->stream));
+    ctx->polys_k = k;
+    ctx->polys_n = n_max;
+    HALO_CATCH(ctx)
+}
+
+int halo_poly_combine_resident(halo_ctx* ctx, const uint64_t alpha[4], uint64_t* degree_out) {
+    if (!ctx || !alpha || !degree_out) return HALO_EINVAL;
+    if (!ctx->polys_k) return fail(ctx, HALO_ESTATE, "halo_poly_combine_resident: no polynomials (call halo_poly_eval_many first)");
+    HALO_TRY(ctx)
+    const uint64_t n = ctx->polys_n ? ctx->polys_n : 1;  // k empty polynomials combine to one zero coefficient
+    ctx->poly_n = 0;
+    if (!reserve_or_nomem(ctx->poly_dev, n * sizeof(fr_t))) return fail(ctx, HALO_ENOMEM, "halo_poly_combine_resident: out of device memory");
+    fr_t a;
+    memcpy(&a, alpha, 32);
+    vec_poly_combine(ctx, ctx->polys_dev.as<fr_t>(), ctx->polys_off.as<uint64_t>(), ctx->polys_k, a, n, ctx->poly_dev.as<fr_t>());
+    ctx->poly_n = n;
+    *degree_out = device_degree(ctx, ctx->poly_dev.as<fr_t>(), n);
+    HALO_CATCH(ctx)
 }
 
 }  // extern "C"

@@ -169,6 +169,10 @@ struct halo_ctx {
     halo::DevBuf lincomb_claims;  // claim descriptors of vec_h_lincomb
     halo::DevBuf combine_in, combine_work, combine_inv_scratch;  // k_point_combine (combine.cu): inputs, work and outputs, inversions
     uint64_t poly_n = 0;
+    // halo_poly_eval_many: the k uploaded polynomials and their k + 1 segment starts, kept for halo_poly_combine_resident
+    // (polys_k = 0: no evaluation to combine); polys_n = the longest of them
+    halo::DevBuf polys_dev, polys_off;
+    uint64_t polys_k = 0, polys_n = 0;
     // buffers of the (single) in-flight PCDL opening, kept across openings: cudaMalloc / cudaFree of 100+ MB per open
     // costs tens of milliseconds
     halo::DevBuf ipa_G, ipa_cs, ipa_zs, ipa_pbar, ipa_tail, ipa_frozen;

@@ -9,6 +9,7 @@
 //   acc.rs:85-94    AccumulatedHPolys::get_poly -> k_h_lincomb with weights alpha^{i+1}, accumulating onto h_0
 //   (batch decider)  sum_j w_j coeffs(h_j) over claims of mixed size -> k_h_lincomb (DESIGN.md K5b)
 //   pcdl.rs:140-142,156  p_bar = q (X - z), p' = p + alpha p_bar -> k_pbar, k_axpy
+//   (batch opening)  p_j(z) of k polynomials, sum_j alpha^j p_j   -> k_poly_eval_many + k_poly_eval_final, k_poly_combine (K3b)
 #include "common.cuh"
 #include "vec.cuh"
 
@@ -92,6 +93,73 @@ void vec_dot(halo_ctx* ctx, const fr_t* d_a, const fr_t* d_b, uint64_t n, fr_t* 
     k_dot_partial<<<blocks, VEC_THREADS, 0, ctx->stream>>>(d_a, d_b, n, d_partials);
     k_dot_final<<<1, VEC_THREADS, 0, ctx->stream>>>(d_partials, blocks, d_out);
     ctx->kernel_launches += 2;
+    HALO_CUDA(cudaGetLastError());
+}
+
+// ---- k polynomials at one point (K3b) ------------------------------------------------------------------------
+// Polynomial j owns coeffs[off[j] .. off[j+1]).  A segment of bps blocks per polynomial, grid-strided over its coefficients:
+// partials[j bps + b]; then one block per polynomial adds its bps partials.
+__global__ void __launch_bounds__(VEC_THREADS) k_poly_eval_many(const fr_t* __restrict__ coeffs, const uint64_t* __restrict__ off,
+                                                                const fr_t* __restrict__ pows, uint32_t bps,
+                                                                fr_t* __restrict__ partials) {
+    __shared__ fr_t sm[VEC_THREADS];
+    const uint32_t seg = blockIdx.x / bps, b = blockIdx.x % bps;
+    const uint64_t o = off[seg], len = off[seg + 1] - o;
+    fr_t acc, t;
+    fp_zero(acc);
+    for (uint64_t i = (uint64_t)b * blockDim.x + threadIdx.x; i < len; i += (uint64_t)bps * blockDim.x) {
+        fp_mul(t, coeffs[o + i], pows[i]);
+        fp_add(acc, acc, t);
+    }
+    block_sum_fr(acc, sm);
+    if (threadIdx.x == 0) partials[blockIdx.x] = acc;
+}
+__global__ void __launch_bounds__(VEC_THREADS) k_poly_eval_final(const fr_t* __restrict__ partials, uint32_t bps, fr_t* __restrict__ out) {
+    __shared__ fr_t sm[VEC_THREADS];
+    const fr_t* p = partials + (uint64_t)blockIdx.x * bps;
+    fr_t acc;
+    fp_zero(acc);
+    for (uint32_t i = threadIdx.x; i < bps; i += blockDim.x) fp_add(acc, acc, p[i]);
+    block_sum_fr(acc, sm);
+    if (threadIdx.x == 0) out[blockIdx.x] = acc;
+}
+
+uint32_t vec_eval_many_blocks(uint64_t k, uint64_t n_max) {
+    uint64_t b = (n_max + VEC_THREADS - 1) / VEC_THREADS, cap = VEC_DOT_MAX_BLOCKS / k;
+    if (b > cap) b = cap;
+    return b ? (uint32_t)b : 1;
+}
+
+void vec_eval_many(halo_ctx* ctx, const fr_t* d_coeffs, const uint64_t* d_off, uint64_t k, uint64_t n_max, const fr_t* d_pows,
+                   fr_t* d_partials, fr_t* d_out) {
+    const uint32_t bps = vec_eval_many_blocks(k, n_max);
+    k_poly_eval_many<<<(unsigned)(k * bps), VEC_THREADS, 0, ctx->stream>>>(d_coeffs, d_off, d_pows, bps, d_partials);
+    k_poly_eval_final<<<(unsigned)k, VEC_THREADS, 0, ctx->stream>>>(d_partials, bps, d_out);
+    ctx->kernel_launches += 2;
+    HALO_CUDA(cudaGetLastError());
+}
+
+// out[i] = sum_j alpha^j p_j[i] by Horner over j (p_j[i] = 0 from off[j+1] - off[j] on): k multiplications per coefficient
+__global__ void __launch_bounds__(VEC_THREADS) k_poly_combine(const fr_t* __restrict__ coeffs, const uint64_t* __restrict__ off,
+                                                              uint32_t k, fr_t alpha, uint64_t n, fr_t* __restrict__ out) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    fr_t acc;
+    fp_zero(acc);
+#pragma unroll 1
+    for (uint32_t j = k; j-- > 0;) {
+        fp_mul(acc, acc, alpha);
+        const uint64_t o = off[j];
+        if (i < off[j + 1] - o) fp_add(acc, acc, coeffs[o + i]);
+    }
+    out[i] = acc;
+}
+
+void vec_poly_combine(halo_ctx* ctx, const fr_t* d_coeffs, const uint64_t* d_off, uint64_t k, const fr_t& alpha, uint64_t n,
+                      fr_t* d_out) {
+    k_poly_combine<<<(unsigned)((n + VEC_THREADS - 1) / VEC_THREADS), VEC_THREADS, 0, ctx->stream>>>(d_coeffs, d_off, (uint32_t)k,
+                                                                                                     alpha, n, d_out);
+    ctx->kernel_launches++;
     HALO_CUDA(cudaGetLastError());
 }
 

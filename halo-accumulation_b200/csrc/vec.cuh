@@ -7,6 +7,14 @@ constexpr uint32_t VEC_DOT_MAX_BLOCKS = 1184;  // 8 CTAs per SM x 148 SMs
 void vec_powers(halo_ctx* ctx, const fr_t& z, uint64_t n, fr_t* d_out);
 // *d_out = sum a[i] b[i]; d_partials: scratch of VEC_DOT_MAX_BLOCKS elements; everything device resident
 void vec_dot(halo_ctx* ctx, const fr_t* d_a, const fr_t* d_b, uint64_t n, fr_t* d_partials, fr_t* d_out);
+// K3b: k polynomials packed back to back, polynomial j = d_coeffs[d_off[j] .. d_off[j+1]) (d_off: k + 1 device starts), its
+// length <= n_max.  vec_eval_many: d_out[j] = <p_j, d_pows> (d_pows: z^0 .. z^(n_max-1)); d_partials holds
+// k * vec_eval_many_blocks(k, n_max) elements.  vec_poly_combine: d_out[i] = sum_j alpha^j p_j[i], i < n.  k < 2^32.
+uint32_t vec_eval_many_blocks(uint64_t k, uint64_t n_max);
+void vec_eval_many(halo_ctx* ctx, const fr_t* d_coeffs, const uint64_t* d_off, uint64_t k, uint64_t n_max, const fr_t* d_pows,
+                   fr_t* d_partials, fr_t* d_out);
+void vec_poly_combine(halo_ctx* ctx, const fr_t* d_coeffs, const uint64_t* d_off, uint64_t k, const fr_t& alpha, uint64_t n,
+                      fr_t* d_out);
 // c[j] += xi_inv c[j+m]; z[j] += xi z[j+m], j < m
 void vec_fold_scalars(halo_ctx* ctx, fr_t* d_c, fr_t* d_z, uint64_t m, const fr_t& xi, const fr_t& xi_inv);
 // One claim of vec_h_lincomb on the device: weight, x[b] = xi_{lg_n - b} for b < lg_n (one above), lg_n.

@@ -113,6 +113,58 @@ int halo_pcdl_open(halo_ctx* ctx, const uint64_t* coeffs, uint64_t n_coeffs, con
     });
 }
 
+int halo_pcdl_open_batch(halo_ctx* ctx, const uint64_t* coeffs, const uint64_t* n_coeffs, uint64_t k, const uint64_t* Cs, uint64_t d,
+                         const uint64_t z[4], const uint64_t* ws, const uint64_t* q, uint64_t n_q, const uint64_t* w_bar,
+                         uint64_t* vs_out, uint64_t C_out[12], uint64_t v_out[4], halo_eval_proof* pi) {
+    return guarded([&] {
+        ensure(k >= 1, HALO_EINVAL, "halo_pcdl_open_batch: nothing to open (k = 0)");
+        ensure(n_coeffs && Cs && vs_out && C_out && v_out && pi, HALO_EINVAL, "halo_pcdl_open_batch: NULL pointer");
+        std::vector<PolyView> ps;
+        std::vector<PallasPoint> C(k);
+        std::vector<PallasScalar> w(ws ? k : 0);
+        ps.reserve(k);
+        uint64_t off = 0;
+        for (uint64_t j = 0; j < k; j++) {
+            ensure(n_coeffs[j] <= UINT64_MAX / 32 - off, HALO_EINVAL, "halo_pcdl_open_batch: packed size overflows");
+            ps.push_back(poly_from(coeffs + 4 * off, n_coeffs[j]));
+            off += n_coeffs[j];
+            C[j] = point_load_checked(Cs + 12 * j, "C_j is not a canonical point on the curve");
+            if (ws) w[j] = scalar_load_checked(ws + 4 * j, "w_j is not a canonical scalar");
+        }
+        ensure(coeffs || off == 0, HALO_EINVAL, "halo_pcdl_open_batch: NULL coefficients");
+        const PallasScalar zs = scalar_load_checked(z, "z is not a canonical scalar");
+        PallasScalar wbs;
+        PolyView qp(nullptr, 0);
+        if (ws) {
+            ensure(w_bar && (q || n_q == 0), HALO_EINVAL, "hiding open needs q and w_bar");
+            wbs = scalar_load(w_bar);
+            qp = poly_from(q, n_q);
+        }
+        pcdl::BatchOpening r = pcdl::open_batch(ctx, ps, C, d, zs, ws ? w.data() : nullptr, ws ? &qp : nullptr, ws ? &wbs : nullptr);
+        for (uint64_t j = 0; j < k; j++) scalar_store(vs_out + 4 * j, r.vs[j]);
+        point_store(C_out, r.C);
+        scalar_store(v_out, r.v);
+        pcdl::proof_to_c(r.pi, *pi);
+    });
+}
+
+int halo_pcdl_batch_claim(halo_ctx* ctx, const uint64_t* Cs, const uint64_t* vs, uint64_t k, const uint64_t z[4], uint64_t C_out[12],
+                          uint64_t v_out[4]) {
+    return guarded([&] {
+        ensure(k >= 1, HALO_EINVAL, "halo_pcdl_batch_claim: no claim (k = 0)");
+        ensure(Cs && vs && C_out && v_out, HALO_EINVAL, "halo_pcdl_batch_claim: NULL pointer");
+        std::vector<PallasPoint> C(k);
+        std::vector<PallasScalar> v(k);
+        for (uint64_t j = 0; j < k; j++) {
+            C[j] = point_load_checked(Cs + 12 * j, "C_j is not a canonical point on the curve");
+            v[j] = scalar_load_checked(vs + 4 * j, "v_j is not a canonical scalar");
+        }
+        const pcdl::BatchClaim r = pcdl::batch_claim(ctx, C, v, scalar_load_checked(z, "z is not a canonical scalar"));
+        point_store(C_out, r.C);
+        scalar_store(v_out, r.v);
+    });
+}
+
 int halo_pcdl_succinct_check(halo_ctx* ctx, const uint64_t C_jac[12], uint64_t d, const uint64_t z[4], const uint64_t v[4],
                              const halo_eval_proof* pi, uint64_t* xis_out, uint64_t U_out[12]) {
     return guarded([&] {

@@ -57,38 +57,53 @@ PallasPoint commit(halo_ctx* ctx, PolyView p, uint64_t d, const PallasScalar* w)
     return pedersen::commit(ctx, w, nullptr, n, p.data(), n_coeffs, true);
 }
 
-std::vector<PallasPoint> commit_batch(halo_ctx* ctx, const std::vector<PolyView>& ps, uint64_t d, const PallasScalar* ws) {
-    const size_t k = ps.size();
+// The polynomials of a batch of degree bound d, validated in order as commit does (the first malformed one throws), and the
+// number of coefficients each uploads: coeffs.resize(n, ZERO) (pcdl.rs:106-107) implies the zero tail.
+static std::vector<uint64_t> batch_lens(halo_ctx* ctx, const std::vector<PolyView>& ps, uint64_t d) {
     const uint64_t n = d + 1;
-    std::vector<uint64_t> lens(k);
-    bool packed = true;  // the uploaded prefixes already lie back to back in memory (no host copy)
-    const PallasScalar* end = nullptr;  // one past the uploaded prefix of the last non-empty polynomial
-    for (size_t j = 0; j < k; j++) {
+    std::vector<uint64_t> lens(ps.size());
+    for (size_t j = 0; j < ps.size(); j++) {
         ensure(is_pow2(n), HALO_EINVAL, "d+1 is not a power of 2");  // pcdl.rs:102
         ensure(degree(ps[j]) <= d, HALO_EINVAL, "p.degree() > d");   // pcdl.rs:103
         ensure(n <= halo_num_generators(ctx), HALO_EINVAL, "d > D");  // pcdl.rs:104
-        lens[j] = ps[j].size() < n ? ps[j].size() : n;  // coeffs.resize(n, ZERO) (pcdl.rs:106-107): the zero tail is implied
+        lens[j] = ps[j].size() < n ? ps[j].size() : n;
+    }
+    return lens;
+}
+
+// The uploaded prefixes (lens[j] coefficients of ps[j]) as one packed array: in place when they already lie back to back in
+// memory, else copied into `copy`.  Null when there is nothing to upload.
+static const PallasScalar* packed_prefixes(const std::vector<PolyView>& ps, const std::vector<uint64_t>& lens,
+                                           std::vector<PallasScalar>& copy) {
+    const size_t k = ps.size();
+    bool packed = true;
+    const PallasScalar* end = nullptr;  // one past the uploaded prefix of the last non-empty polynomial
+    for (size_t j = 0; j < k; j++) {
         if (!lens[j]) continue;  // an empty polynomial uploads nothing, wherever its view points
         if (end && ps[j].data() != end) packed = false;
         end = ps[j].data() + lens[j];
     }
-    if (k == 0) return {};
-    if (k == 1) return {commit(ctx, ps[0], d, ws)};  // the single call, exactly
     size_t first = 0;  // the first polynomial with coefficients to upload anchors the packed buffer
     while (first < k && !lens[first]) first++;
-    std::vector<PallasScalar> copy;
-    const PallasScalar* base = first < k ? ps[first].data() : nullptr;
-    if (!packed) {
-        uint64_t total = 0;
-        for (uint64_t l : lens) total += l;
-        copy.resize(total);
-        uint64_t o = 0;
-        for (size_t j = 0; j < k; j++) {
-            std::copy(ps[j].data(), ps[j].data() + lens[j], copy.begin() + o);
-            o += lens[j];
-        }
-        base = copy.data();
+    if (packed) return first < k ? ps[first].data() : nullptr;
+    uint64_t total = 0;
+    for (uint64_t l : lens) total += l;
+    copy.resize(total);
+    uint64_t o = 0;
+    for (size_t j = 0; j < k; j++) {
+        std::copy(ps[j].data(), ps[j].data() + lens[j], copy.begin() + o);
+        o += lens[j];
     }
+    return copy.data();
+}
+
+std::vector<PallasPoint> commit_batch(halo_ctx* ctx, const std::vector<PolyView>& ps, uint64_t d, const PallasScalar* ws) {
+    const size_t k = ps.size();
+    const std::vector<uint64_t> lens = batch_lens(ctx, ps, d);
+    if (k == 0) return {};
+    if (k == 1) return {commit(ctx, ps[0], d, ws)};  // the single call, exactly
+    std::vector<PallasScalar> copy;
+    const PallasScalar* base = packed_prefixes(ps, lens, copy);
     std::vector<uint64_t> out(12 * k);
     static const PallasScalar none = scalar_zero();
     check_rc(ctx, halo_msm_gens_many(ctx, reinterpret_cast<const uint64_t*>(base ? base : &none), lens.data(), k, out.data()));
@@ -104,19 +119,78 @@ std::vector<PallasPoint> commit_batch(halo_ctx* ctx, const std::vector<PolyView>
 }
 
 static EvalProof open_impl(halo_ctx* ctx, const PolyView* p, uint64_t deg, const PallasPoint& C, uint64_t d, const PallasScalar& z,
-                           const PallasScalar* w, const PolyView* q, const PallasScalar* w_bar);
+                           const PallasScalar* w, const PolyView* q, const PallasScalar* w_bar, PallasScalar* v_out);
 
 EvalProof open(halo_ctx* ctx, PolyView p, const PallasPoint& C, uint64_t d, const PallasScalar& z, const PallasScalar* w,
-               const PolyView* q, const PallasScalar* w_bar) {
-    return open_impl(ctx, &p, degree(p), C, d, z, w, q, w_bar);
+               const PolyView* q, const PallasScalar* w_bar, PallasScalar* v_out) {
+    return open_impl(ctx, &p, degree(p), C, d, z, w, q, w_bar, v_out);
 }
 EvalProof open_resident(halo_ctx* ctx, uint64_t deg, const PallasPoint& C, uint64_t d, const PallasScalar& z,
-                        const PallasScalar* w, const PolyView* q, const PallasScalar* w_bar) {
-    return open_impl(ctx, nullptr, deg, C, d, z, w, q, w_bar);
+                        const PallasScalar* w, const PolyView* q, const PallasScalar* w_bar, PallasScalar* v_out) {
+    return open_impl(ctx, nullptr, deg, C, d, z, w, q, w_bar, v_out);
+}
+
+BatchClaim batch_claim(halo_ctx* ctx, const std::vector<PallasPoint>& Cs, const std::vector<PallasScalar>& vs, const PallasScalar& z) {
+    const size_t k = Cs.size();
+    ensure(k >= 1 && vs.size() == k, HALO_EINVAL, "batch claim: no polynomial");
+    // alpha binds every v_j: a prover could otherwise trade a false v_j against another
+    const std::vector<affine_t> aff = batch_to_affine(Cs);
+    Transcript t;
+    t.scalar(z);
+    for (size_t j = 0; j < k; j++) t.point_affine(aff[j]).scalar(vs[j]);
+    BatchClaim r;
+    r.alpha = t.finish(0);
+    r.powers.resize(k);
+    r.powers[0] = scalar_one();
+    for (size_t j = 1; j < k; j++) r.powers[j] = r.powers[j - 1] * r.alpha;
+    r.v = scalar_zero();
+    for (size_t j = 0; j < k; j++) r.v = r.v + r.powers[j] * vs[j];
+    r.C = point_dot(ctx, r.powers.data(), Cs, k);
+    return r;
+}
+
+BatchOpening open_batch(halo_ctx* ctx, const std::vector<PolyView>& ps, const std::vector<PallasPoint>& Cs, uint64_t d,
+                        const PallasScalar& z, const PallasScalar* ws, const PolyView* q, const PallasScalar* w_bar) {
+    const size_t k = ps.size();
+    ensure(k >= 1 && Cs.size() == k, HALO_EINVAL, "open_batch: no polynomial");
+    const std::vector<uint64_t> lens = batch_lens(ctx, ps, d);
+    if (ws) {  // q is drawn before alpha exists: max_j deg(p_j) coefficients, as `open` wants deg(p) >= 1 of them
+        ensure(q && w_bar, HALO_EINVAL, "hiding open needs the random polynomial q and w_bar");
+        uint64_t max_deg = 0;
+        for (const PolyView& p : ps) max_deg = std::max(max_deg, degree(p));
+        ensure(max_deg >= 1 && q->size() == max_deg, HALO_ELEN, "q must have max_j deg(p_j) coefficients");
+    }
+    BatchOpening r;
+    if (k == 1) {  // the single call, exactly: alpha^0 = 1 makes the claim (C_0, v_0)
+        r.pi = open(ctx, ps[0], Cs[0], d, z, ws, q, w_bar, &r.v);
+        r.vs = {r.v};
+        r.C = Cs[0];
+        return r;
+    }
+    std::vector<PallasScalar> copy;
+    const PallasScalar* base = packed_prefixes(ps, lens, copy);
+    r.vs.resize(k);
+    check_rc(ctx, halo_poly_eval_many(ctx, reinterpret_cast<const uint64_t*>(base), lens.data(), k, d + 1,
+                                      reinterpret_cast<const uint64_t*>(&z), reinterpret_cast<uint64_t*>(r.vs.data())));
+    const BatchClaim bc = batch_claim(ctx, Cs, r.vs, z);
+    PallasScalar w = scalar_zero();
+    if (ws)
+        for (size_t j = 0; j < k; j++) w = w + bc.powers[j] * ws[j];
+    uint64_t deg = 0;
+    check_rc(ctx, halo_poly_combine_resident(ctx, reinterpret_cast<const uint64_t*>(&bc.alpha), &deg));
+    // the top coefficients of p cancel only with negligible probability; the opening then takes the first deg(p) of q
+    const PolyView qd = ws ? PolyView(q->data(), std::min<uint64_t>(deg, q->size())) : PolyView(nullptr, 0);
+    PallasScalar v_dev;
+    r.pi = open_resident(ctx, deg, bc.C, d, z, ws ? &w : nullptr, ws ? &qd : nullptr, w_bar, &v_dev);
+    // the opening evaluates p(z) itself; it must be the claim's sum_j alpha^j v_j
+    ensure(v_dev == bc.v, HALO_EINTERNAL, "open_batch: p(z) of the combined polynomial differs from sum_j alpha^j v_j");
+    r.C = bc.C;
+    r.v = bc.v;
+    return r;
 }
 
 static EvalProof open_impl(halo_ctx* ctx, const PolyView* p, uint64_t deg, const PallasPoint& C, uint64_t d, const PallasScalar& z,
-                           const PallasScalar* w, const PolyView* q, const PallasScalar* w_bar) {
+                           const PallasScalar* w, const PolyView* q, const PallasScalar* w_bar, PallasScalar* v_out) {
     uint64_t n = d + 1;
     ensure(is_pow2(n), HALO_EINVAL, "d+1 is not a power of 2");  // pcdl.rs:130
     ensure(deg <= d, HALO_EINVAL, "p.degree() > d");             // pcdl.rs:131
@@ -140,6 +214,7 @@ static EvalProof open_impl(halo_ctx* ctx, const PolyView* p, uint64_t deg, const
         ~Guard() { halo_ipa_destroy(s); }
     } guard{st};
     PallasScalar v = scalar_load(vbuf);
+    if (v_out) *v_out = v;
 
     EvalProof pi;
     PallasPoint C_prime = C;

@@ -35,12 +35,32 @@ PallasPoint commit(halo_ctx* ctx, PolyView p, uint64_t d, const PallasScalar* w)
 // `commit` of every polynomial (w: one blinding scalar per polynomial, or null): validated in order as commit does, then one
 // halo_msm_gens_many over all of them and w_j S added by one `combine` call (DESIGN.md K2c)
 std::vector<PallasPoint> commit_batch(halo_ctx* ctx, const std::vector<PolyView>& ps, uint64_t d, const PallasScalar* ws);
-// pcdl.rs:120-242; rng draws made explicit: q (deg p coefficients), w_bar
+// pcdl.rs:120-242; rng draws made explicit: q (deg p coefficients), w_bar.  v_out (nullable) receives v = p(z).
 EvalProof open(halo_ctx* ctx, PolyView p, const PallasPoint& C, uint64_t d, const PallasScalar& z, const PallasScalar* w,
-               const PolyView* q, const PallasScalar* w_bar);
+               const PolyView* q, const PallasScalar* w_bar, PallasScalar* v_out = nullptr);
 // Same for a polynomial of degree `deg` that already sits on the device (halo_h_lincomb_resident): acc.rs:209.
 EvalProof open_resident(halo_ctx* ctx, uint64_t deg, const PallasPoint& C, uint64_t d, const PallasScalar& z,
-                        const PallasScalar* w, const PolyView* q, const PallasScalar* w_bar);
+                        const PallasScalar* w, const PolyView* q, const PallasScalar* w_bar, PallasScalar* v_out = nullptr);
+
+// Batch opening at one point (DESIGN.md K3b; the reference has none).  batch_claim reduces the claims (C_j, z, v_j) to one:
+// alpha = rho_0(z, C_0, v_0, .., C_{k-1}, v_{k-1}), C = sum_j alpha^j C_j, v = sum_j alpha^j v_j; powers[j] = alpha^j.
+struct BatchClaim {
+    PallasScalar alpha, v;
+    PallasPoint C;
+    std::vector<PallasScalar> powers;
+};
+BatchClaim batch_claim(halo_ctx* ctx, const std::vector<PallasPoint>& Cs, const std::vector<PallasScalar>& vs, const PallasScalar& z);
+// v_j = p_j(z) for every polynomial, then `open` of p = sum_j alpha^j p_j against the batch claim (C, v), with
+// w = sum_j alpha^j w_j when ws is given; q carries max_j deg(p_j) coefficients, of which the opening uses the first deg(p).
+// The polynomials are validated in order as commit_batch does, before any device work.  k = 1 is `open` itself.
+struct BatchOpening {
+    std::vector<PallasScalar> vs;
+    PallasPoint C;
+    PallasScalar v;
+    EvalProof pi;
+};
+BatchOpening open_batch(halo_ctx* ctx, const std::vector<PolyView>& ps, const std::vector<PallasPoint>& Cs, uint64_t d,
+                        const PallasScalar& z, const PallasScalar* ws, const PolyView* q, const PallasScalar* w_bar);
 // succinct_check (pcdl.rs:252-314) without its group equation, in two halves around C' = C + alpha C_bar - w' S (:272-279) so
 // that a batch can compute every C' with one `combine` call.  succinct_alpha validates (d + 1 a power of two, d <= D, the
 // number of rounds) and returns alpha = rho_0(C, z, v, C_bar) of a hiding proof (zero otherwise); succinct_finish runs the rest

@@ -63,6 +63,35 @@ def open(ctx, p, Cm, d, z, w=None, q=None, w_bar=None):
     return pi
 
 
+def open_batch(ctx, ps, Cs, d, z, ws=None, q=None, w_bar=None):
+    """Opens the polynomials `ps` (commitments Cs, one degree bound d) at one point z with ONE proof (include/halo_pcdl.h
+    halo_pcdl_open_batch; the reference has none) -> (vs, C, v, pi): vs[j] = p_j(z), and (C, d, z, v, pi) is an ordinary
+    claim for `check`, `check_batch` or acc.new_instance.  Hiding with ws (one w_j per polynomial): q holds
+    max_j deg(p_j) coefficients.  With one polynomial this is `open`, bit for bit."""
+    packed, lens = pack(ps)
+    k = len(lens)
+    Cs, z = arr(Cs).reshape(k, 12), arr(z, (4,))
+    wa = arr(ws).reshape(k, 4) if ws is not None else None
+    qa = arr(q).reshape(-1, 4) if q is not None else None
+    wbk, wbp = _host.opt(w_bar)
+    vs = np.zeros((max(1, k), 4), dtype=np.uint64)
+    Cm, v, pi = np.zeros(12, dtype=np.uint64), np.zeros(4, dtype=np.uint64), EvalProof()
+    _host.chk(_host.lib().halo_pcdl_open_batch(ctx._h, p64(packed), p64(lens), C.c_uint64(k), p64(Cs), C.c_uint64(d), p64(z),
+                                               p64(wa) if wa is not None else None, p64(qa) if qa is not None else None,
+                                               C.c_uint64(qa.shape[0] if qa is not None else 0), wbp, p64(vs), p64(Cm), p64(v),
+                                               C.byref(pi)))
+    return vs[:k], Cm, v, pi
+
+
+def batch_claim(ctx, Cs, z, vs):
+    """The verifier's reduction of the claims (C_j, z, vs[j]) of `open_batch` to its one claim -> (C, v)."""
+    Cs, z = arr(Cs).reshape(-1, 12), arr(z, (4,))
+    vs = arr(vs).reshape(Cs.shape[0], 4)
+    Cm, v = np.zeros(12, dtype=np.uint64), np.zeros(4, dtype=np.uint64)
+    _host.chk(_host.lib().halo_pcdl_batch_claim(ctx._h, p64(Cs), p64(vs), C.c_uint64(Cs.shape[0]), p64(z), p64(Cm), p64(v)))
+    return Cm, v
+
+
 def succinct_check(ctx, Cm, d, z, v, pi):
     """pcdl.rs:252-314 -> (HPoly, U); raises Rejected"""
     Cm, z, v = arr(Cm, (12,)), arr(z, (4,)), arr(v, (4,))

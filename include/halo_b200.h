@@ -271,6 +271,21 @@ int halo_h_lincomb(halo_ctx *ctx, const uint64_t *h0 /*[n_h0][4]*/, uint64_t n_h
 int halo_h_lincomb_resident(halo_ctx *ctx, const uint64_t *h0, uint64_t n_h0, const uint64_t *alphas, const uint64_t *xis,
                             uint64_t m, uint32_t lg_n, uint64_t *degree_out);
 
+/* ---- K3b: k polynomials opened at one point (halo_pcdl_open_batch, include/halo_pcdl.h) ----------------- */
+/* vs_out[j] = p_j(z) for k polynomials packed back to back (polynomial j has n_coeffs[j] <= n coefficients), in one segmented
+ * evaluation: the coefficients are uploaded once (pageable memory staged as by halo_msm_gens), z^0 .. z^(max_j n_coeffs[j] - 1)
+ * built on the device, then two launches for all k.  The polynomials stay on the device for halo_poly_combine_resident; their
+ * buffer (sum_j n_coeffs[j] * 32 bytes) stays in the context until it is destroyed, like the opening's buffers.
+ * HALO_EINVAL: NULL pointers, k = 0 or k >= 2^31, n beyond the resident generators, n_coeffs[j] > n (nothing runs).
+ * HALO_ENOMEM: no device memory for the upload; nothing is written and no evaluation is left to combine. */
+int halo_poly_eval_many(halo_ctx *ctx, const uint64_t *coeffs /*packed, [sum n_coeffs][4]*/, const uint64_t *n_coeffs /*[k]*/,
+                        uint64_t k, uint64_t n, const uint64_t z[4], uint64_t *vs_out /*[k][4]*/);
+/* p = sum_j alpha^j p_j over the polynomials of the last halo_poly_eval_many (one launch; coefficients of p_j past
+ * n_coeffs[j] are zero), left on the device for halo_ipa_begin_resident; *degree_out = its degree (DensePolynomial::degree).
+ * May be called again with another alpha.  HALO_ESTATE: no preceding evaluation on this context.  HALO_ENOMEM: no device
+ * memory for p; the context then holds no resident polynomial. */
+int halo_poly_combine_resident(halo_ctx *ctx, const uint64_t alpha[4], uint64_t *degree_out);
+
 /* ---- K3 / K4 / K7: the rounds of PCDL.open (pcdl.rs:183-231) ----------------------------------------- */
 typedef struct halo_ipa halo_ipa;
 /* Uploads the coefficients of p (zero-padded to n, pcdl.rs:183-184), copies GS[0..n) (pcdl.rs:185), builds

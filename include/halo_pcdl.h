@@ -82,6 +82,35 @@ int halo_pcdl_commit_batch(halo_ctx *ctx, const uint64_t *coeffs /*packed*/, con
 int halo_pcdl_open(halo_ctx *ctx, const uint64_t *coeffs, uint64_t n_coeffs, const uint64_t C_jac[12], uint64_t d,
                    const uint64_t z[4], const uint64_t *w /*nullable*/, const uint64_t *q, uint64_t n_q,
                    const uint64_t *w_bar, halo_eval_proof *pi);
+/* Batch opening at one point (an extension: the reference opens one polynomial at a time, DESIGN.md K3b).  For k >= 1
+ * polynomials p_j of one degree bound d, packed as in halo_pcdl_commit_batch, their commitments C_j (as commit returns them,
+ * C_j = commit(p_j) + w_j S) and one point z:
+ *   v_j   = p_j(z)                                                  -> vs_out[j]
+ *   alpha = rho_0(z, C_0, v_0, C_1, v_1, .., C_{k-1}, v_{k-1})      (tag 0; z, every v_j as a scalar, every C_j compressed)
+ *   C = sum_j alpha^j C_j, v = sum_j alpha^j v_j                    -> C_out, v_out
+ *   p = sum_j alpha^j p_j, and with ws: w = sum_j alpha^j w_j
+ *   pi = halo_pcdl_open(p, C, d, z, w, q, w_bar)                    -> pi
+ * (C, d, z, v, pi) is an ordinary PCDL claim: halo_pcdl_check, halo_pcdl_check_batch and the accumulation scheme take it
+ * unchanged.  alpha binds every v_j.  If some p_j(z) != v_j, the combined claim is true for at most k - 1 values of alpha,
+ * so a false batch passes with probability <= (k - 1) / r plus the soundness error of one PCDL check.
+ * Hiding iff ws != NULL: then q holds n_q = max_j deg(p_j) coefficients (what is known before alpha exists; the opening
+ * uses the first deg(p) of them, all of them unless the top coefficients cancel) and w_bar is the second draw.  k = 1 is
+ * halo_pcdl_open itself, bit for bit (C = C_0, v = v_0).  The uploaded polynomials stay in the context's pooled buffer
+ * (halo_poly_eval_many).
+ * Returns HALO_EINVAL, before any device work and before any output is written, for k = 0, NULL pointers, the first
+ * malformed polynomial in order (d + 1 not a power of two, deg > d, d >= the resident generators), a C_j off the curve or
+ * not canonical, a w_j or z not canonical; HALO_ELEN for n_q != max_j deg(p_j) or deg = 0 with hiding (as open);
+ * HALO_EINTERNAL when the opening's own p(z) differs from v (a bug, not a decision). */
+int halo_pcdl_open_batch(halo_ctx *ctx, const uint64_t *coeffs /*packed*/, const uint64_t *n_coeffs /*[k]*/, uint64_t k,
+                         const uint64_t *Cs /*[k][12]*/, uint64_t d, const uint64_t z[4], const uint64_t *ws /*[k][4] or NULL*/,
+                         const uint64_t *q, uint64_t n_q, const uint64_t *w_bar, uint64_t *vs_out /*[k][4]*/, uint64_t C_out[12],
+                         uint64_t v_out[4], halo_eval_proof *pi);
+/* The verifier's side of halo_pcdl_open_batch: the claims (C_j, z, v_j) reduced to the one claim (C, v) above (alpha from the
+ * same transcript), to be decided by halo_pcdl_check / _succinct_check / _check_batch or accumulated.  C_j = O (the zero
+ * polynomial without hiding) is allowed.  HALO_EINVAL: k = 0, NULL pointers, a C_j off the curve or not canonical, a v_j or
+ * z not canonical. */
+int halo_pcdl_batch_claim(halo_ctx *ctx, const uint64_t *Cs /*[k][12]*/, const uint64_t *vs /*[k][4]*/, uint64_t k,
+                          const uint64_t z[4], uint64_t C_out[12], uint64_t v_out[4]);
 /* pcdl.rs:252-314; on accept writes the HPoly challenges xis[lg_n+1][4] and U. */
 int halo_pcdl_succinct_check(halo_ctx *ctx, const uint64_t C_jac[12], uint64_t d, const uint64_t z[4], const uint64_t v[4],
                              const halo_eval_proof *pi, uint64_t *xis_out, uint64_t U_out[12]);
