@@ -30,6 +30,13 @@ __global__ void __launch_bounds__(256) k_mark_infinity(affine_t* __restrict__ ba
     if (i < n && inf[i]) affine_set_inf(bases[i]);
 }
 
+// The caller's infinity flags of n staged bases to d_inf, then the flagged bases set to infinity, on `st`
+static void mark_infinity(halo_ctx* ctx, cudaStream_t st, affine_t* d_bases, uint8_t* d_inf, const uint8_t* inf_flags, uint64_t n) {
+    HALO_CUDA(cudaMemcpyAsync(d_inf, inf_flags, n, cudaMemcpyHostToDevice, st));
+    k_mark_infinity<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_bases, d_inf, n);
+    ctx->kernel_launches++;
+}
+
 __global__ void __launch_bounds__(128) k_jac_to_affine(const jac_t* __restrict__ in, affine_t* __restrict__ out, uint64_t n) {
     uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
@@ -673,16 +680,13 @@ struct ManyGroup {
     MsmPlan plan;
 };
 
-// Plan of one output of the batch by its length: FIXED base under the conditions of a single MSM, else the variable-base
-// window of a single MSM of that length; groups of short segments then narrow it (many_groups).
-MsmPlan many_seg_plan(halo_ctx* ctx, uint64_t len) { return gens_use_fixed(ctx, len) ? ctx->pre_plan : msm_make_plan(len, ctx->force_c); }
-
 // Outputs in caller order, cut into groups of one plan within the limits above; a group of one output is an ordinary MSM.
+// Each output's plan is that of a single MSM of its length; groups of short segments then narrow it.
 std::vector<ManyGroup> many_groups(halo_ctx* ctx, const std::vector<uint64_t>& jobs, const uint64_t* lens, const uint64_t* starts) {
     std::vector<ManyGroup> gs;
     for (size_t j = 0; j < jobs.size(); j++) {
         const uint64_t len = lens[jobs[j]];
-        const MsmPlan p = many_seg_plan(ctx, len);
+        const MsmPlan p = msm_plan(ctx, len, gens_use_fixed(ctx, len));
         if (!gs.empty()) {
             ManyGroup& g = gs.back();
             const uint64_t segs = g.j1 - g.j0 + 1, ns = g.ns + len, nb = segs * g.plan.NB, entries = ns * (uint64_t)p.W;
@@ -705,32 +709,12 @@ std::vector<ManyGroup> many_groups(halo_ctx* ctx, const std::vector<uint64_t>& j
         // at 8 -- 8 segments 0.77 ms (c = 11, the single-MSM window: 1.07), 64 segments 2.98 ms (4.56).  A batch fills the
         // machine, so the narrow window's smaller bucket reduction wins over the latency-bound single MSM's choice.  At 2^16 (8 /
         // 64 segments) the single-MSM window is within 3 % of the best: kept.  (2^13 .. 2^15: not measured.)
-        if (!g.plan.fixed && !ctx->force_c && segs >= 8 && g.max_len <= 4096 && g.plan.c > 8) g.plan = msm_make_plan(g.max_len, 8);
-        plan_set_segments(g.plan, segs);
+        const bool narrow = !g.plan.fixed && !ctx->force_c && segs >= 8 && g.max_len <= 4096 && g.plan.c > 8;
+        g.plan = msm_plan(ctx, g.max_len, g.plan.fixed, narrow ? 8 : g.plan.c, segs);
     }
     return gs;
 }
 
-// f(0) .. f(k - 1) on up to 16 host threads (the host finish of a group's segments)
-void many_parallel(size_t k, const std::function<void(size_t)>& f) {
-    const size_t hw = std::thread::hardware_concurrency();
-    const size_t T = std::min(k, std::max<size_t>(1, std::min<size_t>(hw, 16)));
-    std::vector<std::thread> th;
-    std::vector<size_t> unspawned;
-    auto work = [&](size_t t) {
-        for (size_t j = t; j < k; j += T) f(j);
-    };
-    for (size_t t = 1; t < T; t++) {
-        try {
-            th.emplace_back(work, t);
-        } catch (const std::system_error&) {
-            unspawned.push_back(t);  // no thread available: this thread takes that share as well
-        }
-    }
-    work(0);
-    for (size_t t : unspawned) work(t);
-    for (auto& x : th) x.join();
-}
 }  // namespace
 
 int halo_msm_gens_many(halo_ctx* ctx, const uint64_t* scalars, const uint64_t* lens, uint64_t k, uint64_t* out_jac) {
@@ -761,14 +745,13 @@ int halo_msm_gens_many(halo_ctx* ctx, const uint64_t* scalars, const uint64_t* l
     std::vector<ManyGroup> groups = many_groups(ctx, jobs, lens, starts.data());
     const size_t G = groups.size();
     auto multi = [&](size_t g) { return groups[g].j1 - groups[g].j0 > 1; };
-    auto n_parts = [](const MsmPlan& p) { return (size_t)3 * (p.fixed ? 1 : p.W) * p.segs; };
     // both buffers at the size of the largest group, before anything is in flight
     uint64_t max_ns = 0;
     size_t max_parts = 0;
     for (size_t g = 0; g < G; g++)
         if (multi(g)) {
             max_ns = std::max(max_ns, groups[g].ns);
-            max_parts = std::max(max_parts, n_parts(groups[g].plan));
+            max_parts = std::max(max_parts, msm_parts(groups[g].plan));
         }
     if (max_ns) {
         async_init(ctx);
@@ -813,24 +796,14 @@ int halo_msm_gens_many(halo_ctx* ctx, const uint64_t* scalars, const uint64_t* l
     };
     // group g's segmented MSM on the context stream, its window partials to the pinned host buffer
     auto launch = [&](size_t g) {
-        ManyGroup& gr = groups[g];
+        const ManyGroup& gr = groups[g];
         halo_ctx::ManyBuf& b = ctx->many[g & 1];
-        MsmPlan& plan = gr.plan;  // msm_enqueue settles the reduction geometry in it
-        const size_t nparts = n_parts(plan);
-        MsmInput in;
-        in.scalars = b.scalars.as<fr_t>();
-        in.n = (uint32_t)gr.ns;
-        in.segs = plan.segs;
+        // FIXED base as the group's plan, which the segment lengths chose, not by the length of the whole group
+        MsmInput in = gens_msm_input(ctx, gr.plan.fixed, b.scalars.as<fr_t>(), 0, gr.ns);
+        in.segs = gr.plan.segs;
         in.seg_off = b.seg_off.as<uint32_t>();
-        if (plan.fixed) {
-            in.bases = ctx->gens_pre.as<affine_t>();
-            in.fixed_stride = (uint32_t)ctx->pre_n;
-        } else {
-            in.bases = ctx->gens.as<affine_t>();
-        }
         HALO_CUDA(cudaStreamWaitEvent(ctx->stream, b.copied, 0));
-        msm_enqueue(ctx, in, plan, b.parts.as<xyzz_t>(), 0);
-        HALO_CUDA(cudaMemcpyAsync(b.h_parts, b.parts.p, nparts * sizeof(xyzz_t), cudaMemcpyDeviceToHost, ctx->stream));
+        msm_enqueue_to_host(ctx, in, gr.plan, b.parts.as<xyzz_t>(), b.h_parts);
         HALO_CUDA(cudaEventRecord(b.done, ctx->stream));
     };
     // host finish of group g, one segment per task (a variable-base finish is ~255 doublings)
@@ -838,7 +811,7 @@ int halo_msm_gens_many(halo_ctx* ctx, const uint64_t* scalars, const uint64_t* l
         const ManyGroup& gr = groups[g];
         halo_ctx::ManyBuf& b = ctx->many[g & 1];
         HALO_CUDA(cudaEventSynchronize(b.done));
-        const size_t per = (size_t)3 * (gr.plan.fixed ? 1 : gr.plan.W);
+        const size_t per = msm_parts(gr.plan) / gr.plan.segs;
         auto one = [&](size_t s) {
             xyzz_t r;
             msm_finish_host(b.h_parts + per * s, gr.plan, r);
@@ -847,7 +820,7 @@ int halo_msm_gens_many(halo_ctx* ctx, const uint64_t* scalars, const uint64_t* l
         if (gr.plan.fixed)
             for (size_t s = 0; s < gr.plan.segs; s++) one(s);
         else
-            many_parallel(gr.plan.segs, one);
+            host_parallel(gr.plan.segs, one);
     };
     // Pipeline: the copy of group g+1 and the host finish of group g-1 run while group g is on the device.  A group of one
     // output drains the pipeline and takes the halo_msm_gens route.
@@ -888,36 +861,24 @@ static int submit_impl(halo_ctx* ctx, const uint64_t* scalars, bool resident, ui
         const bool ahead_on = ctx->tune_sort_ahead > 0 && n >= ((uint64_t)1 << 22);
         // (delaying the sort until the HBM-bound pass-0 gathers of the MSM in front are over measured slower: the
         // throttled sort then no longer fits under what is left of that MSM)
-        MsmInput in;
-        if (resident) {
-            in.scalars = reinterpret_cast<const fr_t*>(scalars);
-            // the caller's producer of the scalars ran on a stream we do not know: like halo_msm_gens_resident, the
-            // contract is that they are complete when this call is made
-        } else {
+        // resident: the caller's producer of the scalars ran on a stream we do not know; like halo_msm_gens_resident, the
+        // contract is that they are complete when this call is made
+        const fr_t* d_scalars = reinterpret_cast<const fr_t*>(scalars);
+        if (!resident) {
             s.scalars.reserve(n * sizeof(fr_t));
             h2d_copy(ctx, s.scalars.p, scalars, n * sizeof(fr_t), ctx->copy_stream);
             HALO_CUDA(cudaEventRecord(s.copied, ctx->copy_stream));
             HALO_CUDA(cudaStreamWaitEvent(ahead_on ? ctx->sort_stream : ctx->stream, s.copied, 0));
-            in.scalars = s.scalars.as<fr_t>();
+            d_scalars = s.scalars.as<fr_t>();
         }
-        in.n = (uint32_t)n;
-        if (gens_use_fixed(ctx, n)) {
-            in.bases = ctx->gens_pre.as<affine_t>();
-            in.fixed_stride = (uint32_t)ctx->pre_n;
-            in.fixed_first = (uint32_t)off;
-            s.plan = ctx->pre_plan;
-        } else {
-            in.bases = ctx->gens.as<affine_t>() + off;
-            s.plan = msm_make_plan(n, ctx->force_c);
-        }
+        const bool fixed = gens_use_fixed(ctx, n);
+        s.plan = msm_plan(ctx, n, fixed);
         ctx->ws.wsums.reserve((size_t)6 * 3 * MSM_MAX_WINDOWS * sizeof(xyzz_t));
         xyzz_t* d_parts = ctx->ws.wsums.as<xyzz_t>() + (size_t)(4 + si) * 3 * MSM_MAX_WINDOWS;  // slots 0-3 belong to msm_batch
         // the sort buffers of this slot were last read by the accumulation of the MSM two submits ago, which the caller
         // has collected (slot free) -- so the sort may start as soon as the scalars have arrived
         SortAhead ahead{&s.sort_ws, ctx->sort_stream, s.sorted, ctx->tune_sort_ahead};
-        msm_enqueue(ctx, in, s.plan, d_parts, 0, ahead_on ? &ahead : nullptr);
-        const int nwin = s.plan.fixed ? 1 : s.plan.W;
-        HALO_CUDA(cudaMemcpyAsync(s.h_parts, d_parts, (size_t)3 * nwin * sizeof(xyzz_t), cudaMemcpyDeviceToHost, ctx->stream));
+        msm_enqueue_to_host(ctx, gens_msm_input(ctx, fixed, d_scalars, off, n), s.plan, d_parts, s.h_parts, 0, ahead_on ? &ahead : nullptr);
         HALO_CUDA(cudaEventRecord(s.done, ctx->stream));
     }
     s.active = true;
@@ -963,10 +924,7 @@ int halo_msm(halo_ctx* ctx, const uint64_t* bases_affine, const uint8_t* inf_fla
         h2d_copy(ctx, ctx->stage_bases.p, bases_affine, n * sizeof(affine_t), ctx->stream);
         if (inf_flags) {
             ctx->stage_misc.reserve(n);
-            HALO_CUDA(cudaMemcpyAsync(ctx->stage_misc.p, inf_flags, n, cudaMemcpyHostToDevice, ctx->stream));
-            k_mark_infinity<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->stage_bases.as<affine_t>(),
-                                                                                 ctx->stage_misc.as<uint8_t>(), n);
-            ctx->kernel_launches++;
+            mark_infinity(ctx, ctx->stream, ctx->stage_bases.as<affine_t>(), ctx->stage_misc.as<uint8_t>(), inf_flags, n);
         }
     }
     xyzz_t r;
@@ -1067,27 +1025,12 @@ int halo_h_msm(halo_ctx* ctx, const uint64_t* xis, uint32_t lg_n, uint64_t out_j
     HALO_CATCH(ctx)
 }
 
-// <GS[0..n), d_scalars>: the FIXED-base tables under the same condition as msm_gens_device
-static MsmInput gens_input(halo_ctx* ctx, const fr_t* d_scalars, uint64_t n) {
-    MsmInput in;
-    in.scalars = d_scalars;
-    in.n = (uint32_t)n;
-    if (ctx->use_fixed && ctx->pre_n == ctx->n_gens && ctx->gens_pre.p && n >= (1u << 17) && n * 8 >= ctx->pre_n) {
-        in.bases = ctx->gens_pre.as<affine_t>();
-        in.fixed_stride = (uint32_t)ctx->pre_n;
-        in.fixed_first = 0;
-    } else {
-        in.bases = ctx->gens.as<affine_t>();
-    }
-    return in;
-}
-
 // <GS[0..n), stage_scalars> and the companion MSM sum_i scalars[i] * bases[i] (i < m, staged in stage_misc) on the two lanes
 // of msm_batch.
 static void h_msm_pair(halo_ctx* ctx, uint64_t n, const uint64_t* bases_affine, const uint8_t* inf_flags, const uint64_t* scalars,
                        uint64_t m, xyzz_t out[2]) {
     MsmInput in[2];
-    in[0] = gens_input(ctx, ctx->stage_scalars.as<fr_t>(), n);
+    in[0] = gens_msm_input(ctx, gens_use_fixed(ctx, n), ctx->stage_scalars.as<fr_t>(), 0, n);
     // companion: bases | scalars | infinity flags staged in stage_misc
     const size_t mm = m ? m : 1;
     ctx->stage_misc.reserve(mm * (sizeof(affine_t) + sizeof(fr_t) + 1));
@@ -1097,11 +1040,7 @@ static void h_msm_pair(halo_ctx* ctx, uint64_t n, const uint64_t* bases_affine, 
     if (m) {
         HALO_CUDA(cudaMemcpyAsync(d_b, bases_affine, m * sizeof(affine_t), cudaMemcpyHostToDevice, ctx->stream));
         HALO_CUDA(cudaMemcpyAsync(d_s, scalars, m * sizeof(fr_t), cudaMemcpyHostToDevice, ctx->stream));
-        if (inf_flags) {
-            HALO_CUDA(cudaMemcpyAsync(d_i, inf_flags, m, cudaMemcpyHostToDevice, ctx->stream));
-            k_mark_infinity<<<(unsigned)((m + 255) / 256), 256, 0, ctx->stream>>>(d_b, d_i, m);
-            ctx->kernel_launches++;
-        }
+        if (inf_flags) mark_infinity(ctx, ctx->stream, d_b, d_i, inf_flags, m);
     }
     in[1].bases = d_b;
     in[1].scalars = d_s;
@@ -1158,11 +1097,9 @@ int halo_h_msm_batch_submit(halo_ctx* ctx, const uint64_t* xis, const uint32_t* 
         b.scalars.reserve(n * sizeof(fr_t));
         vec_h_lincomb(ctx, reinterpret_cast<const fr_t*>(xis), lg_ns, reinterpret_cast<const fr_t*>(weights), k, n, false,
                       b.scalars.as<fr_t>());
-        const MsmInput in = gens_input(ctx, b.scalars.as<fr_t>(), n);
-        b.plan = in.fixed_stride ? ctx->pre_plan : msm_make_plan(n, ctx->force_c);
-        msm_enqueue(ctx, in, b.plan, b.parts.as<xyzz_t>(), 0);
-        const int nwin = b.plan.fixed ? 1 : b.plan.W;
-        HALO_CUDA(cudaMemcpyAsync(b.h_parts, b.parts.p, (size_t)3 * nwin * sizeof(xyzz_t), cudaMemcpyDeviceToHost, ctx->stream));
+        const bool fixed = gens_use_fixed(ctx, n);
+        b.plan = msm_plan(ctx, n, fixed);
+        msm_enqueue_to_host(ctx, gens_msm_input(ctx, fixed, b.scalars.as<fr_t>(), 0, n), b.plan, b.parts.as<xyzz_t>(), b.h_parts);
         HALO_CUDA(cudaEventRecord(b.done, ctx->stream));
     }
     b.active = true;
@@ -1188,19 +1125,13 @@ int halo_h_msm_batch_collect(halo_ctx* ctx, int ticket, const uint64_t* bases_af
         uint8_t* d_i = reinterpret_cast<uint8_t*>(d_s + m);
         HALO_CUDA(cudaMemcpyAsync(d_b, bases_affine, m * sizeof(affine_t), cudaMemcpyHostToDevice, ctx->stream2));
         HALO_CUDA(cudaMemcpyAsync(d_s, scalars, m * sizeof(fr_t), cudaMemcpyHostToDevice, ctx->stream2));
-        if (inf_flags) {
-            HALO_CUDA(cudaMemcpyAsync(d_i, inf_flags, m, cudaMemcpyHostToDevice, ctx->stream2));
-            k_mark_infinity<<<(unsigned)((m + 255) / 256), 256, 0, ctx->stream2>>>(d_b, d_i, m);
-            ctx->kernel_launches++;
-        }
+        if (inf_flags) mark_infinity(ctx, ctx->stream2, d_b, d_i, inf_flags, m);
         MsmInput in;
         in.bases = d_b;
         in.scalars = d_s;
         in.n = (uint32_t)m;
-        MsmPlan plan = msm_make_plan(m, ctx->force_c);
-        msm_enqueue(ctx, in, plan, b.parts.as<xyzz_t>() + HB_SLOT, 1);
-        HALO_CUDA(cudaMemcpyAsync(b.h_parts + HB_SLOT, b.parts.as<xyzz_t>() + HB_SLOT, (size_t)3 * plan.W * sizeof(xyzz_t),
-                                  cudaMemcpyDeviceToHost, ctx->stream2));
+        const MsmPlan plan = msm_plan(ctx, m, false);
+        msm_enqueue_to_host(ctx, in, plan, b.parts.as<xyzz_t>() + HB_SLOT, b.h_parts + HB_SLOT, 1);
         // the companion is the smaller MSM as a rule: its host finish overlaps the generator MSM
         HALO_CUDA(cudaStreamSynchronize(ctx->stream2));
         msm_finish_host(b.h_parts + HB_SLOT, plan, comp);
@@ -1208,16 +1139,7 @@ int halo_h_msm_batch_collect(halo_ctx* ctx, int ticket, const uint64_t* bases_af
     if (!b.empty) {
         HALO_CUDA(cudaEventSynchronize(b.done));
         msm_finish_host(b.h_parts, b.plan, gen);
-        if (ctx->profile) {  // phase timings of the generator MSM (lane 0)
-            float t[5];
-            for (int i = 0; i < 5; i++) HALO_CUDA(cudaEventElapsedTime(&t[i], ctx->ev[i], ctx->ev[i + 1]));
-            ctx->last.digits_ms = t[0];
-            ctx->last.scan_ms = t[1];
-            ctx->last.scatter_ms = t[2];
-            ctx->last.accumulate_ms = t[3];
-            ctx->last.reduce_ms = t[4];
-            HALO_CUDA(cudaEventElapsedTime(&ctx->last.total_ms, ctx->ev[0], ctx->ev[5]));
-        }
+        if (ctx->profile) msm_read_timings(ctx);  // the generator MSM (lane 0)
     }
     xyzz_add(gen, comp);
     out_jac_from_xyzz(gen, out_jac);
@@ -1266,12 +1188,7 @@ int halo_msm_multi(halo_ctx* ctx, const halo_msm_desc* descs, uint32_t count, ui
         if (d.bases_affine) {
             affine_t* d_b = reinterpret_cast<affine_t*>(take(d.n * sizeof(affine_t)));
             HALO_CUDA(cudaMemcpyAsync(d_b, d.bases_affine, d.n * sizeof(affine_t), cudaMemcpyHostToDevice, ctx->stream));
-            if (d.inf_flags) {
-                uint8_t* d_i = reinterpret_cast<uint8_t*>(take(d.n));
-                HALO_CUDA(cudaMemcpyAsync(d_i, d.inf_flags, d.n, cudaMemcpyHostToDevice, ctx->stream));
-                k_mark_infinity<<<(unsigned)((d.n + 255) / 256), 256, 0, ctx->stream>>>(d_b, d_i, d.n);
-                ctx->kernel_launches++;
-            }
+            if (d.inf_flags) mark_infinity(ctx, ctx->stream, d_b, reinterpret_cast<uint8_t*>(take(d.n)), d.inf_flags, d.n);
             ins[k].bases = d_b;
         } else {
             ins[k].bases = ctx->gens.as<affine_t>() + d.off;

@@ -165,15 +165,9 @@ void comm_alloc(halo_comm* c) {
 // The plan every rank uses for an MSM over `n_global` points: FIXED-base when every rank holds tables built with the
 // same window (halo_comm_precompute_generators) and the per-rank slice is large enough, else the variable-base plan of the
 // LARGEST slice -- a function of (n_global, size) only, hence identical on all ranks whatever their own slice length.
-bool comm_use_fixed(const halo_comm* c, uint64_t n_global) {
-    const halo_ctx* ctx = c->ctx;
+MsmPlan comm_plan(const halo_comm* c, uint64_t n_global) {
     const uint64_t slice = (n_global + c->size - 1) / c->size;
-    return ctx->use_fixed && ctx->pre_n == ctx->n_gens && ctx->pre_n != 0 && ctx->gens_pre.p && slice >= (1u << 17) && slice * 8 >= ctx->pre_n;
-}
-MsmPlan comm_plan(const halo_comm* c, uint64_t n_global, bool fixed) {
-    if (fixed) return c->ctx->pre_plan;
-    const uint64_t slice = (n_global + c->size - 1) / c->size;
-    return msm_make_plan(slice ? slice : 1, c->ctx->force_c);
+    return msm_plan(c->ctx, slice ? slice : 1, gens_use_fixed(c->ctx, slice));
 }
 
 // local MSM -> partials behind a header in `send` -> all-gather -> host: check headers, add the ranks' partials
@@ -189,12 +183,10 @@ struct LocalSlice {
 void sharded_msm(halo_comm* c, const LocalSlice* sl, int nsl, uint64_t n_global, xyzz_t& out) {
     halo_ctx* ctx = c->ctx;
     NcclApi* api = nccl_api();
-    const bool fixed = comm_use_fixed(c, n_global);
-    MsmPlan plan = comm_plan(c, n_global, fixed);
-    if (plan.red_quad != (ctx->tune_reduce_quad != 0)) plan_set_reduce(plan, ctx->tune_reduce_quad != 0);
-    const int nwin = plan.fixed ? 1 : plan.W;
-    if (1 + 3 * nwin * nsl > PART_SLOTS) throw NcclError{5, "too many windows for a sliced sharded MSM"};
-    const int used = 1 + 3 * nwin * nsl;
+    const MsmPlan plan = comm_plan(c, n_global);
+    const size_t parts = msm_parts(plan);
+    const size_t used = 1 + parts * nsl;
+    if (used > PART_SLOTS) throw NcclError{5, "too many windows for a sliced sharded MSM"};
     xyzz_t* d_send = c->send.as<xyzz_t>();
     cudaStream_t st = ctx->stream;
     PartHeader& h = *c->h_hdr;
@@ -204,7 +196,7 @@ void sharded_msm(halo_comm* c, const LocalSlice* sl, int nsl, uint64_t n_global,
     h.red_T = (uint32_t)plan.red_T, h.red_log_s = (uint32_t)plan.red_log_s, h.n_sets = (uint32_t)nsl;
     HALO_CUDA(cudaMemcpyAsync(d_send, &h, sizeof h, cudaMemcpyHostToDevice, st));
     for (int k = 0; k < nsl; k++) {
-        xyzz_t* d_parts = d_send + 1 + (size_t)3 * nwin * k;
+        xyzz_t* d_parts = d_send + 1 + parts * k;
         if (sl[k].h_src) {
             // the copy is issued here, slice by slice: staging a PAGEABLE slice blocks this thread, and the kernels of the
             // slices already enqueued run meanwhile
@@ -212,39 +204,27 @@ void sharded_msm(halo_comm* c, const LocalSlice* sl, int nsl, uint64_t n_global,
             HALO_CUDA(cudaEventRecord(sl[k].ready, ctx->copy_stream));
         }
         if (sl[k].ready) HALO_CUDA(cudaStreamWaitEvent(st, sl[k].ready, 0));
-        if (sl[k].n) {
-            MsmInput in;
-            in.scalars = sl[k].d_scalars;
-            in.n = (uint32_t)sl[k].n;
-            if (fixed) {
-                in.bases = ctx->gens_pre.as<affine_t>();
-                in.fixed_stride = (uint32_t)ctx->pre_n;
-                in.fixed_first = (uint32_t)sl[k].off;
-            } else {
-                in.bases = ctx->gens.as<affine_t>() + sl[k].off;
-            }
-            MsmPlan pk = plan;  // (msm_enqueue settles the reduction geometry in its argument: identical for every slice)
-            msm_enqueue(ctx, in, pk, d_parts, 0, nullptr);
-        } else {
-            HALO_CUDA(cudaMemsetAsync(d_parts, 0, (size_t)3 * nwin * sizeof(xyzz_t), st));  // zz = 0: infinity
-        }
+        if (sl[k].n)
+            msm_enqueue(ctx, gens_msm_input(ctx, plan.fixed, sl[k].d_scalars, sl[k].off, sl[k].n), plan, d_parts);
+        else
+            HALO_CUDA(cudaMemsetAsync(d_parts, 0, parts * sizeof(xyzz_t), st));  // zz = 0: infinity
     }
-    const size_t bytes = (size_t)used * sizeof(xyzz_t);
+    const size_t bytes = used * sizeof(xyzz_t);
     HALO_NCCL(api, AllGather(d_send, c->recv.p, bytes, NCCL_UINT8, c->comm, st));
     HALO_CUDA(cudaMemcpyAsync(c->h_recv, c->recv.p, bytes * c->size, cudaMemcpyDeviceToHost, st));
     HALO_CUDA(cudaStreamSynchronize(st));
     // rank r's block starts at h_recv + r * used
-    std::vector<xyzz_t> sum((size_t)3 * nwin);
+    std::vector<xyzz_t> sum(parts);
     for (auto& p : sum) xyzz_set_inf(p);
     for (int r = 0; r < c->size; r++) {
-        const xyzz_t* blk = c->h_recv + (size_t)r * used;
+        const xyzz_t* blk = c->h_recv + r * used;
         PartHeader hr;
         memcpy(&hr, blk, sizeof hr);
         if (hr.magic != PART_MAGIC || hr.c != h.c || hr.W != h.W || hr.fixed != h.fixed || hr.red_slabs != h.red_slabs ||
             hr.red_T != h.red_T || hr.red_log_s != h.red_log_s || hr.n_sets != h.n_sets)
             throw NcclError{5 /* ncclInvalidUsage */, "ranks disagree on the MSM plan (different n_global, tables, window or call on some rank)"};
         for (int k = 0; k < nsl; k++)
-            for (int j = 0; j < 3 * nwin; j++) xyzz_add(sum[j], blk[1 + (size_t)3 * nwin * k + j]);
+            for (size_t j = 0; j < parts; j++) xyzz_add(sum[j], blk[1 + parts * k + j]);
     }
     msm_finish_host(sum.data(), plan, out);
 }
@@ -381,11 +361,10 @@ int halo_msm_gens_sharded(halo_comm* c, const uint64_t* local_scalars, uint64_t 
     // the copies of the later slices run on the copy stream beside the kernels of the earlier ones.  The cuts are a function of
     // n_global and the communicator size only, so every rank makes the same number of slices whatever its own n_local.
     const uint64_t slice = (n_global + c->size - 1) / c->size;
-    const bool fixed = comm_use_fixed(c, n_global);
-    const int nwin = fixed ? 1 : comm_plan(c, n_global, false).W;
+    const size_t parts = msm_parts(comm_plan(c, n_global));
     const int a16 = ctx->tune_split_first_16ths, b16 = ctx->tune_split_second_16ths;
-    const int nsl = (b16 > 0 && a16 + b16 < 16 && 1 + 9 * nwin <= PART_SLOTS) ? 3 : 2;
-    if (ctx->tune_split_blocking > 0 && slice >= ((uint64_t)1 << ctx->tune_split_blocking) && 1 + 3 * nsl * nwin <= PART_SLOTS &&
+    const int nsl = (b16 > 0 && a16 + b16 < 16 && 1 + 3 * parts <= PART_SLOTS) ? 3 : 2;
+    if (ctx->tune_split_blocking > 0 && slice >= ((uint64_t)1 << ctx->tune_split_blocking) && 1 + nsl * parts <= PART_SLOTS &&
         !ctx->slots[0].active && !ctx->slots[1].active) {
         async_init(ctx);
         uint64_t cut[4] = {0, slice / 16 * (uint64_t)a16, nsl == 3 ? slice / 16 * (uint64_t)(a16 + b16) : n_local, n_local};

@@ -109,10 +109,6 @@ struct MsmPlan {
     uint32_t red_slabs = 0;
     bool red_quad = true;  // k_reduce_slabs_quad (quad-cooperative additions) or the one-lane k_reduce_slabs
 };
-void plan_set_reduce(MsmPlan& p, bool quad);
-MsmPlan msm_make_plan(uint64_t n, int force_c);
-// p (a one-segment plan) turned into the plan of `segs` segments of the same window
-void plan_set_segments(MsmPlan& p, uint32_t segs);
 
 struct MsmWorkspace {
     DevBuf counts, offsets, cursor, entries, buckets, wsums, scan_tmp;
@@ -249,7 +245,7 @@ struct halo_ctx {
     int tune_sort2_min_lg = 26;  // measured: 2^24 FIXED 6.15 -> 4.45 ms, 2^23 2.76 -> 2.31, 2^22 1.26 -> 1.29 (profiles/r02_sort2_v3_ab.jsonl)
     int tune_pair_bwd_async = 1;  // pass 0 of the pair tree: 1 = cp.async-staged operands + prefix loaded a step ahead (k_pair_bwd0, 5 CTAs per SM:
                                   // accumulation phase at 2^24 27.39 -> 26.75 ms; profiles/r02_pair_bwd_async_ab.jsonl), 0 = per-lane gathers
-    int tune_reduce_quad = 1;   // 0: one-lane bucket reduction (k_reduce_slabs), for A/B measurements
+    int tune_reduce_quad = 1;   // 0: one-lane bucket reduction (k_reduce_slabs), for A/B measurements; applied by msm_plan
     int tune_pair_passes = -1;  // -1: automatic; 0: XYZZ accumulation only; P > 0: force P pair-tree passes
     // what msm_enqueue chose for the last MSM on each lane (halo_test_msm_route, layout in include/halo_b200_test.h); host
     // bookkeeping only, written next to the decisions themselves

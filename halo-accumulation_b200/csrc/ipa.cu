@@ -368,7 +368,7 @@ static int ipa_begin_impl(halo_ctx* ctx, const uint64_t* coeffs, bool resident, 
         st->n = st->cur = n;
         while (((uint64_t)1 << st->lg_n) < n) st->lg_n++;
         // deferred head (k_fold_multi): pays when the L / R of the deferred rounds can take the FIXED-base path
-        st->fixed_ok = ctx->use_fixed && ctx->pre_n == ctx->n_gens && ctx->gens_pre.p && n >= (1u << 17) && n * 8 >= ctx->pre_n;
+        st->fixed_ok = gens_use_fixed(ctx, n);
         st->defer = ctx->tune_ipa_defer >= 0 ? ctx->tune_ipa_defer : (st->fixed_ok ? 3 : 0);
         if (st->defer > FOLD_MAX_DEFER) st->defer = FOLD_MAX_DEFER;
         if (st->defer > (int)st->lg_n) st->defer = (int)st->lg_n;
@@ -523,13 +523,8 @@ int halo_ipa_round_lr(halo_ipa* st, uint64_t L_jac[12], uint64_t R_jac[12]) {
         in[0].scalars = tL;
         in[1].bases = G;
         in[1].scalars = tR;
-        if (st->deferred && st->stage_over_gens && st->fixed_ok) {  // G is still GS[0..n): shared bucket set over the precomputed multiples
-            for (int k = 0; k < 2; k++) {
-                in[k].bases = ctx->gens_pre.as<affine_t>();
-                in[k].fixed_stride = (uint32_t)ctx->pre_n;
-                in[k].fixed_first = 0;
-            }
-        }
+        if (st->deferred && st->stage_over_gens && st->fixed_ok)  // G is still GS[0..n): shared bucket set over the precomputed multiples
+            for (int k = 0; k < 2; k++) in[k] = gens_msm_input(ctx, true, in[k].scalars, 0, st->M0);
     } else {
         in[0].bases = G;       // L = <c_r, g_l> + dot_l H'
         in[0].scalars = c + m;

@@ -32,7 +32,7 @@ namespace halo {
 // ------------------------------------------------------------------------------------------------
 // plan
 // ------------------------------------------------------------------------------------------------
-void plan_set_reduce(MsmPlan& p, bool quad);
+static void plan_set_reduce(MsmPlan& p, bool quad);
 static void plan_fill(MsmPlan& p, int c, bool fixed) {
     p.c = c;
     p.fixed = fixed;
@@ -46,7 +46,7 @@ static void plan_fill(MsmPlan& p, int c, bool fixed) {
 }
 // bucket reduction geometry: slabs of T * s buckets, T (logical) threads per CTA.  quad: k_reduce_slabs_quad (T <= 128
 // quads, slabs of up to 2048 buckets); else k_reduce_slabs (T <= 256 threads).
-void plan_set_reduce(MsmPlan& p, bool quad) {
+static void plan_set_reduce(MsmPlan& p, bool quad) {
     // Measured (scripts/gpu_reduce_probe.py, profiles/r02_reduce_*): the reduction of one slab is a job for ONE CTA, and a
     // CTA's arithmetic runs on one SM (~0.4 G multiplications/s): with a slab per window, a 22-window MSM of 2048 buckets
     // per window kept 22 of the 148 SMs busy for 0.3 ms.  So windows of >= 1024 buckets are cut into slabs until every SM
@@ -79,12 +79,6 @@ void plan_set_reduce(MsmPlan& p, bool quad) {
     p.red_slabs = p.M / (T << p.red_log_s);
 }
 
-void plan_set_segments(MsmPlan& p, uint32_t segs) {
-    p.NB = p.NB / p.segs * segs;
-    p.segs = segs;
-    plan_set_reduce(p, true);
-}
-
 static int ceil_lg(uint64_t n) {
     int l = 0;
     while (((uint64_t)1 << l) < n) l++;
@@ -94,7 +88,7 @@ static int ceil_lg(uint64_t n) {
 // Window widths below are the measured optima on B200 (scripts/gpu_msm_probe.py sweeps: profiles/r01_msm_window_sweep.txt,
 // re-measured with the two-level / quad-cooperative bucket reduction in profiles/r02_msm_window_sweep_variable.txt):
 // total cost = W * (n mixed adds) + bucket reduction (~2.5 full adds per bucket).
-MsmPlan msm_make_plan(uint64_t n, int force_c) {
+static MsmPlan msm_make_plan(uint64_t n, int force_c) {
     const int lg = ceil_lg(n);
     // (third sweep, with four lanes per bucket below 2^15 buckets and the pair-pass policy by bucket fill:
     // profiles/r02_msm_window_sweep_variable_v3.txt -- smaller windows pay once their buckets are full enough for tree passes)
@@ -117,6 +111,16 @@ MsmPlan msm_make_fixed_plan(uint64_t n, int force_c) {
     while ((double)(255 / c + 1) * (double)n >= 2147483648.0 && c < 24) c++;  // entry = index | sign << 31
     MsmPlan p;
     plan_fill(p, c, true);
+    return p;
+}
+
+// The reduction kernel is part of the plan (msm_finish_host undoes its slab geometry), so the reduce_quad knob is applied
+// here, once, and not where the plan is run.
+MsmPlan msm_plan(const halo_ctx* ctx, uint64_t n, bool fixed, int c, uint32_t segs) {
+    MsmPlan p = fixed ? ctx->pre_plan : msm_make_plan(n, c ? c : ctx->force_c);
+    p.NB *= segs;
+    p.segs = segs;
+    plan_set_reduce(p, ctx->tune_reduce_quad != 0);
     return p;
 }
 
@@ -1279,10 +1283,7 @@ void msm_precompute_tables(halo_ctx* ctx, int force_c) {
 // ------------------------------------------------------------------------------------------------
 // Device part of one MSM.  d_out receives 3 points per window (one "window" in FIXED mode): [E, A2, R2] with
 // window sum S = E + slab * (A2 - R2); a single-slab plan writes S into E and leaves A2 = R2 = infinity.
-void msm_enqueue(halo_ctx* ctx, const MsmInput& in, MsmPlan& plan, xyzz_t* d_out, int lane, const SortAhead* ahead) {
-    // the reduction kernel is part of the plan (its slab geometry is what msm_finish_host undoes): settle it here, in the
-    // caller's copy
-    if (plan.red_quad != (ctx->tune_reduce_quad != 0)) plan_set_reduce(plan, ctx->tune_reduce_quad != 0);
+void msm_enqueue(halo_ctx* ctx, const MsmInput& in, const MsmPlan& plan, xyzz_t* d_out, int lane, const SortAhead* ahead) {
     const uint32_t n = in.n;
     const uint32_t ntot = in.n + in.n_tail;
     // lane 0: the context's stream and workspace.  lane 1: a second stream and workspace, so two latency-bound MSMs of
@@ -1519,7 +1520,7 @@ void msm_enqueue(halo_ctx* ctx, const MsmInput& in, MsmPlan& plan, xyzz_t* d_out
         ctx->kernel_launches += 3;
     }
     mark(4);
-    HALO_CUDA(cudaMemsetAsync(d_out, 0, (size_t)3 * nwin * sizeof(xyzz_t), st));
+    HALO_CUDA(cudaMemsetAsync(d_out, 0, msm_parts(plan) * sizeof(xyzz_t), st));
     const bool quad = plan.red_quad;
     const int maxT = quad ? RQ_MAX_T : REDUCE_THREADS;
     auto reduce = [&](dim3 grid, int T, int log_s, const xyzz_t* src, const xyzz_t* extra, size_t stride, xyzz_t* oA, xyzz_t* oR, xyzz_t* oE,
@@ -1585,6 +1586,43 @@ void msm_finish_host(const xyzz_t* parts, const MsmPlan& plan, xyzz_t& out) {
     out = total;
 }
 
+void msm_enqueue_to_host(halo_ctx* ctx, const MsmInput& in, const MsmPlan& plan, xyzz_t* d_out, xyzz_t* h_out, int lane,
+                         const SortAhead* ahead) {
+    msm_enqueue(ctx, in, plan, d_out, lane, ahead);
+    HALO_CUDA(cudaMemcpyAsync(h_out, d_out, msm_parts(plan) * sizeof(xyzz_t), cudaMemcpyDeviceToHost, lane ? ctx->stream2 : ctx->stream));
+}
+
+void msm_read_timings(halo_ctx* ctx) {
+    float t[5];
+    for (int i = 0; i < 5; i++) HALO_CUDA(cudaEventElapsedTime(&t[i], ctx->ev[i], ctx->ev[i + 1]));
+    ctx->last.digits_ms = t[0];
+    ctx->last.scan_ms = t[1];
+    ctx->last.scatter_ms = t[2];
+    ctx->last.accumulate_ms = t[3];
+    ctx->last.reduce_ms = t[4];
+    HALO_CUDA(cudaEventElapsedTime(&ctx->last.total_ms, ctx->ev[0], ctx->ev[5]));
+}
+
+void host_parallel(size_t k, const std::function<void(size_t)>& f) {
+    const size_t hw = std::thread::hardware_concurrency();
+    const size_t T = std::min(k, std::max<size_t>(1, std::min<size_t>(hw, 16)));
+    std::vector<std::thread> th;
+    std::vector<size_t> unspawned;
+    auto work = [&](size_t t) {
+        for (size_t j = t; j < k; j += T) f(j);
+    };
+    for (size_t t = 1; t < T; t++) {
+        try {
+            th.emplace_back(work, t);
+        } catch (const std::system_error&) {
+            unspawned.push_back(t);  // no thread available: this thread takes that share as well (nothing may unwind across the ABI)
+        }
+    }
+    work(0);
+    for (size_t t : unspawned) work(t);
+    for (auto& x : th) x.join();
+}
+
 // Enqueue `count` MSMs back to back on the context stream (they share the workspace, so they serialise on the
 // stream), then one D2H of all partial sums, one synchronisation, and the host finish per MSM.
 void msm_batch(halo_ctx* ctx, const MsmInput* ins, int count, xyzz_t* outs, const std::function<void()>* while_running) {
@@ -1615,13 +1653,10 @@ void msm_batch(halo_ctx* ctx, const MsmInput* ins, int count, xyzz_t* outs, cons
     }
     for (int k = 0; k < count; k++) {
         if (ins[k].n + ins[k].n_tail == 0) continue;
-        plans[k] = ins[k].fixed_stride ? ctx->pre_plan : msm_make_plan(ins[k].n + ins[k].n_tail, ctx->force_c);
+        plans[k] = msm_plan(ctx, ins[k].n + ins[k].n_tail, ins[k].fixed_stride != 0);
         const int lane = two_lanes ? (k & 1) : 0;
-        cudaStream_t st = lane ? ctx->stream2 : ctx->stream;
-        msm_enqueue(ctx, ins[k], plans[k], d_parts + k * SLOT, lane);
+        msm_enqueue_to_host(ctx, ins[k], plans[k], d_parts + k * SLOT, h_parts + k * SLOT, lane);
         ctx->msm_route[lane][9] = two_lanes ? 1 : 0;
-        const int nwin = plans[k].fixed ? 1 : plans[k].W;
-        HALO_CUDA(cudaMemcpyAsync(h_parts + k * SLOT, d_parts + k * SLOT, (size_t)3 * nwin * sizeof(xyzz_t), cudaMemcpyDeviceToHost, st));
         any = true;
     }
     if (two_lanes) {
@@ -1639,19 +1674,10 @@ void msm_batch(halo_ctx* ctx, const MsmInput* ins, int count, xyzz_t* outs, cons
         early[1] = true;
     }
     if (any) HALO_CUDA(cudaStreamSynchronize(ctx->stream));
-    if (any && ctx->profile) {
-        float t[5];
-        for (int i = 0; i < 5; i++) HALO_CUDA(cudaEventElapsedTime(&t[i], ctx->ev[i], ctx->ev[i + 1]));
-        ctx->last.digits_ms = t[0];
-        ctx->last.scan_ms = t[1];
-        ctx->last.scatter_ms = t[2];
-        ctx->last.accumulate_ms = t[3];
-        ctx->last.reduce_ms = t[4];
-        HALO_CUDA(cudaEventElapsedTime(&ctx->last.total_ms, ctx->ev[0], ctx->ev[5]));
-    }
+    if (any && ctx->profile) msm_read_timings(ctx);
     // the Horner combination of a variable-base MSM is ~255 host doublings (~0.1 ms): the two results of an IPA round
     // (L and R) are finished on two host threads
-    auto finish = [&](int k) {
+    auto finish = [&](size_t k) {
         if (early[k]) return;
         if (ins[k].n + ins[k].n_tail == 0)
             xyzz_set_inf(outs[k]);
@@ -1661,26 +1687,10 @@ void msm_batch(halo_ctx* ctx, const MsmInput* ins, int count, xyzz_t* outs, cons
     // (the results of an IPA round, L and R, and the up to four small MSMs of a verifier batch: one host thread each)
     int heavy = 0;
     for (int k = 0; k < count; k++) heavy += ins[k].n + ins[k].n_tail > 0 && !plans[k].fixed;
-    if (count >= 2 && heavy == count) {
-        std::thread others[MAXB];
-        bool spawned[MAXB] = {false, false, false, false};
-        for (int k = 1; k < count; k++) {
-            try {
-                others[k] = std::thread(finish, k);
-                spawned[k] = true;
-            } catch (const std::system_error&) {  // no thread available: finished below (nothing may unwind across the ABI)
-            }
-        }
-        finish(0);
-        for (int k = 1; k < count; k++) {
-            if (spawned[k])
-                others[k].join();
-            else
-                finish(k);
-        }
-    } else {
+    if (count >= 2 && heavy == count)
+        host_parallel((size_t)count, finish);
+    else
         for (int k = 0; k < count; k++) finish(k);
-    }
 }
 
 void msm_device(halo_ctx* ctx, const affine_t* d_bases, const fr_t* d_scalars, uint64_t n, xyzz_t& out) {
@@ -1692,22 +1702,28 @@ void msm_device(halo_ctx* ctx, const affine_t* d_bases, const fr_t* d_scalars, u
 }
 
 // sum_i scalars[i] * G_{first+i} over the resident generators; takes the FIXED-base path when tables exist and the
-// problem is large enough to amortise the (n-independent) bucket reduction of the wide window.
+// problem is large enough to amortise the (n-independent) bucket reduction of the wide window.  (pre_n != 0: an MSM of n <=
+// n_gens points implies it, but the sharded MSM asks with a slice of n_global, which a rank's resident set need not cover.)
 bool gens_use_fixed(const halo_ctx* ctx, uint64_t n) {
-    return ctx->use_fixed && ctx->pre_n == ctx->n_gens && ctx->gens_pre.p && n >= (1u << 17) && n * 8 >= ctx->pre_n;
+    return ctx->use_fixed && ctx->pre_n == ctx->n_gens && ctx->pre_n != 0 && ctx->gens_pre.p && n >= (1u << 17) && n * 8 >= ctx->pre_n;
 }
 
-void msm_gens_device(halo_ctx* ctx, const fr_t* d_scalars, uint64_t first, uint64_t n, xyzz_t& out) {
+MsmInput gens_msm_input(const halo_ctx* ctx, bool fixed, const fr_t* scalars, uint64_t first, uint64_t n) {
     MsmInput in;
-    in.scalars = d_scalars;
+    in.scalars = scalars;
     in.n = (uint32_t)n;
-    if (gens_use_fixed(ctx, n)) {
+    if (fixed) {
         in.bases = ctx->gens_pre.as<affine_t>();
-        in.fixed_stride = ctx->pre_n;
+        in.fixed_stride = (uint32_t)ctx->pre_n;
         in.fixed_first = (uint32_t)first;
     } else {
         in.bases = ctx->gens.as<affine_t>() + first;
     }
+    return in;
+}
+
+void msm_gens_device(halo_ctx* ctx, const fr_t* d_scalars, uint64_t first, uint64_t n, xyzz_t& out) {
+    const MsmInput in = gens_msm_input(ctx, gens_use_fixed(ctx, n), d_scalars, first, n);
     msm_batch(ctx, &in, 1, &out);
 }
 

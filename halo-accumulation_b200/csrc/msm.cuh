@@ -24,8 +24,16 @@ struct MsmInput {
     const uint32_t* seg_off = nullptr;
 };
 MsmPlan msm_make_fixed_plan(uint64_t n, int force_c);
+// The plan of an MSM of n points: the FIXED-base tables' plan or the variable-base window of n points (c, else the context's
+// forced window, else the measured choice), over `segs` segments, with the context's reduction kernel.  Plans are final when
+// made: msm_enqueue and msm_finish_host read them as they are.
+MsmPlan msm_plan(const halo_ctx* ctx, uint64_t n, bool fixed, int c = 0, uint32_t segs = 1);
+// Window partials an MSM leaves in d_out: (E, A2, R2) per window (one window in FIXED mode) and segment, segment-major
+inline size_t msm_parts(const MsmPlan& p) { return (size_t)3 * (p.fixed ? 1 : p.W) * p.segs; }
 // FIXED base for an MSM of n points over the resident generators (tables present, enough points to amortise the wide window)
 bool gens_use_fixed(const halo_ctx* ctx, uint64_t n);
+// The MSM of n scalars over the resident generators G_first..: over their precomputed multiples when `fixed`
+MsmInput gens_msm_input(const halo_ctx* ctx, bool fixed, const fr_t* scalars, uint64_t first, uint64_t n);
 // Counting sort of an MSM ahead of its accumulation: own stream (high priority), own sort buffers, throttled grid.
 struct SortAhead {
     MsmWorkspace* ws;
@@ -33,9 +41,15 @@ struct SortAhead {
     cudaEvent_t sorted;
     int ctas_per_sm;  // 0: full grid
 };
-// Device part of one MSM: 3 partial points per window (and segment) into d_out (see msm.cu).
-// (`plan` is the caller's copy: the reduction geometry in it is settled here and read back by msm_finish_host)
-void msm_enqueue(halo_ctx* ctx, const MsmInput& in, MsmPlan& plan, xyzz_t* d_out, int lane = 0, const SortAhead* ahead = nullptr);
+// Device part of one MSM: its msm_parts(plan) partial points into d_out (see msm.cu).
+void msm_enqueue(halo_ctx* ctx, const MsmInput& in, const MsmPlan& plan, xyzz_t* d_out, int lane = 0, const SortAhead* ahead = nullptr);
+// msm_enqueue, then the copy of its partials from d_out to the pinned h_out on the lane's stream
+void msm_enqueue_to_host(halo_ctx* ctx, const MsmInput& in, const MsmPlan& plan, xyzz_t* d_out, xyzz_t* h_out, int lane = 0,
+                         const SortAhead* ahead = nullptr);
+// Phase timings of the last MSM on lane 0 under profiling (events recorded by msm_enqueue, complete) into ctx->last
+void msm_read_timings(halo_ctx* ctx);
+// f(0) .. f(k - 1) on up to 16 host threads (host finishes of variable-base MSMs: ~255 doublings each)
+void host_parallel(size_t k, const std::function<void(size_t)>& f);
 // First `passes` levels of the bucket sums as flat pairwise affine additions with batched inversion (msm_pairs.cu).
 const affine_t* pair_tree_enqueue(halo_ctx* ctx, MsmWorkspace& ws, cudaStream_t st, const MsmInput& in, const uint32_t* entries,
                                   const uint32_t* total_slots, uint64_t slots_max, int passes);
