@@ -78,6 +78,11 @@ def lib():
         _lib.halo_pcdl_open_batch.argtypes = [C.c_void_p, u64p, u64p, C.c_uint64, u64p, C.c_uint64, u64p, u64p, u64p, C.c_uint64,
                                               u64p, u64p, u64p, u64p, C.POINTER(EvalProof)]
         _lib.halo_pcdl_batch_claim.argtypes = [C.c_void_p, u64p, u64p, C.c_uint64, u64p, u64p, u64p]
+        _lib.halo_pcdl_open_multi.argtypes = [C.c_void_p, u64p, u64p, C.c_uint64, u64p, C.c_uint64, u64p, C.c_uint64, u64p, u64p,
+                                              C.c_uint64, u64p, u64p, u64p, C.c_uint64, u64p, u64p, u64p, u64p, u64p, u64p, u64p,
+                                              C.POINTER(EvalProof)]
+        _lib.halo_pcdl_multi_claim.argtypes = [C.c_void_p, u64p, C.c_uint64, u64p, C.c_uint64, u64p, u64p, u64p, C.c_uint64, u64p,
+                                               u64p, u64p, u64p, u64p]
         _lib.halo_pcdl_check_batch.argtypes = [C.c_void_p, C.POINTER(Instance), C.c_uint64, u64p, u64p]
         _lib.halo_acc_decider_batch.argtypes = [C.c_void_p, C.POINTER(Accumulator), C.c_uint64, u64p, u64p]
         _lib.halo_acc_verifier_batch.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(Instance), u64p, C.POINTER(Accumulator),

@@ -208,6 +208,8 @@ void halo_ctx_destroy(halo_ctx* ctx) {
     ctx->poly_dev.release();
     ctx->polys_dev.release();
     ctx->polys_off.release();
+    ctx->quot_dev.release();
+    ctx->quot_scratch.release();
     ctx->lincomb_claims.release();
     for (halo::DevBuf* b : {&ctx->combine_in, &ctx->combine_work, &ctx->combine_inv_scratch}) b->release();
     for (halo::DevBuf* b : {&ctx->ipa_G, &ctx->ipa_cs, &ctx->ipa_zs, &ctx->ipa_pbar, &ctx->ipa_tail, &ctx->ipa_frozen,
@@ -1271,30 +1273,54 @@ static bool reserve_or_nomem(DevBuf& b, size_t bytes) {
     }
 }
 
-int halo_poly_eval_many(halo_ctx* ctx, const uint64_t* coeffs, const uint64_t* n_coeffs, uint64_t k, uint64_t n, const uint64_t z[4],
-                        uint64_t* vs_out) {
-    if (!ctx || !n_coeffs || !z || !vs_out) return HALO_EINVAL;
-    if (k == 0 || (k >> 31)) return fail(ctx, HALO_EINVAL, "halo_poly_eval_many: k must be 1 .. 2^31 - 1");
-    if (n > ctx->n_gens) return fail(ctx, HALO_EINVAL, "halo_poly_eval_many: n exceeds the resident generators");
+// Validates k packed polynomials of at most n coefficients and uploads them into the pooled polys_dev; on success they are the
+// context's resident polynomials (polys_k, polys_n = the longest), the quotient of an earlier upload is gone.  The caller's
+// scratch, n_max * extra_per_poly + extra_fixed elements of stage_scalars, is reserved before anything is uploaded.
+static int poly_upload(halo_ctx* ctx, const char* fn, const uint64_t* coeffs, const uint64_t* n_coeffs, uint64_t k, uint64_t n,
+                       uint64_t extra_per_poly, uint64_t extra_fixed) {
+    std::string e(fn);
+    if (!ctx || !n_coeffs) return HALO_EINVAL;
+    if (k == 0 || (k >> 31)) return fail(ctx, HALO_EINVAL, (e + ": k must be 1 .. 2^31 - 1").c_str());
+    if (n > ctx->n_gens) return fail(ctx, HALO_EINVAL, (e + ": n exceeds the resident generators").c_str());
     std::vector<uint64_t> off(k + 1, 0);
     uint64_t n_max = 0;
     for (uint64_t j = 0; j < k; j++) {
-        if (n_coeffs[j] > n) return fail(ctx, HALO_EINVAL, "halo_poly_eval_many: a polynomial has more than n coefficients");
+        if (n_coeffs[j] > n) return fail(ctx, HALO_EINVAL, (e + ": a polynomial has more than n coefficients").c_str());
         off[j + 1] = off[j] + n_coeffs[j];  // k < 2^31 polynomials of at most n < 2^32 coefficients: no wrap
         n_max = std::max(n_max, n_coeffs[j]);
     }
     const uint64_t total = off[k];
     if (!coeffs && total) return HALO_EINVAL;
-    if (total > (UINT64_MAX >> 6)) return fail(ctx, HALO_ENOMEM, "halo_poly_eval_many: out of device memory");
-    ctx->polys_k = 0;  // the previous evaluation is gone from here on, whatever the outcome
+    if (total > (UINT64_MAX >> 6)) return fail(ctx, HALO_ENOMEM, (e + ": out of device memory").c_str());
+    ctx->polys_k = 0;  // the previous upload is gone from here on, whatever the outcome
+    ctx->quot_ready = false;
     HALO_TRY(ctx)
-    const uint32_t bps = vec_eval_many_blocks(k, n_max);
     if (!reserve_or_nomem(ctx->polys_dev, (total ? total : 1) * sizeof(fr_t)) ||
         !reserve_or_nomem(ctx->polys_off, (k + 1) * sizeof(uint64_t)) ||
-        !reserve_or_nomem(ctx->stage_scalars, (n_max + (uint64_t)bps * k + k) * sizeof(fr_t)))
-        return fail(ctx, HALO_ENOMEM, "halo_poly_eval_many: out of device memory");
+        !reserve_or_nomem(ctx->stage_scalars, (n_max * extra_per_poly + extra_fixed) * sizeof(fr_t) + 1))
+        return fail(ctx, HALO_ENOMEM, (e + ": out of device memory").c_str());
     HALO_CUDA(cudaMemcpyAsync(ctx->polys_off.p, off.data(), (k + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
     h2d_copy(ctx, ctx->polys_dev.p, coeffs, total * sizeof(fr_t), ctx->stream);
+    ctx->polys_k = k;
+    ctx->polys_n = n_max;
+    ctx->polys_starts = std::move(off);
+    HALO_CATCH(ctx)
+}
+
+int halo_poly_upload(halo_ctx* ctx, const uint64_t* coeffs, const uint64_t* n_coeffs, uint64_t k, uint64_t n) {
+    return poly_upload(ctx, "halo_poly_upload", coeffs, n_coeffs, k, n, 0, 0);
+}
+
+int halo_poly_eval_many(halo_ctx* ctx, const uint64_t* coeffs, const uint64_t* n_coeffs, uint64_t k, uint64_t n, const uint64_t z[4],
+                        uint64_t* vs_out) {
+    if (!ctx || !n_coeffs || !z || !vs_out) return HALO_EINVAL;
+    if (k == 0 || (k >> 31)) return fail(ctx, HALO_EINVAL, "halo_poly_eval_many: k must be 1 .. 2^31 - 1");
+    uint64_t n_max = 0;
+    for (uint64_t j = 0; j < k; j++) n_max = std::max(n_max, std::min(n_coeffs[j], n));
+    const uint32_t bps = vec_eval_many_blocks(k, n_max);
+    const int rc = poly_upload(ctx, "halo_poly_eval_many", coeffs, n_coeffs, k, n, 1, (uint64_t)bps * k + k);
+    if (rc) return rc;
+    HALO_TRY(ctx)
     fr_t zz;
     memcpy(&zz, z, 32);
     fr_t* pows = ctx->stage_scalars.as<fr_t>();
@@ -1304,8 +1330,6 @@ int halo_poly_eval_many(halo_ctx* ctx, const uint64_t* coeffs, const uint64_t* n
     vec_eval_many(ctx, ctx->polys_dev.as<fr_t>(), ctx->polys_off.as<uint64_t>(), k, n_max, pows, partials, vs);
     HALO_CUDA(cudaMemcpyAsync(vs_out, vs, k * sizeof(fr_t), cudaMemcpyDeviceToHost, ctx->stream));
     HALO_CUDA(cudaStreamSynchronize(ctx->stream));
-    ctx->polys_k = k;
-    ctx->polys_n = n_max;
     HALO_CATCH(ctx)
 }
 
@@ -1319,6 +1343,160 @@ int halo_poly_combine_resident(halo_ctx* ctx, const uint64_t alpha[4], uint64_t*
     fr_t a;
     memcpy(&a, alpha, 32);
     vec_poly_combine(ctx, ctx->polys_dev.as<fr_t>(), ctx->polys_off.as<uint64_t>(), ctx->polys_k, a, n, ctx->poly_dev.as<fr_t>());
+    ctx->poly_n = n;
+    *degree_out = device_degree(ctx, ctx->poly_dev.as<fr_t>(), n);
+    HALO_CATCH(ctx)
+}
+
+// ---- K3c: k polynomials opened at several points ---------------------------------------------------------------
+// Descriptors and scratch of one run of the K3c kernels, carved out of ctx->quot_scratch.  Points t < T each get a power
+// table; group g sums its terms (j, w) over the resident polynomials.
+struct QuotRun {
+    std::vector<QuotGroup> groups;
+    std::vector<QuotTerm> terms;
+    std::vector<fr_t> zthr;
+    QuotGroup* d_groups = nullptr;
+    QuotTerm* d_terms = nullptr;
+    fr_t *d_zthr = nullptr, *d_kloc = nullptr, *d_agg = nullptr, *d_kblk = nullptr, *d_rem = nullptr;
+};
+
+// One table per point; the points are checked by the caller
+static void quot_points(QuotRun& r, const uint64_t* zs, uint64_t T) {
+    r.zthr.resize(T * VEC_QUOT_ZTHR);
+    for (uint64_t t = 0; t < T; t++) {
+        fr_t z, zb;
+        memcpy(&z, zs + 4 * t, 32);
+        vec_quot_tables(z, zb, &r.zthr[t * VEC_QUOT_ZTHR]);
+    }
+}
+
+static QuotGroup quot_group(const uint64_t* zs, uint64_t t, const fr_t& s, uint32_t first, uint32_t count, const std::vector<fr_t>& zthr) {
+    QuotGroup g{};
+    memcpy(&g.z, zs + 4 * t, 32);
+    g.s = s;
+    fp_mul(g.zblk, zthr[t * VEC_QUOT_ZTHR + VEC_QUOT_ZTHR - 1], zthr[t * VEC_QUOT_ZTHR + 1]);
+    g.first = first;
+    g.count = count;
+    g.tab = (uint32_t)t;
+    return g;
+}
+
+static QuotTerm quot_term(const std::vector<uint64_t>& off, uint64_t j, const fr_t* w) {  // w = NULL: weight one
+    QuotTerm e{};
+    e.off = off[j];
+    e.len = off[j + 1] - off[j];
+    if (w) {
+        e.w = *w;
+    } else {
+        fp_one(e.w);
+        e.unit = 1;
+    }
+    return e;
+}
+
+// Reserves the scratch (false: no device memory) and uploads the descriptors
+static bool quot_stage(halo_ctx* ctx, QuotRun& r, uint64_t nblk, bool carries) {
+    const uint64_t G = r.groups.size();
+    auto al = [](uint64_t b) { return (b + 255) & ~(uint64_t)255; };
+    const uint64_t b_groups = al(G * sizeof(QuotGroup)), b_terms = al(r.terms.size() * sizeof(QuotTerm)),
+                   b_zthr = al(r.zthr.size() * sizeof(fr_t)), b_kloc = carries ? al(G * nblk * VEC_QUOT_ZTHR * sizeof(fr_t)) : 0,
+                   b_agg = al(G * nblk * sizeof(fr_t)), b_kblk = carries ? b_agg : 0, b_rem = al(G * sizeof(fr_t));
+    if (!reserve_or_nomem(ctx->quot_scratch, b_groups + b_terms + b_zthr + b_kloc + b_agg + b_kblk + b_rem)) return false;
+    char* p = static_cast<char*>(ctx->quot_scratch.p);
+    r.d_groups = reinterpret_cast<QuotGroup*>(p);
+    r.d_terms = reinterpret_cast<QuotTerm*>(p += b_groups);
+    r.d_zthr = reinterpret_cast<fr_t*>(p += b_terms);
+    r.d_kloc = carries ? reinterpret_cast<fr_t*>(p + b_zthr) : nullptr;
+    r.d_agg = reinterpret_cast<fr_t*>(p += b_zthr + b_kloc);
+    r.d_kblk = carries ? reinterpret_cast<fr_t*>(p + b_agg) : nullptr;
+    r.d_rem = reinterpret_cast<fr_t*>(p += b_agg + b_kblk);
+    HALO_CUDA(cudaMemcpyAsync(r.d_groups, r.groups.data(), G * sizeof(QuotGroup), cudaMemcpyHostToDevice, ctx->stream));
+    HALO_CUDA(cudaMemcpyAsync(r.d_terms, r.terms.data(), r.terms.size() * sizeof(QuotTerm), cudaMemcpyHostToDevice, ctx->stream));
+    HALO_CUDA(cudaMemcpyAsync(r.d_zthr, r.zthr.data(), r.zthr.size() * sizeof(fr_t), cudaMemcpyHostToDevice, ctx->stream));
+    return true;
+}
+
+static int check_queries(halo_ctx* ctx, const char* fn, const uint64_t* zs, uint64_t T, const uint64_t* q_poly, const uint64_t* q_point,
+                         uint64_t m) {
+    std::string e(fn);
+    if (!zs || !q_poly || !q_point) return fail(ctx, HALO_EINVAL, (e + ": NULL pointer").c_str());
+    if (T == 0 || T > HALO_MULTI_MAX_POINTS) return fail(ctx, HALO_EINVAL, (e + ": T must be 1 .. HALO_MULTI_MAX_POINTS").c_str());
+    if (m == 0 || (m >> 31)) return fail(ctx, HALO_EINVAL, (e + ": m must be 1 .. 2^31 - 1").c_str());
+    if (!ctx->polys_k) return fail(ctx, HALO_ESTATE, (e + ": no resident polynomials (call halo_poly_upload first)").c_str());
+    for (uint64_t i = 0; i < m; i++)
+        if (q_poly[i] >= ctx->polys_k || q_point[i] >= T) return fail(ctx, HALO_EINVAL, (e + ": a query index is out of range").c_str());
+    return HALO_OK;
+}
+
+int halo_poly_eval_queries(halo_ctx* ctx, const uint64_t* zs, uint64_t T, const uint64_t* q_poly, const uint64_t* q_point, uint64_t m,
+                           uint64_t* vs_out) {
+    if (!ctx || !vs_out) return HALO_EINVAL;
+    if (int rc = check_queries(ctx, "halo_poly_eval_queries", zs, T, q_poly, q_point, m)) return rc;
+    HALO_TRY(ctx)
+    const std::vector<uint64_t>& off = ctx->polys_starts;
+    QuotRun r;
+    quot_points(r, zs, T);
+    fr_t one;
+    fp_one(one);
+    for (uint64_t i = 0; i < m; i++) {
+        r.groups.push_back(quot_group(zs, q_point[i], one, (uint32_t)i, 1, r.zthr));
+        r.terms.push_back(quot_term(off, q_poly[i], nullptr));
+    }
+    const uint64_t n = ctx->polys_n, nblk = vec_quot_blocks(n);
+    if (!quot_stage(ctx, r, nblk, false)) return fail(ctx, HALO_ENOMEM, "halo_poly_eval_queries: out of device memory");
+    vec_quot_eval(ctx, ctx->polys_dev.as<fr_t>(), r.d_groups, (uint32_t)m, r.d_terms, r.d_zthr, n, r.d_agg, r.d_rem);
+    HALO_CUDA(cudaMemcpyAsync(vs_out, r.d_rem, m * sizeof(fr_t), cudaMemcpyDeviceToHost, ctx->stream));
+    HALO_CUDA(cudaStreamSynchronize(ctx->stream));
+    HALO_CATCH(ctx)
+}
+
+int halo_poly_quotient(halo_ctx* ctx, const uint64_t* zs, const uint64_t* scales, uint64_t T, const uint64_t* q_poly,
+                       const uint64_t* q_point, const uint64_t* weights, uint64_t m, uint64_t* rems_out, uint64_t Q_out[12]) {
+    if (!ctx || !scales || !weights || !rems_out || !Q_out) return HALO_EINVAL;
+    if (int rc = check_queries(ctx, "halo_poly_quotient", zs, T, q_poly, q_point, m)) return rc;
+    ctx->quot_ready = false;
+    HALO_TRY(ctx)
+    const std::vector<uint64_t>& off = ctx->polys_starts;
+    QuotRun r;
+    quot_points(r, zs, T);
+    for (uint64_t t = 0; t < T; t++) {  // point t's terms in query order
+        const uint32_t first = (uint32_t)r.terms.size();
+        for (uint64_t i = 0; i < m; i++)
+            if (q_point[i] == t) r.terms.push_back(quot_term(off, q_poly[i], reinterpret_cast<const fr_t*>(weights + 4 * i)));
+        fr_t s;
+        memcpy(&s, scales + 4 * t, 32);
+        r.groups.push_back(quot_group(zs, t, s, first, (uint32_t)r.terms.size() - first, r.zthr));
+    }
+    const uint64_t n = ctx->polys_n, nblk = vec_quot_blocks(n), n_q = n ? n - 1 : 0;
+    if (!quot_stage(ctx, r, nblk, true) || !reserve_or_nomem(ctx->quot_dev, (n_q ? n_q : 1) * sizeof(fr_t)))
+        return fail(ctx, HALO_ENOMEM, "halo_poly_quotient: out of device memory");
+    vec_quotient(ctx, ctx->polys_dev.as<fr_t>(), r.d_groups, (uint32_t)T, r.d_terms, r.d_zthr, n, r.d_kloc, r.d_agg, r.d_kblk, r.d_rem,
+                 ctx->quot_dev.as<fr_t>());
+    std::vector<fr_t> rems(T);
+    HALO_CUDA(cudaMemcpyAsync(rems.data(), r.d_rem, T * sizeof(fr_t), cudaMemcpyDeviceToHost, ctx->stream));
+    xyzz_t Q;
+    msm_gens_device(ctx, ctx->quot_dev.as<fr_t>(), 0, n_q, Q);  // synchronises the stream
+    memcpy(rems_out, rems.data(), T * sizeof(fr_t));
+    out_jac_from_xyzz(Q, Q_out);
+    ctx->quot_n = n_q;
+    ctx->quot_ready = true;
+    HALO_CATCH(ctx)
+}
+
+int halo_poly_lincomb_resident(halo_ctx* ctx, const uint64_t* cs, const uint64_t c_q[4], uint64_t* degree_out) {
+    if (!ctx || !cs || !c_q || !degree_out) return HALO_EINVAL;
+    if (!ctx->polys_k || !ctx->quot_ready)
+        return fail(ctx, HALO_ESTATE, "halo_poly_lincomb_resident: no quotient of the resident polynomials (call halo_poly_quotient first)");
+    HALO_TRY(ctx)
+    const uint64_t n = ctx->polys_n ? ctx->polys_n : 1;
+    ctx->poly_n = 0;
+    if (!reserve_or_nomem(ctx->poly_dev, n * sizeof(fr_t)) || !reserve_or_nomem(ctx->stage_scalars, ctx->polys_k * sizeof(fr_t)))
+        return fail(ctx, HALO_ENOMEM, "halo_poly_lincomb_resident: out of device memory");
+    HALO_CUDA(cudaMemcpyAsync(ctx->stage_scalars.p, cs, ctx->polys_k * sizeof(fr_t), cudaMemcpyHostToDevice, ctx->stream));
+    fr_t cq;
+    memcpy(&cq, c_q, 32);
+    vec_poly_lincomb(ctx, ctx->polys_dev.as<fr_t>(), ctx->polys_off.as<uint64_t>(), ctx->stage_scalars.as<fr_t>(), ctx->polys_k,
+                     ctx->quot_dev.as<fr_t>(), ctx->quot_n, cq, n, ctx->poly_dev.as<fr_t>());
     ctx->poly_n = n;
     *degree_out = device_degree(ctx, ctx->poly_dev.as<fr_t>(), n);
     HALO_CATCH(ctx)

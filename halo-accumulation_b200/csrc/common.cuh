@@ -165,10 +165,16 @@ struct halo_ctx {
     halo::DevBuf lincomb_claims;  // claim descriptors of vec_h_lincomb
     halo::DevBuf combine_in, combine_work, combine_inv_scratch;  // k_point_combine (combine.cu): inputs, work and outputs, inversions
     uint64_t poly_n = 0;
-    // halo_poly_eval_many: the k uploaded polynomials and their k + 1 segment starts, kept for halo_poly_combine_resident
-    // (polys_k = 0: no evaluation to combine); polys_n = the longest of them
+    // halo_poly_upload / halo_poly_eval_many: the k uploaded polynomials and their k + 1 segment starts, kept for the
+    // evaluations, the quotient and the combinations (polys_k = 0: none resident); polys_n = the longest of them
     halo::DevBuf polys_dev, polys_off;
     uint64_t polys_k = 0, polys_n = 0;
+    std::vector<uint64_t> polys_starts;  // host copy of polys_off
+    // halo_poly_quotient: q of the resident polynomials, kept for halo_poly_lincomb_resident (quot_ready: q belongs to the
+    // current upload), and the scratch of the K3c kernels (descriptors, carries)
+    halo::DevBuf quot_dev, quot_scratch;
+    uint64_t quot_n = 0;
+    bool quot_ready = false;
     // buffers of the (single) in-flight PCDL opening, kept across openings: cudaMalloc / cudaFree of 100+ MB per open
     // costs tens of milliseconds
     halo::DevBuf ipa_G, ipa_cs, ipa_zs, ipa_pbar, ipa_tail, ipa_frozen;

@@ -492,4 +492,16 @@ int halo_test_h_lincomb_bench(halo_ctx* ctx, uint32_t lg_n, uint64_t k, float* m
     a.release();
     T_CATCH(ctx)
 }
+
+int halo_test_read_quotient(halo_ctx* ctx, uint64_t* out, uint64_t cap, uint64_t* n_out) {
+    if (!ctx || !n_out || (!out && cap)) return HALO_EINVAL;
+    if (!ctx->quot_ready) return HALO_ESTATE;
+    T_TRY(ctx)
+    *n_out = ctx->quot_n;
+    if (cap >= ctx->quot_n && ctx->quot_n) {
+        HALO_CUDA(cudaMemcpyAsync(out, ctx->quot_dev.p, ctx->quot_n * sizeof(fr_t), cudaMemcpyDeviceToHost, ctx->stream));
+        HALO_CUDA(cudaStreamSynchronize(ctx->stream));
+    }
+    T_CATCH(ctx)
+}
 }

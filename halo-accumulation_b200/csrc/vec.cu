@@ -10,6 +10,8 @@
 //   (batch decider)  sum_j w_j coeffs(h_j) over claims of mixed size -> k_h_lincomb (DESIGN.md K5b)
 //   pcdl.rs:140-142,156  p_bar = q (X - z), p' = p + alpha p_bar -> k_pbar, k_axpy
 //   (batch opening)  p_j(z) of k polynomials, sum_j alpha^j p_j   -> k_poly_eval_many + k_poly_eval_final, k_poly_combine (K3b)
+//   (multi-point opening) sum_t s_t (f_t - f_t(z_t)) / (X - z_t), p_j(z_t) of m queries, sum_j c_j p_j + c_q q
+//                    -> k_quot_chunks + k_quot_carry (+ k_quot_write), k_poly_lincomb (K3c)
 #include "common.cuh"
 #include "vec.cuh"
 
@@ -159,6 +161,225 @@ void vec_poly_combine(halo_ctx* ctx, const fr_t* d_coeffs, const uint64_t* d_off
                       fr_t* d_out) {
     k_poly_combine<<<(unsigned)((n + VEC_THREADS - 1) / VEC_THREADS), VEC_THREADS, 0, ctx->stream>>>(d_coeffs, d_off, (uint32_t)k,
                                                                                                      alpha, n, d_out);
+    ctx->kernel_launches++;
+    HALO_CUDA(cudaGetLastError());
+}
+
+// ---- K3c: division by X - z and evaluation, as a chunked scan ---------------------------------------------------------
+// A group is g = sum of its terms w p_j (coefficients synthesised on the fly, never stored).  The quotient h = g / (X - z)
+// obeys h_{i-1} = g_i + z h_i from the top down; the remainder is g(z).  A thread owns QB consecutive coefficients (its chunk
+// c), a block QT chunks:
+//   k_quot_chunks: S_c = sum_l g_{cB+l} z^l (Horner), then a block suffix scan gives the carry into each chunk from the chunks
+//                  above it in the block (kloc) and the block's aggregate (agg);
+//   k_quot_carry:  one block per group scans the aggregates: the carry into each block (kblk) and g(z) = the full suffix (rem);
+//   k_quot_write:  each chunk starts from its carry kloc + z^(QB (QT - 1 - t)) kblk and writes h downward; q (+)= s h.
+// Evaluation is the first two kernels without kloc / kblk.
+constexpr int QB = 16;
+constexpr int QT = 256;
+
+__device__ __forceinline__ void quot_synth(fr_t& g, const fr_t* __restrict__ coeffs, const QuotTerm* __restrict__ terms,
+                                           uint32_t first, uint32_t count, uint64_t i) {
+    fp_zero(g);
+#pragma unroll 1
+    for (uint32_t e = first; e < first + count; e++) {
+        const QuotTerm& tm = terms[e];
+        if (i >= tm.len) continue;
+        if (tm.unit) {
+            fp_add(g, g, coeffs[tm.off + i]);
+        } else {
+            fr_t t;
+            fp_mul(t, coeffs[tm.off + i], tm.w);
+            fp_add(g, g, t);
+        }
+    }
+}
+
+// In-block inclusive suffix scan of v over the QT threads: v_t <- sum_{u >= t} v_u Z^(u - t), where pw[d] = Z^d for d < QT
+__device__ __forceinline__ void block_suffix_scan(fr_t& v, fr_t* sm, const fr_t* __restrict__ pw) {
+    const int t = threadIdx.x;
+    sm[t] = v;
+    __syncthreads();
+#pragma unroll 1
+    for (int d = 1; d < QT; d <<= 1) {
+        fr_t o;
+        const bool has = t + d < QT;
+        if (has) {
+            fp_mul(o, sm[t + d], pw[d]);
+            fp_add(v, v, o);
+        }
+        __syncthreads();
+        sm[t] = v;
+        __syncthreads();
+    }
+}
+
+__global__ void __launch_bounds__(QT) k_quot_chunks(const fr_t* __restrict__ coeffs, const QuotGroup* __restrict__ groups,
+                                                    const QuotTerm* __restrict__ terms, const fr_t* __restrict__ zthr,
+                                                    uint32_t nblk, fr_t* __restrict__ kloc, fr_t* __restrict__ agg) {
+    __shared__ fr_t sm[QT];
+    const uint32_t g = blockIdx.x / nblk, b = blockIdx.x % nblk;
+    const QuotGroup& gr = groups[g];
+    const fr_t z = gr.z;
+    const uint64_t lo = ((uint64_t)b * QT + threadIdx.x) * QB;
+    fr_t acc, x;
+    fp_zero(acc);
+#pragma unroll 1
+    for (int l = QB - 1; l >= 0; l--) {
+        quot_synth(x, coeffs, terms, gr.first, gr.count, lo + l);
+        fp_mul(acc, acc, z);
+        fp_add(acc, acc, x);
+    }
+    const fr_t* pw = zthr + (uint64_t)gr.tab * QT;
+    block_suffix_scan(acc, sm, pw);
+    if (kloc) {
+        fr_t c;
+        if (threadIdx.x + 1 < QT)
+            c = sm[threadIdx.x + 1];
+        else
+            fp_zero(c);
+        kloc[(uint64_t)g * nblk * QT + (uint64_t)b * QT + threadIdx.x] = c;
+    }
+    if (threadIdx.x == 0) agg[(uint64_t)g * nblk + b] = acc;
+}
+
+__global__ void __launch_bounds__(QT) k_quot_carry(const QuotGroup* __restrict__ groups, const fr_t* __restrict__ agg, uint32_t nblk,
+                                                   fr_t* __restrict__ kblk, fr_t* __restrict__ rem) {
+    __shared__ fr_t sm[QT];
+    __shared__ fr_t pw[QT];
+    const uint32_t g = blockIdx.x, t = threadIdx.x;
+    const fr_t zb = groups[g].zblk;  // z^(QB QT): one block's span
+    const fr_t* a = agg + (uint64_t)g * nblk;
+    const uint32_t r = (nblk + QT - 1) / QT, lo = t * r, hi = min(lo + r, nblk);
+    fr_t acc;
+    fp_zero(acc);
+#pragma unroll 1
+    for (uint32_t i = hi; i-- > lo;) {
+        fp_mul(acc, acc, zb);
+        fp_add(acc, acc, a[i]);
+    }
+    if (t == 0) {  // pw[d] = zb^(r d): the distance of d runs
+        fr_t m, e;
+        fp_one(m);
+        e = zb;
+        for (uint32_t s = r; s; s >>= 1) {
+            if (s & 1) fp_mul(m, m, e);
+            fp_sqr(e, e);
+        }
+        fp_one(e);
+        for (int d = 0; d < QT; d++) {
+            pw[d] = e;
+            fp_mul(e, e, m);
+        }
+    }
+    __syncthreads();
+    block_suffix_scan(acc, sm, pw);
+    if (t == 0) rem[g] = acc;
+    if (!kblk) return;
+    fr_t c;
+    if (t + 1 < QT)
+        c = sm[t + 1];
+    else
+        fp_zero(c);
+#pragma unroll 1
+    for (uint32_t i = hi; i-- > lo;) {
+        kblk[(uint64_t)g * nblk + i] = c;
+        fp_mul(c, c, zb);
+        fp_add(c, c, a[i]);
+    }
+}
+
+__global__ void __launch_bounds__(QT) k_quot_write(const fr_t* __restrict__ coeffs, const QuotGroup* __restrict__ groups,
+                                                   uint32_t n_groups, const QuotTerm* __restrict__ terms, const fr_t* __restrict__ zthr,
+                                                   uint32_t nblk, const fr_t* __restrict__ kloc, const fr_t* __restrict__ kblk,
+                                                   uint64_t n_q, fr_t* __restrict__ q) {
+    const uint32_t b = blockIdx.x, t = threadIdx.x;
+    const uint64_t lo = ((uint64_t)b * QT + t) * QB;
+    if (lo >= n_q) return;
+#pragma unroll 1
+    for (uint32_t g = 0; g < n_groups; g++) {
+        const QuotGroup& gr = groups[g];
+        const fr_t z = gr.z, s = gr.s;
+        fr_t acc, x, o;
+        fp_mul(acc, kblk[(uint64_t)g * nblk + b], zthr[(uint64_t)gr.tab * QT + (QT - 1 - t)]);
+        fp_add(acc, acc, kloc[(uint64_t)g * nblk * QT + (uint64_t)b * QT + t]);  // h_{lo + QB - 1}
+#pragma unroll 1
+        for (int l = QB - 1; l >= 0; l--) {
+            const uint64_t i = lo + l;  // acc = h_i
+            if (i < n_q) {
+                fp_mul(o, acc, s);
+                if (g) fp_add(o, o, q[i]);
+                q[i] = o;
+            }
+            if (l) {
+                quot_synth(x, coeffs, terms, gr.first, gr.count, i);
+                fp_mul(acc, acc, z);
+                fp_add(acc, acc, x);
+            }
+        }
+    }
+}
+
+uint32_t vec_quot_blocks(uint64_t n) {
+    const uint64_t b = (n + (uint64_t)QB * QT - 1) / ((uint64_t)QB * QT);
+    return b ? (uint32_t)b : 1;
+}
+
+void vec_quot_tables(const fr_t& z, fr_t& zblk, fr_t* zthr) {
+    fr_t zq = z;
+    for (int i = 1; i < QB; i <<= 1) fp_sqr(zq, zq);  // z^QB (QB a power of two)
+    fp_one(zthr[0]);
+    for (int u = 1; u < QT; u++) fp_mul(zthr[u], zthr[u - 1], zq);
+    fp_mul(zblk, zthr[QT - 1], zq);
+}
+
+void vec_quot_eval(halo_ctx* ctx, const fr_t* d_coeffs, const QuotGroup* d_groups, uint32_t n_groups, const QuotTerm* d_terms,
+                   const fr_t* d_zthr, uint64_t n, fr_t* d_agg, fr_t* d_rem) {
+    const uint32_t nblk = vec_quot_blocks(n);
+    k_quot_chunks<<<(unsigned)((uint64_t)n_groups * nblk), QT, 0, ctx->stream>>>(d_coeffs, d_groups, d_terms, d_zthr, nblk, nullptr,
+                                                                                 d_agg);
+    k_quot_carry<<<n_groups, QT, 0, ctx->stream>>>(d_groups, d_agg, nblk, nullptr, d_rem);
+    ctx->kernel_launches += 2;
+    HALO_CUDA(cudaGetLastError());
+}
+
+void vec_quotient(halo_ctx* ctx, const fr_t* d_coeffs, const QuotGroup* d_groups, uint32_t n_groups, const QuotTerm* d_terms,
+                  const fr_t* d_zthr, uint64_t n, fr_t* d_kloc, fr_t* d_agg, fr_t* d_kblk, fr_t* d_rem, fr_t* d_q) {
+    const uint32_t nblk = vec_quot_blocks(n);
+    k_quot_chunks<<<(unsigned)((uint64_t)n_groups * nblk), QT, 0, ctx->stream>>>(d_coeffs, d_groups, d_terms, d_zthr, nblk, d_kloc,
+                                                                                 d_agg);
+    k_quot_carry<<<n_groups, QT, 0, ctx->stream>>>(d_groups, d_agg, nblk, d_kblk, d_rem);
+    ctx->kernel_launches += 2;
+    if (n > 1) {
+        k_quot_write<<<nblk, QT, 0, ctx->stream>>>(d_coeffs, d_groups, n_groups, d_terms, d_zthr, nblk, d_kloc, d_kblk, n - 1, d_q);
+        ctx->kernel_launches++;
+    }
+    HALO_CUDA(cudaGetLastError());
+}
+
+// out[i] = sum_j c_j p_j[i] + c_q q[i] (p_j[i] = 0 from off[j+1] - off[j] on, q[i] = 0 from n_q on)
+__global__ void __launch_bounds__(VEC_THREADS) k_poly_lincomb(const fr_t* __restrict__ coeffs, const uint64_t* __restrict__ off,
+                                                              const fr_t* __restrict__ cs, uint32_t k, const fr_t* __restrict__ q,
+                                                              uint64_t n_q, fr_t c_q, uint64_t n, fr_t* __restrict__ out) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    fr_t acc, t;
+    fp_zero(acc);
+    if (i < n_q) fp_mul(acc, q[i], c_q);
+#pragma unroll 1
+    for (uint32_t j = 0; j < k; j++) {
+        const uint64_t o = off[j];
+        if (i < off[j + 1] - o) {
+            fp_mul(t, coeffs[o + i], cs[j]);
+            fp_add(acc, acc, t);
+        }
+    }
+    out[i] = acc;
+}
+
+void vec_poly_lincomb(halo_ctx* ctx, const fr_t* d_coeffs, const uint64_t* d_off, const fr_t* d_cs, uint64_t k, const fr_t* d_q,
+                      uint64_t n_q, const fr_t& c_q, uint64_t n, fr_t* d_out) {
+    k_poly_lincomb<<<(unsigned)((n + VEC_THREADS - 1) / VEC_THREADS), VEC_THREADS, 0, ctx->stream>>>(d_coeffs, d_off, d_cs, (uint32_t)k,
+                                                                                                     d_q, n_q, c_q, n, d_out);
     ctx->kernel_launches++;
     HALO_CUDA(cudaGetLastError());
 }

@@ -165,6 +165,82 @@ int halo_pcdl_batch_claim(halo_ctx* ctx, const uint64_t* Cs, const uint64_t* vs,
     });
 }
 
+// The caller's points and queries of a multi-point opening (validated in pcdl::multi_validate)
+static void multi_inputs(const uint64_t* zs, uint64_t T, const uint64_t* q_poly, const uint64_t* q_point, uint64_t m,
+                         std::vector<PallasScalar>& z, std::vector<uint64_t>& qp, std::vector<uint64_t>& qt) {
+    z.resize(T);
+    for (uint64_t t = 0; t < T; t++) z[t] = scalar_load_checked(zs + 4 * t, "z_t is not a canonical scalar");
+    qp.assign(q_poly, q_poly + m);
+    qt.assign(q_point, q_point + m);
+}
+
+int halo_pcdl_open_multi(halo_ctx* ctx, const uint64_t* coeffs, const uint64_t* n_coeffs, uint64_t k, const uint64_t* Cs, uint64_t d,
+                         const uint64_t* zs, uint64_t T, const uint64_t* q_poly, const uint64_t* q_point, uint64_t m, const uint64_t* ws,
+                         const uint64_t* w_Q, const uint64_t* q, uint64_t n_q, const uint64_t* w_bar, uint64_t* vs_out, uint64_t Q_out[12],
+                         uint64_t* us_out, uint64_t C_out[12], uint64_t x_out[4], uint64_t v_out[4], halo_eval_proof* pi) {
+    return guarded([&] {
+        ensure(k >= 1 && T >= 1 && m >= 1, HALO_EINVAL, "halo_pcdl_open_multi: k, T and m must be at least 1");
+        ensure(n_coeffs && Cs && zs && q_poly && q_point && vs_out && Q_out && us_out && C_out && x_out && v_out && pi, HALO_EINVAL,
+               "halo_pcdl_open_multi: NULL pointer");
+        std::vector<PolyView> ps;
+        std::vector<PallasPoint> C(k);
+        std::vector<PallasScalar> w(ws ? k : 0);
+        ps.reserve(k);
+        uint64_t off = 0;
+        for (uint64_t j = 0; j < k; j++) {
+            ensure(n_coeffs[j] <= UINT64_MAX / 32 - off, HALO_EINVAL, "halo_pcdl_open_multi: packed size overflows");
+            ps.push_back(poly_from(coeffs + 4 * off, n_coeffs[j]));
+            off += n_coeffs[j];
+        }
+        ensure(coeffs || off == 0, HALO_EINVAL, "halo_pcdl_open_multi: NULL coefficients");
+        for (uint64_t j = 0; j < k; j++) {
+            C[j] = point_load_checked(Cs + 12 * j, "C_j is not a canonical point on the curve");
+            if (ws) w[j] = scalar_load_checked(ws + 4 * j, "w_j is not a canonical scalar");
+        }
+        std::vector<PallasScalar> z;
+        std::vector<uint64_t> qp, qt;
+        multi_inputs(zs, T, q_poly, q_point, m, z, qp, qt);
+        PallasScalar wq, wbs;
+        PolyView qv(nullptr, 0);
+        if (ws) {
+            ensure(w_Q && w_bar && (q || n_q == 0), HALO_EINVAL, "hiding open needs w_Q, q and w_bar");
+            wq = scalar_load_checked(w_Q, "w_Q is not a canonical scalar");
+            wbs = scalar_load_checked(w_bar, "w_bar is not a canonical scalar");
+            qv = poly_from(q, n_q);
+        }
+        const pcdl::MultiOpening r = pcdl::open_multi(ctx, ps, C, d, z, qp, qt, ws ? w.data() : nullptr, ws ? &wq : nullptr,
+                                                      ws ? &qv : nullptr, ws ? &wbs : nullptr);
+        for (uint64_t i = 0; i < m; i++) scalar_store(vs_out + 4 * i, r.vs[i]);
+        point_store(Q_out, r.Q);
+        for (uint64_t t = 0; t < T; t++) scalar_store(us_out + 4 * t, r.us[t]);
+        point_store(C_out, r.claim.C);
+        scalar_store(x_out, r.claim.x3);
+        scalar_store(v_out, r.claim.v);
+        pcdl::proof_to_c(r.pi, *pi);
+    });
+}
+
+int halo_pcdl_multi_claim(halo_ctx* ctx, const uint64_t* Cs, uint64_t k, const uint64_t* zs, uint64_t T, const uint64_t* q_poly,
+                          const uint64_t* q_point, const uint64_t* vs, uint64_t m, const uint64_t Q[12], const uint64_t* us,
+                          uint64_t C_out[12], uint64_t x_out[4], uint64_t v_out[4]) {
+    return guarded([&] {
+        ensure(k >= 1 && T >= 1 && m >= 1, HALO_EINVAL, "halo_pcdl_multi_claim: k, T and m must be at least 1");
+        ensure(Cs && zs && q_poly && q_point && vs && Q && us && C_out && x_out && v_out, HALO_EINVAL, "halo_pcdl_multi_claim: NULL pointer");
+        std::vector<PallasPoint> C(k);
+        for (uint64_t j = 0; j < k; j++) C[j] = point_load_checked(Cs + 12 * j, "C_j is not a canonical point on the curve");
+        std::vector<PallasScalar> z, v(m), u(T);
+        std::vector<uint64_t> qp, qt;
+        multi_inputs(zs, T, q_poly, q_point, m, z, qp, qt);
+        for (uint64_t i = 0; i < m; i++) v[i] = scalar_load_checked(vs + 4 * i, "v_i is not a canonical scalar");
+        const PallasPoint Qp = point_load_checked(Q, "Q is not a canonical point on the curve");
+        for (uint64_t t = 0; t < T; t++) u[t] = scalar_load_checked(us + 4 * t, "u_t is not a canonical scalar");
+        const pcdl::MultiClaim r = pcdl::multi_claim(ctx, C, z, qp, qt, v, Qp, u);
+        point_store(C_out, r.C);
+        scalar_store(x_out, r.x3);
+        scalar_store(v_out, r.v);
+    });
+}
+
 int halo_pcdl_succinct_check(halo_ctx* ctx, const uint64_t C_jac[12], uint64_t d, const uint64_t z[4], const uint64_t v[4],
                              const halo_eval_proof* pi, uint64_t* xis_out, uint64_t U_out[12]) {
     return guarded([&] {

@@ -189,6 +189,166 @@ BatchOpening open_batch(halo_ctx* ctx, const std::vector<PolyView>& ps, const st
     return r;
 }
 
+// ---- K3c: several points -------------------------------------------------------------------------------------------
+// Every point and polynomial in some query, points distinct, no (j, t) pair twice
+static void multi_validate(size_t k, const std::vector<PallasScalar>& zs, const std::vector<uint64_t>& q_poly,
+                           const std::vector<uint64_t>& q_point) {
+    const size_t T = zs.size(), m = q_poly.size();
+    ensure(k >= 1 && T >= 1 && m >= 1 && q_point.size() == m, HALO_EINVAL, "multi-point opening: k, T and m must be at least 1");
+    ensure(T <= HALO_MULTI_MAX_POINTS, HALO_EINVAL, "multi-point opening: more than HALO_MULTI_MAX_POINTS points");
+    for (size_t t = 0; t < T; t++)
+        for (size_t u = 0; u < t; u++) ensure(!(zs[t] == zs[u]), HALO_EINVAL, "multi-point opening: duplicate points");
+    std::vector<std::pair<uint64_t, uint64_t>> pairs(m);
+    std::vector<uint8_t> poly_used(k, 0), point_used(T, 0);
+    for (size_t i = 0; i < m; i++) {
+        ensure(q_poly[i] < k && q_point[i] < T, HALO_EINVAL, "multi-point opening: a query index is out of range");
+        pairs[i] = {q_poly[i], q_point[i]};
+        poly_used[q_poly[i]] = point_used[q_point[i]] = 1;
+    }
+    std::sort(pairs.begin(), pairs.end());
+    ensure(std::adjacent_find(pairs.begin(), pairs.end()) == pairs.end(), HALO_EINVAL, "multi-point opening: a (j, t) pair repeats");
+    ensure(std::count(poly_used.begin(), poly_used.end(), 0) == 0, HALO_EINVAL, "multi-point opening: a polynomial is in no query");
+    ensure(std::count(point_used.begin(), point_used.end(), 0) == 0, HALO_EINVAL, "multi-point opening: a point is in no query");
+}
+
+static std::vector<PallasScalar> powers_of(const PallasScalar& x, size_t n) {
+    std::vector<PallasScalar> p(n);
+    if (n) p[0] = scalar_one();
+    for (size_t i = 1; i < n; i++) p[i] = p[i - 1] * x;
+    return p;
+}
+
+// x1 = rho_2(u64 k, u64 T, u64 m, C_0 .. C_{k-1}, z_0 .. z_{T-1}, (u64 j_i, u64 t_i, v_i) for every query)
+static PallasScalar multi_x1(const std::vector<PallasPoint>& Cs, const std::vector<PallasScalar>& zs, const std::vector<uint64_t>& q_poly,
+                             const std::vector<uint64_t>& q_point, const std::vector<PallasScalar>& vs) {
+    Transcript t;
+    t.u64(Cs.size()).u64(zs.size()).u64(q_poly.size());
+    for (const affine_t& a : batch_to_affine(Cs)) t.point_affine(a);
+    for (const PallasScalar& z : zs) t.scalar(z);
+    for (size_t i = 0; i < q_poly.size(); i++) t.u64(q_poly[i]).u64(q_point[i]).scalar(vs[i]);
+    return t.finish(2);
+}
+
+// v_hat_t = sum_{i: t_i = t} x1^i v_i
+static std::vector<PallasScalar> multi_vhat(size_t T, const std::vector<uint64_t>& q_point, const std::vector<PallasScalar>& vs,
+                                            const std::vector<PallasScalar>& pw1) {
+    std::vector<PallasScalar> vh(T, scalar_zero());
+    for (size_t i = 0; i < q_point.size(); i++) vh[q_point[i]] = vh[q_point[i]] + pw1[i] * vs[i];
+    return vh;
+}
+
+static void multi_x3_check(const PallasScalar& x3, const std::vector<PallasScalar>& zs) {
+    for (const PallasScalar& z : zs) ensure(!(x3 == z), HALO_EINTERNAL, "multi-point opening: x3 is one of the points");
+}
+
+// Steps 9-10 of the definition from x1, x2, x3 and the u_t
+static MultiClaim multi_final(halo_ctx* ctx, const std::vector<PallasPoint>& Cs, const std::vector<PallasScalar>& zs,
+                              const std::vector<uint64_t>& q_poly, const std::vector<uint64_t>& q_point, const std::vector<PallasScalar>& pw1,
+                              const std::vector<PallasScalar>& vh, const PallasScalar& x2, const PallasScalar& x3, const PallasPoint& Q,
+                              const std::vector<PallasScalar>& us) {
+    const size_t k = Cs.size(), T = zs.size();
+    Transcript tr;
+    tr.scalar(x3);
+    for (const PallasScalar& u : us) tr.scalar(u);
+    const PallasScalar x4 = tr.finish(2);
+    const std::vector<PallasScalar> pw2 = powers_of(x2, T), pw4 = powers_of(x4, T + 1);
+    std::vector<PallasScalar> den(T);
+    for (size_t t = 0; t < T; t++) den[t] = x3 - zs[t];
+    batch_inverse(den);
+    MultiClaim r;
+    r.x3 = x3;
+    r.v = scalar_zero();
+    for (size_t t = 0; t < T; t++) r.v = r.v + pw2[t] * (us[t] - vh[t]) * den[t] + pw4[t + 1] * us[t];  // q_hat + sum x4^(t+1) u_t
+    r.cs.assign(k, scalar_zero());
+    for (size_t i = 0; i < q_poly.size(); i++) r.cs[q_poly[i]] = r.cs[q_poly[i]] + pw4[q_point[i] + 1] * pw1[i];
+    std::vector<PallasPoint> pts(1, Q);
+    pts.insert(pts.end(), Cs.begin(), Cs.end());
+    std::vector<PallasScalar> sc(1, scalar_one());
+    sc.insert(sc.end(), r.cs.begin(), r.cs.end());
+    r.C = point_dot(ctx, sc.data(), pts, k + 1);
+    return r;
+}
+
+MultiClaim multi_claim(halo_ctx* ctx, const std::vector<PallasPoint>& Cs, const std::vector<PallasScalar>& zs,
+                       const std::vector<uint64_t>& q_poly, const std::vector<uint64_t>& q_point, const std::vector<PallasScalar>& vs,
+                       const PallasPoint& Q, const std::vector<PallasScalar>& us) {
+    multi_validate(Cs.size(), zs, q_poly, q_point);
+    ensure(vs.size() == q_poly.size() && us.size() == zs.size(), HALO_EINVAL, "multi_claim: one v per query and one u per point");
+    const PallasScalar x1 = multi_x1(Cs, zs, q_poly, q_point, vs);
+    const std::vector<PallasScalar> pw1 = powers_of(x1, q_poly.size());
+    const PallasScalar x2 = Transcript().scalar(x1).finish(2);
+    const PallasScalar x3 = Transcript().scalar(x2).point(Q).finish(2);
+    multi_x3_check(x3, zs);
+    return multi_final(ctx, Cs, zs, q_poly, q_point, pw1, multi_vhat(zs.size(), q_point, vs, pw1), x2, x3, Q, us);
+}
+
+MultiOpening open_multi(halo_ctx* ctx, const std::vector<PolyView>& ps, const std::vector<PallasPoint>& Cs, uint64_t d,
+                        const std::vector<PallasScalar>& zs, const std::vector<uint64_t>& q_poly, const std::vector<uint64_t>& q_point,
+                        const PallasScalar* ws, const PallasScalar* w_Q, const PolyView* q, const PallasScalar* w_bar) {
+    const size_t k = ps.size(), T = zs.size(), m = q_poly.size();
+    ensure(k >= 1 && Cs.size() == k, HALO_EINVAL, "open_multi: no polynomial");
+    const std::vector<uint64_t> lens = batch_lens(ctx, ps, d);
+    multi_validate(k, zs, q_poly, q_point);
+    if (ws) {  // q is drawn before any challenge exists: max_j deg(p_j) coefficients, as in open_batch
+        ensure(w_Q && q && w_bar, HALO_EINVAL, "hiding open needs w_Q, the random polynomial q and w_bar");
+        uint64_t max_deg = 0;
+        for (const PolyView& p : ps) max_deg = std::max(max_deg, degree(p));
+        ensure(max_deg >= 1 && q->size() == max_deg, HALO_ELEN, "q must have max_j deg(p_j) coefficients");
+    }
+    std::vector<PallasScalar> copy;
+    const PallasScalar* base = packed_prefixes(ps, lens, copy);
+    check_rc(ctx, halo_poly_upload(ctx, reinterpret_cast<const uint64_t*>(base), lens.data(), k, d + 1));
+    const uint64_t* zp = reinterpret_cast<const uint64_t*>(zs.data());
+    MultiOpening r;
+    r.vs.resize(m);
+    check_rc(ctx, halo_poly_eval_queries(ctx, zp, T, q_poly.data(), q_point.data(), m, reinterpret_cast<uint64_t*>(r.vs.data())));
+
+    const PallasScalar x1 = multi_x1(Cs, zs, q_poly, q_point, r.vs);
+    const std::vector<PallasScalar> pw1 = powers_of(x1, m), vh = multi_vhat(T, q_point, r.vs, pw1);
+    const PallasScalar x2 = Transcript().scalar(x1).finish(2);
+    const std::vector<PallasScalar> pw2 = powers_of(x2, T);
+    std::vector<PallasScalar> rems(T);
+    uint64_t Qb[12];
+    check_rc(ctx, halo_poly_quotient(ctx, zp, reinterpret_cast<const uint64_t*>(pw2.data()), T, q_poly.data(), q_point.data(),
+                                     reinterpret_cast<const uint64_t*>(pw1.data()), m, reinterpret_cast<uint64_t*>(rems.data()), Qb));
+    for (size_t t = 0; t < T; t++)  // f_t(z_t), the remainder of the division, must be the claimed v_hat_t
+        ensure(rems[t] == vh[t], HALO_EINTERNAL, "open_multi: a remainder of the division differs from sum x1^i v_i");
+    r.Q = point_load(Qb);
+    if (ws) {
+        PallasPoint S, H;
+        params_SH(ctx, S, H);
+        r.Q = r.Q + S * (*w_Q);
+    }
+    const PallasScalar x3 = Transcript().scalar(x2).point(r.Q).finish(2);
+    multi_x3_check(x3, zs);
+
+    // u_t = f_t(x3) from every polynomial at x3
+    std::vector<uint64_t> all(k), zero(k, 0);
+    for (size_t j = 0; j < k; j++) all[j] = j;
+    std::vector<PallasScalar> ev(k);
+    check_rc(ctx, halo_poly_eval_queries(ctx, reinterpret_cast<const uint64_t*>(&x3), 1, all.data(), zero.data(), k,
+                                         reinterpret_cast<uint64_t*>(ev.data())));
+    r.us.assign(T, scalar_zero());
+    for (size_t i = 0; i < m; i++) r.us[q_point[i]] = r.us[q_point[i]] + pw1[i] * ev[q_poly[i]];
+    r.claim = multi_final(ctx, Cs, zs, q_poly, q_point, pw1, vh, x2, x3, r.Q, r.us);
+
+    PallasScalar w = scalar_zero();
+    if (ws) {
+        w = *w_Q;
+        for (size_t j = 0; j < k; j++) w = w + r.claim.cs[j] * ws[j];
+    }
+    const PallasScalar one = scalar_one();
+    uint64_t deg = 0;
+    check_rc(ctx, halo_poly_lincomb_resident(ctx, reinterpret_cast<const uint64_t*>(r.claim.cs.data()),
+                                             reinterpret_cast<const uint64_t*>(&one), &deg));
+    const PolyView qd = ws ? PolyView(q->data(), std::min<uint64_t>(deg, q->size())) : PolyView(nullptr, 0);
+    PallasScalar v_dev;
+    r.pi = open_resident(ctx, deg, r.claim.C, d, x3, ws ? &w : nullptr, ws ? &qd : nullptr, w_bar, &v_dev);
+    // the opening evaluates P(x3) itself; it must be the claim's v
+    ensure(v_dev == r.claim.v, HALO_EINTERNAL, "open_multi: P(x3) of the combined polynomial differs from v");
+    return r;
+}
+
 static EvalProof open_impl(halo_ctx* ctx, const PolyView* p, uint64_t deg, const PallasPoint& C, uint64_t d, const PallasScalar& z,
                            const PallasScalar* w, const PolyView* q, const PallasScalar* w_bar, PallasScalar* v_out) {
     uint64_t n = d + 1;

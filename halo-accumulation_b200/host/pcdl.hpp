@@ -61,6 +61,30 @@ struct BatchOpening {
 };
 BatchOpening open_batch(halo_ctx* ctx, const std::vector<PolyView>& ps, const std::vector<PallasPoint>& Cs, uint64_t d,
                         const PallasScalar& z, const PallasScalar* ws, const PolyView* q, const PallasScalar* w_bar);
+
+// Batch opening at several points (DESIGN.md K3c, include/halo_pcdl.h halo_pcdl_open_multi; the reference has none).  Query i
+// opens polynomial q_poly[i] at zs[q_point[i]].  multi_claim is the verifier's side: the claims (C_j, z_t, v_i) with the
+// prover's Q and u_t reduced to the one PCDL claim (C, x3, v); c_j are the weights of P = q + sum_j c_j p_j.  Both validate
+// the queries (HALO_EINVAL) and fail with HALO_EINTERNAL when x3 is one of the points.
+struct MultiClaim {
+    PallasPoint C;
+    PallasScalar x3, v;
+    std::vector<PallasScalar> cs;
+};
+MultiClaim multi_claim(halo_ctx* ctx, const std::vector<PallasPoint>& Cs, const std::vector<PallasScalar>& zs,
+                       const std::vector<uint64_t>& q_poly, const std::vector<uint64_t>& q_point, const std::vector<PallasScalar>& vs,
+                       const PallasPoint& Q, const std::vector<PallasScalar>& us);
+// vs[i] = p_{q_poly[i]}(z_{q_point[i]}), the quotient's commitment Q, us[t] = f_t(x3) and the proof of the final claim.  Hiding
+// iff ws is given: w_Q blinds Q, q holds max_j deg(p_j) coefficients (the opening uses the first deg(P)), w_bar as in open.
+struct MultiOpening {
+    std::vector<PallasScalar> vs, us;
+    PallasPoint Q;
+    MultiClaim claim;
+    EvalProof pi;
+};
+MultiOpening open_multi(halo_ctx* ctx, const std::vector<PolyView>& ps, const std::vector<PallasPoint>& Cs, uint64_t d,
+                        const std::vector<PallasScalar>& zs, const std::vector<uint64_t>& q_poly, const std::vector<uint64_t>& q_point,
+                        const PallasScalar* ws, const PallasScalar* w_Q, const PolyView* q, const PallasScalar* w_bar);
 // succinct_check (pcdl.rs:252-314) without its group equation, in two halves around C' = C + alpha C_bar - w' S (:272-279) so
 // that a batch can compute every C' with one `combine` call.  succinct_alpha validates (d + 1 a power of two, d <= D, the
 // number of rounds) and returns alpha = rho_0(C, z, v, C_bar) of a hiding proof (zero otherwise); succinct_finish runs the rest

@@ -92,6 +92,50 @@ def batch_claim(ctx, Cs, z, vs):
     return Cm, v
 
 
+def _queries(queries):
+    q = np.ascontiguousarray(queries, dtype=np.uint64).reshape(-1, 2)
+    return np.ascontiguousarray(q[:, 0]), np.ascontiguousarray(q[:, 1])
+
+
+def open_multi(ctx, ps, Cs, d, zs, queries, ws=None, w_Q=None, q=None, w_bar=None):
+    """Opens the polynomials `ps` (commitments Cs, one degree bound d) at several points with ONE proof (include/halo_pcdl.h
+    halo_pcdl_open_multi; the reference has none).  queries: (j, t) pairs, polynomial j at point zs[t] -> (vs, Q, us, C, x, v,
+    pi): vs[i] = p_j(z_t) of query i, Q the quotient's commitment, us[t] = f_t(x), and (C, d, x, v, pi) an ordinary claim for
+    `check`, `check_batch` or acc.new_instance.  Hiding with ws (one w_j per polynomial): then w_Q, q (max_j deg(p_j)
+    coefficients) and w_bar are the caller's draws."""
+    packed, lens = pack(ps)
+    k = len(lens)
+    Cs, zs = arr(Cs).reshape(k, 12), arr(zs).reshape(-1, 4)
+    qp, qt = _queries(queries)
+    m, T = qp.shape[0], zs.shape[0]
+    wa = arr(ws).reshape(k, 4) if ws is not None else None
+    qa = arr(q).reshape(-1, 4) if q is not None else None
+    wqk, wqp = _host.opt(w_Q)
+    wbk, wbp = _host.opt(w_bar)
+    vs, us = np.zeros((max(1, m), 4), dtype=np.uint64), np.zeros((max(1, T), 4), dtype=np.uint64)
+    Q, Cm, x, v, pi = np.zeros(12, dtype=np.uint64), np.zeros(12, dtype=np.uint64), np.zeros(4, dtype=np.uint64), \
+        np.zeros(4, dtype=np.uint64), EvalProof()
+    _host.chk(_host.lib().halo_pcdl_open_multi(ctx._h, p64(packed), p64(lens), C.c_uint64(k), p64(Cs), C.c_uint64(d), p64(zs),
+                                               C.c_uint64(T), p64(qp), p64(qt), C.c_uint64(m), p64(wa) if wa is not None else None,
+                                               wqp, p64(qa) if qa is not None else None,
+                                               C.c_uint64(qa.shape[0] if qa is not None else 0), wbp, p64(vs), p64(Q), p64(us),
+                                               p64(Cm), p64(x), p64(v), C.byref(pi)))
+    return vs[:m], Q, us[:T], Cm, x, v, pi
+
+
+def multi_claim(ctx, Cs, zs, queries, vs, Q, us):
+    """The verifier's reduction of the claims of `open_multi` (commitments, points, (j, t) queries, their values, the
+    quotient's commitment Q and the u_t) to its one claim -> (C, x, v)."""
+    Cs, zs = arr(Cs).reshape(-1, 12), arr(zs).reshape(-1, 4)
+    qp, qt = _queries(queries)
+    vs, Q, us = arr(vs).reshape(qp.shape[0], 4), arr(Q, (12,)), arr(us).reshape(zs.shape[0], 4)
+    Cm, x, v = np.zeros(12, dtype=np.uint64), np.zeros(4, dtype=np.uint64), np.zeros(4, dtype=np.uint64)
+    _host.chk(_host.lib().halo_pcdl_multi_claim(ctx._h, p64(Cs), C.c_uint64(Cs.shape[0]), p64(zs), C.c_uint64(zs.shape[0]),
+                                                p64(qp), p64(qt), p64(vs), C.c_uint64(qp.shape[0]), p64(Q), p64(us), p64(Cm),
+                                                p64(x), p64(v)))
+    return Cm, x, v
+
+
 def succinct_check(ctx, Cm, d, z, v, pi):
     """pcdl.rs:252-314 -> (HPoly, U); raises Rejected"""
     Cm, z, v = arr(Cm, (12,)), arr(z, (4,)), arr(v, (4,))

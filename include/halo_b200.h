@@ -286,6 +286,30 @@ int halo_poly_eval_many(halo_ctx *ctx, const uint64_t *coeffs /*packed, [sum n_c
  * memory for p; the context then holds no resident polynomial. */
 int halo_poly_combine_resident(halo_ctx *ctx, const uint64_t alpha[4], uint64_t *degree_out);
 
+/* ---- K3c: k polynomials opened at several points (halo_pcdl_open_multi, include/halo_pcdl.h) ----------- */
+#define HALO_MULTI_MAX_POINTS 64
+/* The upload half of halo_poly_eval_many: the k packed polynomials become the context's resident polynomials, with the same
+ * errors; an earlier upload and its quotient are gone whatever the outcome. */
+int halo_poly_upload(halo_ctx *ctx, const uint64_t *coeffs /*packed, [sum n_coeffs][4]*/, const uint64_t *n_coeffs /*[k]*/,
+                     uint64_t k, uint64_t n);
+/* vs_out[i] = p_{q_poly[i]}(zs[q_point[i]]) over the resident polynomials, for m queries in two launches (k_quot_chunks,
+ * k_quot_carry).  HALO_EINVAL: NULL pointers, T = 0 or T > HALO_MULTI_MAX_POINTS, m = 0 or m >= 2^31, q_poly[i] >= k or
+ * q_point[i] >= T.  HALO_ESTATE: nothing uploaded.  HALO_ENOMEM: no device memory for the scratch; nothing is written. */
+int halo_poly_eval_queries(halo_ctx *ctx, const uint64_t *zs /*[T][4]*/, uint64_t T, const uint64_t *q_poly /*[m]*/,
+                           const uint64_t *q_point /*[m]*/, uint64_t m, uint64_t *vs_out /*[m][4]*/);
+/* With f_t = sum_{i: q_point[i] = t} weights[i] p_{q_poly[i]} over the resident polynomials (n = the longest of them):
+ *   q = sum_t scales[t] (f_t - f_t(z_t)) / (X - z_t), n - 1 coefficients, kept on the device;
+ *   rems_out[t] = f_t(z_t), the remainders;  Q_out = <GS[0..n-1), q> by the generator-MSM route of halo_msm_gens.
+ * The division is a chunked scan in three launches (k_quot_chunks, k_quot_carry, k_quot_write).  Errors as
+ * halo_poly_eval_queries; on any error no quotient is left for halo_poly_lincomb_resident. */
+int halo_poly_quotient(halo_ctx *ctx, const uint64_t *zs /*[T][4]*/, const uint64_t *scales /*[T][4]*/, uint64_t T,
+                       const uint64_t *q_poly /*[m]*/, const uint64_t *q_point /*[m]*/, const uint64_t *weights /*[m][4]*/, uint64_t m,
+                       uint64_t *rems_out /*[T][4]*/, uint64_t Q_out[12]);
+/* P = sum_j cs[j] p_j + c_q q over the resident polynomials and the quotient of the last halo_poly_quotient (one launch,
+ * k_poly_lincomb), left on the device for halo_ipa_begin_resident; *degree_out = its degree.  HALO_ESTATE: no quotient of
+ * the current upload.  HALO_ENOMEM: no device memory for P; the context then holds no resident polynomial. */
+int halo_poly_lincomb_resident(halo_ctx *ctx, const uint64_t *cs /*[k][4]*/, const uint64_t c_q[4], uint64_t *degree_out);
+
 /* ---- K3 / K4 / K7: the rounds of PCDL.open (pcdl.rs:183-231) ----------------------------------------- */
 typedef struct halo_ipa halo_ipa;
 /* Uploads the coefficients of p (zero-padded to n, pcdl.rs:183-184), copies GS[0..n) (pcdl.rs:185), builds

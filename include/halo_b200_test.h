@@ -64,6 +64,9 @@ int halo_test_glv_decompose_jsf(const uint64_t xi[4], int8_t d1[136], int8_t d2[
  * halo_b200.h because only that library calls it; removing or changing it breaks those entry points. */
 int halo_test_point_combine(halo_ctx *ctx, int path, const uint64_t *P_jac, const uint64_t *Q_jac, const uint64_t *a,
                             const uint64_t *b, uint64_t n, uint64_t *out_affine);
+/* K3c: *n_out = the number of coefficients of the quotient q that the last halo_poly_quotient left on the device; when
+ * cap >= *n_out they are copied to out[*n_out][4] (Montgomery limbs).  HALO_ESTATE: no quotient of the current upload. */
+int halo_test_read_quotient(halo_ctx *ctx, uint64_t *out, uint64_t cap, uint64_t *n_out);
 #ifdef __cplusplus
 }
 #endif

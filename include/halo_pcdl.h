@@ -111,6 +111,58 @@ int halo_pcdl_open_batch(halo_ctx *ctx, const uint64_t *coeffs /*packed*/, const
  * z not canonical. */
 int halo_pcdl_batch_claim(halo_ctx *ctx, const uint64_t *Cs /*[k][12]*/, const uint64_t *vs /*[k][4]*/, uint64_t k,
                           const uint64_t z[4], uint64_t C_out[12], uint64_t v_out[4]);
+/* Batch opening at several points (an extension: the reference opens one polynomial at one point, DESIGN.md K3c; the
+ * multi-point reduction of Halo 2, after Boneh-Drake-Fisch-Gabizon 2020).
+ *
+ * Inputs: k >= 1 polynomials p_0 .. p_{k-1} of one degree bound d, packed as in halo_pcdl_commit_batch; their commitments
+ * C_j, as commit returns them; T >= 1 distinct points z_0 .. z_{T-1} (T <= HALO_MULTI_MAX_POINTS); m >= 1 queries
+ * (j_i, t_i) = (q_poly[i], q_point[i]): polynomial j_i is opened at point z_{t_i}; optionally the blinding scalars w_j.
+ * Every point and every polynomial must appear in at least one query, and no (j, t) pair may repeat.
+ * All challenges use the transcript of host/group.hpp with tag 2 (rho_2), apart from PCDL's tag 0 and ASDL's tag 1; each
+ * record is a u64 little-endian, a compressed point or a canonical scalar.
+ *   1. v_i = p_{j_i}(z_{t_i}) for i < m                                                      -> vs_out[i]
+ *   2. x1 = rho_2(u64 k, u64 T, u64 m, C_0 .. C_{k-1}, z_0 .. z_{T-1}, then for each query i: u64 j_i, u64 t_i, v_i)
+ *   3. for each point t, over its queries in query order: f_t = sum_{i: t_i = t} x1^i p_{j_i}, v^_t = sum x1^i v_i,
+ *      C^_t = sum x1^i C_{j_i}, w^_t = sum x1^i w_{j_i}
+ *   4. x2 = rho_2(x1)
+ *   5. q = sum_t x2^t (f_t - v^_t) / (X - z_t): exact division for honest claims, deg q <= d - 1.  The quotient of f_t by
+ *      (X - z_t) does not depend on v^_t; the remainder of that division is f_t(z_t) and must equal v^_t.
+ *   6. Q = commit(q, d, w_Q), the ordinary PCDL commitment (hiding with the caller's draw w_Q)       -> Q_out
+ *   7. x3 = rho_2(x2, Q); if x3 equals some z_t the call fails with HALO_EINTERNAL (probability <= T / r)  -> x_out
+ *   8. u_t = f_t(x3) for t < T                                                                 -> us_out[t]
+ *   9. x4 = rho_2(x3, u_0 .. u_{T-1})
+ *  10. the final claim: P = q + sum_t x4^(t+1) f_t = q + sum_j c_j p_j with c_j = sum_{i: j_i = j} x4^(t_i+1) x1^i;
+ *      C = Q + sum_j c_j C_j; v = q^ + sum_t x4^(t+1) u_t with q^ = sum_t x2^t (u_t - v^_t) / (x3 - z_t);
+ *      w = w_Q + sum_j c_j w_j when hiding                                                     -> C_out, v_out
+ *  11. pi = halo_pcdl_open(P, C, d, x3, w, q_rand, w_bar), the opening unchanged               -> pi
+ * (C, d, x3, v, pi) is an ordinary PCDL claim: halo_pcdl_check, halo_pcdl_check_batch and the accumulation scheme take it
+ * unchanged.  The verifier's side is halo_pcdl_multi_claim.
+ * Hiding applies iff ws != NULL; the caller's draws are, in order, w_Q, q_rand with n_q = max_j deg(p_j) coefficients (as
+ * in halo_pcdl_open_batch; the opening takes the first deg(P) of them) and w_bar.
+ * Soundness: if some v_i is false, then with probability >= 1 - (m - 1)/r over x1 some f_t(z_t) != v^_t; then with
+ * probability >= 1 - (T - 1)/r over x2 the sum of step 5 has a pole and is no polynomial; Q is bound before x3; over x4 the
+ * final claim forces q'(x3) = q^ and u_t = f_t(x3) for every t, except with probability T/r; and the committed q' agrees with
+ * the rational function at x3 with probability at most (d + T)/r.  Total <= (m + 3T + d)/r plus the soundness error of one
+ * PCDL check (DESIGN.md K3c).
+ * Returns, before any device work and before any output is written: HALO_EINVAL for k, T or m = 0, NULL pointers, the first
+ * malformed polynomial in order (as halo_pcdl_open_batch), a C_j off the curve or not canonical, a z_t, w_j, w_Q or w_bar
+ * that is not canonical, duplicate points, a query index out of range, a duplicate (j, t) pair, an unused point or
+ * polynomial; HALO_ELEN for n_q != max_j deg(p_j) or max deg = 0 with hiding.  HALO_EINTERNAL when a remainder differs from
+ * v^_t or the opening's own P(x3) from v (bugs, not decisions), or x3 is one of the points. */
+int halo_pcdl_open_multi(halo_ctx *ctx, const uint64_t *coeffs /*packed*/, const uint64_t *n_coeffs /*[k]*/, uint64_t k,
+                         const uint64_t *Cs /*[k][12]*/, uint64_t d, const uint64_t *zs /*[T][4]*/, uint64_t T,
+                         const uint64_t *q_poly /*[m]*/, const uint64_t *q_point /*[m]*/, uint64_t m,
+                         const uint64_t *ws /*[k][4] or NULL*/, const uint64_t *w_Q, const uint64_t *q, uint64_t n_q,
+                         const uint64_t *w_bar, uint64_t *vs_out /*[m][4]*/, uint64_t Q_out[12], uint64_t *us_out /*[T][4]*/,
+                         uint64_t C_out[12], uint64_t x_out[4], uint64_t v_out[4], halo_eval_proof *pi);
+/* The verifier's side of halo_pcdl_open_multi: recomputes x1 .. x4 and reduces the claims (C_j, z_t, v_i) with the prover's
+ * Q and u_t to the one claim (C, x3, v) above (host arithmetic and one point_dot of k + 1 points), to be decided by
+ * halo_pcdl_check / _check_batch or accumulated.  HALO_EINVAL as halo_pcdl_open_multi for the commitments, points and
+ * queries, and for a v_i, u_t or Q that is not canonical; HALO_EINTERNAL when x3 is one of the points. */
+int halo_pcdl_multi_claim(halo_ctx *ctx, const uint64_t *Cs /*[k][12]*/, uint64_t k, const uint64_t *zs /*[T][4]*/, uint64_t T,
+                          const uint64_t *q_poly /*[m]*/, const uint64_t *q_point /*[m]*/, const uint64_t *vs /*[m][4]*/, uint64_t m,
+                          const uint64_t Q[12], const uint64_t *us /*[T][4]*/, uint64_t C_out[12], uint64_t x_out[4],
+                          uint64_t v_out[4]);
 /* pcdl.rs:252-314; on accept writes the HPoly challenges xis[lg_n+1][4] and U. */
 int halo_pcdl_succinct_check(halo_ctx *ctx, const uint64_t C_jac[12], uint64_t d, const uint64_t z[4], const uint64_t v[4],
                              const halo_eval_proof *pi, uint64_t *xis_out, uint64_t U_out[12]);
