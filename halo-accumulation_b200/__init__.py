@@ -12,7 +12,16 @@ import numpy as np
 from . import _build
 from ._capi import HaloError, arr, load, p64, pack, u8p
 
-__all__ = ["Context", "Comm", "MultiGpu", "HaloError", "build", "points_sum", "points_equal", "comm_slice"]
+__all__ = ["Context", "Comm", "MultiGpu", "HaloError", "build", "points_sum", "points_equal", "comm_slice", "domain_root"]
+
+
+def domain_root(lg_n):
+    """omega_{2^lg_n} = 5^((r - 1) / 2^lg_n) in Montgomery form (include/halo_b200.h K8), lg_n <= 32."""
+    out = np.zeros(4, dtype=np.uint64)
+    rc = load().halo_domain_root(C.c_uint32(lg_n), p64(out))
+    if rc != 0:
+        raise HaloError(rc, f"halo_domain_root: lg_n = {lg_n} above 32")
+    return out
 
 
 def points_sum(points_jac):
@@ -226,6 +235,29 @@ class Context:
         out = np.zeros((max(1, len(lens)), 12), dtype=np.uint64)
         self._chk(self._lib.halo_msm_gens_many(self._h, p64(packed), p64(lens), C.c_uint64(len(lens)), p64(out)))
         return out[:len(lens)]
+
+    def ntt(self, a, lg_n=None, inverse=False, shift=None):
+        """halo_ntt (DESIGN.md K8): k vectors (k, n_in, 4) -> (k, 2^lg_n, 4), forward or inverse transform over the coset
+        shift * H, H of order 2^lg_n (lg_n = None: n_in rounded up to a power of two).  A (n_in, 4) vector gives (2^lg_n, 4)."""
+        a = arr(a)
+        one = a.ndim == 2
+        a = a.reshape(1 if one else a.shape[0], -1, 4)
+        k, n_in = a.shape[:2]
+        if lg_n is None:
+            lg_n = max(0, (n_in - 1).bit_length())
+        out = np.zeros((max(1, k), 1 << lg_n, 4), dtype=np.uint64)
+        sh = arr(shift, (4,)) if shift is not None else None
+        src = a.reshape(-1, 4) if a.size else np.zeros((1, 4), dtype=np.uint64)
+        self._chk(self._lib.halo_ntt(self._h, p64(src), C.c_uint64(n_in), C.c_uint64(k), C.c_uint32(lg_n), int(bool(inverse)),
+                                     p64(sh) if sh is not None else None, p64(out)))
+        return out[0] if one else out[:k]
+
+    def ntt_resident(self, d_ptr, k, lg_n, inverse=False, shift=None):
+        """halo_ntt_resident: the same in place on k * 2^lg_n scalars at a CUDA pointer (e.g. a torch tensor's data_ptr(),
+        complete when called)."""
+        sh = arr(shift, (4,)) if shift is not None else None
+        self._chk(self._lib.halo_ntt_resident(self._h, C.c_void_p(d_ptr), C.c_uint64(k), C.c_uint32(lg_n), int(bool(inverse)),
+                                              p64(sh) if sh is not None else None))
 
     def msm_gens_submit(self, scalars, off=0):
         """Pipelined halo_msm_gens: returns a ticket; `scalars` must stay alive (ideally pinned) until collect."""

@@ -66,6 +66,11 @@ def load():
     lib.halo_h_msm_batch_submit.argtypes = [C.c_void_p, u64p, C.POINTER(C.c_uint32), u64p, C.c_uint64, C.POINTER(C.c_int)]
     lib.halo_h_msm_batch_collect.argtypes = [C.c_void_p, C.c_int, u64p, u8p, u64p, C.c_uint64, u64p]
     lib.halo_msm_gens_many.argtypes = [C.c_void_p, u64p, u64p, C.c_uint64, u64p]
+    lib.halo_domain_root.argtypes = [C.c_uint32, u64p]
+    lib.halo_ntt.argtypes = [C.c_void_p, u64p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_int, u64p, u64p]
+    lib.halo_ntt_resident.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_int, u64p]
+    lib.halo_poly_upload_evals.argtypes = [C.c_void_p, u64p, C.c_uint64, C.c_uint64, u64p]
+    lib.halo_poly_commit_resident.argtypes = [C.c_void_p, u64p]
     lib.halo_test_point_combine.argtypes = [C.c_void_p, C.c_int, u64p, u64p, u64p, u64p, C.c_uint64, u64p]
     if lib.halo_curve_name().decode() != _build.CURVE:
         raise RuntimeError(f"{path} was built for {lib.halo_curve_name().decode()}, HALO_B200_CURVE asks for {_build.CURVE}")

@@ -81,6 +81,10 @@ def lib():
         _lib.halo_pcdl_open_multi.argtypes = [C.c_void_p, u64p, u64p, C.c_uint64, u64p, C.c_uint64, u64p, C.c_uint64, u64p, u64p,
                                               C.c_uint64, u64p, u64p, u64p, C.c_uint64, u64p, u64p, u64p, u64p, u64p, u64p, u64p,
                                               C.POINTER(EvalProof)]
+        _lib.halo_pcdl_commit_evals.argtypes = [C.c_void_p, u64p, C.c_uint64, C.c_uint64, u64p, u64p]
+        _lib.halo_pcdl_open_multi_evals.argtypes = [C.c_void_p, u64p, C.c_uint64, u64p, C.c_uint64, u64p, C.c_uint64, u64p, u64p,
+                                                    C.c_uint64, u64p, u64p, u64p, C.c_uint64, u64p, u64p, u64p, u64p, u64p, u64p,
+                                                    u64p, C.POINTER(EvalProof)]
         _lib.halo_pcdl_multi_claim.argtypes = [C.c_void_p, u64p, C.c_uint64, u64p, C.c_uint64, u64p, u64p, u64p, C.c_uint64, u64p,
                                                u64p, u64p, u64p, u64p]
         _lib.halo_pcdl_check_batch.argtypes = [C.c_void_p, C.POINTER(Instance), C.c_uint64, u64p, u64p]

@@ -8,6 +8,7 @@
 #include "../../include/halo_b200.h"
 #include "common.cuh"
 #include "msm.cuh"
+#include "ntt.cuh"
 #include "params.cuh"
 #include "vec.cuh"
 
@@ -210,6 +211,8 @@ void halo_ctx_destroy(halo_ctx* ctx) {
     ctx->polys_off.release();
     ctx->quot_dev.release();
     ctx->quot_scratch.release();
+    for (halo::DevBuf* b : {&ctx->ntt_dit, &ctx->ntt_scale, &ctx->ntt_a, &ctx->ntt_b, &ctx->ntt_deg}) b->release();
+    for (halo::DevBuf& b : ctx->ntt_tw) b.release();
     ctx->lincomb_claims.release();
     for (halo::DevBuf* b : {&ctx->combine_in, &ctx->combine_work, &ctx->combine_inv_scratch}) b->release();
     for (halo::DevBuf* b : {&ctx->ipa_G, &ctx->ipa_cs, &ctx->ipa_zs, &ctx->ipa_pbar, &ctx->ipa_tail, &ctx->ipa_frozen,
@@ -719,10 +722,10 @@ std::vector<ManyGroup> many_groups(halo_ctx* ctx, const std::vector<uint64_t>& j
 
 }  // namespace
 
-int halo_msm_gens_many(halo_ctx* ctx, const uint64_t* scalars, const uint64_t* lens, uint64_t k, uint64_t* out_jac) {
-    if (!ctx) return HALO_EINVAL;
-    if (k == 0) return HALO_OK;
-    if (!scalars || !lens || !out_jac) return HALO_EINVAL;
+// The body of halo_msm_gens_many for either source of the packed scalars: host memory (`scalars`, copied group by group on the
+// copy stream) or device memory (`d_scalars`, used in place).  One grouping, plan and finish for both.
+static int gens_many_impl(halo_ctx* ctx, const uint64_t* scalars, const fr_t* d_scalars, const uint64_t* lens, uint64_t k,
+                          uint64_t* out_jac) {
     std::vector<uint64_t> starts, jobs;  // packed position of every output; the outputs with scalars
     try {
         starts.resize(k);
@@ -763,7 +766,7 @@ int halo_msm_gens_many(halo_ctx* ctx, const uint64_t* scalars, const uint64_t* l
                 HALO_CUDA(cudaEventCreateWithFlags(&b.done, cudaEventDisableTiming));
                 HALO_CUDA(cudaMallocHost(reinterpret_cast<void**>(&b.h_seg_off), (size_t)(MANY_MAX_SEGS + 1) * 4));
             }
-            b.scalars.reserve(max_ns * sizeof(fr_t));
+            if (!d_scalars) b.scalars.reserve(max_ns * sizeof(fr_t));
             b.seg_off.reserve((size_t)(MANY_MAX_SEGS + 1) * 4);
             b.parts.reserve(max_parts * sizeof(xyzz_t));
             if (b.h_parts_cap < max_parts) {
@@ -784,7 +787,8 @@ int halo_msm_gens_many(halo_ctx* ctx, const uint64_t* scalars, const uint64_t* l
             cudaStreamSynchronize(c->stream);
         }
     } drain{max_ns ? ctx : nullptr};
-    // group g's scalars and segment starts into buffer g & 1 on the copy stream, once the group two back has released it
+    // group g's scalars (host source) and segment starts into buffer g & 1 on the copy stream, once the group two back has
+    // released it
     auto issue_copy = [&](size_t g) {
         const ManyGroup& gr = groups[g];
         halo_ctx::ManyBuf& b = ctx->many[g & 1];
@@ -793,7 +797,7 @@ int halo_msm_gens_many(halo_ctx* ctx, const uint64_t* scalars, const uint64_t* l
         HALO_CUDA(cudaStreamWaitEvent(ctx->copy_stream, b.done, 0));
         for (uint32_t s = 0; s <= segs; s++) b.h_seg_off[s] = (uint32_t)((s < segs ? starts[jobs[gr.j0 + s]] : gr.s0 + gr.ns) - gr.s0);
         HALO_CUDA(cudaMemcpyAsync(b.seg_off.p, b.h_seg_off, (size_t)(segs + 1) * 4, cudaMemcpyHostToDevice, ctx->copy_stream));
-        h2d_copy(ctx, b.scalars.p, scalars + 4 * gr.s0, gr.ns * sizeof(fr_t), ctx->copy_stream);
+        if (!d_scalars) h2d_copy(ctx, b.scalars.p, scalars + 4 * gr.s0, gr.ns * sizeof(fr_t), ctx->copy_stream);
         HALO_CUDA(cudaEventRecord(b.copied, ctx->copy_stream));
     };
     // group g's segmented MSM on the context stream, its window partials to the pinned host buffer
@@ -801,7 +805,7 @@ int halo_msm_gens_many(halo_ctx* ctx, const uint64_t* scalars, const uint64_t* l
         const ManyGroup& gr = groups[g];
         halo_ctx::ManyBuf& b = ctx->many[g & 1];
         // FIXED base as the group's plan, which the segment lengths chose, not by the length of the whole group
-        MsmInput in = gens_msm_input(ctx, gr.plan.fixed, b.scalars.as<fr_t>(), 0, gr.ns);
+        MsmInput in = gens_msm_input(ctx, gr.plan.fixed, d_scalars ? d_scalars + gr.s0 : b.scalars.as<fr_t>(), 0, gr.ns);
         in.segs = gr.plan.segs;
         in.seg_off = b.seg_off.as<uint32_t>();
         HALO_CUDA(cudaStreamWaitEvent(ctx->stream, b.copied, 0));
@@ -833,7 +837,8 @@ int halo_msm_gens_many(halo_ctx* ctx, const uint64_t* scalars, const uint64_t* l
             if (pend != SIZE_MAX) finish(pend);
             pend = SIZE_MAX;
             const uint64_t j = jobs[groups[g].j0];
-            const int rc = halo_msm_gens(ctx, scalars + 4 * starts[j], 0, lens[j], out_jac + 12 * j);
+            const int rc = d_scalars ? halo_msm_gens_resident(ctx, d_scalars + starts[j], 0, lens[j], out_jac + 12 * j)
+                                     : halo_msm_gens(ctx, scalars + 4 * starts[j], 0, lens[j], out_jac + 12 * j);
             if (rc) return rc;
         } else {
             launch(g);
@@ -846,6 +851,13 @@ int halo_msm_gens_many(halo_ctx* ctx, const uint64_t* scalars, const uint64_t* l
     }
     if (pend != SIZE_MAX) finish(pend);
     HALO_CATCH(ctx)
+}
+
+int halo_msm_gens_many(halo_ctx* ctx, const uint64_t* scalars, const uint64_t* lens, uint64_t k, uint64_t* out_jac) {
+    if (!ctx) return HALO_EINVAL;
+    if (k == 0) return HALO_OK;
+    if (!scalars || !lens || !out_jac) return HALO_EINVAL;
+    return gens_many_impl(ctx, scalars, nullptr, lens, k, out_jac);
 }
 
 // Shared body of the two submit entry points: host scalars are copied on the copy stream first; device-resident
@@ -1499,6 +1511,116 @@ int halo_poly_lincomb_resident(halo_ctx* ctx, const uint64_t* cs, const uint64_t
                      ctx->quot_dev.as<fr_t>(), ctx->quot_n, cq, n, ctx->poly_dev.as<fr_t>());
     ctx->poly_n = n;
     *degree_out = device_degree(ctx, ctx->poly_dev.as<fr_t>(), n);
+    HALO_CATCH(ctx)
+}
+
+int halo_poly_commit_resident(halo_ctx* ctx, uint64_t* out_jac) {
+    if (!ctx || !out_jac) return HALO_EINVAL;
+    if (!ctx->polys_k) return fail(ctx, HALO_ESTATE, "halo_poly_commit_resident: no resident polynomials (call halo_poly_upload first)");
+    std::vector<uint64_t> lens(ctx->polys_k);
+    for (uint64_t j = 0; j < ctx->polys_k; j++) lens[j] = ctx->polys_starts[j + 1] - ctx->polys_starts[j];
+    return gens_many_impl(ctx, nullptr, ctx->polys_dev.as<fr_t>(), lens.data(), ctx->polys_k, out_jac);
+}
+
+// ---- K8: number-theoretic transforms over the scalar field (ntt.cu) -------------------------------------------------------
+int halo_domain_root(uint32_t lg_n, uint64_t out[4]) {
+    if (!out || lg_n > NTT_MAX_LG) return HALO_EINVAL;
+    const fr_t w = ntt_root(lg_n);
+    memcpy(out, w.v, sizeof w.v);
+    return HALO_OK;
+}
+
+// The checks every transform entry point shares; *g = the shift's residue when there is one
+static int ntt_check(halo_ctx* ctx, const char* fn, uint64_t k, uint32_t lg_n, const uint64_t shift[4], fr_t* g) {
+    const std::string e(fn);
+    if (lg_n > NTT_MAX_LG) return fail(ctx, HALO_EINVAL, (e + ": lg_n above 32").c_str());
+    const uint64_t n = (uint64_t)1 << lg_n;
+    if (n > ctx->max_n) return fail(ctx, HALO_EINVAL, (e + ": 2^lg_n exceeds the context's max_n").c_str());
+    if (k > UINT64_MAX / sizeof(fr_t) / n) return fail(ctx, HALO_EINVAL, (e + ": k * 2^lg_n scalars overflow").c_str());
+    if (shift) {
+        uint32_t m[8], t[8];
+        memcpy(g->v, shift, sizeof g->v);
+        fp_mod_limbs<ScalarParams>(m);
+        if (fp_is_zero(*g) || !sub8(t, g->v, m)) return fail(ctx, HALO_EINVAL, (e + ": the shift is zero or not canonical").c_str());
+    }
+    return HALO_OK;
+}
+
+int halo_ntt(halo_ctx* ctx, const uint64_t* in, uint64_t n_in, uint64_t k, uint32_t lg_n, int inverse, const uint64_t shift[4],
+             uint64_t* out) {
+    if (!ctx) return HALO_EINVAL;
+    fr_t g;
+    if (int rc = ntt_check(ctx, "halo_ntt", k, lg_n, shift, &g)) return rc;
+    const uint64_t n = (uint64_t)1 << lg_n;
+    if (n_in > n) return fail(ctx, HALO_EINVAL, "halo_ntt: n_in exceeds 2^lg_n");
+    if (inverse && n_in != n) return fail(ctx, HALO_ELEN, "halo_ntt: an inverse transform needs n_in = 2^lg_n");
+    if (k == 0) return HALO_OK;
+    if (!out || (!in && n_in)) return HALO_EINVAL;
+    HALO_TRY(ctx)
+    // the input is staged into the buffer the first pass does not write (one pass over a full vector: in place)
+    const bool in_a = ntt_stage_in_a(lg_n) || (ntt_passes(lg_n) == 1 && n_in == n);
+    const uint64_t b_len = ntt_passes(lg_n) > 1 ? k * n : in_a ? 0 : k * n_in;
+    if (!reserve_or_nomem(ctx->ntt_a, k * n * sizeof(fr_t)) || !reserve_or_nomem(ctx->ntt_b, (b_len ? b_len : 1) * sizeof(fr_t)) ||
+        !ntt_prepare(ctx, lg_n, inverse, shift ? &g : nullptr))
+        return fail(ctx, HALO_ENOMEM, "halo_ntt: out of device memory");
+    fr_t* src = in_a ? ctx->ntt_a.as<fr_t>() : ctx->ntt_b.as<fr_t>();
+    h2d_copy(ctx, src, in, k * n_in * sizeof(fr_t), ctx->stream);
+    ntt_run(ctx, src, n_in, ctx->ntt_a.as<fr_t>(), ctx->ntt_b.as<fr_t>(), k, lg_n, inverse, shift != nullptr);
+    HALO_CUDA(cudaMemcpyAsync(out, ctx->ntt_a.p, k * n * sizeof(fr_t), cudaMemcpyDeviceToHost, ctx->stream));
+    HALO_CUDA(cudaStreamSynchronize(ctx->stream));
+    HALO_CATCH(ctx)
+}
+
+int halo_ntt_resident(halo_ctx* ctx, void* d_vecs, uint64_t k, uint32_t lg_n, int inverse, const uint64_t shift[4]) {
+    if (!ctx) return HALO_EINVAL;
+    fr_t g;
+    if (int rc = ntt_check(ctx, "halo_ntt_resident", k, lg_n, shift, &g)) return rc;
+    if (k == 0) return HALO_OK;
+    if (!d_vecs) return HALO_EINVAL;
+    const uint64_t n = (uint64_t)1 << lg_n;
+    const uint32_t P = ntt_passes(lg_n);
+    HALO_TRY(ctx)
+    if ((P > 1 && !reserve_or_nomem(ctx->ntt_b, k * n * sizeof(fr_t))) || !ntt_prepare(ctx, lg_n, inverse, shift ? &g : nullptr))
+        return fail(ctx, HALO_ENOMEM, "halo_ntt_resident: out of device memory");
+    fr_t* a = static_cast<fr_t*>(d_vecs);
+    const fr_t* src = a;  // one pass: in place; an even number of passes ends where it starts
+    if (P > 1 && !ntt_stage_in_a(lg_n)) {  // an odd number of passes above one starts from a copy
+        HALO_CUDA(cudaMemcpyAsync(ctx->ntt_b.p, d_vecs, k * n * sizeof(fr_t), cudaMemcpyDeviceToDevice, ctx->stream));
+        src = ctx->ntt_b.as<fr_t>();
+    }
+    ntt_run(ctx, src, n, a, ctx->ntt_b.as<fr_t>(), k, lg_n, inverse, shift != nullptr);
+    HALO_CUDA(cudaStreamSynchronize(ctx->stream));
+    HALO_CATCH(ctx)
+}
+
+int halo_poly_upload_evals(halo_ctx* ctx, const uint64_t* evals, uint64_t k, uint64_t n, uint64_t* degrees_out) {
+    if (!ctx || !evals || !degrees_out) return HALO_EINVAL;
+    if (k == 0 || (k >> 31)) return fail(ctx, HALO_EINVAL, "halo_poly_upload_evals: k must be 1 .. 2^31 - 1");
+    if (!n || (n & (n - 1))) return fail(ctx, HALO_EINVAL, "halo_poly_upload_evals: n is not a power of two");
+    if (n > ctx->n_gens) return fail(ctx, HALO_EINVAL, "halo_poly_upload_evals: n exceeds the resident generators");
+    uint32_t lg = 0;
+    while (((uint64_t)1 << lg) < n) lg++;
+    if (int rc = ntt_check(ctx, "halo_poly_upload_evals", k, lg, nullptr, nullptr)) return rc;
+    ctx->polys_k = 0;  // the previous upload is gone from here on, whatever the outcome
+    ctx->quot_ready = false;
+    HALO_TRY(ctx)
+    std::vector<uint64_t> off(k + 1), deg(k);
+    for (uint64_t j = 0; j <= k; j++) off[j] = j * n;
+    if (!reserve_or_nomem(ctx->polys_dev, k * n * sizeof(fr_t)) || !reserve_or_nomem(ctx->polys_off, (k + 1) * sizeof(uint64_t)) ||
+        !reserve_or_nomem(ctx->ntt_b, (ntt_passes(lg) > 1 ? k * n : 1) * sizeof(fr_t)) ||
+        !reserve_or_nomem(ctx->ntt_deg, k * sizeof(uint64_t)) || !ntt_prepare(ctx, lg, true, nullptr))
+        return fail(ctx, HALO_ENOMEM, "halo_poly_upload_evals: out of device memory");
+    fr_t* src = ntt_passes(lg) > 1 && !ntt_stage_in_a(lg) ? ctx->ntt_b.as<fr_t>() : ctx->polys_dev.as<fr_t>();
+    h2d_copy(ctx, src, evals, k * n * sizeof(fr_t), ctx->stream);
+    ntt_run(ctx, src, n, ctx->polys_dev.as<fr_t>(), ctx->ntt_b.as<fr_t>(), k, lg, true, false);
+    ntt_degrees(ctx, ctx->polys_dev.as<fr_t>(), k, n, ctx->ntt_deg.as<uint64_t>());
+    HALO_CUDA(cudaMemcpyAsync(ctx->polys_off.p, off.data(), (k + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
+    HALO_CUDA(cudaMemcpyAsync(deg.data(), ctx->ntt_deg.p, k * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    HALO_CUDA(cudaStreamSynchronize(ctx->stream));
+    for (uint64_t j = 0; j < k; j++) degrees_out[j] = deg[j] ? deg[j] - 1 : 0;  // highest non-zero index + 1, 0: none
+    ctx->polys_k = k;
+    ctx->polys_n = n;
+    ctx->polys_starts = std::move(off);
     HALO_CATCH(ctx)
 }
 

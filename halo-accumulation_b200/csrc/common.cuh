@@ -175,6 +175,10 @@ struct halo_ctx {
     halo::DevBuf quot_dev, quot_scratch;
     uint64_t quot_n = 0;
     bool quot_ready = false;
+    // K8 (ntt.cu): twiddle tables (omega_{2^11}^x; per size lg the two-level table of omega_{2^lg}), built once; the coset /
+    // scale table of the last call; the staging and ping-pong vectors of the passes; the degrees of halo_poly_upload_evals
+    halo::DevBuf ntt_dit, ntt_tw[33], ntt_scale, ntt_a, ntt_b, ntt_deg;
+    bool ntt_attr = false;  // k_ntt_pass may use 64 KiB of dynamic shared memory on this context's device
     // buffers of the (single) in-flight PCDL opening, kept across openings: cudaMalloc / cudaFree of 100+ MB per open
     // costs tens of milliseconds
     halo::DevBuf ipa_G, ipa_cs, ipa_zs, ipa_pbar, ipa_tail, ipa_frozen;

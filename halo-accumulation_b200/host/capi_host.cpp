@@ -1,4 +1,6 @@
 // host/capi_host.cpp -- C view (include/halo_pcdl.h) of the C++ host layer, for ctypes / C callers.
+#include <functional>
+
 #include "../../include/halo_pcdl.h"
 
 #include "acc.hpp"
@@ -95,6 +97,17 @@ int halo_pcdl_commit_batch(halo_ctx* ctx, const uint64_t* coeffs, const uint64_t
     });
 }
 
+int halo_pcdl_commit_evals(halo_ctx* ctx, const uint64_t* evals, uint64_t k, uint64_t d, const uint64_t* ws, uint64_t* out_jac) {
+    return guarded([&] {
+        if (k == 0) return;
+        ensure(evals && out_jac, HALO_EINVAL, "halo_pcdl_commit_evals: NULL pointer");
+        ensure(d < UINT64_MAX && k <= UINT64_MAX / 32 / (d + 1), HALO_EINVAL, "halo_pcdl_commit_evals: k (d + 1) scalars overflow");
+        const std::vector<PallasPoint> C = pcdl::commit_evals(ctx, reinterpret_cast<const PallasScalar*>(evals), k, d,
+                                                              reinterpret_cast<const PallasScalar*>(ws));
+        for (uint64_t j = 0; j < k; j++) point_store(out_jac + 12 * j, C[j]);
+    });
+}
+
 int halo_pcdl_open(halo_ctx* ctx, const uint64_t* coeffs, uint64_t n_coeffs, const uint64_t C_jac[12], uint64_t d,
                    const uint64_t z[4], const uint64_t* w, const uint64_t* q, uint64_t n_q, const uint64_t* w_bar,
                    halo_eval_proof* pi) {
@@ -174,6 +187,42 @@ static void multi_inputs(const uint64_t* zs, uint64_t T, const uint64_t* q_poly,
     qt.assign(q_point, q_point + m);
 }
 
+// The body of the two multi-point entry points after their polynomials: the caller's commitments, points, queries and draws
+// in, the opening of `open` out
+using MultiOpen = std::function<pcdl::MultiOpening(const std::vector<PallasPoint>&, const std::vector<PallasScalar>&, const std::vector<uint64_t>&,
+                                                   const std::vector<uint64_t>&, const PallasScalar*, const PallasScalar*, const PolyView*,
+                                                   const PallasScalar*)>;
+static void open_multi_c(uint64_t k, const uint64_t* Cs, const uint64_t* zs, uint64_t T, const uint64_t* q_poly, const uint64_t* q_point,
+                         uint64_t m, const uint64_t* ws, const uint64_t* w_Q, const uint64_t* q, uint64_t n_q, const uint64_t* w_bar,
+                         uint64_t* vs_out, uint64_t Q_out[12], uint64_t* us_out, uint64_t C_out[12], uint64_t x_out[4], uint64_t v_out[4],
+                         halo_eval_proof* pi, const MultiOpen& open) {
+    std::vector<PallasPoint> C(k);
+    std::vector<PallasScalar> w(ws ? k : 0);
+    for (uint64_t j = 0; j < k; j++) {
+        C[j] = point_load_checked(Cs + 12 * j, "C_j is not a canonical point on the curve");
+        if (ws) w[j] = scalar_load_checked(ws + 4 * j, "w_j is not a canonical scalar");
+    }
+    std::vector<PallasScalar> z;
+    std::vector<uint64_t> qp, qt;
+    multi_inputs(zs, T, q_poly, q_point, m, z, qp, qt);
+    PallasScalar wq, wbs;
+    PolyView qv(nullptr, 0);
+    if (ws) {
+        ensure(w_Q && w_bar && (q || n_q == 0), HALO_EINVAL, "hiding open needs w_Q, q and w_bar");
+        wq = scalar_load_checked(w_Q, "w_Q is not a canonical scalar");
+        wbs = scalar_load_checked(w_bar, "w_bar is not a canonical scalar");
+        qv = poly_from(q, n_q);
+    }
+    const pcdl::MultiOpening r = open(C, z, qp, qt, ws ? w.data() : nullptr, ws ? &wq : nullptr, ws ? &qv : nullptr, ws ? &wbs : nullptr);
+    for (uint64_t i = 0; i < m; i++) scalar_store(vs_out + 4 * i, r.vs[i]);
+    point_store(Q_out, r.Q);
+    for (uint64_t t = 0; t < T; t++) scalar_store(us_out + 4 * t, r.us[t]);
+    point_store(C_out, r.claim.C);
+    scalar_store(x_out, r.claim.x3);
+    scalar_store(v_out, r.claim.v);
+    pcdl::proof_to_c(r.pi, *pi);
+}
+
 int halo_pcdl_open_multi(halo_ctx* ctx, const uint64_t* coeffs, const uint64_t* n_coeffs, uint64_t k, const uint64_t* Cs, uint64_t d,
                          const uint64_t* zs, uint64_t T, const uint64_t* q_poly, const uint64_t* q_point, uint64_t m, const uint64_t* ws,
                          const uint64_t* w_Q, const uint64_t* q, uint64_t n_q, const uint64_t* w_bar, uint64_t* vs_out, uint64_t Q_out[12],
@@ -183,8 +232,6 @@ int halo_pcdl_open_multi(halo_ctx* ctx, const uint64_t* coeffs, const uint64_t* 
         ensure(n_coeffs && Cs && zs && q_poly && q_point && vs_out && Q_out && us_out && C_out && x_out && v_out && pi, HALO_EINVAL,
                "halo_pcdl_open_multi: NULL pointer");
         std::vector<PolyView> ps;
-        std::vector<PallasPoint> C(k);
-        std::vector<PallasScalar> w(ws ? k : 0);
         ps.reserve(k);
         uint64_t off = 0;
         for (uint64_t j = 0; j < k; j++) {
@@ -193,30 +240,27 @@ int halo_pcdl_open_multi(halo_ctx* ctx, const uint64_t* coeffs, const uint64_t* 
             off += n_coeffs[j];
         }
         ensure(coeffs || off == 0, HALO_EINVAL, "halo_pcdl_open_multi: NULL coefficients");
-        for (uint64_t j = 0; j < k; j++) {
-            C[j] = point_load_checked(Cs + 12 * j, "C_j is not a canonical point on the curve");
-            if (ws) w[j] = scalar_load_checked(ws + 4 * j, "w_j is not a canonical scalar");
-        }
-        std::vector<PallasScalar> z;
-        std::vector<uint64_t> qp, qt;
-        multi_inputs(zs, T, q_poly, q_point, m, z, qp, qt);
-        PallasScalar wq, wbs;
-        PolyView qv(nullptr, 0);
-        if (ws) {
-            ensure(w_Q && w_bar && (q || n_q == 0), HALO_EINVAL, "hiding open needs w_Q, q and w_bar");
-            wq = scalar_load_checked(w_Q, "w_Q is not a canonical scalar");
-            wbs = scalar_load_checked(w_bar, "w_bar is not a canonical scalar");
-            qv = poly_from(q, n_q);
-        }
-        const pcdl::MultiOpening r = pcdl::open_multi(ctx, ps, C, d, z, qp, qt, ws ? w.data() : nullptr, ws ? &wq : nullptr,
-                                                      ws ? &qv : nullptr, ws ? &wbs : nullptr);
-        for (uint64_t i = 0; i < m; i++) scalar_store(vs_out + 4 * i, r.vs[i]);
-        point_store(Q_out, r.Q);
-        for (uint64_t t = 0; t < T; t++) scalar_store(us_out + 4 * t, r.us[t]);
-        point_store(C_out, r.claim.C);
-        scalar_store(x_out, r.claim.x3);
-        scalar_store(v_out, r.claim.v);
-        pcdl::proof_to_c(r.pi, *pi);
+        open_multi_c(k, Cs, zs, T, q_poly, q_point, m, ws, w_Q, q, n_q, w_bar, vs_out, Q_out, us_out, C_out, x_out, v_out, pi,
+                     [&](auto& C, auto& z, auto& qp, auto& qt, auto w, auto wq, auto qv, auto wb) {
+                         return pcdl::open_multi(ctx, ps, C, d, z, qp, qt, w, wq, qv, wb);
+                     });
+    });
+}
+
+int halo_pcdl_open_multi_evals(halo_ctx* ctx, const uint64_t* evals, uint64_t k, const uint64_t* Cs, uint64_t d, const uint64_t* zs,
+                               uint64_t T, const uint64_t* q_poly, const uint64_t* q_point, uint64_t m, const uint64_t* ws,
+                               const uint64_t* w_Q, const uint64_t* q, uint64_t n_q, const uint64_t* w_bar, uint64_t* vs_out,
+                               uint64_t Q_out[12], uint64_t* us_out, uint64_t C_out[12], uint64_t x_out[4], uint64_t v_out[4],
+                               halo_eval_proof* pi) {
+    return guarded([&] {
+        ensure(k >= 1 && T >= 1 && m >= 1, HALO_EINVAL, "halo_pcdl_open_multi_evals: k, T and m must be at least 1");
+        ensure(evals && Cs && zs && q_poly && q_point && vs_out && Q_out && us_out && C_out && x_out && v_out && pi, HALO_EINVAL,
+               "halo_pcdl_open_multi_evals: NULL pointer");
+        const PallasScalar* e = reinterpret_cast<const PallasScalar*>(evals);
+        open_multi_c(k, Cs, zs, T, q_poly, q_point, m, ws, w_Q, q, n_q, w_bar, vs_out, Q_out, us_out, C_out, x_out, v_out, pi,
+                     [&](auto& C, auto& z, auto& qp, auto& qt, auto w, auto wq, auto qv, auto wb) {
+                         return pcdl::open_multi_evals(ctx, e, C, d, z, qp, qt, w, wq, qv, wb);
+                     });
     });
 }
 

@@ -97,6 +97,20 @@ static const PallasScalar* packed_prefixes(const std::vector<PolyView>& ps, cons
     return copy.data();
 }
 
+// The k Jacobian results of a batch MSM as commitments; hiding (ws): pedersen.rs:15-16, C_j + w_j S for every j in ONE combine
+// (host threads or k_point_combine by the output count)
+static std::vector<PallasPoint> commitments_hiding(halo_ctx* ctx, const std::vector<uint64_t>& out, size_t k, const PallasScalar* ws) {
+    std::vector<PallasPoint> C(k);
+    for (size_t j = 0; j < k; j++) C[j] = point_load(&out[12 * j]);
+    if (ws) {
+        CombineList cl;
+        for (size_t j = 0; j < k; j++) cl.push(C[j], point_zero(), scalar_zero(), ws[j]);
+        const std::vector<affine_t> r = cl.run(ctx);
+        for (size_t j = 0; j < k; j++) xyzz_from_affine(C[j].p, r[j]);
+    }
+    return C;
+}
+
 std::vector<PallasPoint> commit_batch(halo_ctx* ctx, const std::vector<PolyView>& ps, uint64_t d, const PallasScalar* ws) {
     const size_t k = ps.size();
     const std::vector<uint64_t> lens = batch_lens(ctx, ps, d);
@@ -107,15 +121,18 @@ std::vector<PallasPoint> commit_batch(halo_ctx* ctx, const std::vector<PolyView>
     std::vector<uint64_t> out(12 * k);
     static const PallasScalar none = scalar_zero();
     check_rc(ctx, halo_msm_gens_many(ctx, reinterpret_cast<const uint64_t*>(base ? base : &none), lens.data(), k, out.data()));
-    std::vector<PallasPoint> C(k);
-    for (size_t j = 0; j < k; j++) C[j] = point_load(&out[12 * j]);
-    if (ws) {  // pedersen.rs:15-16: C_j + w_j S for every j in ONE combine (host threads or k_point_combine by the output count)
-        CombineList cl;
-        for (size_t j = 0; j < k; j++) cl.push(C[j], point_zero(), scalar_zero(), ws[j]);
-        const std::vector<affine_t> r = cl.run(ctx);
-        for (size_t j = 0; j < k; j++) xyzz_from_affine(C[j].p, r[j]);
-    }
-    return C;
+    return commitments_hiding(ctx, out, k, ws);
+}
+
+std::vector<PallasPoint> commit_evals(halo_ctx* ctx, const PallasScalar* evals, size_t k, uint64_t d, const PallasScalar* ws) {
+    const uint64_t n = d + 1;
+    ensure(is_pow2(n), HALO_EINVAL, "d+1 is not a power of 2");   // pcdl.rs:102 (deg p_j <= d by construction)
+    ensure(n <= halo_num_generators(ctx), HALO_EINVAL, "d > D");  // pcdl.rs:104
+    if (k == 0) return {};
+    std::vector<uint64_t> degs(k), out(12 * k);
+    check_rc(ctx, halo_poly_upload_evals(ctx, reinterpret_cast<const uint64_t*>(evals), k, n, degs.data()));
+    check_rc(ctx, halo_poly_commit_resident(ctx, out.data()));
+    return commitments_hiding(ctx, out, k, ws);
 }
 
 static EvalProof open_impl(halo_ctx* ctx, const PolyView* p, uint64_t deg, const PallasPoint& C, uint64_t d, const PallasScalar& z,
@@ -282,10 +299,14 @@ MultiClaim multi_claim(halo_ctx* ctx, const std::vector<PallasPoint>& Cs, const 
     return multi_final(ctx, Cs, zs, q_poly, q_point, pw1, multi_vhat(zs.size(), q_point, vs, pw1), x2, x3, Q, us);
 }
 
+static MultiOpening open_multi_resident(halo_ctx* ctx, const std::vector<PallasPoint>& Cs, uint64_t d, const std::vector<PallasScalar>& zs,
+                                        const std::vector<uint64_t>& q_poly, const std::vector<uint64_t>& q_point, const PallasScalar* ws,
+                                        const PallasScalar* w_Q, const PolyView* q, const PallasScalar* w_bar);
+
 MultiOpening open_multi(halo_ctx* ctx, const std::vector<PolyView>& ps, const std::vector<PallasPoint>& Cs, uint64_t d,
                         const std::vector<PallasScalar>& zs, const std::vector<uint64_t>& q_poly, const std::vector<uint64_t>& q_point,
                         const PallasScalar* ws, const PallasScalar* w_Q, const PolyView* q, const PallasScalar* w_bar) {
-    const size_t k = ps.size(), T = zs.size(), m = q_poly.size();
+    const size_t k = ps.size();
     ensure(k >= 1 && Cs.size() == k, HALO_EINVAL, "open_multi: no polynomial");
     const std::vector<uint64_t> lens = batch_lens(ctx, ps, d);
     multi_validate(k, zs, q_poly, q_point);
@@ -298,6 +319,32 @@ MultiOpening open_multi(halo_ctx* ctx, const std::vector<PolyView>& ps, const st
     std::vector<PallasScalar> copy;
     const PallasScalar* base = packed_prefixes(ps, lens, copy);
     check_rc(ctx, halo_poly_upload(ctx, reinterpret_cast<const uint64_t*>(base), lens.data(), k, d + 1));
+    return open_multi_resident(ctx, Cs, d, zs, q_poly, q_point, ws, w_Q, q, w_bar);
+}
+
+MultiOpening open_multi_evals(halo_ctx* ctx, const PallasScalar* evals, const std::vector<PallasPoint>& Cs, uint64_t d,
+                              const std::vector<PallasScalar>& zs, const std::vector<uint64_t>& q_poly, const std::vector<uint64_t>& q_point,
+                              const PallasScalar* ws, const PallasScalar* w_Q, const PolyView* q, const PallasScalar* w_bar) {
+    const size_t k = Cs.size();
+    ensure(k >= 1, HALO_EINVAL, "open_multi_evals: no polynomial");
+    ensure(is_pow2(d + 1), HALO_EINVAL, "d+1 is not a power of 2");    // pcdl.rs:102 (deg p_j <= d by construction)
+    ensure(d + 1 <= halo_num_generators(ctx), HALO_EINVAL, "d > D");  // pcdl.rs:104
+    multi_validate(k, zs, q_poly, q_point);
+    if (ws) {  // q is drawn before the degrees are known: d coefficients, the most any degree can be
+        ensure(w_Q && q && w_bar, HALO_EINVAL, "hiding open needs w_Q, the random polynomial q and w_bar");
+        ensure(q->size() == d, HALO_ELEN, "q must have d coefficients");
+    }
+    std::vector<uint64_t> degs(k);
+    check_rc(ctx, halo_poly_upload_evals(ctx, reinterpret_cast<const uint64_t*>(evals), k, d + 1, degs.data()));
+    if (ws) ensure(*std::max_element(degs.begin(), degs.end()) >= 1, HALO_ELEN, "hiding open of polynomials of degree 0");
+    return open_multi_resident(ctx, Cs, d, zs, q_poly, q_point, ws, w_Q, q, w_bar);
+}
+
+// Everything of the multi-point opening after the upload of the polynomials (validated by the caller)
+static MultiOpening open_multi_resident(halo_ctx* ctx, const std::vector<PallasPoint>& Cs, uint64_t d, const std::vector<PallasScalar>& zs,
+                                        const std::vector<uint64_t>& q_poly, const std::vector<uint64_t>& q_point, const PallasScalar* ws,
+                                        const PallasScalar* w_Q, const PolyView* q, const PallasScalar* w_bar) {
+    const size_t k = Cs.size(), T = zs.size(), m = q_poly.size();
     const uint64_t* zp = reinterpret_cast<const uint64_t*>(zs.data());
     MultiOpening r;
     r.vs.resize(m);

@@ -35,6 +35,9 @@ PallasPoint commit(halo_ctx* ctx, PolyView p, uint64_t d, const PallasScalar* w)
 // `commit` of every polynomial (w: one blinding scalar per polynomial, or null): validated in order as commit does, then one
 // halo_msm_gens_many over all of them and w_j S added by one `combine` call (DESIGN.md K2c)
 std::vector<PallasPoint> commit_batch(halo_ctx* ctx, const std::vector<PolyView>& ps, uint64_t d, const PallasScalar* ws);
+// commit_batch of the k polynomials whose d + 1 evaluations over H_{d+1} are evals[j] ([k][d + 1]; DESIGN.md K8): one batched
+// inverse transform and one segmented MSM over the coefficients on the device.  d is validated as commit_batch does.
+std::vector<PallasPoint> commit_evals(halo_ctx* ctx, const PallasScalar* evals, size_t k, uint64_t d, const PallasScalar* ws);
 // pcdl.rs:120-242; rng draws made explicit: q (deg p coefficients), w_bar.  v_out (nullable) receives v = p(z).
 EvalProof open(halo_ctx* ctx, PolyView p, const PallasPoint& C, uint64_t d, const PallasScalar& z, const PallasScalar* w,
                const PolyView* q, const PallasScalar* w_bar, PallasScalar* v_out = nullptr);
@@ -85,6 +88,12 @@ struct MultiOpening {
 MultiOpening open_multi(halo_ctx* ctx, const std::vector<PolyView>& ps, const std::vector<PallasPoint>& Cs, uint64_t d,
                         const std::vector<PallasScalar>& zs, const std::vector<uint64_t>& q_poly, const std::vector<uint64_t>& q_point,
                         const PallasScalar* ws, const PallasScalar* w_Q, const PolyView* q, const PallasScalar* w_bar);
+// open_multi of the polynomials given by their d + 1 evaluations over H_{d+1} (evals: [k][d + 1], DESIGN.md K8): the upload is
+// one batched inverse transform on the device, the rest is open_multi's code.  Hiding: q holds d coefficients (the degrees are
+// known only after the upload); the opening uses the first deg(P) of them, as open_multi does.
+MultiOpening open_multi_evals(halo_ctx* ctx, const PallasScalar* evals, const std::vector<PallasPoint>& Cs, uint64_t d,
+                              const std::vector<PallasScalar>& zs, const std::vector<uint64_t>& q_poly, const std::vector<uint64_t>& q_point,
+                              const PallasScalar* ws, const PallasScalar* w_Q, const PolyView* q, const PallasScalar* w_bar);
 // succinct_check (pcdl.rs:252-314) without its group equation, in two halves around C' = C + alpha C_bar - w' S (:272-279) so
 // that a batch can compute every C' with one `combine` call.  succinct_alpha validates (d + 1 a power of two, d <= D, the
 // number of rounds) and returns alpha = rho_0(C, z, v, C_bar) of a hiding proof (zero otherwise); succinct_finish runs the rest

@@ -50,6 +50,20 @@ def commit_batch(ctx, ps, d, ws=None):
     return out[:k]
 
 
+def commit_evals(ctx, evals, d, ws=None):
+    """`commit_batch` of the polynomials given by their d + 1 evaluations over H_{d+1} (evals: (k, d + 1, 4), row j =
+    p_j(omega^i), omega = domain_root(lg(d + 1))) -> (k, 12).  The interpolation is one batched transform on the device
+    (include/halo_pcdl.h halo_pcdl_commit_evals)."""
+    e = arr(evals).reshape(-1, d + 1, 4)
+    k = e.shape[0]
+    wa = arr(ws).reshape(k, 4) if ws is not None else None
+    out = np.zeros((max(1, k), 12), dtype=np.uint64)
+    src = e.reshape(-1, 4) if k else np.zeros((1, 4), dtype=np.uint64)
+    _host.chk(_host.lib().halo_pcdl_commit_evals(ctx._h, p64(src), C.c_uint64(k), C.c_uint64(d), p64(wa) if wa is not None else None,
+                                                 p64(out)))
+    return out[:k]
+
+
 def open(ctx, p, Cm, d, z, w=None, q=None, w_bar=None):
     """pcdl.rs:120-242.  The reference's rng draws are explicit: q (deg p coefficients) and w_bar when hiding."""
     p, Cm, z = arr(p).reshape(-1, 4), arr(Cm, (12,)), arr(z, (4,))
@@ -120,6 +134,31 @@ def open_multi(ctx, ps, Cs, d, zs, queries, ws=None, w_Q=None, q=None, w_bar=Non
                                                wqp, p64(qa) if qa is not None else None,
                                                C.c_uint64(qa.shape[0] if qa is not None else 0), wbp, p64(vs), p64(Q), p64(us),
                                                p64(Cm), p64(x), p64(v), C.byref(pi)))
+    return vs[:m], Q, us[:T], Cm, x, v, pi
+
+
+def open_multi_evals(ctx, evals, Cs, d, zs, queries, ws=None, w_Q=None, q=None, w_bar=None):
+    """`open_multi` of the polynomials given by their d + 1 evaluations over H_{d+1} (evals: (k, d + 1, 4)), with the same
+    result tuple.  Hiding: q holds d coefficients (include/halo_pcdl.h halo_pcdl_open_multi_evals), of which the opening uses
+    the first deg(P)."""
+    e = arr(evals).reshape(-1, d + 1, 4)
+    k = e.shape[0]
+    Cs, zs = arr(Cs).reshape(k, 12), arr(zs).reshape(-1, 4)
+    qp, qt = _queries(queries)
+    m, T = qp.shape[0], zs.shape[0]
+    wa = arr(ws).reshape(k, 4) if ws is not None else None
+    qa = arr(q).reshape(-1, 4) if q is not None else None
+    wqk, wqp = _host.opt(w_Q)
+    wbk, wbp = _host.opt(w_bar)
+    vs, us = np.zeros((max(1, m), 4), dtype=np.uint64), np.zeros((max(1, T), 4), dtype=np.uint64)
+    Q, Cm, x, v, pi = np.zeros(12, dtype=np.uint64), np.zeros(12, dtype=np.uint64), np.zeros(4, dtype=np.uint64), \
+        np.zeros(4, dtype=np.uint64), EvalProof()
+    _host.chk(_host.lib().halo_pcdl_open_multi_evals(ctx._h, p64(e.reshape(-1, 4)), C.c_uint64(k), p64(Cs), C.c_uint64(d), p64(zs),
+                                                     C.c_uint64(T), p64(qp), p64(qt), C.c_uint64(m),
+                                                     p64(wa) if wa is not None else None, wqp,
+                                                     p64(qa) if qa is not None else None,
+                                                     C.c_uint64(qa.shape[0] if qa is not None else 0), wbp, p64(vs), p64(Q), p64(us),
+                                                     p64(Cm), p64(x), p64(v), C.byref(pi)))
     return vs[:m], Q, us[:T], Cm, x, v, pi
 
 

@@ -310,6 +310,39 @@ int halo_poly_quotient(halo_ctx *ctx, const uint64_t *zs /*[T][4]*/, const uint6
  * the current upload.  HALO_ENOMEM: no device memory for P; the context then holds no resident polynomial. */
 int halo_poly_lincomb_resident(halo_ctx *ctx, const uint64_t *cs /*[k][4]*/, const uint64_t c_q[4], uint64_t *degree_out);
 
+/* ---- K8: polynomials in evaluation form (number-theoretic transforms over the scalar field, csrc/ntt.cu) ----------------
+ * r = the scalar-field modulus of the build (Pallas: Fr; Vesta: Pallas' Fq); both fields have 2-adicity 32.
+ *   omega_{2^s} = 5^((r - 1) / 2^s) mod r, 0 <= s <= 32 (5 is a quadratic non-residue in both fields; GENERATOR = 5 and
+ *   root = 5^t of pasta_curves' ROOT_OF_UNITY and arkworks' TWO_ADIC_ROOT_OF_UNITY, a rule not checked against those crates
+ *   here).  omega_n = omega_{2^32}^(2^(32 - lg n)), omega_n^(n/2) = -1.  The canonical omega_{2^32}:
+ *     Pallas build: 0x2de6a9b8746d3f589e5c4dfd492ae26e9bb97ea3c106f049a70e2c1102b6d05f
+ *     Vesta build:  0x2bce74deac30ebda362120830561f81aea322bf2b7bb7584bdad6fabd87ea32f
+ * Transforms of n = 2^lg_n scalars in natural order over the coset g H, H = <omega_n>, g = the shift (1 if NULL):
+ *   forward  e_i = sum_j a_j (g omega_n^i)^j   (a may be shorter than n: n_in <= n, missing coefficients are zero)
+ *   inverse  a_j = g^-j n^-1 sum_i e_i omega_n^(-i j)   (n_in = n)
+ * Scalars are Montgomery limbs of canonical residues, as everywhere; the transform is exact.  k vectors run as ONE batch:
+ * ceil(lg_n / 11) launches of k_ntt_pass whatever k (DESIGN.md K8).  Errors: HALO_EINVAL for NULL pointers with k > 0,
+ * lg_n > 32, 2^lg_n above the context's max_n, n_in > 2^lg_n, a shift that is zero or not canonical, k 2^lg_n 32 bytes
+ * overflowing; HALO_ELEN for an inverse transform with n_in != 2^lg_n; HALO_ENOMEM when the device has no memory for the
+ * data or the tables (nothing written).  k = 0 does nothing.  Element values are not validated. */
+/* omega_{2^lg_n} in Montgomery form (host only, no context).  HALO_EINVAL for lg_n > 32. */
+int halo_domain_root(uint32_t lg_n, uint64_t out[4]);
+/* k vectors: forward (inverse = 0) or inverse transform over the coset shift H, H of order 2^lg_n; shift NULL = 1. */
+int halo_ntt(halo_ctx *ctx, const uint64_t *in /*[k][n_in][4]*/, uint64_t n_in, uint64_t k, uint32_t lg_n, int inverse,
+             const uint64_t shift[4], uint64_t *out /*[k][2^lg_n][4]*/);
+/* The same in place on a CUDA device buffer of k 2^lg_n scalars (complete when the call is made; synchronous, as
+ * halo_msm_gens_resident). */
+int halo_ntt_resident(halo_ctx *ctx, void *d_vecs, uint64_t k, uint32_t lg_n, int inverse, const uint64_t shift[4]);
+/* Evaluation-form upload: k columns of n = 2^lg values (evaluations over H of order n) become the context's resident
+ * polynomials (the state halo_poly_upload leaves: k polynomials of n coefficients, no quotient) by ONE batched inverse
+ * transform in place; degrees_out[j] = deg p_j (DensePolynomial::degree), found on the device in one launch.
+ * HALO_EINVAL: NULL pointers, k = 0 or k >= 2^31, n not a power of two or beyond max_n or the resident generators.
+ * HALO_ENOMEM: nothing written.  An earlier upload and its quotient are gone whatever the outcome. */
+int halo_poly_upload_evals(halo_ctx *ctx, const uint64_t *evals /*[k][n][4]*/, uint64_t k, uint64_t n, uint64_t *degrees_out /*[k]*/);
+/* k MSMs over the resident polynomials: out_jac[j] = <GS[0..len_j), p_j>, by the segmented route of halo_msm_gens_many with
+ * the coefficients read in place.  HALO_ESTATE: nothing uploaded. */
+int halo_poly_commit_resident(halo_ctx *ctx, uint64_t *out_jac /*[k][12]*/);
+
 /* ---- K3 / K4 / K7: the rounds of PCDL.open (pcdl.rs:183-231) ----------------------------------------- */
 typedef struct halo_ipa halo_ipa;
 /* Uploads the coefficients of p (zero-padded to n, pcdl.rs:183-184), copies GS[0..n) (pcdl.rs:185), builds

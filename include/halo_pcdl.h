@@ -78,6 +78,12 @@ int halo_pcdl_commit(halo_ctx *ctx, const uint64_t *coeffs, uint64_t n_coeffs, u
  * before any output is written.  One halo_msm_gens_many for all of them; the hiding terms w_j S in one combined step. */
 int halo_pcdl_commit_batch(halo_ctx *ctx, const uint64_t *coeffs /*packed*/, const uint64_t *n_coeffs /*[k]*/, uint64_t k, uint64_t d,
                            const uint64_t *ws /*[k][4] or NULL*/, uint64_t *out_jac /*[k][12]*/);
+/* K8: halo_pcdl_commit_batch of the k polynomials whose d + 1 evaluations over H_{d+1} are evals[j] (include/halo_b200.h K8):
+ * one batched inverse transform (halo_poly_upload_evals), one segmented MSM over the resident coefficients
+ * (halo_poly_commit_resident), then C_j + w_j S for the hiding ones in one combine.  d + 1 must be a power of two within the
+ * resident generators (HALO_EINVAL, checked before any device work); every degree is <= d by construction.  k = 0 does nothing. */
+int halo_pcdl_commit_evals(halo_ctx *ctx, const uint64_t *evals /*[k][d+1][4]*/, uint64_t k, uint64_t d, const uint64_t *ws /*[k][4] or NULL*/,
+                           uint64_t *out_jac /*[k][12]*/);
 /* pcdl.rs:120-242; hiding iff w != NULL, then q (n_q = deg p coefficients) and w_bar are the rng draws. */
 int halo_pcdl_open(halo_ctx *ctx, const uint64_t *coeffs, uint64_t n_coeffs, const uint64_t C_jac[12], uint64_t d,
                    const uint64_t z[4], const uint64_t *w /*nullable*/, const uint64_t *q, uint64_t n_q,
@@ -155,6 +161,19 @@ int halo_pcdl_open_multi(halo_ctx *ctx, const uint64_t *coeffs /*packed*/, const
                          const uint64_t *ws /*[k][4] or NULL*/, const uint64_t *w_Q, const uint64_t *q, uint64_t n_q,
                          const uint64_t *w_bar, uint64_t *vs_out /*[m][4]*/, uint64_t Q_out[12], uint64_t *us_out /*[T][4]*/,
                          uint64_t C_out[12], uint64_t x_out[4], uint64_t v_out[4], halo_eval_proof *pi);
+/* K8: the same opening of k polynomials given in evaluation form (include/halo_b200.h K8): evals[j] holds p_j(omega^i),
+ * i < d + 1, omega = omega_{d+1}.  The polynomials come from ONE batched inverse transform on the device
+ * (halo_poly_upload_evals); everything after that is halo_pcdl_open_multi's code.  Hiding: q holds n_q = d coefficients, the
+ * most any degree can be (halo_pcdl_open_multi: max_j deg p_j); the opening uses its first deg(P) <= max_j deg p_j, so the result
+ * equals halo_pcdl_open_multi of the interpolated polynomials with q[0 .. max_j deg p_j) field by field.  Errors as
+ * halo_pcdl_open_multi, with d + 1 a power of two and HALO_ELEN for n_q != d before any device work; a maximum degree of 0
+ * with hiding is HALO_ELEN after the upload (the degrees are known only then), with nothing written. */
+int halo_pcdl_open_multi_evals(halo_ctx *ctx, const uint64_t *evals /*[k][d+1][4]*/, uint64_t k, const uint64_t *Cs /*[k][12]*/,
+                               uint64_t d, const uint64_t *zs /*[T][4]*/, uint64_t T, const uint64_t *q_poly /*[m]*/,
+                               const uint64_t *q_point /*[m]*/, uint64_t m, const uint64_t *ws /*[k][4] or NULL*/, const uint64_t *w_Q,
+                               const uint64_t *q /*[n_q][4]*/, uint64_t n_q, const uint64_t *w_bar, uint64_t *vs_out /*[m][4]*/,
+                               uint64_t Q_out[12], uint64_t *us_out /*[T][4]*/, uint64_t C_out[12], uint64_t x_out[4], uint64_t v_out[4],
+                               halo_eval_proof *pi);
 /* The verifier's side of halo_pcdl_open_multi: recomputes x1 .. x4 and reduces the claims (C_j, z_t, v_i) with the prover's
  * Q and u_t to the one claim (C, x3, v) above (host arithmetic and one point_dot of k + 1 points), to be decided by
  * halo_pcdl_check / _check_batch or accumulated.  HALO_EINVAL as halo_pcdl_open_multi for the commitments, points and
